@@ -62,6 +62,10 @@ def parse_args():
     ap.add_argument("--flags", type=int, default=0)
     ap.add_argument("--plan-bases", type=float, default=0, help="profiling aid: plan the partitions for this many bases (a slice of C4 then runs "
                     "phase A with the full job's bin counts; phase B sees proportionally smaller partitions)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float64): the summary, the histogram of the "
+                         "histogram configurations, and for the export configurations the (filtered, key-sorted) table entries whose "
+                         "key %% ceil(bases / 1e6) == 0, keys split into 32-bit halves")
     return ap.parse_args()
 
 
@@ -143,6 +147,38 @@ def expected_windows_uniform(total: int, records: int, k: int) -> int:
     return (records - 1) * max(0, rec_len - k + 1) + max(0, last - k + 1)
 
 
+# --------------------------------------------------------------------------------------------- --dump-outputs
+DUMP_LIMIT_BYTES = 64 << 20
+TABLE_SAMPLE_BASES = 1_000_000   # the dumped table sample keeps about one entry per this many input bases
+
+
+def table_sample(counter, cfg, min_count: int, world: int):
+    """The key-space sample key % ceil(bases / 1e6) == 0 of the (key, count) table a caller would export, key-sorted over all
+    ranks.  The modulus depends on the arguments only, so two builds sample the same keys."""
+    import numpy as np
+    m = max(1, -(-cfg["bases"] // TABLE_SAMPLE_BASES))
+    keys, counts = counter.export_shard(m, 0, min_count, True)
+    if world > 1:
+        import torch.distributed as dist
+        parts = [None] * world
+        dist.all_gather_object(parts, (keys, counts))
+        keys = np.concatenate([p[0] for p in parts]); counts = np.concatenate([p[1] for p in parts])
+        order = np.argsort(keys, kind="stable")
+        keys, counts = keys[order], counts[order]
+    return {"table_keys_hi": keys >> np.uint64(32), "table_keys_lo": keys & np.uint64(0xFFFFFFFF), "table_counts": counts}
+
+
+def write_outputs(out_dir: str, arrays: dict):
+    """Each array as out_dir/<name>.npy in float64 (exact: every value is an integer below 2^53)."""
+    import numpy as np
+    total = sum(8 * np.asarray(a).size for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES} byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a).astype(np.float64))
+
+
 # --------------------------------------------------------------------------------------------- reference arm
 def cpu_sample(cfg, sample_bases: int):
     """A bounded sample of the configuration's own generator for the CPU arm: (seq, qual, offsets, description)."""
@@ -185,9 +221,11 @@ def run_reference(args, rank: int):
     t0 = time.perf_counter()
     windows = 0
     for _ in range(args.steps):
-        w, _d = orc.reference_path_count(k, seq, qual, offsets, min_quality=q, threads=cores)
+        w, d = orc.reference_path_count(k, seq, qual, offsets, min_quality=q, threads=cores)
         windows += w
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"summary": [w, d]})   # n_windows, n_distinct of the last step
     value = windows / dt
     sample = f"{what}, k={k}, per step; restated reference CPU path (oracle/kmer_oracle.c orc_reference_path_count)"
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -336,7 +374,7 @@ def main():
     ev0 = torch.cuda.Event(enable_timing=True); ev1 = torch.cuda.Event(enable_timing=True)
     ev0.record()
     for _ in range(args.steps):
-        step_device()
+        res = step_device()
     ev1.record()
     barrier()
     launches = L.kmg_kernel_launches() - launches0
@@ -350,6 +388,14 @@ def main():
             raise SystemExit(f"PARITY FAILURE: counted {exp_windows} windows, expected {cfg['reads'] * (READ_LEN - k + 1)}")
     elif summary["n_windows"] != exp_windows:
         raise SystemExit(f"PARITY FAILURE: counted {summary['n_windows']} windows, expected {exp_windows}")
+    if args.dump_outputs:   # before the legs below reset the table
+        out = {"summary": [summary["n_windows"], summary["n_distinct"], summary["max_count"]]}
+        if res is not None:
+            out["histogram_values"], out["histogram_frequencies"] = res
+        else:
+            out.update(table_sample(engine.counter, cfg, min_count, world))
+        if rank == 0:
+            write_outputs(args.dump_outputs, out)
     local = summary.get("local", summary)
     value = exp_windows / (ms_per_step * 1e-3)
 
