@@ -108,8 +108,8 @@ struct kmg_ctx {
   std::vector<Run> runs;      // pending, not yet consolidated
   Run result;                 // consolidated (key, count) run
   bool has_result = false;
-  bool spec_coarse_ok = !getenv("KMG_NO_SPECULATION");  // same for the level-1 scatter
-  bool spec_fine_ok = !getenv("KMG_NO_SPECULATION");  // level-2 scatter without a count pass until a partition overflows its share
+  bool spec_coarse_ok = true;  // same for the level-1 scatter
+  bool spec_fine_ok = true;  // level-2 scatter without a count pass until a partition overflows its share
   size_t total_mem = 0;                      // device memory size (cudaMemGetInfo is slow; asked once)
   void *d_scan_tmp = nullptr;                // CUB scan scratch for scan_tmp_items items
   size_t scan_tmp_bytes = 0;
@@ -367,9 +367,7 @@ kmg_status decide_mode(kmg_ctx *c, uint64_t first_call_windows) {
     c->n_coarse = 1u << (lg / 2);
     c->n_sub = 1u << (lg - lg / 2);
   } else {
-    uint64_t target = TARGET_KEYS_PER_PART;
-    if (const char *t = getenv("KMG_TARGET_KEYS")) target = std::max<uint64_t>(256, strtoull(t, nullptr, 10));  // tuning experiments only
-    const uint64_t want = std::max<uint64_t>(4, (hint + target - 1) / target);
+    const uint64_t want = std::max<uint64_t>(4, (hint + TARGET_KEYS_PER_PART - 1) / TARGET_KEYS_PER_PART);
     uint64_t p1 = 1;
     while (p1 * p1 < want) ++p1;
     p1 = std::min<uint64_t>(p1, 2048);
@@ -747,20 +745,18 @@ kmg_status consolidate(kmg_ctx *c, bool recompact) {
   for (auto *r : in) if (!r->d_counts) raw_entries += r->n;
   // Direct emit (count_partitions_smem_kernel<false, true>): only unweighted runs of keys that are mostly distinct (a genome, not a
   // deep read set), partitions within the plan.  Its output holds one entry per input entry.
-  static const bool no_direct = getenv("KMG_NO_DIRECT") != nullptr;  // ablation
-  bool direct = !no_direct && !recompact && raw_entries == total && c->dedup_ratio >= 0.5 && max_total <= 0xffffu &&
+  bool direct = !recompact && raw_entries == total && c->dedup_ratio >= 0.5 && max_total <= 0xffffu &&
                 total / std::max<uint32_t>(P, 1) <= SMEM_TABLE_SLOTS / 2 && !(c->cfg.flags & KMG_FLAG_NO_PREAGG);
   // Sieve variant (count_partitions_sieve_kernel): same precondition; it leaves the partitions it cannot take (too many repeated keys,
   // more than one batch of entries) to the compacting variant, so no bound on the largest partition is needed.
-  static const bool no_sieve = getenv("KMG_NO_SIEVE") != nullptr;  // ablation
-  bool sieve = !no_sieve && !recompact && raw_entries == total && c->dedup_ratio >= 0.5 &&
+  bool sieve = !recompact && raw_entries == total && c->dedup_ratio >= 0.5 &&
                total / std::max<uint32_t>(P, 1) <= SIEVE_MAX_ENTRIES * 15 / 16 && !(c->cfg.flags & KMG_FLAG_NO_PREAGG);
   uint32_t *d_redo = nullptr;
   unsigned long long *d_redo_base = nullptr;
   if (sieve && (pool_alloc(c, &d_redo, (size_t)P * 8) != cudaSuccess || pool_alloc(c, &d_redo_base, (size_t)P * 8) != cudaSuccess)) {  // d_redo: partition numbers, then range lengths
     cudaGetLastError(); pool_free(c, d_redo); pool_free(c, d_redo_base); d_redo = nullptr; d_redo_base = nullptr; sieve = false;
   }
-  bool sieve_padded = sieve && getenv("KMG_NO_SIEVE_TMA") == nullptr;
+  bool sieve_padded = sieve;
   for (auto *r : in) sieve_padded = sieve_padded && r->padded;
   uint64_t out_cap = std::max<uint64_t>(total, 1) + (sieve_padded ? (uint64_t)P * R : 0);  // padded segments: up to one filler entry per partition and run
   if (recompact) out_cap = std::min<uint64_t>(out_cap, c->result.n_valid + (1ull << 20));
@@ -1013,8 +1009,7 @@ kmg_status scan_packed(kmg_ctx *c, uint64_t n_words_total, bool has_start) {
     if (ms != KMG_OK) return ms;
   }
   if (c->mode == kmg_ctx::MODE_PARTITIONED) {
-    static const bool no_sparse = getenv("KMG_NO_SPARSE") != nullptr;  // ablation
-    if (incoming_exact && !no_sparse && !c->shm && incoming * 8 < n_words_total * 32 && incoming < (1ull << 32) - 1) {
+    if (incoming_exact && !c->shm && incoming * 8 < n_words_total * 32 && incoming < (1ull << 32) - 1) {
       // sparse route: fewer than one window in eight survives the quality filter -- scan + compact the surviving keys, then partition
       // those (the scatter kernels would pay their per-sub-tile work for every tile of the input)
       if (incoming == 0) return KMG_OK;
@@ -1247,7 +1242,6 @@ KMG_EXPORT kmg_status kmg_create(const kmg_config *cfg, kmg_ctx **out) {
     if (_e != cudaSuccess) { cuda_fail(c, _e, #call); return bail(_e == cudaErrorMemoryAllocation ? KMG_ERR_OOM : KMG_ERR_CUDA); } \
   } while (0)
   CUC(cudaSetDevice(c->device));
-  if (const char *dbg = getenv("KMG_DEBUG")) set_debug((uint32_t)atoi(dbg));
   if (cfg->stream) c->stream = (cudaStream_t)cfg->stream;
   else { CUC(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking)); c->own_stream = true; }
   CUC(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
@@ -1980,9 +1974,7 @@ KMG_EXPORT kmg_status kmg_shard_join(kmg_ctx *c, uint32_t world, uint32_t rank, 
     const uint64_t want = std::max<uint64_t>(4, (per_rank + TARGET_KEYS_PER_PART - 1) / TARGET_KEYS_PER_PART);
     uint64_t p1 = 1;
     while (p1 * p1 < want) ++p1;
-    uint64_t g_max = SHARD_MAX_BINS;  // world * P1 global bins in one scatter (the single-scan rows kernel's limit)
-    if (const char *e = getenv("KMG_SHARD_BINS")) g_max = std::min<uint64_t>(std::max<uint64_t>(strtoull(e, nullptr, 10), world), SHARD_MAX_BINS);
-    p1 = std::min<uint64_t>(p1, g_max / world);
+    p1 = std::min<uint64_t>(p1, SHARD_MAX_BINS / world);  // world * P1 global bins in one scatter (the single-scan rows kernel's limit)
     c->n_coarse = (uint32_t)std::max<uint64_t>(p1, 1);
     c->n_sub = (uint32_t)std::min<uint64_t>((want + c->n_coarse - 1) / c->n_coarse, 2048);
     kmg_status st = init_partitioned(c);

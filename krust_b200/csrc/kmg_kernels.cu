@@ -21,9 +21,6 @@
 
 namespace kmg {
 
-__constant__ uint32_t g_dbg = 0;  // ablation switches for tools/ablate.py (KMG_DEBUG env): 1 no stores, 2 no histogram pass, 4 no scatter pass
-void set_debug(uint32_t v) { cudaMemcpyToSymbol(g_dbg, &v, sizeof v); }
-
 // =================================================================================================
 // K8 ingest: ASCII (+ Phred+33 quality) -> packed bases + valid mask.  One thread per 32-base word.
 // =================================================================================================
@@ -173,7 +170,7 @@ __device__ __forceinline__ void issue_tile(const ScanInput &in, TileSmem *dst, u
 // Walk the 32 windows ending in word `i` of the staged tile, handing groups of G canonical keys to
 // the emitter.  fwd/rc are rolled one base at a time; canonical = min(fwd, rc) which equals the
 // reference's bytewise lexicographic choice (src/kmer.rs:348-365) because A<C<G<T in both orders.
-template <int G, class Emit, bool UNIFORM = false>
+template <int G, class Emit>
 __device__ __forceinline__ uint32_t scan_word(const TileSmem *ts, int i, int k, bool has_start, Emit &emit) {
   const uint64_t prev = ts->bases[LEAD_BASE_WORDS + i - 1];
   const uint64_t cur = ts->bases[LEAD_BASE_WORDS + i];
@@ -181,7 +178,7 @@ __device__ __forceinline__ uint32_t scan_word(const TileSmem *ts, int i, int k, 
   uint32_t sprev = 0, scur = 0;
   if (has_start) { sprev = ts->start[LEAD_MASK_WORDS + i - 1]; scur = ts->start[LEAD_MASK_WORDS + i]; }
   const uint32_t ok = window_ok_mask(vprev, vcur, sprev, scur, k, has_start);
-  if (!UNIFORM && ok == 0) return 0;  // UNIFORM: every lane of the warp walks all groups (the emitter uses warp collectives)
+  if (ok == 0) return 0;
   const uint64_t mask = kmer_mask(k);
   const int rc_shift = 2 * (k - 1);
   uint64_t fwd = prev & mask;
@@ -199,7 +196,7 @@ __device__ __forceinline__ uint32_t scan_word(const TileSmem *ts, int i, int k, 
       key[j] = fwd < rc ? fwd : rc;
       okg |= ((ok >> (31 - e)) & 1u) << j;
     }
-    if (UNIFORM || okg) emit.template group<G>(key, okg);
+    if (okg) emit.template group<G>(key, okg);
   }
   return __popc(ok);
 }
@@ -417,33 +414,6 @@ struct PartScatterEmit {
   }
 };
 
-// Warp-level multisplit emitter (the scheme radix sorts use): every warp owns a private cursor per partition, lanes
-// that hit the same partition find each other with __match_any_sync, the lowest of them advances the cursor by
-// the group size with a plain load/store, everybody takes base + (number of lower peers).  No returning shared
-// atomics: those execute lane-serially (~2 cycles per lane) and bounded the ATOMS-based scatter at ~8 cycles
-// per key per SM.  Must be called by all 32 lanes (scan_word<..., UNIFORM = true>).
-struct PartWarpScatterEmit {
-  uint32_t *wcur;  // smem: THIS warp's absolute next index in `out` per partition
-  uint64_t *out;
-  uint32_t n_parts;
-  template <int G>
-  __device__ __forceinline__ void group(const uint64_t (&key)[G], uint32_t okg) {
-    const uint32_t lane = threadIdx.x & 31u, lt = (1u << lane) - 1u;
-#pragma unroll
-    for (int j = 0; j < G; ++j) {
-      const bool ok = (okg >> j) & 1u;
-      const uint32_t p = ok ? part_of(key[j], n_parts) : (0x80000000u | lane);  // invalid lanes match only themselves
-      const uint32_t peers = __match_any_sync(0xffffffffu, p);
-      const int leader = __ffs(peers) - 1;
-      uint32_t base = 0;
-      if (ok && (int)lane == leader) { base = wcur[p]; wcur[p] = base + __popc(peers); }
-      base = __shfl_sync(0xffffffffu, base, leader);
-      __syncwarp();  // the leader's cursor update is visible to the next group's leaders
-      if (ok && !(g_dbg & 1u)) __stcs(out + (base + __popc(peers & lt)), key[j]);
-    }
-  }
-};
-
 // Synchronously stage one tile (used at pass boundaries where there is nothing to overlap with).
 __device__ __forceinline__ void wait_stage(uint64_t *bars, int stage, uint32_t &phase0, uint32_t &phase1) {
   if (stage == 0) { mbar_wait(&bars[0], phase0); phase0 ^= 1; } else { mbar_wait(&bars[1], phase1); phase1 ^= 1; }
@@ -599,62 +569,7 @@ __global__ void __launch_bounds__(SCATTER_THREADS, 2) partition_scatter_kernel(S
   }
 }
 
-// pass 2, warp-multisplit variant (used when NW x n_parts cursors fit in shared memory): per tile, every warp
-// histograms ITS windows into a private array, a per-partition prefix over the warps turns the counts into
-// absolute cursors (one global reservation per (tile, partition)), then the tile is re-scanned and scattered
-// with PartWarpScatterEmit.
-constexpr int WSCATTER_THREADS = 256;
-constexpr int WSCATTER_WARPS = WSCATTER_THREADS / 32;
-__global__ void __launch_bounds__(WSCATTER_THREADS) partition_scatter_warp_kernel(ScanInput in, uint32_t n_parts,
-                                                                                  const unsigned long long *part_start,
-                                                                                  unsigned long long *part_cursor, uint64_t *out) {
-  extern __shared__ __align__(128) uint8_t smem_raw[];
-  TileSmem *stages = reinterpret_cast<TileSmem *>(smem_raw);
-  __shared__ __align__(8) uint64_t bars[2];
-  uint32_t *whist = reinterpret_cast<uint32_t *>(smem_raw + 2 * sizeof(TileSmem));  // [WSCATTER_WARPS][n_parts]
-  const int tid = threadIdx.x, warp = tid >> 5;
-  uint32_t *mine = whist + (size_t)warp * n_parts;
-  const bool has_start = in.start != nullptr;
-  if (tid == 0) { mbar_init(&bars[0], 1); mbar_init(&bars[1], 1); mbar_fence_init(); }
-  for (uint32_t i = tid; i < n_parts * WSCATTER_WARPS; i += WSCATTER_THREADS) whist[i] = 0;
-  __syncthreads();
-  uint64_t tile = blockIdx.x;
-  int stage = 0;
-  uint32_t phase0 = 0, phase1 = 0;
-  if (tile < in.n_tiles && tid == 0) issue_tile(in, &stages[0], &bars[0], tile);
-  for (; tile < in.n_tiles; tile += gridDim.x) {
-    const uint64_t next = tile + gridDim.x;
-    if (next < in.n_tiles && tid == 0) issue_tile(in, &stages[stage ^ 1], &bars[stage ^ 1], next);
-    wait_stage(bars, stage, phase0, phase1);
-    const TileSmem *ts = &stages[stage];
-    if (!(g_dbg & 2u)) {
-      PartCountEmit e{mine, n_parts};  // warp-private histogram (ATOMS.POPC.INC, no return value)
-#pragma unroll 1
-      for (int r = 0; r < TILE_WORDS / WSCATTER_THREADS; ++r) scan_word<8>(ts, r * WSCATTER_THREADS + tid, in.k, has_start, e);
-    }
-    __syncthreads();
-    for (uint32_t p = tid; p < n_parts; p += WSCATTER_THREADS) {  // counts -> absolute cursors, warp after warp
-      uint32_t cnt[WSCATTER_WARPS], total = 0;
-#pragma unroll
-      for (int w = 0; w < WSCATTER_WARPS; ++w) { cnt[w] = whist[(size_t)w * n_parts + p]; total += cnt[w]; }
-      uint32_t run = total ? (uint32_t)(part_start[p] + atomicAdd(part_cursor + p, (unsigned long long)total)) : 0u;
-#pragma unroll
-      for (int w = 0; w < WSCATTER_WARPS; ++w) { whist[(size_t)w * n_parts + p] = run; run += cnt[w]; }
-    }
-    __syncthreads();
-    if (!(g_dbg & 4u)) {
-      PartWarpScatterEmit e{mine, out, n_parts};
-#pragma unroll 1
-      for (int r = 0; r < TILE_WORDS / WSCATTER_THREADS; ++r) scan_word<8, PartWarpScatterEmit, true>(ts, r * WSCATTER_THREADS + tid, in.k, has_start, e);
-    }
-    __syncthreads();
-    for (uint32_t i = tid; i < n_parts * WSCATTER_WARPS; i += WSCATTER_THREADS) whist[i] = 0;
-    __syncthreads();
-    stage ^= 1;
-  }
-}
-
-// pass 2, STAGED variant (default): measured with ablation switches (tools/ablate.py), 60 % of the scatter pass
+// pass 2, STAGED variant: measured with ablation switches on an earlier unstaged scatter, 60 % of the scatter pass
 // was the stores themselves -- a warp store of 32 keys to 32 different partitions is 32 separate L2 transactions.
 // Here each sub-tile's keys are first ranked into a shared-memory staging buffer in partition order, then copied
 // out by consecutive lanes: a warp instruction now covers a few contiguous runs (one sector per ~4 keys).
@@ -784,8 +699,7 @@ __global__ void __launch_bounds__(STAGE_THREADS, 1) partition_scatter_staged_ker
   }
 }
 
-// pass 2, ROWS variant (up to 2048 partitions; this first form is kept as the KMG_ROWS_LEGACY=1 baseline, partition_scatter_rows2_kernel
-// below is what runs): ONE scan of the input.  Every partition owns a row of
+// pass 2, ROWS variant (up to 2048 partitions): ONE scan of the input.  Every partition owns a row of
 // 2^cl key slots in shared memory; a window's key is ranked inside its partition by one shared atomic (with return)
 // and dropped into the row, the few keys whose row is full (partition sizes per sub-tile are Poisson around 9/16 of
 // a row) go to a small overflow list with their rank.  Then one global reservation per partition and a copy-out
@@ -797,31 +711,6 @@ constexpr int ROWS_THREADS = 1024;
 constexpr int ROWS_SUB_WORDS = ROWS_THREADS / 4;   // 8192 windows per sub-tile
 constexpr int ROWS_SLOTS = 16384;                  // n_parts rows of 2^cl keys (128 KiB; also the staging buffer of the exact route)
 constexpr int ROWS_OVERFLOW = 1536;   // keys whose row was full (repeat-rich reads put ~200 per sub-tile there; beyond it the sub-tile takes the exact route)
-template <bool MIXED>
-struct RowsEmit {
-  uint32_t *cnt;
-  uint64_t *rows, *ov_key;
-  uint32_t *ov_meta, *ov_n;
-  uint32_t n_parts, cap;
-  template <int G>
-  __device__ __forceinline__ void group(const uint64_t (&key)[G], uint32_t okg) {
-    uint32_t p[G], r[G];
-    uint64_t v[G];
-#pragma unroll
-    for (int j = 0; j < G; ++j) { const uint64_t m = mix64(key[j]); p[j] = coarse_of_mix(m, n_parts); v[j] = MIXED ? m : key[j]; }
-#pragma unroll
-    for (int j = 0; j < G; ++j) { r[j] = 0; if ((okg >> j) & 1u) r[j] = atomicAdd(cnt + p[j], 1u); }
-#pragma unroll
-    for (int j = 0; j < G; ++j) {
-      if (!((okg >> j) & 1u)) continue;
-      if (r[j] < cap) rows[p[j] * cap + r[j]] = v[j];
-      else {
-        const uint32_t o = atomicAdd(ov_n, 1u);
-        if (o < (uint32_t)ROWS_OVERFLOW) { ov_key[o] = v[j]; ov_meta[o] = (p[j] << 16) | r[j]; }  // r < 8192, p < 2048
-      }
-    }
-  }
-};
 // the 8 windows ending at bases 8g .. 8g+7 of word i
 template <class Emit>
 __device__ __forceinline__ void scan_octet(const TileSmem *ts, int i, int g, int k, bool has_start, Emit &emit) {
@@ -850,98 +739,10 @@ __device__ __forceinline__ void scan_octet(const TileSmem *ts, int i, int g, int
   }
   emit.template group<8>(key, okg);
 }
-template <bool MIXED>
-__global__ void __launch_bounds__(ROWS_THREADS, 1) partition_scatter_rows_kernel(ScanInput in, uint32_t n_parts, uint32_t cap, uint32_t magic,
-                                                                                  const unsigned long long *part_start,
-                                                                                  unsigned long long *part_cursor, uint64_t *out) {
-  extern __shared__ __align__(128) uint8_t smem_raw[];
-  TileSmem *stages = reinterpret_cast<TileSmem *>(smem_raw);
-  __shared__ __align__(8) uint64_t bars[2];
-  __shared__ uint32_t s_scan[ROWS_THREADS / 32 + 1], s_ovn;
-  uint64_t *rows = reinterpret_cast<uint64_t *>(smem_raw + 2 * sizeof(TileSmem));
-  uint64_t *ov_key = rows + ROWS_SLOTS;
-  uint32_t *ov_meta = reinterpret_cast<uint32_t *>(ov_key + ROWS_OVERFLOW);
-  uint32_t *cnt = ov_meta + ROWS_OVERFLOW, *s_off = cnt + n_parts, *g_base = s_off + n_parts;
-  const uint32_t n_slots = n_parts * cap;  // x / cap == __umulhi(x, magic) for x < 2^16
-  const int tid = threadIdx.x;
-  const bool has_start = in.start != nullptr;
-  if (tid == 0) { mbar_init(&bars[0], 1); mbar_init(&bars[1], 1); mbar_fence_init(); s_ovn = 0; }
-  for (uint32_t p = tid; p < n_parts; p += ROWS_THREADS) cnt[p] = 0;
-  __syncthreads();
-  uint64_t tile = blockIdx.x;
-  int stage = 0;
-  uint32_t phase0 = 0, phase1 = 0;
-  if (tile < in.n_tiles && tid == 0) issue_tile(in, &stages[0], &bars[0], tile);
-  for (; tile < in.n_tiles; tile += gridDim.x) {
-    const uint64_t next = tile + gridDim.x;
-    if (next < in.n_tiles && tid == 0) issue_tile(in, &stages[stage ^ 1], &bars[stage ^ 1], next);
-    wait_stage(bars, stage, phase0, phase1);
-    const TileSmem *ts = &stages[stage];
-    for (int sub = 0; sub < TILE_WORDS / ROWS_SUB_WORDS; ++sub) {
-      const int w0 = sub * ROWS_SUB_WORDS;
-      {
-        RowsEmit<MIXED> e{cnt, rows, ov_key, ov_meta, &s_ovn, n_parts, cap};
-        scan_octet(ts, w0 + (tid >> 2), tid & 3, in.k, has_start, e);
-      }
-      __syncthreads();
-      const uint32_t n_ov = s_ovn;
-      if (n_ov > (uint32_t)ROWS_OVERFLOW) {  // block-uniform: skewed sub-tile, take the exact route
-        for (uint32_t p = tid; p < n_parts; p += ROWS_THREADS) cnt[p] = 0;
-        __syncthreads();
-        stage_subtile_exact<ROWS_THREADS, MIXED>(ts, w0, ROWS_SUB_WORDS, in, has_start, n_parts, part_start, part_cursor, out, rows, cnt, s_off,
-                                          g_base, s_scan);
-      } else {
-        for (uint32_t p = tid; p < n_parts; p += ROWS_THREADS) {
-          const uint32_t h = cnt[p];
-          g_base[p] = part_reserve(in, part_start, part_cursor, p, h);
-          if (g_base[p] == NO_BASE) cnt[p] = 0;  // refused: nothing of this partition is written
-        }
-        __syncthreads();
-        // copy-out, lanes along the rows (contiguous destinations).  Rows of up to 24 slots (more than ~680 partitions): EIGHT LANES PER
-        // ROW, the row's size and base fetched once per lane and row, up to three predicated slot copies, no slot -> row division and no
-        // loop (the flat walk over all slots cost ~20 instructions per slot visit and 1.4 of 4.4 warp-instr per window,
-        // profiles/r2_v1_lines.txt; a half-warp per row with a strided loop was worse still: 2.2).
-        // (two slots per lane through one 16-byte row load was measured SLOWER, 44.8 vs 40.9 ms of phase A on C4: the stores of a warp
-        //  then stride by 16 bytes and touch twice the sectors)
-        if (cap <= 24u) {
-          const uint32_t l = tid & 7u;
-#pragma unroll 2
-          for (uint32_t p = tid >> 3; p < n_parts; p += ROWS_THREADS / 8) {
-            const uint32_t c = min(cnt[p], cap);
-            uint64_t *dst = out + (uint64_t)g_base[p] + l;
-            const uint64_t *row = rows + p * cap + l;
-            if (l == 0u) cnt[p] = 0;  // all eight lanes have read it (same instruction): the row is handed back clean, no separate pass + barrier
-            if (l < c) __stcs(dst, row[0]);
-            if (l + 8u < c) __stcs(dst + 8, row[8]);
-            if (c > 16u && l + 16u < c) __stcs(dst + 16, row[16]);
-          }
-        } else {
-#pragma unroll 4
-          for (uint32_t x = tid; x < n_slots; x += ROWS_THREADS) {
-            const uint32_t p = __umulhi(x, magic), e = x - p * cap;
-            if (e < cnt[p]) __stcs(out + (uint64_t)g_base[p] + e, rows[x]);
-          }
-        }
-        for (uint32_t o = tid; o < n_ov; o += ROWS_THREADS) {
-          const uint32_t meta = ov_meta[o];
-          if (g_base[meta >> 16] != NO_BASE) __stcs(out + (uint64_t)g_base[meta >> 16] + (meta & 0xffffu), ov_key[o]);
-        }
-        if (cap > 24u) {
-          __syncthreads();
-          for (uint32_t p = tid; p < n_parts; p += ROWS_THREADS) cnt[p] = 0;
-        }
-      }
-      if (tid == 0) s_ovn = 0;
-      __syncthreads();
-    }
-    stage ^= 1;
-  }
-}
 
-// The rows kernel with its inner loops written against 32-bit shared-space addresses (kmg_device.cuh: atoms_add / sts64_if /
-// copy64_if_lt): same phases and barriers as partition_scatter_rows_kernel.  An octet whose eight windows all count (the normal
-// case inside a record) is ranked without per-window tests, a row store is one predicated STS, overflow keys are handled after
-// the eight stores from a bit mask, the copy-out is three predicated load + store pairs per row.
+// The inner loops are written against 32-bit shared-space addresses (kmg_device.cuh: atoms_add / sts64_if / copy64_if_lt).  An
+// octet whose eight windows all count (the normal case inside a record) is ranked without per-window tests, a row store is one
+// predicated STS, overflow keys are handled after the eight stores from a bit mask, the copy-out is three predicated load + store pairs per row.
 template <bool MIXED>
 struct RowsEmit2 {
   uint32_t cnt_s, rows_s;  // shared-space addresses
@@ -1031,7 +832,13 @@ __global__ void __launch_bounds__(ROWS_THREADS, 1) partition_scatter_rows2_kerne
           if (g_base[p] == NO_BASE) cnt[p] = 0;  // refused: nothing of this partition is written
         }
         __syncthreads();
-        if (cap <= 24u) {  // eight lanes per row, lanes along the row (see partition_scatter_rows_kernel)
+        // copy-out, lanes along the rows (contiguous destinations).  Rows of up to 24 slots (more than ~680 partitions): EIGHT LANES PER
+        // ROW, the row's size and base fetched once per lane and row, up to three predicated slot copies, no slot -> row division and no
+        // loop (the flat walk over all slots cost ~20 instructions per slot visit and 1.4 of 4.4 warp-instr per window,
+        // profiles/r2_v1_lines.txt; a half-warp per row with a strided loop was worse still: 2.2).
+        // (two slots per lane through one 16-byte row load was measured SLOWER, 44.8 vs 40.9 ms of phase A on C4: the stores of a warp
+        //  then stride by 16 bytes and touch twice the sectors)
+        if (cap <= 24u) {
           const uint32_t l = tid & 7u;
 #pragma unroll 2
           for (uint32_t p = tid >> 3; p < n_parts; p += ROWS_THREADS / 8) {
@@ -1506,15 +1313,9 @@ cudaError_t launch_scan_dense(const ScanInput &in, unsigned long long *dense, un
   return cudaGetLastError();
 }
 
-bool rows_legacy() {  // KMG_ROWS_LEGACY=1: the round-3 rows kernels (A/B baseline)
-  static const bool on = [] { const char *v = getenv("KMG_ROWS_LEGACY"); return v && atoi(v) != 0; }();
-  return on;
-}
-
 bool scan_scatter_supports_cap(uint32_t n_parts) {  // the rows / staged kernels honour ScanInput::part_cap
   const size_t stsmem = 2 * sizeof(TileSmem) + (size_t)STAGE_KEYS * 8 + 3 * (size_t)n_parts * sizeof(uint32_t);
-  const char *v = getenv("KMG_SCATTER");
-  return (!v || atoi(v) == 0) && (n_parts <= (uint32_t)ROWS_SLOTS / 8 || stsmem <= 220 * 1024);
+  return n_parts <= (uint32_t)ROWS_SLOTS / 8 || stsmem <= 220 * 1024;
 }
 
 cudaError_t launch_scan_partition(const ScanInput &in, uint32_t n_parts, bool scatter, unsigned long long *part_counts,
@@ -1524,37 +1325,24 @@ cudaError_t launch_scan_partition(const ScanInput &in, uint32_t n_parts, bool sc
   const size_t smem = 2 * sizeof(TileSmem) + (size_t)n_parts * sizeof(uint32_t);
   const uint64_t max_ctas = (uint64_t)num_sms() * (smem > 100 * 1024 ? 1 : smem > 72 * 1024 ? 2 : SCAN_CTAS_PER_SM);
   cudaError_t e;
-  const size_t wsmem = 2 * sizeof(TileSmem) + (size_t)WSCATTER_WARPS * n_parts * sizeof(uint32_t);
   const size_t stsmem = 2 * sizeof(TileSmem) + (size_t)STAGE_KEYS * 8 + 3 * (size_t)n_parts * sizeof(uint32_t);
   const size_t rwsmem = 2 * sizeof(TileSmem) + (size_t)ROWS_SLOTS * 8 + (size_t)ROWS_OVERFLOW * 12 + 3 * (size_t)n_parts * sizeof(uint32_t);
-  if (scatter && n_parts <= (uint32_t)ROWS_SLOTS / 8 && !getenv("KMG_SCATTER")) {  // single-scan rows variant (default)
+  if (scatter && n_parts <= (uint32_t)ROWS_SLOTS / 8) {  // single-scan rows variant
     const uint32_t cap = std::min<uint32_t>((uint32_t)ROWS_SLOTS / n_parts, ROWS_SUB_WORDS * 32);  // mean fill 8192 / (n_parts * cap) ~ 0.5
     const uint32_t magic = (uint32_t)(((1ull << 32) + cap - 1) / cap);
     const unsigned grid = (unsigned)std::min<uint64_t>(in.n_tiles, (uint64_t)num_sms());
-    if (!rows_legacy()) {
-      if ((e = mixed ? set_smem(partition_scatter_rows2_kernel<true>, rwsmem) : set_smem(partition_scatter_rows2_kernel<false>, rwsmem)) != cudaSuccess) return e;
-      g_launches.fetch_add(1, std::memory_order_relaxed);
-      if (mixed) partition_scatter_rows2_kernel<true><<<grid, ROWS_THREADS, rwsmem, s>>>(in, n_parts, cap, magic, part_start, part_cursor, out);
-      else partition_scatter_rows2_kernel<false><<<grid, ROWS_THREADS, rwsmem, s>>>(in, n_parts, cap, magic, part_start, part_cursor, out);
-      return cudaGetLastError();
-    }
-    if ((e = mixed ? set_smem(partition_scatter_rows_kernel<true>, rwsmem) : set_smem(partition_scatter_rows_kernel<false>, rwsmem)) != cudaSuccess) return e;
+    if ((e = mixed ? set_smem(partition_scatter_rows2_kernel<true>, rwsmem) : set_smem(partition_scatter_rows2_kernel<false>, rwsmem)) != cudaSuccess) return e;
     g_launches.fetch_add(1, std::memory_order_relaxed);
-    if (mixed) partition_scatter_rows_kernel<true><<<grid, ROWS_THREADS, rwsmem, s>>>(in, n_parts, cap, magic, part_start, part_cursor, out);
-    else partition_scatter_rows_kernel<false><<<grid, ROWS_THREADS, rwsmem, s>>>(in, n_parts, cap, magic, part_start, part_cursor, out);
-  } else if (scatter && stsmem <= 220 * 1024 && !(getenv("KMG_SCATTER") && atoi(getenv("KMG_SCATTER")) != 0)) {  // staged variant (KMG_SCATTER=0, or > 2048 partitions)
+    if (mixed) partition_scatter_rows2_kernel<true><<<grid, ROWS_THREADS, rwsmem, s>>>(in, n_parts, cap, magic, part_start, part_cursor, out);
+    else partition_scatter_rows2_kernel<false><<<grid, ROWS_THREADS, rwsmem, s>>>(in, n_parts, cap, magic, part_start, part_cursor, out);
+  } else if (scatter && stsmem <= 220 * 1024) {  // staged variant (> 2048 partitions)
     const unsigned grid = (unsigned)std::min<uint64_t>(in.n_tiles, (uint64_t)num_sms());
     if ((e = mixed ? set_smem(partition_scatter_staged_kernel<true>, stsmem) : set_smem(partition_scatter_staged_kernel<false>, stsmem)) != cudaSuccess) return e;
     g_launches.fetch_add(1, std::memory_order_relaxed);
     if (mixed) partition_scatter_staged_kernel<true><<<grid, STAGE_THREADS, stsmem, s>>>(in, n_parts, part_start, part_cursor, out);
     else partition_scatter_staged_kernel<false><<<grid, STAGE_THREADS, stsmem, s>>>(in, n_parts, part_start, part_cursor, out);
   } else if (scatter && mixed) {
-    return cudaErrorInvalidValue;  // > 8192-ish partitions with mixed output: no kernel variant (the plan never asks for it)
-  } else if (scatter && wsmem <= 110 * 1024 && !(getenv("KMG_SCATTER") && atoi(getenv("KMG_SCATTER")) == 2)) {  // warp-multisplit variant: >= 2 CTAs/SM
-    if ((e = set_smem(partition_scatter_warp_kernel, wsmem)) != cudaSuccess) return e;
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    const uint64_t ctas = (uint64_t)num_sms() * (wsmem <= 72 * 1024 ? 3 : 2);
-    partition_scatter_warp_kernel<<<(unsigned)std::min(in.n_tiles, ctas), WSCATTER_THREADS, wsmem, s>>>(in, n_parts, part_start, part_cursor, out);
+    return cudaErrorInvalidValue;  // > 5100-ish partitions with mixed output: no kernel variant (the plan never asks for it)
   } else if (scatter) {
     if ((e = set_smem(partition_scatter_kernel, smem)) != cudaSuccess) return e;
     g_launches.fetch_add(1, std::memory_order_relaxed);

@@ -154,7 +154,6 @@ cudaError_t launch_keys_coarse(const uint64_t *d_keys, const uint64_t *d_counts,
                                unsigned long long *coarse_counts, const unsigned long long *coarse_start,
                                unsigned long long *coarse_cursor, uint64_t *out_keys, uint64_t *out_counts, cudaStream_t s);
 cudaError_t launch_refine(const RefineParams &P, bool scatter, cudaStream_t s);
-bool rows_legacy();  // KMG_ROWS_LEGACY=1: the round-3 rows kernels of A1 / A2 (A/B baseline)
 bool refine_single_pass_available(uint32_t n_sub, bool weighted);  // the rows kernel applies (it can run without a count pass)
 cudaError_t launch_fill_strided(uint64_t *d, uint64_t n, uint64_t stride, cudaStream_t s);  // d[i] = i * stride
 cudaError_t launch_sum_lens(const CountParams &P, unsigned long long *d_totals, unsigned long long *d_max, cudaStream_t s);
@@ -174,7 +173,6 @@ cudaError_t launch_pad_segments(uint64_t *keys, const uint64_t *seg_start, const
 // tmp == nullptr: returns the scratch size needed for n items in *tmp_bytes.  Asynchronous on s.
 cudaError_t exclusive_sum_u64(const uint64_t *d_in, uint64_t *d_out, uint64_t n, void *tmp, size_t *tmp_bytes, cudaStream_t s);
 int num_sms();
-void set_debug(uint32_t v);  // ablation switches (tools/ablate.py)
 cudaError_t launch_table_init(HashTable t, cudaStream_t s, uint64_t empty = ~0ull);  // empty: EMPTY_KEY, or EMPTY_MIX for phase B scratch
 cudaError_t launch_insert_keys(HashTable t, const uint64_t *d_keys, const uint64_t *d_counts, uint64_t n,
                                unsigned long long *counters, cudaStream_t s);

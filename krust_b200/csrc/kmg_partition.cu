@@ -217,6 +217,13 @@ __device__ __forceinline__ void refine_tile_two_pass(const RefineParams &P, cons
   for (uint32_t s = tid; s < P.n_sub; s += THREADS) hist[s] = 0;
 }
 
+// the key range [begin, begin + m) of tile g, which lies in coarse partition c
+__device__ __forceinline__ void refine_tile_range(const RefineParams &P, uint32_t g, uint32_t c, uint64_t &begin, uint32_t &m) {
+  begin = P.coarse_start[c] + (uint64_t)(g - P.tile_prefix[c]) * REFINE_TILE;
+  const uint64_t end_c = P.coarse_len ? P.coarse_start[c] + P.coarse_len[c] : P.coarse_start[c + 1];
+  m = (uint32_t)(end_c - begin < (uint64_t)REFINE_TILE ? end_c - begin : (uint64_t)REFINE_TILE);
+}
+
 // which coarse partition owns tile g (largest c with tile_prefix[c] <= g), and the tile's key range
 __device__ __forceinline__ void refine_locate_tile(const RefineParams &P, uint32_t g, uint32_t *s_c, uint32_t &c, uint64_t &begin, uint32_t &m) {
   if (threadIdx.x == 0) {
@@ -226,15 +233,25 @@ __device__ __forceinline__ void refine_locate_tile(const RefineParams &P, uint32
   }
   __syncthreads();
   c = *s_c;
-  begin = P.coarse_start[c] + (uint64_t)(g - P.tile_prefix[c]) * REFINE_TILE;
-  const uint64_t end_c = P.coarse_len ? P.coarse_start[c] + P.coarse_len[c] : P.coarse_start[c + 1];
-  m = (uint32_t)(end_c - begin < (uint64_t)REFINE_TILE ? end_c - begin : (uint64_t)REFINE_TILE);
+  refine_tile_range(P, g, c, begin, m);
+}
+
+// the coarse partition of tile g, searched from `hint` (the partition of the tile located before it): consecutive tiles of a
+// CTA mostly share their partition or lie in the next non-empty one
+__device__ __forceinline__ uint32_t refine_partition_from(const RefineParams &P, uint32_t g, uint32_t hint) {
+  if (P.tile_prefix[hint] > g || hint >= P.n_coarse) hint = 0;
+  if (P.tile_prefix[hint + 1] <= g) {  // not in the same or the next non-empty partition: binary search
+    uint32_t lo = hint, hi = P.n_coarse;
+    while (hi - lo > 1) { const uint32_t mid = (lo + hi) >> 1; if (P.tile_prefix[mid] <= g) lo = mid; else hi = mid; }
+    hint = lo;
+  }
+  return hint;
 }
 
 template <bool SCATTER>
 __global__ void __launch_bounds__(REFINE_THREADS) refine_kernel(RefineParams P) {
   extern __shared__ __align__(16) uint8_t rsm[];
-  // count pass: one histogram.  scatter pass (weighted keys, or KMG_REFINE=legacy): the tile's keys are ranked into a
+  // count pass: one histogram.  scatter pass (weighted keys): the tile's keys are ranked into a
   // shared-memory staging buffer in sub-bin order and copied out by consecutive lanes (scattered 8-byte stores, one L2
   // transaction each, were 60 % of the unstaged kernels).
   uint64_t *staging = reinterpret_cast<uint64_t *>(rsm);                                // SCATTER only: REFINE_TILE keys
@@ -280,29 +297,13 @@ __global__ void __launch_bounds__(REFINE_ROWS_THREADS, 1) refine_rows_kernel(Ref
   const uint32_t g_begin = blockIdx.x * per_cta, g_end = min(g_begin + per_cta, P.n_tiles);
   if (g_begin >= g_end) return;
   uint32_t c_hint = 0;  // thread 0: coarse partition of the tile located last
-  auto locate = [&](uint32_t g, int slot) {  // thread 0 publishes the partition of tile g
-    if (tid == 0) {
-      if (P.tile_prefix[c_hint] > g || c_hint >= P.n_coarse) c_hint = 0;
-      if (P.tile_prefix[c_hint + 1] <= g) {  // not in the same or the next non-empty partition: binary search
-        uint32_t lo = c_hint, hi = P.n_coarse;
-        while (hi - lo > 1) { const uint32_t mid = (lo + hi) >> 1; if (P.tile_prefix[mid] <= g) lo = mid; else hi = mid; }
-        c_hint = lo;
-      }
-      s_c[slot] = c_hint;
-    }
-  };
-  auto tile_range = [&](uint32_t g, uint32_t c, uint64_t &begin, uint32_t &m) {
-    begin = P.coarse_start[c] + (uint64_t)(g - P.tile_prefix[c]) * REFINE_TILE;
-    const uint64_t end_c = P.coarse_len ? P.coarse_start[c] + P.coarse_len[c] : P.coarse_start[c + 1];
-    m = (uint32_t)(end_c - begin < (uint64_t)REFINE_TILE ? end_c - begin : (uint64_t)REFINE_TILE);
-  };
   for (uint32_t s = tid; s < P.n_sub; s += REFINE_ROWS_THREADS) cnt[s] = 0;
   if (tid == 0) s_ovn = 0;
-  locate(g_begin, 0);
+  if (tid == 0) s_c[0] = c_hint = refine_partition_from(P, g_begin, c_hint);
   __syncthreads();
   uint32_t c = s_c[0], m;
   uint64_t begin;
-  tile_range(g_begin, c, begin, m);
+  refine_tile_range(P, g_begin, c, begin, m);
   uint64_t key[U];
   {
     const uint64_t *kb = refine_keys_of(P, c) + begin;
@@ -334,7 +335,7 @@ __global__ void __launch_bounds__(REFINE_ROWS_THREADS, 1) refine_rows_kernel(Ref
       }
     }
     const int nslot = (g - g_begin + 1) & 1;
-    if (g + 1 < g_end) locate(g + 1, nslot);
+    if (g + 1 < g_end && tid == 0) s_c[nslot] = c_hint = refine_partition_from(P, g + 1, c_hint);
     __syncthreads();
     const uint32_t n_ov = s_ovn;
     const bool exact = n_ov > REFINE_ROWS_OVERFLOW;  // block-uniform: skewed tile, take the exact route
@@ -354,7 +355,7 @@ __global__ void __launch_bounds__(REFINE_ROWS_THREADS, 1) refine_rows_kernel(Ref
     uint64_t begin_next = 0;
     if (g + 1 < g_end) {
       c_next = s_c[nslot];
-      tile_range(g + 1, c_next, begin_next, m_next);
+      refine_tile_range(P, g + 1, c_next, begin_next, m_next);
       const uint64_t *kb = refine_keys_of(P, c_next) + begin_next + tid;
       uint32_t mn = m_next;
       asm volatile("" : "+l"(kb), "+r"(mn));  // pinned in registers: the compiler otherwise re-derives the tile's base (segment tables, source select) for every load
@@ -397,8 +398,8 @@ __global__ void __launch_bounds__(REFINE_ROWS_THREADS, 1) refine_rows_kernel(Ref
   }
 }
 
-// The rows scheme as it runs by default (refine_rows_kernel above stays for fewer than 128 sub-bins and as the KMG_ROWS_LEGACY=1
-// baseline).  What the measurements on C4 said (profiles/r4_summary.md), in the order they were made:
+// The rows scheme for 128 sub-bins and more when the keys are local (refine_rows_kernel above takes fewer sub-bins and keys pulled
+// from other GPUs).  What the measurements on C4 said (profiles/r4_summary.md), in the order they were made:
 //   * cutting the instructions per key by a third (32-bit shared-space addresses, predicated stores and copies instead of
 //     BSSY / BRA / BSYNC regions that re-derive the shared window per key) changed nothing: 20.0 -> 19.9 ms.  Not issue bound.
 //   * TILE ORDER is what mattered: with a contiguous tile range per CTA the grid appends to 148 x 928 output regions at once and
@@ -440,7 +441,9 @@ __global__ void __launch_bounds__(REFINE_ROWS_THREADS, 1) refine_rows4_kernel(Re
   // tile order: P.pad = C > 0 -> INTERLEAVED in chunks of C tile pairs (pair q holds tiles 2q, 2q + 1; CTA b takes pairs
   // [b*C, b*C + C) of every block of gridDim * C pairs): the whole grid works in a handful of coarse bins and appends to the same
   // few thousand output regions at a time, which is what DRAM wants (C4, A2: 20.0 ms with contiguous ranges, 16.7 ms interleaved);
-  // C > 1 keeps the CTAs from reserving in the same sub-bins at the same instant.  P.pad = 0: a contiguous range of tiles per CTA.
+  // C > 1 keeps the CTAs from reserving in the same sub-bins at the same instant.  P.pad = 0 (a contiguous range of tiles per CTA)
+  // is never launched: launch_refine sets C >= 1.  The branches for it stay because the kernel compiled without them measured
+  // slower on a B200 (A2 +0.6 % on C4, +2 % on C1: the register allocation of the whole loop changes).
   const uint32_t C = P.pad;
   const bool il = C != 0;
   uint32_t pi = 0;  // interleaved: this CTA's pair counter
@@ -448,23 +451,7 @@ __global__ void __launch_bounds__(REFINE_ROWS_THREADS, 1) refine_rows4_kernel(Re
   const uint32_t per_cta = (P.n_tiles + gridDim.x - 1) / gridDim.x;
   const uint32_t g_begin = il ? 2u * pair_of(0) : blockIdx.x * per_cta, g_end = il ? P.n_tiles : min(g_begin + per_cta, P.n_tiles);
   if (g_begin >= g_end) return;
-  uint32_t c_hint = 0;
-  auto locate = [&](uint32_t g, int slot) {  // thread 0 publishes the partition of tile g
-    if (tid == 0) {
-      if (P.tile_prefix[c_hint] > g || c_hint >= P.n_coarse) c_hint = 0;
-      if (P.tile_prefix[c_hint + 1] <= g) {
-        uint32_t lo = c_hint, hi = P.n_coarse;
-        while (hi - lo > 1) { const uint32_t mid = (lo + hi) >> 1; if (P.tile_prefix[mid] <= g) lo = mid; else hi = mid; }
-        c_hint = lo;
-      }
-      s_c[slot] = c_hint;
-    }
-  };
-  auto tile_range = [&](uint32_t g, uint32_t c, uint64_t &begin, uint32_t &m) {
-    begin = P.coarse_start[c] + (uint64_t)(g - P.tile_prefix[c]) * REFINE_TILE;
-    const uint64_t end_c = P.coarse_len ? P.coarse_start[c] + P.coarse_len[c] : P.coarse_start[c + 1];
-    m = (uint32_t)(end_c - begin < (uint64_t)REFINE_TILE ? end_c - begin : (uint64_t)REFINE_TILE);
-  };
+  uint32_t c_hint = 0;  // thread 0: coarse partition of the tile located last
   // batch `half` (0 / 1) of the tile whose keys start at kb and which holds m keys
   auto load_batch = [&](uint64_t (&k)[U], const uint64_t *kb, uint32_t m, uint32_t half) {
     const uint64_t *p = kb + half * R4_BATCH + tid;
@@ -516,11 +503,11 @@ __global__ void __launch_bounds__(REFINE_ROWS_THREADS, 1) refine_rows4_kernel(Re
   };
   for (uint32_t s = tid; s < P.n_sub; s += T) cnt[s] = 0;
   if (tid == 0) s_ovn = 0;
-  locate(g_begin, 0);
+  if (tid == 0) s_c[0] = c_hint = refine_partition_from(P, g_begin, c_hint);
   __syncthreads();
   uint32_t c = s_c[0], m;
   uint64_t begin;
-  tile_range(g_begin, c, begin, m);
+  refine_tile_range(P, g_begin, c, begin, m);
   uint64_t kA[U], kB[U];
   load_batch(kA, refine_keys_of(P, c) + begin, m, 0);
   load_batch(kB, refine_keys_of(P, c) + begin, m, 1);
@@ -534,7 +521,7 @@ __global__ void __launch_bounds__(REFINE_ROWS_THREADS, 1) refine_rows4_kernel(Re
     uint64_t begin2 = 0;
     uint32_t m2 = 0;
     const uint64_t *kbase = refine_keys_of(P, c);
-    if (two) tile_range(g + 1, c, begin2, m2);
+    if (two) refine_tile_range(P, g + 1, c, begin2, m2);
     if (!P.n_src) {  // L2 prefetch of this CTA's NEXT group (one 128-byte line per thread = two tiles), assuming it lies in the same
                      // partition (it does for all but one group in ~200): its loads then wait for L2, not for DRAM
       const uint64_t end_c = P.coarse_len ? P.coarse_start[c] + P.coarse_len[c] : P.coarse_start[c + 1];
@@ -555,7 +542,7 @@ __global__ void __launch_bounds__(REFINE_ROWS_THREADS, 1) refine_rows4_kernel(Re
     uint32_t g_next = g + (two ? 2u : 1u);
     if (il && ((g & 1u) || two || g + 1 >= g_end)) g_next = 2u * pair_of(++pi);
     slot ^= 1;
-    if (g_next < g_end) locate(g_next, slot);
+    if (g_next < g_end && tid == 0) s_c[slot] = c_hint = refine_partition_from(P, g_next, c_hint);
     __syncthreads();
     const uint32_t n_ov = s_ovn;
     const bool exact = n_ov > (uint32_t)R4_OVERFLOW;  // block-uniform: skewed group, take the exact route tile by tile
@@ -579,7 +566,7 @@ __global__ void __launch_bounds__(REFINE_ROWS_THREADS, 1) refine_rows4_kernel(Re
     uint64_t begin_next = 0;
     if (g_next < g_end) {
       c_next = s_c[slot];
-      tile_range(g_next, c_next, begin_next, m_next);
+      refine_tile_range(P, g_next, c_next, begin_next, m_next);
       const uint64_t *kb = refine_keys_of(P, c_next) + begin_next;
       load_batch(kA, kb, m_next, 0);
       load_batch(kB, kb, m_next, 1);
@@ -609,11 +596,7 @@ __global__ void __launch_bounds__(REFINE_ROWS_THREADS, 1) refine_rows4_kernel(Re
   }
 }
 
-static bool refine_legacy() {
-  static const bool legacy = [] { const char *v = getenv("KMG_REFINE"); return v && v[0] == 'l'; }();  // ablation: KMG_REFINE=legacy
-  return legacy;
-}
-bool refine_single_pass_available(uint32_t n_sub, bool weighted) { return !weighted && !refine_legacy() && n_sub <= REFINE_ROWS_SLOTS / 8; }
+bool refine_single_pass_available(uint32_t n_sub, bool weighted) { return !weighted && n_sub <= REFINE_ROWS_SLOTS / 8; }
 
 __global__ void fill_strided_kernel(uint64_t *d, uint64_t n, uint64_t stride) {
   for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) d[i] = i * stride;
@@ -638,17 +621,15 @@ cudaError_t launch_refine(const RefineParams &P_in, bool scatter, cudaStream_t s
     // big rows, drained once per two tiles, tiles interleaved over the grid -- for LOCAL keys.  When the keys are pulled from other
     // GPUs (n_src) the round-3 kernel stays: measured on two GPUs (profiles/r4_summary.md) it pulls and refines a step's keys in
     // 10.4 ms against 12.4 ms (13.7 ms with one tile per drain): NVLink, not the drain pattern, sets its pace.
-    if (!rows_legacy() && P.n_sub >= 128u && P.n_src == 0) {
+    if (P.n_sub >= 128u && P.n_src == 0) {
       const uint32_t n_slots = (uint32_t)((R4_SMEM - (size_t)R4_OVERFLOW * 12 - 3 * (size_t)P.n_sub * sizeof(uint32_t)) / 8) & ~1u;
       P.row_cap = n_slots / P.n_sub;
       const uint32_t tg = rows_overflow_fraction(2.0 * REFINE_TILE / P.n_sub, P.row_cap) <= 0.035 ? 2u : 1u;  // two tiles per drain unless the rows would overflow too often
       const size_t smem4 = (size_t)n_slots * 8 + (size_t)R4_OVERFLOW * 12 + 3 * (size_t)P.n_sub * sizeof(uint32_t);
       const unsigned grid = (unsigned)std::min<uint64_t>(P.n_tiles, (uint64_t)num_sms());
       // chunk of the interleaved tile order: 16 pairs, less when the input is so small that some CTAs would get nothing
-      static const int chunk_env = [] { const char *v = getenv("KMG_A2_INTERLEAVE"); return v ? atoi(v) : -1; }();  // tuning: 0 = contiguous ranges
-      uint32_t chunk = 16;
-      while (chunk > 1 && (uint64_t)grid * chunk * 8 > P.n_tiles) chunk >>= 1;
-      P.pad = chunk_env >= 0 ? (uint32_t)chunk_env : chunk;
+      P.pad = 16;
+      while (P.pad > 1 && (uint64_t)grid * P.pad * 8 > P.n_tiles) P.pad >>= 1;
       auto kern = P.in_keys ? refine_rows4_kernel<true> : refine_rows4_kernel<false>;
       if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem4)) != cudaSuccess) return e;
       g_launches.fetch_add(1, std::memory_order_relaxed);

@@ -31,24 +31,19 @@ print(f"generated {n} bases in {time.perf_counter() - t0:.1f} s", flush=True)
 
 h = torch.from_numpy(seq).pin_memory()
 h_np = h.numpy()
-for name, flags in (("auto", 0), ("no-speculation", None)):
-    import os
-    if flags is None:
-        os.environ["KMG_NO_SPECULATION"] = "1"
-        flags = 0
-    with kb.GpuKmerCounter(k, flags=flags) as c:
-        best = 1e9
-        for it in range(3):
-            c.reset()
-            torch.cuda.synchronize()
-            t0 = time.perf_counter()
-            c.count_batch(h_np, None, offsets)
-            s = c.finalize(True)
-            vals, freqs = c.histogram(1)
-            best = min(best, time.perf_counter() - t0)
-        print(f"{name:15s}: {best * 1e3:8.1f} ms  {s['n_windows'] / best / 1e9:6.2f} G k-mers/s  windows {s['n_windows']} distinct {s['n_distinct']} "
-              f"max {s['max_count']} consolidations {s['n_grows']} | phase A {s['scan_ns'] / 1e6:.1f} ms, phase B {s['consolidate_ns'] / 1e6:.1f} ms", flush=True)
-        gpu_hist = (vals.copy(), freqs.copy())
+with kb.GpuKmerCounter(k) as c:
+    best = 1e9
+    for it in range(3):
+        c.reset()
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        c.count_batch(h_np, None, offsets)
+        s = c.finalize(True)
+        vals, freqs = c.histogram(1)
+        best = min(best, time.perf_counter() - t0)
+    print(f"{'auto':15s}: {best * 1e3:8.1f} ms  {s['n_windows'] / best / 1e9:6.2f} G k-mers/s  windows {s['n_windows']} distinct {s['n_distinct']} "
+          f"max {s['max_count']} consolidations {s['n_grows']} | phase A {s['scan_ns'] / 1e6:.1f} ms, phase B {s['consolidate_ns'] / 1e6:.1f} ms", flush=True)
+    gpu_hist = (vals.copy(), freqs.copy())
 if "--stream" in sys.argv:
     # the same genome fed record by record with no size hint: the plan is made from the first call alone
     rec = [(int(offsets[i]), int(offsets[i + 1])) for i in range(len(offsets) - 1)]

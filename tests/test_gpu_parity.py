@@ -299,7 +299,7 @@ def test_extract_and_insert_equal_direct_count():
     offsets = torch.from_numpy(offsets_np.astype(np.int64)).to(dev)
     for k in (11, 21, 32):
         oracle = orc.count_batch(k, host, None, offsets_np, mode="rolling")
-        for n_shards in (1, 2, 8, 64):
+        for n_shards in (1, 2, 8, 64, 4096, 8192):  # 4096: the staged scatter kernel, 8192: partition_scatter_kernel
             out = torch.empty(len(host), dtype=torch.int64, device=dev)
             with kb.GpuKmerCounter(k) as c:
                 counts = c.extract_keys_device(seq.data_ptr(), len(host), n_shards, out.data_ptr(), len(host),

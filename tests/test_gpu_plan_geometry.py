@@ -184,7 +184,7 @@ def _source_constant(path: str, name: str) -> int:
 
 def test_row_reciprocal_is_exact_for_every_planned_row_size():
     """The scatter kernels map a row slot x to its row as __umulhi(x, magic) with magic = ceil(2^32 / cap) (the flat copy-outs
-    of partition_scatter_rows(2)_kernel and refine_rows_kernel): that equals x / cap for every slot of every row size a plan can
+    of partition_scatter_rows2_kernel and refine_rows_kernel): that equals x / cap for every slot of every row size a plan can
     produce -- A1 rows of min(16384 / P1, 8192) slots for P1 in 1..2048, refine_rows rows of min(16384 / P2, 8192) slots for every
     P2 it may run with (1..127 from a plan, up to 2048 for keys pulled from other GPUs)."""
     rows_slots = _source_constant("kmg_kernels.cu", "ROWS_SLOTS")
