@@ -66,6 +66,7 @@ struct Run {
   uint64_t n = 0;        // entries (a consolidated run may hold skipped filler entries, see count_partitions_smem_kernel)
   uint64_t n_valid = 0;  // consolidated runs: distinct keys
   bool padded = false;   // speculative layout: segments start on 16-byte boundaries and an EMPTY_MIX entry follows every segment of odd length
+  uint64_t part_cap = 0;  // raw run in the speculative layout: partition p owns entries [p * part_cap, (p + 1) * part_cap); 0: exact layout
 };
 
 struct kmg_ctx {
@@ -488,6 +489,7 @@ kmg_status refine_to_run(kmg_ctx *c, uint64_t *d_ckeys, uint64_t *d_ccounts, con
     if (!h_flag) {
       cleanup();
       r.n = n;
+      r.part_cap = cap_f;
       if (!(cap_f & 1ull) && launch_pad_segments(r.d_keys, r.d_seg_start, r.d_seg_len, P, c->stream) == cudaSuccess) r.padded = true;
       if (split) { *split->out = std::move(r); return KMG_OK; }
       guard.release();  // the run is complete: a consolidation triggered by add_run may re-split it with the others
@@ -758,6 +760,14 @@ kmg_status consolidate(kmg_ctx *c, bool recompact) {
   }
   bool sieve_padded = sieve;
   for (auto *r : in) sieve_padded = sieve_padded && r->padded;
+  // In place (count_partitions_sieve_tma_kernel<true, true>): one raw run in the speculative layout is counted where it lies.  The
+  // result takes over its keys and segment starts and gets a count for every slot of the layout (0: repeat, pad entry or slack), so
+  // phase B writes 8 bytes per slot instead of 16 per entry and no second key array is held.  Each fallback below leaves the route
+  // for the copying one: the kernel never writes the keys, so the input is intact until the compacting variant has run.  The
+  // partitions it hands over are compacted into their own capacity, which is only safe while that variant cannot overflow: a
+  // capacity of at most two batches (2 x 4096 entries) fits its 8192-slot table and, at 256 claims per warp and batch, its warp lists.
+  bool in_place = sieve_padded && R == 1 && in[0]->part_cap != 0 && in[0]->part_cap <= 2ull * SMEM_COUNT_THREADS * 8;
+  const uint64_t in_place_n = in_place ? (uint64_t)P * in[0]->part_cap : 0;
   uint64_t out_cap = std::max<uint64_t>(total, 1) + (sieve_padded ? (uint64_t)P * R : 0);  // padded segments: up to one filler entry per partition and run
   if (recompact) out_cap = std::min<uint64_t>(out_cap, c->result.n_valid + (1ull << 20));
   else if (total > (1ull << 28) && !direct && !sieve) {
@@ -770,22 +780,28 @@ kmg_status consolidate(kmg_ctx *c, bool recompact) {
     if (ae != cudaSuccess) { pool_free(c, out.d_keys); pool_free(c, out.d_counts); out.d_keys = out.d_counts = nullptr; cudaGetLastError(); }
     return ae;
   };
-  if (e == cudaSuccess) {
-    e = alloc_out(out_cap);
-    if (e != cudaSuccess && out_cap > (1ull << 26)) {  // not even the estimate fits: take what is there
+  auto alloc_copy_out = [&]() -> cudaError_t {
+    cudaError_t ae = alloc_out(out_cap);
+    if (ae != cudaSuccess && out_cap > (1ull << 26)) {  // not even the estimate fits: take what is there
       size_t free_b = 0, total_b = 0;
       pool_release_idle(c);
       cudaMemGetInfo(&free_b, &total_b);
       const uint64_t room = free_b > (3ull << 30) ? (free_b - (2ull << 30)) / 16 : 0;
-      if (room >= (1ull << 26)) { out_cap = std::min(out_cap, room); e = alloc_out(out_cap); }
+      if (room >= (1ull << 26)) { out_cap = std::min(out_cap, room); ae = alloc_out(out_cap); }
     }
+    prm.out_keys = out.d_keys; prm.out_counts = out.d_counts; prm.out_cap = out_cap; prm.part_cap = 0;
+    return ae;
+  };
+  if (e == cudaSuccess && in_place) {
+    if (pool_alloc(c, &out.d_counts, in_place_n * 8) == cudaSuccess) {
+      prm.out_keys = in[0]->d_keys; prm.out_counts = out.d_counts; prm.out_cap = in_place_n; prm.part_cap = (uint32_t)in[0]->part_cap;
+    } else { cudaGetLastError(); in_place = false; }
   }
+  if (e == cudaSuccess && !in_place) e = alloc_copy_out();
   if (e == cudaSuccess) e = pool_alloc(c, &out.d_seg_start, (size_t)P * 8);
   if (e == cudaSuccess) e = pool_alloc(c, &out.d_seg_len, (size_t)P * 8);
   if (e != cudaSuccess) { pool_free(c, d_order); pool_free(c, d_redo); pool_free(c, d_redo_base); free_run(c, out); return cuda_fail(c, e, "cudaMalloc(consolidated run)"); }
-  prm.out_keys = out.d_keys; prm.out_counts = out.d_counts;
   prm.out_seg_start = out.d_seg_start; prm.out_seg_len = out.d_seg_len;
-  prm.out_cap = out_cap;
 
   if (!c->d_hist) {
     e = cudaMalloc(&c->d_hist, (HIST_DENSE_BINS + 1) * sizeof(unsigned long long));
@@ -829,6 +845,12 @@ kmg_status consolidate(kmg_ctx *c, bool recompact) {
     bool weighted = max_total > ((2ull * SMEM_COUNT_THREADS * 8) << split_log2);  // partitions oversized beyond the split want the pre-aggregating variant
     for (uint32_t r = 0; r < R; ++r) weighted |= in[r]->d_counts != nullptr;
     if (weighted || split_log2 || !use_smem) direct = sieve = false;
+    if (in_place && !sieve) {  // the copying route takes over
+      pool_free(c, out.d_counts); out.d_counts = nullptr;
+      in_place = false;
+      if (e == cudaSuccess) e = alloc_copy_out();
+    }
+    static const bool dbg_sieve = getenv("KMG_DEBUG_SIEVE") != nullptr;
     unsigned long long h_sync[4] = {0, 0, 0, 0};
     if (sieve) {
       prm.redo_list = d_redo; prm.redo_count = reinterpret_cast<uint32_t *>(d_sync + 3) + 1;
@@ -841,6 +863,7 @@ kmg_status consolidate(kmg_ctx *c, bool recompact) {
       if (e == cudaSuccess && (n_redo > sieve_redo_limit_host(P) || (uint32_t)h_sync[3])) {
         // duplicate-rich input (the reserved ranges of the partitions handed back are lost as fillers, the padded variant stops early):
         // the launch is repeated without the sieve
+        if (dbg_sieve) fprintf(stderr, "[kmg] sieve: %u partitions, %u handed back, repeated without the sieve, %s\n", P, n_redo, in_place ? "leaves the in-place route" : "copied");
         pool_free(c, d_scratch); pool_free(c, d_sync);
         sieve = sieve_padded = direct = false;
         c->dedup_ratio = std::min(c->dedup_ratio, 0.49);
@@ -859,8 +882,9 @@ kmg_status consolidate(kmg_ctx *c, bool recompact) {
         if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
         c->sieve_redo += n_redo;
       }
-      static const bool dbg_sieve = getenv("KMG_DEBUG_SIEVE") != nullptr;
-      if (dbg_sieve) fprintf(stderr, "[kmg] sieve: %u partitions, %u left to the compacting variant, %llu entries, %llu distinct\n", P, n_redo, (unsigned long long)h_sync[0], (unsigned long long)h_sync[2]);
+      if (dbg_sieve)
+        fprintf(stderr, "[kmg] sieve: %u partitions, %u left to the compacting variant, %llu entries, %llu distinct, %s\n", P, n_redo,
+                in_place ? (unsigned long long)in_place_n : (unsigned long long)h_sync[0], (unsigned long long)h_sync[2], in_place ? "in place" : "copied");
     } else {
       if (e == cudaSuccess) e = use_smem ? launch_count_partitions_smem(prm, weighted, direct, c->stream) : launch_count_partitions(prm, grid, c->stream);
       timer_end(c, tmr);
@@ -884,6 +908,13 @@ kmg_status consolidate(kmg_ctx *c, bool recompact) {
     }
     n_out = h_sync[0]; n_valid = h_sync[2];
     if (!(h_sync[1] >> 32)) break;  // no overflow
+    if (sieve && in_place) {
+      // Not reached: the route is only taken for capacities the compacting variant always holds (see above).  Its other
+      // partitions were compacted into the input, so the launch cannot be repeated from it.
+      c->poisoned = true;
+      st = fail(c, KMG_ERR_STATE, "phase B in place: the compacting variant overflowed on a partition of the speculative layout (the context must be reset)");
+      break;
+    }
     if (sieve) { sieve = false; continue; }    // a left-over partition was beyond the compacting variant too: the whole launch is repeated without the sieve
     if (direct) { direct = false; continue; }  // a partition beyond the direct variant's limits: the compacting variant takes the launch
     if (attempt >= 16 || c->scratch_log2 >= 30) { st = fail(c, KMG_ERR_TABLE_FULL, "partition table overflow could not be resolved"); break; }
@@ -896,6 +927,11 @@ kmg_status consolidate(kmg_ctx *c, bool recompact) {
   pool_free(c, d_order); pool_free(c, d_redo); pool_free(c, d_redo_base);
   if (st != KMG_OK) { free_run(c, out); return st; }
   out.n = n_out; out.n_valid = n_valid;
+  if (in_place) {  // the result takes over the input run's keys and layout (free_run below leaves them alone)
+    out.n = in_place_n;
+    out.d_keys = in[0]->d_keys; in[0]->d_keys = nullptr;
+    pool_free(c, out.d_seg_start); out.d_seg_start = in[0]->d_seg_start; in[0]->d_seg_start = nullptr;
+  }
   if (raw_entries > (1ull << 24)) {  // distinct keys the raw runs added per raw entry (an upper estimate: keys already in the result count as new)
     const uint64_t before = total - raw_entries;
     c->dedup_ratio = std::min(1.0, (double)(n_valid > before / 2 ? n_valid - before / 2 : 0) / (double)raw_entries);
@@ -904,8 +940,9 @@ kmg_status consolidate(kmg_ctx *c, bool recompact) {
   for (auto &r : c->runs) free_run(c, r);
   c->runs.clear();
   c->pending_bytes = 0;
-  // give back the slack (upper bound was one slot per input entry) when it is worth a copy
-  if (out.n && out.n < total / 2) {
+  // give back the slack (upper bound was one slot per input entry) when it is worth a copy (an in-place result has no spare
+  // allocation: its slack is the layout's)
+  if (!in_place && out.n && out.n < total / 2) {
     uint64_t *k2 = nullptr, *c2 = nullptr;
     if (pool_alloc(c, &k2, out.n * 8) == cudaSuccess && pool_alloc(c, &c2, out.n * 8) == cudaSuccess) {
       cudaMemcpyAsync(k2, out.d_keys, out.n * 8, cudaMemcpyDeviceToDevice, c->stream);

@@ -927,7 +927,7 @@ __global__ void rehash_kernel(HashTable from, HashTable to, unsigned long long *
 
 // A "view" unifies both table kinds for the read-side kernels: entry i is (key, count); empty if count == 0.
 __device__ __forceinline__ bool view_get(const TableView &v, uint64_t i, uint64_t &key, uint64_t &count) {
-  if (v.pair_keys) { key = unmix64(v.pair_keys[i]); count = v.pair_counts[i]; return count != 0; }  // runs hold mixed keys; count 0: filler entry of a multi-pass partition
+  if (v.pair_keys) { key = unmix64(v.pair_keys[i]); count = v.pair_counts[i]; return count != 0; }  // runs hold mixed keys; count 0: filler entry, repeat left in place or slack of a strided layout (any key)
   if (v.dense) { key = i; count = v.dense[i]; return count != 0; }
   ulonglong2 s = reinterpret_cast<const ulonglong2 *>(v.slots)[i];
   key = s.x; count = s.y + 1;  // slots store occurrences - 1
@@ -1120,8 +1120,8 @@ __global__ void __launch_bounds__(256) query_kernel(TableView v, HashTable t, co
       if (g / n_coarse == shard_rank) {  // a sharded table answers for its own keys only
         const uint64_t p = (uint64_t)(g - shard_rank * n_coarse) * n_sub + sub_of_mix(m, n_sub);
         const uint64_t b = seg_start[p], e = b + seg_len[p];
-        for (uint64_t j = b + lane; j < e; j += 32)
-          if (v.pair_keys[j] == m) found = v.pair_counts[j];
+        for (uint64_t j = b + lane; j < e; j += 32)  // a repeat that phase B left in place holds the key once more, with count 0
+          if (v.pair_keys[j] == m) found |= v.pair_counts[j];
       }
     } else if (t.slots && lane == 0) {
       uint64_t slot = slot_of(key, t.cap);

@@ -88,7 +88,11 @@ struct RefineParams {
 };
 struct CountParams {
   uint32_t n_parts, R, scratch_log2, preagg;
-  uint32_t split_log2, pad0;         // shared-memory kernel: partitions larger than a table are counted in up to 2^split_log2 passes
+  uint32_t split_log2;               // shared-memory kernel: partitions larger than a table are counted in up to 2^split_log2 passes
+  // padded sieve, in place (one raw run in a strided layout: partition p owns entries [p * part_cap, (p + 1) * part_cap)): the
+  // output run IS the input run.  Its keys are never written -- a repeated key's further entries keep their key and get count 0 --
+  // and the counts cover every partition's whole capacity (0 behind the segment).  0: the keys are copied to out_keys.
+  uint32_t part_cap;
   ConsRun runs[CONS_MAX_RUNS];
   const uint32_t *order;             // partitions in processing order (largest first); nullptr = 0, 1, 2, ...
   uint64_t *scratch;                 // gridDim.x private tables of 2^scratch_log2 (key, count-1) slots, clean
@@ -166,7 +170,7 @@ cudaError_t launch_count_partitions_smem(const CountParams &P, bool weighted, bo
 // other key is copied to the output in place.  Partitions it cannot take are listed in P.redo_list for the variants above.
 constexpr uint32_t SIEVE_MAX_ENTRIES = 4096;  // entries of one partition the sieve variant takes (one batch)
 // padded: every input run has 16-byte aligned segments padded to an even length (launch_pad_segments) -- the copies then go
-// through the TMA unit and the output segments are the padded inputs
+// through the TMA unit and the output segments are the padded inputs.  With P.part_cap set the padded variant runs in place.
 cudaError_t launch_count_partitions_sieve(const CountParams &P, bool padded, cudaStream_t s);
 uint32_t sieve_redo_limit_host(uint32_t n_parts);  // more partitions handed back than this: the padded variant stopped early, repeat the launch without the sieve
 cudaError_t launch_pad_segments(uint64_t *keys, const uint64_t *seg_start, const uint64_t *seg_len, uint32_t n_parts, cudaStream_t s);

@@ -139,12 +139,20 @@ __device__ __forceinline__ const uint64_t *refine_keys_of(const RefineParams &P,
 
 // One tile, exact two-pass procedure: histogram -> (count: add to fine_counts | scatter: prefix, one global reservation
 // per sub-bin, rank the keys into `staging` in sub-bin order, coalesced copy-out).  hist[] is zero on entry and on exit.
-template <int THREADS, bool SCATTER>
+// FILLERS: the input may be a consolidated run (refine_kernel; the rows kernels only see raw runs, which hold no fillers).
+template <int THREADS, bool SCATTER, bool FILLERS = false>
 __device__ __forceinline__ void refine_tile_two_pass(const RefineParams &P, const uint64_t *__restrict__ kbase, const uint64_t begin, const uint32_t m, const uint64_t f0, const uint32_t sub_base,
                                                      uint64_t *staging, uint64_t *staging_c, uint32_t *hist, uint32_t *s_off,
                                                      uint32_t *g_base, uint32_t *s_scan) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   constexpr int U = 8;  // keys in flight per thread
+  // sub-bin of a mixed key of the tile.  A consolidated run being re-split holds filler entries inside its segments (EMPTY_MIX
+  // with count 0: the pad entry of an odd segment, a repeat of the copying sieve); their mix lies in no particular partition, so
+  // they stay fillers in the last sub-bin of their own partition instead of indexing past hist[].
+  auto bin_of = [&](uint64_t mixed) {
+    const uint32_t b = sub_of_mix(mixed, P.sub_total) - sub_base;
+    return FILLERS ? min(b, P.n_sub - 1u) : b;
+  };
   for (uint32_t i0 = 0; i0 < m; i0 += U * THREADS) {
     uint64_t key[U];
 #pragma unroll
@@ -153,7 +161,7 @@ __device__ __forceinline__ void refine_tile_two_pass(const RefineParams &P, cons
       key[j] = i < m ? (SCATTER ? kbase[begin + i] : __ldcs(kbase + begin + i)) : EMPTY_KEY;
     }
 #pragma unroll
-    for (int j = 0; j < U; ++j) if (i0 + j * THREADS + tid < m) atomicAdd(hist + (sub_of_mix(P.in_keys ? mix64(key[j]) : key[j], P.sub_total) - sub_base), 1u);
+    for (int j = 0; j < U; ++j) if (i0 + j * THREADS + tid < m) atomicAdd(hist + bin_of(P.in_keys ? mix64(key[j]) : key[j]), 1u);
   }
   __syncthreads();
   if (!SCATTER) {
@@ -199,7 +207,7 @@ __device__ __forceinline__ void refine_tile_two_pass(const RefineParams &P, cons
       cnt[j] = (i < m && P.counts) ? __ldcs(P.counts + begin + i) : 1ull;
     }
 #pragma unroll
-    for (int j = 0; j < U; ++j) { if (P.in_keys) key[j] = mix64(key[j]); sb[j] = sub_of_mix(key[j], P.sub_total) - sub_base; o[j] = 0; if (i0 + j * THREADS + tid < m) o[j] = atomicAdd(hist + sb[j], 1u); }
+    for (int j = 0; j < U; ++j) { if (P.in_keys) key[j] = mix64(key[j]); sb[j] = bin_of(key[j]); o[j] = 0; if (i0 + j * THREADS + tid < m) o[j] = atomicAdd(hist + sb[j], 1u); }
 #pragma unroll
     for (int j = 0; j < U; ++j)
       if (i0 + j * THREADS + tid < m) { staging[o[j]] = key[j]; if (P.counts) staging_c[o[j]] = cnt[j]; }
@@ -207,7 +215,7 @@ __device__ __forceinline__ void refine_tile_two_pass(const RefineParams &P, cons
   __syncthreads();
   for (uint32_t i = tid; i < m; i += THREADS) {  // coalesced copy-out; destination recomputed from the key
     const uint64_t key = staging[i];
-    const uint32_t sbin = sub_of_mix(key, P.sub_total) - sub_base;  // staged values are mixed keys
+    const uint32_t sbin = bin_of(key);  // staged values are mixed keys
     if (g_base[sbin] == NO_BASE) continue;
     const uint64_t dst = (uint64_t)g_base[sbin] + (i - s_off[sbin]);
     P.out_keys[dst] = key;
@@ -267,7 +275,7 @@ __global__ void __launch_bounds__(REFINE_THREADS) refine_kernel(RefineParams P) 
     uint64_t begin;
     refine_locate_tile(P, g, &s_c, c, begin, m);
     const uint32_t cb = c / P.in_group;  // coarse bin of input partition c
-    refine_tile_two_pass<REFINE_THREADS, SCATTER>(P, refine_keys_of(P, c), begin, m, (uint64_t)cb * P.n_sub, (cb % P.sub_old) * P.n_sub, staging, staging_c, hist, s_off, g_base, s_scan);
+    refine_tile_two_pass<REFINE_THREADS, SCATTER, true>(P, refine_keys_of(P, c), begin, m, (uint64_t)cb * P.n_sub, (cb % P.sub_old) * P.n_sub, staging, staging_c, hist, s_off, g_base, s_scan);
     __syncthreads();
   }
 }
@@ -1213,7 +1221,8 @@ __global__ void __launch_bounds__(SMEM_COUNT_THREADS, 2) count_partitions_smem_k
     // ---- compact: the partition gets one contiguous output range (one global atomic), each warp a sub-range of it
     uint32_t pre, pass_d;
     {
-      const uint32_t v = lane < NW ? min(s_wn[lane], WLIST) : 0u;
+      const uint32_t raw = lane < NW ? s_wn[lane] : 0u, v = min(raw, WLIST);
+      const bool lost = __any_sync(0xffffffffu, raw > WLIST);  // some warp's list overflowed: the partition's results are void
       uint32_t incl = v;
 #pragma unroll
       for (int o = 1; o < NW; o <<= 1) { const uint32_t u = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += u; }
@@ -1224,6 +1233,10 @@ __global__ void __launch_bounds__(SMEM_COUNT_THREADS, 2) count_partitions_smem_k
         if (b == NO_SPACE) {
           b = atomicAdd(P.out_cursor, (unsigned long long)d);
           if (b + d > P.out_cap) { atomicExch(P.nospace_flag, 1u); b = NO_SPACE; }
+        } else if (lost || *reinterpret_cast<volatile uint32_t *>(P.error_flag)) {
+          // void results stay out of a pre-reserved range: on the in-place route it is the partition's input, which the host's
+          // fallback reads again (this CTA's table overflow was flagged before the barrier above)
+          b = NO_SPACE;
         }
         P.out_seg_start[p] = b; P.out_seg_len[p] = d;
         s_base = b; s_run = 0;
@@ -1251,8 +1264,8 @@ __global__ void __launch_bounds__(SMEM_COUNT_THREADS, 2) count_partitions_smem_k
         if (P.hist) hist_note(ok, cnt, s_hist, P, lane);
       }
     }
-    if (n_pass == 1 && P.pre_base && P.pre_base[work] != NO_SPACE) {  // the rest of the pre-reserved range: entries every reader skips
-      const unsigned long long b = P.pre_base[work];
+    if (n_pass == 1 && P.pre_base && P.pre_base[work] != NO_SPACE && s_base != NO_SPACE) {  // the rest of the pre-reserved range: entries every reader skips
+      const unsigned long long b = s_base;
       for (uint32_t i = pass_d + tid; i < P.pre_len[work]; i += SMEM_COUNT_THREADS) { __stcs(P.out_keys + b + i, (uint64_t)EMPTY_MIX); __stcs(P.out_counts + b + i, (uint64_t)0); }
     }
     __syncthreads();  // table clean before the next pass / partition (and every warp has read the list counters)
@@ -1529,6 +1542,11 @@ __global__ void __launch_bounds__(SV_THREADS, 2) count_partitions_sieve_kernel(C
 //   * two 512-thread CTAs per SM, so one CTA's barriers overlap the other's work; output ranges are reserved when the segment
 //     table is fetched (two partitions ahead), so no global atomic sits on the critical path.
 // The output segment is the padded input: entries (EMPTY, 0) are fillers every reader skips.
+// IN_PLACE (one raw run in a strided layout, P.part_cap): the stored keys would be byte-identical to the loaded ones except for
+// the rare repeats, so the output run keeps the input's key array and layout and only counts are written -- 8 B in and 8 B per
+// slot of capacity out per key instead of 8 in and 16 out.  A repeat keeps its key and gets count 0; the pad entry and the slack
+// behind the segment get count 0 too, so whole-array readers skip them whatever keys sit there.  The keys are never written, so
+// every fallback of the host (early stop, the launch without the sieve) rereads an intact input.
 // ---------------------------------------------------------------------------------------------------
 constexpr int SVT_THREADS = 512, SVT_G = 8, SVT_NS = 2, SVT_META = 3;
 __host__ __device__ __forceinline__ uint32_t sieve_redo_limit_impl(uint32_t n_parts) { return n_parts / 8 + 64; }
@@ -1546,8 +1564,9 @@ template <int N>
 __device__ __forceinline__ void tma_wait_group_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
-template <bool ONE_RUN>
+template <bool ONE_RUN, bool IN_PLACE>
 __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_kernel(CountParams P) {
+  static_assert(ONE_RUN || !IN_PLACE, "in place: the output segment is the one input segment");
   extern __shared__ __align__(128) unsigned char svt_raw[];
   constexpr int G = SVT_G, T = SVT_THREADS, NS = SVT_NS, NM = SVT_META;
   unsigned long long *stage = reinterpret_cast<unsigned long long *>(svt_raw);  // [NS][SVT_CAP] keys
@@ -1596,7 +1615,8 @@ __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_ker
     const uint32_t state = w >= P.n_parts ? 0u : (big || npad > SVT_CAP) ? 2u : npad ? 1u : 0u;
     if (lane < (int)R) { m_src[sl][lane] = reinterpret_cast<uint64_t>(P.runs[lane].keys + b); m_len[sl][lane] = pl; }
     if (lane == 0) {
-      if (state == 1u) { pend_ob = atomicAdd(P.out_cursor, (unsigned long long)npad); pend_npad = npad; pend_slot = sl; }
+      if (IN_PLACE) m_base[sl] = b;  // the output segment is the input segment
+      else if (state == 1u) { pend_ob = atomicAdd(P.out_cursor, (unsigned long long)npad); pend_npad = npad; pend_slot = sl; }
       m_npad[sl] = npad; m_np[sl] = np; m_work[sl] = w; m_state[sl] = state;
     }
     __syncwarp();
@@ -1656,9 +1676,14 @@ __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_ker
       if (lane == 0) handed_back = *reinterpret_cast<volatile uint32_t *>(P.redo_count);  // looked at when this iteration ends
     }
     if (state != 1u) {
+      if (IN_PLACE && state == 0u)  // an empty partition: its whole capacity is slack
+        for (uint32_t i = tid; i < P.part_cap; i += T) __stcs(P.out_counts + base + i, 0ull);
       if (tid == 0) {
-        if (state == 0u) { P.out_seg_start[p] = 0; P.out_seg_len[p] = 0; }
-        else { const uint32_t ri = atomicAdd(P.redo_count, 1u); P.redo_list[ri] = p; P.redo_base[ri] = NO_SPACE; P.redo_len[ri] = 0; }
+        if (state == 0u) { if (!IN_PLACE) P.out_seg_start[p] = 0; P.out_seg_len[p] = 0; }
+        else {  // in place, the compacting variant writes the partition into its own capacity
+          const uint32_t ri = atomicAdd(P.redo_count, 1u);
+          P.redo_list[ri] = p; P.redo_base[ri] = IN_PLACE ? base : NO_SPACE; P.redo_len[ri] = IN_PLACE ? P.part_cap : 0u;
+        }
         tma_wait_group_read<0>();
         issue((int)((it + 1) % NM), ks ^ 1);  // the next partition's keys
       }
@@ -1680,7 +1705,7 @@ __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_ker
           key[j] = st[min(idx, last)];  // rows past the end re-read the last entry and stay dead
           const bool lv = ONE_RUN ? idx < np : (idx < npad && key[j] != EMPTY_MIX);  // not the pad entry behind a segment of odd length
           live |= (lv ? 1u : 0u) << j;
-          if (fits && idx < npad) __stcs(P.out_counts + base + idx, lv ? 1ull : 0ull);
+          if (fits && idx < (IN_PLACE ? P.part_cap : npad)) __stcs(P.out_counts + base + idx, lv ? 1ull : 0ull);
           const uint32_t lo = (uint32_t)key[j];
           old[j] = lv ? atomicOr(&bm[(lo >> 5) & (SV_BM_WORDS - 1)], __funnelshift_l(0u, 1u, lo)) : 0u;
         }
@@ -1689,6 +1714,8 @@ __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_ker
           const uint32_t lo = (uint32_t)key[j];
           if (__funnelshift_r(old[j], 0u, lo) & 1u) atomicOr(&s_bloom[(lo >> 5) & (SVT_BLOOM_WORDS - 1)], __funnelshift_l(0u, 1u, lo));
         }
+        if (IN_PLACE)  // the capacity may exceed one batch
+          for (uint32_t i = (uint32_t)G * T + tid; i < P.part_cap; i += T) __stcs(P.out_counts + base + i, 0ull);
       }
       if (tid == 0) {  // the other key stage: its last store has had this pass to leave shared memory
         tma_wait_group_read<0>();
@@ -1747,7 +1774,7 @@ __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_ker
             }
             if (st[cur - 1u] == k) {  // the owner of a slot is never patched: its key stays readable
               atomicAdd(&Lcnt[s], 1u);
-              st[idx] = EMPTY_MIX;
+              if (!IN_PLACE) st[idx] = EMPTY_MIX;
               if (fits) P.out_counts[base + idx] = 0ull;  // after this entry's own 1 (two barriers ago)
               atomicAdd(&s_holes, 1u);  // of this partition
               break;
@@ -1756,7 +1783,7 @@ __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_ker
           }
         }
       }
-      fence_proxy_async_smem();  // this thread's patches of the stage, ahead of the bulk store
+      if (!IN_PLACE) fence_proxy_async_smem();  // this thread's patches of the stage, ahead of the bulk store
       __syncthreads();           // D: L's counters are final
       const bool fail = nq > SVT_Q || s_fail != 0;
       if (!fail) {
@@ -1776,13 +1803,19 @@ __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_ker
           Lslot[my_slot[u]] = 0; Lcnt[my_slot[u]] = 0;
         }
         if (tid == 0) {
-          if (fits) tma_store_1d(P.out_keys + base, st, npad * 8u);
-          P.out_seg_start[p] = fits ? base : 0; P.out_seg_len[p] = npad;
+          if (!IN_PLACE) {
+            if (fits) tma_store_1d(P.out_keys + base, st, npad * 8u);
+            P.out_seg_start[p] = fits ? base : 0;
+          }
+          P.out_seg_len[p] = npad;
           my_entries += np - s_holes;
         }
       } else {  // too many repeated keys: the partition goes to the compacting variant, which writes into the range reserved here
         for (uint32_t i = tid; i < SVT_L_SLOTS; i += T) { Lslot[i] = 0; Lcnt[i] = 0; }
-        if (tid == 0) { const uint32_t ri = atomicAdd(P.redo_count, 1u); P.redo_list[ri] = p; P.redo_base[ri] = base; P.redo_len[ri] = npad; }
+        if (tid == 0) {
+          const uint32_t ri = atomicAdd(P.redo_count, 1u);
+          P.redo_list[ri] = p; P.redo_base[ri] = base; P.redo_len[ri] = IN_PLACE ? P.part_cap : npad;
+        }
       }
       if (tid < (int)SVT_BLOOM_WORDS) s_bloom[tid] = 0;
     }
@@ -1821,7 +1854,9 @@ cudaError_t launch_count_partitions_sieve(const CountParams &P, bool padded, cud
   if (P.n_parts == 0) return cudaSuccess;
   if (!P.redo_list || !P.redo_count || !P.redo_base || !P.redo_len) return cudaErrorInvalidValue;
   if (padded) {
-    auto kern = P.R == 1 ? count_partitions_sieve_tma_kernel<true> : count_partitions_sieve_tma_kernel<false>;
+    if (P.part_cap && P.R != 1) return cudaErrorInvalidValue;
+    auto kern = P.part_cap ? count_partitions_sieve_tma_kernel<true, true>
+                : P.R == 1 ? count_partitions_sieve_tma_kernel<true, false> : count_partitions_sieve_tma_kernel<false, false>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SVT_SMEM);
     if (e != cudaSuccess) return e;
     g_launches.fetch_add(1, std::memory_order_relaxed);
