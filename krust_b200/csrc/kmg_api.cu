@@ -760,7 +760,7 @@ kmg_status consolidate(kmg_ctx *c, bool recompact) {
   }
   bool sieve_padded = sieve;
   for (auto *r : in) sieve_padded = sieve_padded && r->padded;
-  // In place (count_partitions_sieve_tma_kernel<true, true>): one raw run in the speculative layout is counted where it lies.  The
+  // In place (count_partitions_sieve_in_place_kernel): one raw run in the speculative layout is counted where it lies.  The
   // result takes over its keys and segment starts and gets a count for every slot of the layout (0: repeat, pad entry or slack), so
   // phase B writes 8 bytes per slot instead of 16 per entry and no second key array is held.  Each fallback below leaves the route
   // for the copying one: the kernel never writes the keys, so the input is intact until the compacting variant has run.  The

@@ -1541,12 +1541,8 @@ __global__ void __launch_bounds__(SV_THREADS, 2) count_partitions_sieve_kernel(C
 //     (32-bit CAS; the key of a slot is read from the stage): first claimant = the entry that stays, the others become fillers;
 //   * two 512-thread CTAs per SM, so one CTA's barriers overlap the other's work; output ranges are reserved when the segment
 //     table is fetched (two partitions ahead), so no global atomic sits on the critical path.
-// The output segment is the padded input: entries (EMPTY, 0) are fillers every reader skips.
-// IN_PLACE (one raw run in a strided layout, P.part_cap): the stored keys would be byte-identical to the loaded ones except for
-// the rare repeats, so the output run keeps the input's key array and layout and only counts are written -- 8 B in and 8 B per
-// slot of capacity out per key instead of 8 in and 16 out.  A repeat keeps its key and gets count 0; the pad entry and the slack
-// behind the segment get count 0 too, so whole-array readers skip them whatever keys sit there.  The keys are never written, so
-// every fallback of the host (early stop, the launch without the sieve) rereads an intact input.
+// The output segment is the padded input: entries (EMPTY, 0) are fillers every reader skips.  The in-place variant of this scheme
+// (count_partitions_sieve_in_place_kernel) follows it.
 // ---------------------------------------------------------------------------------------------------
 constexpr int SVT_THREADS = 512, SVT_G = 8, SVT_NS = 2, SVT_META = 3;
 __host__ __device__ __forceinline__ uint32_t sieve_redo_limit_impl(uint32_t n_parts) { return n_parts / 8 + 64; }
@@ -1564,9 +1560,13 @@ template <int N>
 __device__ __forceinline__ void tma_wait_group_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
-template <bool ONE_RUN, bool IN_PLACE>
+__device__ __forceinline__ void hist_add(uint32_t *s_hist, const CountParams &P, unsigned long long cnt) {
+  if (cnt < (unsigned long long)HIST_CTA_BINS) atomicAdd(&s_hist[cnt], 1u);
+  else if (cnt < (unsigned long long)HIST_DENSE_BINS) atomicAdd(P.hist + cnt, 1ull);
+  else { const unsigned long long o = atomicAdd(P.hist + HIST_DENSE_BINS, 1ull); if (o < P.hist_overflow_cap) P.hist_overflow[o] = cnt; }
+}
+template <bool ONE_RUN>
 __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_kernel(CountParams P) {
-  static_assert(ONE_RUN || !IN_PLACE, "in place: the output segment is the one input segment");
   extern __shared__ __align__(128) unsigned char svt_raw[];
   constexpr int G = SVT_G, T = SVT_THREADS, NS = SVT_NS, NM = SVT_META;
   unsigned long long *stage = reinterpret_cast<unsigned long long *>(svt_raw);  // [NS][SVT_CAP] keys
@@ -1615,8 +1615,7 @@ __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_ker
     const uint32_t state = w >= P.n_parts ? 0u : (big || npad > SVT_CAP) ? 2u : npad ? 1u : 0u;
     if (lane < (int)R) { m_src[sl][lane] = reinterpret_cast<uint64_t>(P.runs[lane].keys + b); m_len[sl][lane] = pl; }
     if (lane == 0) {
-      if (IN_PLACE) m_base[sl] = b;  // the output segment is the input segment
-      else if (state == 1u) { pend_ob = atomicAdd(P.out_cursor, (unsigned long long)npad); pend_npad = npad; pend_slot = sl; }
+      if (state == 1u) { pend_ob = atomicAdd(P.out_cursor, (unsigned long long)npad); pend_npad = npad; pend_slot = sl; }
       m_npad[sl] = npad; m_np[sl] = np; m_work[sl] = w; m_state[sl] = state;
     }
     __syncwarp();
@@ -1676,13 +1675,11 @@ __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_ker
       if (lane == 0) handed_back = *reinterpret_cast<volatile uint32_t *>(P.redo_count);  // looked at when this iteration ends
     }
     if (state != 1u) {
-      if (IN_PLACE && state == 0u)  // an empty partition: its whole capacity is slack
-        for (uint32_t i = tid; i < P.part_cap; i += T) __stcs(P.out_counts + base + i, 0ull);
       if (tid == 0) {
-        if (state == 0u) { if (!IN_PLACE) P.out_seg_start[p] = 0; P.out_seg_len[p] = 0; }
-        else {  // in place, the compacting variant writes the partition into its own capacity
+        if (state == 0u) { P.out_seg_start[p] = 0; P.out_seg_len[p] = 0; }
+        else {
           const uint32_t ri = atomicAdd(P.redo_count, 1u);
-          P.redo_list[ri] = p; P.redo_base[ri] = IN_PLACE ? base : NO_SPACE; P.redo_len[ri] = IN_PLACE ? P.part_cap : 0u;
+          P.redo_list[ri] = p; P.redo_base[ri] = NO_SPACE; P.redo_len[ri] = 0u;
         }
         tma_wait_group_read<0>();
         issue((int)((it + 1) % NM), ks ^ 1);  // the next partition's keys
@@ -1705,7 +1702,7 @@ __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_ker
           key[j] = st[min(idx, last)];  // rows past the end re-read the last entry and stay dead
           const bool lv = ONE_RUN ? idx < np : (idx < npad && key[j] != EMPTY_MIX);  // not the pad entry behind a segment of odd length
           live |= (lv ? 1u : 0u) << j;
-          if (fits && idx < (IN_PLACE ? P.part_cap : npad)) __stcs(P.out_counts + base + idx, lv ? 1ull : 0ull);
+          if (fits && idx < npad) __stcs(P.out_counts + base + idx, lv ? 1ull : 0ull);
           const uint32_t lo = (uint32_t)key[j];
           old[j] = lv ? atomicOr(&bm[(lo >> 5) & (SV_BM_WORDS - 1)], __funnelshift_l(0u, 1u, lo)) : 0u;
         }
@@ -1714,8 +1711,6 @@ __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_ker
           const uint32_t lo = (uint32_t)key[j];
           if (__funnelshift_r(old[j], 0u, lo) & 1u) atomicOr(&s_bloom[(lo >> 5) & (SVT_BLOOM_WORDS - 1)], __funnelshift_l(0u, 1u, lo));
         }
-        if (IN_PLACE)  // the capacity may exceed one batch
-          for (uint32_t i = (uint32_t)G * T + tid; i < P.part_cap; i += T) __stcs(P.out_counts + base + i, 0ull);
       }
       if (tid == 0) {  // the other key stage: its last store has had this pass to leave shared memory
         tma_wait_group_read<0>();
@@ -1774,7 +1769,7 @@ __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_ker
             }
             if (st[cur - 1u] == k) {  // the owner of a slot is never patched: its key stays readable
               atomicAdd(&Lcnt[s], 1u);
-              if (!IN_PLACE) st[idx] = EMPTY_MIX;
+              st[idx] = EMPTY_MIX;
               if (fits) P.out_counts[base + idx] = 0ull;  // after this entry's own 1 (two barriers ago)
               atomicAdd(&s_holes, 1u);  // of this partition
               break;
@@ -1783,7 +1778,7 @@ __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_ker
           }
         }
       }
-      if (!IN_PLACE) fence_proxy_async_smem();  // this thread's patches of the stage, ahead of the bulk store
+      fence_proxy_async_smem();  // this thread's patches of the stage, ahead of the bulk store
       __syncthreads();           // D: L's counters are final
       const bool fail = nq > SVT_Q || s_fail != 0;
       if (!fail) {
@@ -1794,19 +1789,13 @@ __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_ker
           const unsigned long long cnt = 1ull + Lcnt[my_slot[u]];
           if (cnt > 1) {
             if (fits) P.out_counts[base + my_idx[u]] = cnt;
-            if (P.hist) {
-              if (cnt < (unsigned long long)HIST_CTA_BINS) atomicAdd(&s_hist[cnt], 1u);
-              else if (cnt < (unsigned long long)HIST_DENSE_BINS) atomicAdd(P.hist + cnt, 1ull);
-              else { const unsigned long long o = atomicAdd(P.hist + HIST_DENSE_BINS, 1ull); if (o < P.hist_overflow_cap) P.hist_overflow[o] = cnt; }
-            }
+            if (P.hist) hist_add(s_hist, P, cnt);
           }
           Lslot[my_slot[u]] = 0; Lcnt[my_slot[u]] = 0;
         }
         if (tid == 0) {
-          if (!IN_PLACE) {
-            if (fits) tma_store_1d(P.out_keys + base, st, npad * 8u);
-            P.out_seg_start[p] = fits ? base : 0;
-          }
+          if (fits) tma_store_1d(P.out_keys + base, st, npad * 8u);
+          P.out_seg_start[p] = fits ? base : 0;
           P.out_seg_len[p] = npad;
           my_entries += np - s_holes;
         }
@@ -1814,7 +1803,7 @@ __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_ker
         for (uint32_t i = tid; i < SVT_L_SLOTS; i += T) { Lslot[i] = 0; Lcnt[i] = 0; }
         if (tid == 0) {
           const uint32_t ri = atomicAdd(P.redo_count, 1u);
-          P.redo_list[ri] = p; P.redo_base[ri] = base; P.redo_len[ri] = IN_PLACE ? P.part_cap : npad;
+          P.redo_list[ri] = p; P.redo_base[ri] = base; P.redo_len[ri] = npad;
         }
       }
       if (tid < (int)SVT_BLOOM_WORDS) s_bloom[tid] = 0;
@@ -1831,6 +1820,223 @@ __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_ker
     tma_wait_group_read<0>();
     if (my_entries) atomicAdd(P.out_distinct, my_entries);
   }
+  if (P.hist) hist_flush(s_hist, P, tid);
+}
+
+// ---------------------------------------------------------------------------------------------------
+// The sieve in place (one raw run in a strided layout, P.part_cap): the stored keys would be byte-identical to the loaded ones
+// except for the rare repeats, so the output run keeps the input's key array and layout and only counts are written -- 8 B in and
+// 8 B per slot of capacity out per key instead of 8 in and 16 out.  A repeat keeps its key and gets count 0; the pad entry and the
+// slack behind the segment get count 0 too, so whole-array readers skip them whatever keys sit there.  The keys are never written,
+// so every fallback of the host (early stop, the launch without the sieve) rereads an intact input.
+// The passes are those of the TMA sieve above.  Without a bulk store the stage only has to live until the queue is resolved, so a
+// CTA has one key stage and keeps no keys in registers across its barriers (pass 2 and the queue re-read the stage); the next
+// partition's bulk load is issued right after barrier D.  The shared memory a second stage would take holds more partitions in
+// flight instead: four 256-thread CTAs per SM, whose chains of a bulk load and four block barriers per partition overlap.  The bit
+// map is 2^16 bits: a partition of ~3500 keys has ~90 suspects and a queue of ~300 entries, well inside SVT_Q and SVT_L_MAX.
+// ---------------------------------------------------------------------------------------------------
+constexpr int SVI_THREADS = 256, SVI_G = 16, SVI_BATCH = 8, SVI_CTAS_PER_SM = 4;
+constexpr uint32_t SVI_BM_WORDS = 1u << (16 - 5);  // 8 KiB
+static_assert(SVI_THREADS * SVI_G == (int)SVT_CAP, "one stage per partition");
+constexpr size_t SVI_SMEM = (size_t)SVT_CAP * 8 + (size_t)SVI_BM_WORDS * 4 + (size_t)SVT_L_SLOTS * 8 + (size_t)SVT_Q * 2;
+
+__global__ void __launch_bounds__(SVI_THREADS, SVI_CTAS_PER_SM) count_partitions_sieve_in_place_kernel(CountParams P) {
+  extern __shared__ __align__(128) unsigned char svi_raw[];
+  constexpr int G = SVI_G, T = SVI_THREADS, NM = SVT_META;
+  unsigned long long *st = reinterpret_cast<unsigned long long *>(svi_raw);  // [SVT_CAP] keys
+  const uint32_t *st32 = reinterpret_cast<const uint32_t *>(st);             // st32[2 * i]: low half of key i
+  uint32_t *bm = reinterpret_cast<uint32_t *>(st + SVT_CAP);                 // bit map
+  uint32_t *Lslot = bm + SVI_BM_WORDS;
+  uint32_t *Lcnt = Lslot + SVT_L_SLOTS;
+  uint16_t *Q = reinterpret_cast<uint16_t *>(Lcnt + SVT_L_SLOTS);
+  __shared__ __align__(8) uint64_t bar;
+  __shared__ unsigned long long m_base[NM];  // the partition's segment: its first slot in the input (and output) run
+  __shared__ uint32_t m_npad[NM], m_np[NM], m_work[NM], m_state[NM];  // state: 0 empty, 1 staged, 2 left to the compacting variant
+  __shared__ uint32_t s_hist[HIST_CTA_BINS], s_bloom[SVT_BLOOM_WORDS];
+  __shared__ uint32_t s_nq, s_nL, s_fail, s_holes;
+  const int tid = threadIdx.x;
+
+  // thread 0 only: the segment table of work item w is loaded when an iteration starts and published when it ends
+  auto fetch = [&](uint32_t w, uint64_t &b, uint64_t &len) {
+    b = 0; len = 0;
+    if (w < P.n_parts) {
+      const uint32_t p = P.order ? P.order[w] : w;
+      b = P.runs[0].seg_start[p]; len = P.runs[0].seg_len[p];
+    }
+  };
+  auto publish = [&](int sl, uint32_t w, uint64_t b, uint64_t len) {
+    const uint32_t np = len > (uint64_t)SVT_CAP ? 0u : (uint32_t)len;
+    m_base[sl] = b; m_npad[sl] = (np + 1u) & ~1u; m_np[sl] = np; m_work[sl] = w;
+    m_state[sl] = w >= P.n_parts ? 0u : len > (uint64_t)SVT_CAP ? 2u : np ? 1u : 0u;
+  };
+  auto issue = [&](int sl) {  // the bulk load of the partition in metadata slot sl into the key stage
+    if (m_state[sl] != 1u) return;
+    mbar_expect_tx(&bar, m_npad[sl] * 8u);
+    tma_load_1d(st, P.runs[0].keys + m_base[sl], m_npad[sl] * 8u, &bar);
+  };
+
+  if (tid < HIST_CTA_BINS) s_hist[tid] = 0;
+  if (tid < (int)SVT_BLOOM_WORDS) s_bloom[tid] = 0;
+  for (uint32_t i = tid; i < SVT_L_SLOTS; i += T) { Lslot[i] = 0; Lcnt[i] = 0; }
+  for (uint32_t i = tid; i < SVI_BM_WORDS; i += T) bm[i] = 0;
+  uint32_t w_ahead = 0;  // thread 0: the work item two after the current one
+  if (tid == 0) {
+    s_nq = 0; s_nL = 0; s_fail = 0; s_holes = 0;
+    mbar_init(&bar, 1);
+    mbar_fence_init();
+    const uint32_t w0 = atomicAdd(P.next, 1u), w1 = atomicAdd(P.next, 1u);
+    w_ahead = atomicAdd(P.next, 1u);
+    uint64_t b, len;
+    fetch(w0, b, len); publish(0, w0, b, len);
+    fetch(w1, b, len); publish(1, w1, b, len);
+    issue(0);
+  }
+  __syncthreads();
+
+  unsigned long long my_entries = 0;  // tid 0: distinct keys of the partitions this CTA counted
+  uint32_t ph = 0;                    // parity of the key stage's next completion
+  for (uint32_t it = 0;; ++it) {
+    const int sl = (int)(it % NM), sl_next = (int)((it + 1) % NM);
+    const uint32_t work = m_work[sl];
+    if (work >= P.n_parts) break;
+    const uint32_t state = m_state[sl], npad = m_npad[sl], np = m_np[sl];
+    const unsigned long long base = m_base[sl];
+    const uint32_t p = P.order ? P.order[work] : work;
+    uint32_t wn = 0, handed_back = 0;
+    uint64_t nb = 0, nlen = 0;
+    if (tid == 0) {
+      wn = w_ahead;
+      fetch(wn, nb, nlen);
+      if (wn < P.n_parts) w_ahead = atomicAdd(P.next, 1u);
+      handed_back = *reinterpret_cast<volatile uint32_t *>(P.redo_count);  // looked at when this iteration ends
+    }
+    if (state != 1u) {
+      if (state == 0u)  // an empty partition: its whole capacity is slack
+        for (uint32_t i = tid; i < P.part_cap; i += T) __stcs(P.out_counts + base + i, 0ull);
+      if (tid == 0) {
+        if (state == 0u) P.out_seg_len[p] = 0;
+        else {  // the compacting variant writes the partition into its own capacity
+          const uint32_t ri = atomicAdd(P.redo_count, 1u);
+          P.redo_list[ri] = p; P.redo_base[ri] = base; P.redo_len[ri] = P.part_cap;
+        }
+        issue(sl_next);
+      }
+    } else {
+      // the previous partition's queue / table counters: everybody read them before barrier A, nobody touches them before barrier B
+      if (tid == 0) { s_nq = 0; s_nL = 0; s_fail = 0; s_holes = 0; }
+      mbar_wait(&bar, ph);
+      ph ^= 1u;
+      // ---- pass 1: read the staged keys' low halves, write the counts (1 per live entry), test-and-set in the bit map
+      const uint32_t last = npad - 1u;
+      uint32_t live = 0;
+#pragma unroll
+      for (int h = 0; h < G; h += SVI_BATCH) {
+        uint32_t lo[SVI_BATCH], old[SVI_BATCH];
+#pragma unroll
+        for (int j = 0; j < SVI_BATCH; ++j) {
+          const uint32_t idx = (uint32_t)(h + j) * T + tid;
+          lo[j] = st32[2u * min(idx, last)];  // rows past the end re-read the last entry and stay dead
+          const bool lv = idx < np;           // not the pad entry behind a segment of odd length
+          live |= (lv ? 1u : 0u) << (h + j);
+          if (idx < P.part_cap) __stcs(P.out_counts + base + idx, lv ? 1ull : 0ull);
+          old[j] = lv ? atomicOr(&bm[(lo[j] >> 5) & (SVI_BM_WORDS - 1)], __funnelshift_l(0u, 1u, lo[j])) : 0u;
+        }
+#pragma unroll
+        for (int j = 0; j < SVI_BATCH; ++j)  // a suspect (its bit was already set) marks the filter
+          if (__funnelshift_r(old[j], 0u, lo[j]) & 1u) atomicOr(&s_bloom[(lo[j] >> 5) & (SVT_BLOOM_WORDS - 1)], __funnelshift_l(0u, 1u, lo[j]));
+      }
+      for (uint32_t i = (uint32_t)G * T + tid; i < P.part_cap; i += T) __stcs(P.out_counts + base + i, 0ull);  // the capacity may exceed one stage
+      __syncthreads();  // B: bit map and filter complete
+      {
+        uint4 *bm4 = reinterpret_cast<uint4 *>(bm);
+#pragma unroll
+        for (uint32_t i = 0; i < SVI_BM_WORDS / 4 / T; ++i) bm4[i * T + tid] = make_uint4(0u, 0u, 0u, 0u);
+      }
+      // ---- pass 2: the entries the filter flags are queued
+      {
+        uint32_t hit = 0;
+#pragma unroll
+        for (int j = 0; j < G; ++j) {
+          const uint32_t lo = st32[2u * min((uint32_t)j * T + tid, last)];
+          hit |= ((s_bloom[(lo >> 5) & (SVT_BLOOM_WORDS - 1)] & __funnelshift_l(0u, 1u, lo)) ? 1u : 0u) << j;
+        }
+        hit &= live;
+        if (hit) {
+          uint32_t q = atomicAdd(&s_nq, (uint32_t)__popc(hit));
+          while (hit) {
+            const uint32_t j = (uint32_t)__ffs((int)hit) - 1u;
+            if (q < SVT_Q) Q[q] = (uint16_t)(j * T + tid);
+            ++q;
+            hit &= hit - 1u;
+          }
+        }
+      }
+      __syncthreads();  // C: the queue is complete
+      const uint32_t nq = s_nq;
+      // ---- resolve the queue: entry e claims a slot of L for its key or meets the entry that did
+      if (nq <= SVT_Q)
+        for (uint32_t e = tid; e < nq; e += T) {
+          const uint32_t idx = Q[e];
+          const unsigned long long k = st[idx];
+          uint32_t s = (uint32_t)(k >> 32) & (SVT_L_SLOTS - 1);
+          for (uint32_t t = 0;; ++t) {
+            if (t > SVT_L_SLOTS) { atomicExch(&s_fail, 1u); break; }
+            uint32_t cur = *reinterpret_cast<volatile uint32_t *>(&Lslot[s]);
+            if (cur == 0u) {
+              if (*reinterpret_cast<volatile uint32_t *>(&s_fail)) break;  // bounds the entries: every thread has at most one claim past this test
+              cur = atomicCAS(&Lslot[s], 0u, idx + 1u);
+              if (cur == 0u) {
+                if (atomicAdd(&s_nL, 1u) >= SVT_L_MAX) atomicExch(&s_fail, 1u);
+                break;
+              }
+            }
+            if (st[cur - 1u] == k) {
+              atomicAdd(&Lcnt[s], 1u);
+              P.out_counts[base + idx] = 0ull;  // after this entry's own 1 (two barriers ago)
+              atomicAdd(&s_holes, 1u);          // of this partition
+              break;
+            }
+            s = (s + 1u) & (SVT_L_SLOTS - 1);
+          }
+        }
+      __syncthreads();  // D: L's counters are final; nobody reads the stage any more
+      if (tid == 0) issue(sl_next);
+      const bool fail = nq > SVT_Q || s_fail != 0;
+      {  // the entries that own a slot of L carry their key's count; L is cleaned (one slot quad per thread)
+        static_assert(SVT_L_SLOTS == 4 * T, "one uint4 of L per thread");
+        uint4 *ls4 = reinterpret_cast<uint4 *>(Lslot) + tid, *lc4 = reinterpret_cast<uint4 *>(Lcnt) + tid;
+        const uint4 ls = *ls4, lc = *lc4;
+        if (!fail && (lc.x | lc.y | lc.z | lc.w)) {
+          const uint32_t own[4] = {ls.x, ls.y, ls.z, ls.w}, more[4] = {lc.x, lc.y, lc.z, lc.w};
+#pragma unroll
+          for (int u = 0; u < 4; ++u) {
+            if (!more[u]) continue;
+            const unsigned long long cnt = 1ull + more[u];
+            P.out_counts[base + own[u] - 1u] = cnt;
+            if (P.hist) hist_add(s_hist, P, cnt);
+          }
+        }
+        if (ls.x | ls.y | ls.z | ls.w) { *ls4 = make_uint4(0u, 0u, 0u, 0u); *lc4 = make_uint4(0u, 0u, 0u, 0u); }
+      }
+      if (tid == 0) {
+        if (!fail) {
+          P.out_seg_len[p] = npad;
+          my_entries += np - s_holes;
+        } else {  // too many repeated keys: the compacting variant writes the partition into its own capacity
+          const uint32_t ri = atomicAdd(P.redo_count, 1u);
+          P.redo_list[ri] = p; P.redo_base[ri] = base; P.redo_len[ri] = P.part_cap;
+        }
+      }
+      s_bloom[tid % SVT_BLOOM_WORDS] = 0;  // by every thread: a predicate kept across the loop would cost a register
+    }
+    if (tid == 0) {
+      // a duplicate-rich input (most partitions handed back) is not this variant's business: stop early, the host repeats the launch without it
+      if (handed_back > sieve_redo_limit(P.n_parts)) { wn = 0xffffffffu; nb = 0; nlen = 0; }
+      publish((int)((it + 2) % NM), wn, nb, nlen);
+    }
+    __syncthreads();  // A
+  }
+  if (tid == 0 && my_entries) atomicAdd(P.out_distinct, my_entries);
   if (P.hist) hist_flush(s_hist, P, tid);
 }
 
@@ -1854,9 +2060,16 @@ cudaError_t launch_count_partitions_sieve(const CountParams &P, bool padded, cud
   if (P.n_parts == 0) return cudaSuccess;
   if (!P.redo_list || !P.redo_count || !P.redo_base || !P.redo_len) return cudaErrorInvalidValue;
   if (padded) {
-    if (P.part_cap && P.R != 1) return cudaErrorInvalidValue;
-    auto kern = P.part_cap ? count_partitions_sieve_tma_kernel<true, true>
-                : P.R == 1 ? count_partitions_sieve_tma_kernel<true, false> : count_partitions_sieve_tma_kernel<false, false>;
+    if (P.part_cap) {
+      if (P.R != 1) return cudaErrorInvalidValue;
+      cudaError_t e = cudaFuncSetAttribute(count_partitions_sieve_in_place_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SVI_SMEM);
+      if (e != cudaSuccess) return e;
+      g_launches.fetch_add(1, std::memory_order_relaxed);
+      count_partitions_sieve_in_place_kernel<<<(unsigned)std::min<uint64_t>(P.n_parts, (uint64_t)num_sms() * SVI_CTAS_PER_SM), SVI_THREADS,
+                                               SVI_SMEM, s>>>(P);
+      return cudaGetLastError();
+    }
+    auto kern = P.R == 1 ? count_partitions_sieve_tma_kernel<true> : count_partitions_sieve_tma_kernel<false>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SVT_SMEM);
     if (e != cudaSuccess) return e;
     g_launches.fetch_add(1, std::memory_order_relaxed);
