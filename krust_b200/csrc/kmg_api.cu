@@ -60,12 +60,12 @@ struct Staging {
 
 // A run is a partition-indexed list of keys (phase A output, every key counts 1) or of (key, count)
 // pairs (phase B output / weighted inserts).  All runs of a context share the same partition count;
-// partition p of a run is entries [seg_start[p], seg_start[p] + seg_len[p]).
+// partition p of a run is entries [seg_start[p], seg_start[p] + seg_len[p]).  A run built by refine_to_run (a raw run, or weighted
+// keys) is padded: its segments start on 16-byte boundaries and an EMPTY_MIX key follows every segment of odd length.
 struct Run {
   uint64_t *d_keys = nullptr, *d_counts = nullptr, *d_seg_start = nullptr, *d_seg_len = nullptr;
   uint64_t n = 0;        // entries (a consolidated run may hold skipped filler entries, see count_partitions_smem_kernel)
   uint64_t n_valid = 0;  // consolidated runs: distinct keys
-  bool padded = false;   // speculative layout: segments start on 16-byte boundaries and an EMPTY_MIX entry follows every segment of odd length
   uint64_t part_cap = 0;  // raw run in the speculative layout: partition p owns entries [p * part_cap, (p + 1) * part_cap); 0: exact layout
 };
 
@@ -337,6 +337,9 @@ void timers_collect(kmg_ctx *c) {
 // (kernels and rationale: kmg_partition.cu).
 // =================================================================================================
 constexpr uint64_t TARGET_KEYS_PER_PART = 3600;  // <= 4096 with 8 sigma to spare: one upsert round per partition; load ~0.44
+// entries one refine_to_run call takes: the exact layout places them at 32-bit positions, with room for one pad entry per
+// partition (at most 2048 x 2048)
+constexpr uint64_t REFINE_MAX_ENTRIES = (1ull << 32) - 2048ull * 2048;
 
 // n_coarse / n_sub are set: allocate the partitioned pipeline's bookkeeping
 kmg_status init_partitioned(kmg_ctx *c) {
@@ -434,6 +437,16 @@ kmg_status refine_to_run(kmg_ctx *c, uint64_t *d_ckeys, uint64_t *d_ccounts, con
   uint64_t *d_cstart = nullptr, *d_clen = nullptr;
   uint32_t *d_tprefix = nullptr;
   auto cleanup = [&]() { if (owns) { pool_free(c, d_ckeys); pool_free(c, d_ccounts); } pool_free(c, d_cstart); pool_free(c, d_clen); pool_free(c, d_tprefix); };
+  if (n + P > (1ull << 32)) { cleanup(); return fail(c, KMG_ERR_STATE, "refine: more entries than 32-bit positions hold with a pad entry per partition"); }
+  // both layouts end here: the pad entries behind odd segments, then the run is handed over
+  auto finish = [&]() -> kmg_status {
+    const cudaError_t pe = launch_pad_segments(r.d_keys, r.d_seg_start, r.d_seg_len, P, c->stream);
+    if (pe != cudaSuccess) { free_run(c, r); return cuda_fail(c, pe, "pad segments"); }
+    r.n = n;
+    if (split) { *split->out = std::move(r); return KMG_OK; }
+    guard.release();  // the run is complete: a consolidation triggered by add_run may re-split it with the others
+    return add_run(c, std::move(r));
+  };
   std::vector<uint32_t> tprefix(P1 + 1, 0);
   uint64_t tiles = 0;
   for (uint32_t p = 0; p < P1; ++p) { tprefix[p] = (uint32_t)tiles; tiles += (len_of(p) + REFINE_TILE - 1) / REFINE_TILE; }
@@ -488,12 +501,8 @@ kmg_status refine_to_run(kmg_ctx *c, uint64_t *d_ckeys, uint64_t *d_ccounts, con
     if (e != cudaSuccess) { cleanup(); free_run(c, r); return cuda_fail(c, e, "refine scatter (speculative layout)"); }
     if (!h_flag) {
       cleanup();
-      r.n = n;
       r.part_cap = cap_f;
-      if (!(cap_f & 1ull) && launch_pad_segments(r.d_keys, r.d_seg_start, r.d_seg_len, P, c->stream) == cudaSuccess) r.padded = true;
-      if (split) { *split->out = std::move(r); return KMG_OK; }
-      guard.release();  // the run is complete: a consolidation triggered by add_run may re-split it with the others
-      return add_run(c, std::move(r));
+      return finish();
     }
     c->spec_fine_ok = false;
     pool_free(c, r.d_keys); r.d_keys = nullptr;
@@ -514,10 +523,12 @@ kmg_status refine_to_run(kmg_ctx *c, uint64_t *d_ckeys, uint64_t *d_ccounts, con
     c->scan_tmp_items = P;
   }
 
-  if (e == cudaSuccess) e = exclusive_sum_u64(r.d_seg_len, r.d_seg_start, P, c->d_scan_tmp, &c->scan_tmp_bytes, c->stream);
+  // segment p starts at the prefix of the lengths rounded up to even: room for its pad entry, and a 16-byte aligned start
+  if (e == cudaSuccess) e = launch_even_lengths(r.d_seg_len, r.d_seg_start, P, c->stream);
+  if (e == cudaSuccess) e = exclusive_sum_u64(r.d_seg_start, r.d_seg_start, P, c->d_scan_tmp, &c->scan_tmp_bytes, c->stream);
   if (e != cudaSuccess) { cleanup(); free_run(c, r); return cuda_fail(c, e, "refine count"); }
-  kmg_status s = alloc_or_consolidate(c, reinterpret_cast<void **>(&r.d_keys), n * 8, "fine keys");
-  if (s == KMG_OK && d_ccounts) s = alloc_or_consolidate(c, reinterpret_cast<void **>(&r.d_counts), n * 8, "fine counts");
+  kmg_status s = alloc_or_consolidate(c, reinterpret_cast<void **>(&r.d_keys), (n + P) * 8, "fine keys");
+  if (s == KMG_OK && d_ccounts) s = alloc_or_consolidate(c, reinterpret_cast<void **>(&r.d_counts), (n + P) * 8, "fine counts");
   if (s != KMG_OK) { cleanup(); free_run(c, r); return s; }
   rp.out_keys = r.d_keys; rp.out_counts = r.d_counts;
   const size_t tmr4 = timer_begin(c, 2);
@@ -526,10 +537,7 @@ kmg_status refine_to_run(kmg_ctx *c, uint64_t *d_ckeys, uint64_t *d_ccounts, con
   if (e == cudaSuccess && sync) e = cudaStreamSynchronize(c->stream);
   cleanup();
   if (e != cudaSuccess) { free_run(c, r); return cuda_fail(c, e, "refine scatter"); }
-  r.n = n;
-  if (split) { *split->out = std::move(r); return KMG_OK; }
-  guard.release();
-  return add_run(c, std::move(r));
+  return finish();
 }
 
 // A1 over the packed stream: coarse count pass, exact offsets, coarse scatter; then A2.
@@ -538,7 +546,7 @@ kmg_status scan_to_run(kmg_ctx *c, uint64_t n_words_total, bool has_start) {
   if (c->feed_kind == 2) return fail(c, KMG_ERR_STATE, "context holds blocks adopted from a sender (kmg_adopt_coarse_device): it cannot also scan input itself");
   c->feed_kind = 1;
   const uint64_t n_tiles = n_words_total / TILE_WORDS;
-  const uint64_t max_tiles = ((1ull << 32) - 1) / ((uint64_t)TILE_WORDS * 32);  // < 2^32 windows per launch
+  const uint64_t max_tiles = REFINE_MAX_ENTRIES / ((uint64_t)TILE_WORDS * 32);  // < 2^32 windows per launch, one refine_to_run each
   const uint32_t P1 = c->n_coarse;
   unsigned long long *d_cnt = c->d_part, *d_start = c->d_part + MAX_PARTS, *d_cur = c->d_part + 2 * MAX_PARTS;
   for (uint64_t tile0 = 0; tile0 < n_tiles; tile0 += max_tiles) {
@@ -615,7 +623,7 @@ kmg_status keys_to_run(kmg_ctx *c, const uint64_t *d_keys, const uint64_t *d_cou
   c->feed_kind = 1;
   const uint32_t P1 = c->n_coarse;
   unsigned long long *d_cnt = c->d_part, *d_start = c->d_part + MAX_PARTS, *d_cur = c->d_part + 2 * MAX_PARTS;
-  const uint64_t max_n = (1ull << 32) - 1;
+  const uint64_t max_n = REFINE_MAX_ENTRIES;
   for (uint64_t i0 = 0; i0 < n; i0 += max_n) {
     const uint64_t m = std::min(max_n, n - i0);
     const size_t tmr = timer_begin(c, 0);
@@ -646,7 +654,7 @@ kmg_status resplit_runs(kmg_ctx *c, uint32_t m) {
   std::vector<Run *> all;
   if (c->has_result && c->result.n) all.push_back(&c->result);
   for (auto &r : c->runs) all.push_back(&r);
-  for (auto *r : all) if (r->n >= (1ull << 32) - 1) return KMG_OK;  // refine launches index with 32 bits: leave it to the multi-pass kernel
+  for (auto *r : all) if (r->n > REFINE_MAX_ENTRIES) return KMG_OK;  // refine launches index with 32 bits: leave it to the multi-pass kernel
   c->in_resplit = true;
   kmg_status st = KMG_OK;
   std::vector<uint64_t> off(P_old + 1), lens(P_old);
@@ -749,7 +757,7 @@ kmg_status consolidate(kmg_ctx *c, bool recompact) {
   // deep read set), partitions within the plan.  Its output holds one entry per input entry.
   bool direct = !recompact && raw_entries == total && c->dedup_ratio >= 0.5 && max_total <= 0xffffu &&
                 total / std::max<uint32_t>(P, 1) <= SMEM_TABLE_SLOTS / 2 && !(c->cfg.flags & KMG_FLAG_NO_PREAGG);
-  // Sieve variant (count_partitions_sieve_kernel): same precondition; it leaves the partitions it cannot take (too many repeated keys,
+  // Sieve variant (count_partitions_sieve_tma_kernel): same precondition; it leaves the partitions it cannot take (too many repeated keys,
   // more than one batch of entries) to the compacting variant, so no bound on the largest partition is needed.
   bool sieve = !recompact && raw_entries == total && c->dedup_ratio >= 0.5 &&
                total / std::max<uint32_t>(P, 1) <= SIEVE_MAX_ENTRIES * 15 / 16 && !(c->cfg.flags & KMG_FLAG_NO_PREAGG);
@@ -758,17 +766,15 @@ kmg_status consolidate(kmg_ctx *c, bool recompact) {
   if (sieve && (pool_alloc(c, &d_redo, (size_t)P * 8) != cudaSuccess || pool_alloc(c, &d_redo_base, (size_t)P * 8) != cudaSuccess)) {  // d_redo: partition numbers, then range lengths
     cudaGetLastError(); pool_free(c, d_redo); pool_free(c, d_redo_base); d_redo = nullptr; d_redo_base = nullptr; sieve = false;
   }
-  bool sieve_padded = sieve;
-  for (auto *r : in) sieve_padded = sieve_padded && r->padded;
   // In place (count_partitions_sieve_in_place_kernel): one raw run in the speculative layout is counted where it lies.  The
   // result takes over its keys and segment starts and gets a count for every slot of the layout (0: repeat, pad entry or slack), so
   // phase B writes 8 bytes per slot instead of 16 per entry and no second key array is held.  Each fallback below leaves the route
   // for the copying one: the kernel never writes the keys, so the input is intact until the compacting variant has run.  The
   // partitions it hands over are compacted into their own capacity, which is only safe while that variant cannot overflow: a
   // capacity of at most two batches (2 x 4096 entries) fits its 8192-slot table and, at 256 claims per warp and batch, its warp lists.
-  bool in_place = sieve_padded && R == 1 && in[0]->part_cap != 0 && in[0]->part_cap <= 2ull * SMEM_COUNT_THREADS * 8;
+  bool in_place = sieve && R == 1 && in[0]->part_cap != 0 && in[0]->part_cap <= 2ull * SMEM_COUNT_THREADS * 8;
   const uint64_t in_place_n = in_place ? (uint64_t)P * in[0]->part_cap : 0;
-  uint64_t out_cap = std::max<uint64_t>(total, 1) + (sieve_padded ? (uint64_t)P * R : 0);  // padded segments: up to one filler entry per partition and run
+  uint64_t out_cap = std::max<uint64_t>(total, 1) + (sieve ? (uint64_t)P * R : 0);  // padded segments: up to one filler entry per partition and run
   if (recompact) out_cap = std::min<uint64_t>(out_cap, c->result.n_valid + (1ull << 20));
   else if (total > (1ull << 28) && !direct && !sieve) {
     const uint64_t est = (total - raw_entries) + (uint64_t)((double)raw_entries * std::min(1.0, c->dedup_ratio * 1.25 + 0.02)) + (1ull << 24);
@@ -855,17 +861,17 @@ kmg_status consolidate(kmg_ctx *c, bool recompact) {
     if (sieve) {
       prm.redo_list = d_redo; prm.redo_count = reinterpret_cast<uint32_t *>(d_sync + 3) + 1;
       prm.redo_len = d_redo + P; prm.redo_base = d_redo_base;
-      if (e == cudaSuccess) e = launch_count_partitions_sieve(prm, sieve_padded, c->stream);
+      if (e == cudaSuccess) e = launch_count_partitions_sieve(prm, c->stream);
       timer_end(c, tmr);
       if (e == cudaSuccess) e = cudaMemcpyAsync(h_sync, d_sync, 32, cudaMemcpyDeviceToHost, c->stream);
       if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
       const uint32_t n_redo = (uint32_t)(h_sync[3] >> 32);
       if (e == cudaSuccess && (n_redo > sieve_redo_limit_host(P) || (uint32_t)h_sync[3])) {
-        // duplicate-rich input (the reserved ranges of the partitions handed back are lost as fillers, the padded variant stops early):
+        // duplicate-rich input (the reserved ranges of the partitions handed back are lost as fillers, the sieve stops early):
         // the launch is repeated without the sieve
         if (dbg_sieve) fprintf(stderr, "[kmg] sieve: %u partitions, %u handed back, repeated without the sieve, %s\n", P, n_redo, in_place ? "leaves the in-place route" : "copied");
         pool_free(c, d_scratch); pool_free(c, d_sync);
-        sieve = sieve_padded = direct = false;
+        sieve = direct = false;
         c->dedup_ratio = std::min(c->dedup_ratio, 0.49);
         continue;
       }
@@ -1738,7 +1744,7 @@ KMG_EXPORT kmg_status kmg_adopt_coarse_device(kmg_ctx *c, const uint64_t *d_keys
   if (c->shm) return fail(c, KMG_ERR_STATE, "context belongs to a shard group: feed it with kmg_shard_count_ascii(_device)");
   if (c->mode != kmg_ctx::MODE_PARTITIONED) return fail(c, KMG_ERR_STATE, "call kmg_partition_plan first");
   if (n_bins != c->n_coarse) return fail(c, KMG_ERR_INVALID_ARG, "n_bins must equal the context's coarse partition count");
-  if (n >= (1ull << 32)) return fail(c, KMG_ERR_INVALID_ARG, "at most 2^32-1 keys per call");
+  if (n > REFINE_MAX_ENTRIES) return fail(c, KMG_ERR_INVALID_ARG, "at most 2^32 - 2^22 keys per call");
   std::vector<uint64_t> off(n_bins + 1, 0);
   for (uint32_t b = 0; b < n_bins; ++b) off[b + 1] = off[b] + bin_counts[b];
   if (off[n_bins] != n) return fail(c, KMG_ERR_INVALID_ARG, "bin_counts do not add up to n");
@@ -2022,7 +2028,7 @@ KMG_EXPORT kmg_status kmg_shard_join(kmg_ctx *c, uint32_t world, uint32_t rank, 
   const uint64_t G = (uint64_t)world * c->n_coarse;
   const uint64_t round_max = round_up(c->batch_bases, (uint64_t)TILE_WORDS * 32);  // rounds are padded to whole tiles
   const double mu = (double)round_max / (double)G;
-  c->sh_recv_entries = std::min<uint64_t>(round_max + G * (uint64_t)(7.0 * std::sqrt(mu) + 96.0), (1ull << 32) - 1);
+  c->sh_recv_entries = std::min<uint64_t>(round_max + G * (uint64_t)(7.0 * std::sqrt(mu) + 96.0), REFINE_MAX_ENTRIES);
   CU(c, cudaMalloc(&c->sh_recv, 2 * c->sh_recv_entries * 8));
   // ---- shared segment: rank 0 creates, the others attach
   const std::string name = std::string("/kmg-") + group;

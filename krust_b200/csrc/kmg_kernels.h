@@ -89,7 +89,7 @@ struct RefineParams {
 struct CountParams {
   uint32_t n_parts, R, scratch_log2, preagg;
   uint32_t split_log2;               // shared-memory kernel: partitions larger than a table are counted in up to 2^split_log2 passes
-  // padded sieve, in place (one raw run in a strided layout: partition p owns entries [p * part_cap, (p + 1) * part_cap)): the
+  // sieve in place (one raw run in a strided layout: partition p owns entries [p * part_cap, (p + 1) * part_cap)): the
   // output run IS the input run.  Its keys are never written -- a repeated key's further entries keep their key and get count 0 --
   // and the counts cover every partition's whole capacity (0 behind the segment).  0: the keys are copied to out_keys.
   uint32_t part_cap;
@@ -168,12 +168,14 @@ cudaError_t launch_count_partitions(const CountParams &P, unsigned grid, cudaStr
 cudaError_t launch_count_partitions_smem(const CountParams &P, bool weighted, bool direct, cudaStream_t s);
 // sieve: unweighted, mostly distinct keys -- a bitmap finds the few keys that MAY repeat, only those enter a (small) table; every
 // other key is copied to the output in place.  Partitions it cannot take are listed in P.redo_list for the variants above.
+// The input runs are raw runs, whose segments are 16-byte aligned and padded to an even length (launch_pad_segments): the copies go
+// through the TMA unit and the output segments are the padded inputs.  With P.part_cap set the sieve runs in place.
 constexpr uint32_t SIEVE_MAX_ENTRIES = 4096;  // entries of one partition the sieve variant takes (one batch)
-// padded: every input run has 16-byte aligned segments padded to an even length (launch_pad_segments) -- the copies then go
-// through the TMA unit and the output segments are the padded inputs.  With P.part_cap set the padded variant runs in place.
-cudaError_t launch_count_partitions_sieve(const CountParams &P, bool padded, cudaStream_t s);
-uint32_t sieve_redo_limit_host(uint32_t n_parts);  // more partitions handed back than this: the padded variant stopped early, repeat the launch without the sieve
+cudaError_t launch_count_partitions_sieve(const CountParams &P, cudaStream_t s);
+uint32_t sieve_redo_limit_host(uint32_t n_parts);  // more partitions handed back than this: the sieve stopped early, repeat the launch without it
+// keys[seg_start[p] + seg_len[p]] = EMPTY_MIX for every segment of odd length (the layout must leave room for it)
 cudaError_t launch_pad_segments(uint64_t *keys, const uint64_t *seg_start, const uint64_t *seg_len, uint32_t n_parts, cudaStream_t s);
+cudaError_t launch_even_lengths(const uint64_t *seg_len, uint64_t *even_len, uint32_t n_parts, cudaStream_t s);  // even_len[p] = seg_len[p] rounded up to even
 // tmp == nullptr: returns the scratch size needed for n items in *tmp_bytes.  Asynchronous on s.
 cudaError_t exclusive_sum_u64(const uint64_t *d_in, uint64_t *d_out, uint64_t n, void *tmp, size_t *tmp_bytes, cudaStream_t s);
 int num_sms();

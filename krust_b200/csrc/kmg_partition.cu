@@ -10,9 +10,10 @@
 //   A2  coarse bin -> P2 sub-bins each (P = P1*P2 fine)           (refine_rows4_kernel: big rows, tiles interleaved over the grid;
 //                                                                  refine_rows_kernel: few sub-bins, and keys pulled from other GPUs;
 //                                                                  refine_kernel<> = exact route)
-//   B   one CTA per fine partition: count, emit, histogram        (count_partitions_sieve(_tma)_kernel: bit-map sieve for mostly
-//                                                                  distinct keys; count_partitions_smem_kernel: table variant for
-//                                                                  weighted / repeat-rich runs; count_partitions_kernel = L2-scratch
+//   B   one CTA per fine partition: count, emit, histogram        (count_partitions_sieve_tma_kernel, and _in_place_kernel for one
+//                                                                  raw run in the speculative layout: bit-map sieve for raw runs of
+//                                                                  mostly distinct keys; count_partitions_smem_kernel: table variant
+//                                                                  for weighted / repeat-rich runs; count_partitions_kernel = L2-scratch
 //                                                                  fallback)
 //
 // The streams between the stages hold MIXED keys v = mix64(key) (kmg_device.cuh): coarse bin = top bits of v's high
@@ -1290,247 +1291,14 @@ __global__ void __launch_bounds__(SMEM_COUNT_THREADS, 2) count_partitions_smem_k
 }
 
 // ---------------------------------------------------------------------------------------------------
-// phase B, sieve variant (unweighted runs of mostly distinct keys: a genome).  The table variants above pay a compare-and-swap
-// protocol for EVERY key although almost every key of such a partition occurs once.  Here a key first sets its bit in a 2^18-bit
-// map (one shared atomic OR, no retry, no divergence): with ~3600 keys per partition only ~0.7 % of them find the bit already
-// set.  Those SUSPECTS -- real repeats and chance collisions alike -- are put into a small side table L.  After a barrier every
-// key looks itself up in L (one 8-byte shared load that almost always sees an empty slot):
-//   * not in L  -> the key occurs exactly once: it is copied to the output AT ITS INPUT POSITION with count 1 (coalesced);
-//   * in L      -> it bumps the entry's counter; the first to do so lends the entry its position, the others write a filler
-//                  entry (EMPTY, 0) that every reader skips.  L's entries are written out with their final counts at the end.
-// So the output segment has one entry per input entry and the count-of-counts falls out of L alone.  A partition with more
-// suspects than L holds, or more entries than one batch, is appended to P.redo_list and left to the compacting variant.
-// The next partition's segment table is fetched one partition ahead (registers -> the other half of a double buffer).
-// ---------------------------------------------------------------------------------------------------
-constexpr uint32_t SV_BM_LOG2 = 18;
-constexpr uint32_t SV_BM_WORDS = 1u << (SV_BM_LOG2 - 5);  // 32 KiB
-constexpr uint32_t SV_L_SLOTS = 4096;                     // 32 KiB of keys + 16 KiB of counters + 8 KiB of positions
-constexpr uint32_t SV_L_MAX = 2048;                       // entries L may hold (+ 4 KiB: the list of used slots)
-constexpr int SV_THREADS = 512, SV_G = 8;
-static_assert(SV_THREADS * SV_G == (int)SIEVE_MAX_ENTRIES, "one batch per partition");
-
-__device__ __noinline__ void sieve_insert(unsigned long long *Lkey, uint16_t *Lused, uint32_t *n_used, uint32_t *fail, unsigned long long k,
-                                          uint32_t slot_mask = SV_L_SLOTS - 1, uint32_t max_used = SV_L_MAX) {
-  if (*reinterpret_cast<volatile uint32_t *>(fail)) return;  // bounds the entries: every thread has at most one insertion past this test
-  uint32_t s = (uint32_t)(k >> 32) & slot_mask;
-  for (uint32_t t = 0; t <= slot_mask; ++t) {
-    unsigned long long cur = *reinterpret_cast<volatile unsigned long long *>(&Lkey[s]);
-    if (cur == EMPTY_MIX) cur = atomicCAS(&Lkey[s], EMPTY_MIX, k);
-    if (cur == k) return;
-    if (cur == EMPTY_MIX) {
-      const uint32_t i = atomicAdd(n_used, 1u);
-      if (i < max_used) Lused[i] = (uint16_t)s; else atomicExch(fail, 1u);
-      return;
-    }
-    s = (s + 1) & slot_mask;
-  }
-  atomicExch(fail, 1u);
-}
-// slot of k in L, or SV_L_SLOTS when it is not there (L is read-only by now)
-__device__ __noinline__ uint32_t sieve_find(const unsigned long long *Lkey, unsigned long long k, uint32_t slot_mask = SV_L_SLOTS - 1) {
-  uint32_t s = (uint32_t)(k >> 32) & slot_mask;
-  for (uint32_t t = 0; t <= slot_mask; ++t) {
-    const unsigned long long cur = Lkey[s];
-    if (cur == k) return s;
-    if (cur == EMPTY_MIX) break;
-    s = (s + 1) & slot_mask;
-  }
-  return SV_L_SLOTS;
-}
-
-template <bool ONE_RUN>  // every partition is one contiguous segment (the whole input went through one scatter round)
-__global__ void __launch_bounds__(SV_THREADS, 2) count_partitions_sieve_kernel(CountParams P) {
-  extern __shared__ __align__(16) unsigned long long sv_smem[];
-  unsigned long long *Lkey = sv_smem;
-  uint32_t *Lcnt = reinterpret_cast<uint32_t *>(Lkey + SV_L_SLOTS);
-  uint32_t *bm = Lcnt + SV_L_SLOTS;
-  uint16_t *Lpos = reinterpret_cast<uint16_t *>(bm + SV_BM_WORDS);
-  uint16_t *Lused = Lpos + SV_L_SLOTS;
-  __shared__ uint64_t seg_begin[2][CONS_MAX_RUNS];
-  __shared__ uint64_t seg_prefix[2][CONS_MAX_RUNS + 1];
-  __shared__ uint32_t s_work[2], s_hist[HIST_CTA_BINS];
-  __shared__ uint32_t s_nL, s_fail, s_holes;
-  __shared__ unsigned long long s_base;
-  constexpr int G = SV_G;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const uint32_t R = P.R;
-
-  // warp 0: segment table of work item w -> buffer `buf` (b / len already loaded by the lanes)
-  auto publish = [&](int buf, uint32_t w, uint64_t b, uint64_t len) {
-    uint64_t incl = len;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { const uint64_t v = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += v; }
-    if (lane < (int)R) { seg_begin[buf][lane] = b; seg_prefix[buf][lane] = incl - len; }
-    if (lane == (int)R - 1) seg_prefix[buf][R] = incl;
-    if (lane == 0) s_work[buf] = w;
-  };
-  auto fetch = [&](uint32_t w, uint64_t &b, uint64_t &len) {
-    b = 0; len = 0;
-    if (w < P.n_parts && lane < (int)R) {
-      const uint32_t p = P.order ? P.order[w] : w;
-      b = P.runs[lane].seg_start[p]; len = P.runs[lane].seg_len[p];
-    }
-  };
-
-  if (tid < HIST_CTA_BINS) s_hist[tid] = 0;
-  for (uint32_t i = tid; i < SV_L_SLOTS; i += SV_THREADS) { Lkey[i] = EMPTY_MIX; Lcnt[i] = 0; }
-  for (uint32_t i = tid; i < SV_BM_WORDS; i += SV_THREADS) bm[i] = 0;
-  if (tid == 0) { s_nL = 0; s_fail = 0; s_holes = 0; }
-  uint32_t w_next = 0;  // lane 0 of warp 0: the work item after the current one
-  if (warp == 0) {
-    uint32_t w0 = 0;
-    if (lane == 0) { w0 = atomicAdd(P.next, 1u); w_next = atomicAdd(P.next, 1u); }
-    w0 = __shfl_sync(0xffffffffu, w0, 0);
-    uint64_t b, len;
-    fetch(w0, b, len);
-    publish(0, w0, b, len);
-  }
-  __syncthreads();
-
-  unsigned long long my_entries = 0;  // tid 0: entries of the partitions this CTA counted
-  for (int cur = 0;; cur ^= 1) {
-    const uint32_t work = s_work[cur];
-    if (work >= P.n_parts) break;
-    // the next partition's segment table: loads issued now, published at the end of this iteration
-    uint32_t wn = 0;
-    uint64_t nb = 0, nlen = 0;
-    if (warp == 0) {
-      wn = __shfl_sync(0xffffffffu, w_next, 0);
-      fetch(wn, nb, nlen);
-      if (lane == 0 && wn < P.n_parts) w_next = atomicAdd(P.next, 1u);
-    }
-    const uint64_t *sb = seg_begin[cur], *sp = seg_prefix[cur];
-    const uint32_t p = P.order ? P.order[work] : work;
-    const uint64_t n_p = sp[R];
-    bool counted = false;
-    if (n_p == 0) {
-      if (tid == 0) { P.out_seg_start[p] = 0; P.out_seg_len[p] = 0; }
-    } else if (n_p > (uint64_t)SIEVE_MAX_ENTRIES) {  // block-uniform
-      if (tid == 0) { const uint32_t ri = atomicAdd(P.redo_count, 1u); P.redo_list[ri] = p; P.redo_base[ri] = NO_SPACE; P.redo_len[ri] = 0; }
-    } else {
-      // ---- load the partition (one batch: G keys per thread, entry idx = j * SV_THREADS + tid)
-      unsigned long long key[G];
-      uint32_t live = 0;
-      {
-        uint32_t r = 0;
-        uint64_t hi = sp[1];
-        const uint64_t *kq = P.runs[0].keys + sb[0];
-#pragma unroll
-        for (int j = 0; j < G; ++j) {
-          const uint32_t idx = (uint32_t)j * SV_THREADS + tid;
-          key[j] = EMPTY_MIX;
-          if (idx < n_p) {
-            if (!ONE_RUN) while (idx >= hi) { ++r; hi = sp[r + 1]; kq = P.runs[r].keys + sb[r] - sp[r]; }
-            key[j] = __ldcs(kq + idx);
-            live |= 1u << j;
-          }
-        }
-      }
-      // ---- pass 1: test-and-set in the bit map; suspects enter L
-      {
-        uint32_t old[G];
-#pragma unroll
-        for (int j = 0; j < G; ++j) {
-          const uint32_t lo = (uint32_t)key[j];
-          old[j] = 0;
-          if (live >> j & 1u) old[j] = atomicOr(&bm[(lo >> 5) & (SV_BM_WORDS - 1)], 1u << (lo & 31u));
-        }
-        uint32_t sus = 0;
-#pragma unroll
-        for (int j = 0; j < G; ++j) sus |= ((old[j] >> ((uint32_t)key[j] & 31u)) & 1u) << j;
-        if (sus) {
-#pragma unroll
-          for (int j = 0; j < G; ++j) if (sus >> j & 1u) sieve_insert(Lkey, Lused, &s_nL, &s_fail, key[j]);
-        }
-      }
-      __syncthreads();  // B: L is complete
-      const bool fail = s_fail != 0;
-      const uint32_t nL = s_nL;
-      {  // the bit map is not needed any more: clean it for the next partition
-        uint4 *bm4 = reinterpret_cast<uint4 *>(bm);
-#pragma unroll
-        for (uint32_t i = 0; i < SV_BM_WORDS / 4 / SV_THREADS; ++i) bm4[i * SV_THREADS + tid] = make_uint4(0u, 0u, 0u, 0u);
-      }
-      if (fail) {
-        for (uint32_t i = tid; i < SV_L_SLOTS; i += SV_THREADS) { Lkey[i] = EMPTY_MIX; Lcnt[i] = 0; }
-        __syncthreads();  // every thread has read s_fail / s_nL
-        if (tid == 0) { const uint32_t ri = atomicAdd(P.redo_count, 1u); P.redo_list[ri] = p; P.redo_base[ri] = NO_SPACE; P.redo_len[ri] = 0; s_nL = 0; s_fail = 0; }
-      } else {
-        counted = true;
-        if (tid == 0) {
-          unsigned long long ob = atomicAdd(P.out_cursor, (unsigned long long)n_p);
-          if (ob + n_p > P.out_cap) { atomicExch(P.nospace_flag, 1u); ob = NO_SPACE; }
-          s_base = ob;
-        }
-        // ---- pass 2: every key looks itself up in L
-        uint32_t rep = 0, hole = 0;
-        if (nL) {
-          uint32_t hit = 0;
-#pragma unroll
-          for (int j = 0; j < G; ++j) hit |= (Lkey[(uint32_t)(key[j] >> 32) & (SV_L_SLOTS - 1)] != EMPTY_MIX ? 1u : 0u) << j;
-          hit &= live;
-          if (hit) {
-#pragma unroll
-            for (int j = 0; j < G; ++j) {
-              if (!(hit >> j & 1u)) continue;
-              const uint32_t s = sieve_find(Lkey, key[j]);
-              if (s == SV_L_SLOTS) continue;
-              if (atomicAdd(&Lcnt[s], 1u) == 0u) { Lpos[s] = (uint16_t)((uint32_t)j * SV_THREADS + tid); rep |= 1u << j; }
-              else hole |= 1u << j;
-            }
-            if (hole) atomicAdd(&s_holes, (uint32_t)__popc(hole));
-          }
-        }
-        __syncthreads();  // C: s_base, L's counters and positions are final
-        const unsigned long long base = s_base;
-        const bool fits = base != NO_SPACE;
-        if (fits) {
-          uint64_t *ok = P.out_keys + base + tid, *oc = P.out_counts + base + tid;
-          if ((rep | hole) == 0u) {
-#pragma unroll
-            for (int j = 0; j < G; ++j)
-              if (live >> j & 1u) { __stcs(ok + j * SV_THREADS, (uint64_t)key[j]); __stcs(oc + j * SV_THREADS, (uint64_t)1); }
-          } else {
-#pragma unroll
-            for (int j = 0; j < G; ++j)
-              if ((live & ~rep) >> j & 1u) {
-                const bool h = hole >> j & 1u;
-                __stcs(ok + j * SV_THREADS, h ? (uint64_t)EMPTY_MIX : (uint64_t)key[j]);
-                __stcs(oc + j * SV_THREADS, h ? (uint64_t)0 : (uint64_t)1);
-              }
-          }
-        }
-        // L's entries go out with their counts (at the position their first claimant lent them), and L is cleaned
-        for (uint32_t i = tid; i < nL; i += SV_THREADS) {
-          const uint32_t s = Lused[i];
-          const unsigned long long cnt = Lcnt[s];
-          if (fits) { __stcs(P.out_keys + base + Lpos[s], (uint64_t)Lkey[s]); __stcs(P.out_counts + base + Lpos[s], (uint64_t)cnt); }
-          if (P.hist && cnt > 1) {
-            if (cnt < (unsigned long long)HIST_CTA_BINS) atomicAdd(&s_hist[cnt], 1u);
-            else if (cnt < (unsigned long long)HIST_DENSE_BINS) atomicAdd(P.hist + cnt, 1ull);
-            else { const unsigned long long o = atomicAdd(P.hist + HIST_DENSE_BINS, 1ull); if (o < P.hist_overflow_cap) P.hist_overflow[o] = cnt; }
-          }
-          Lkey[s] = EMPTY_MIX; Lcnt[s] = 0;
-        }
-        if (tid == 0) {
-          P.out_seg_start[p] = fits ? base : 0; P.out_seg_len[p] = n_p;
-          my_entries += n_p;
-          s_nL = 0;
-        }
-      }
-    }
-    (void)counted;
-    if (warp == 0) publish(cur ^ 1, wn, nb, nlen);
-    __syncthreads();  // A: next segment table published; L and the bit map are clean
-  }
-  if (tid == 0 && my_entries) atomicAdd(P.out_distinct, my_entries - (unsigned long long)s_holes);
-  if (P.hist) hist_flush(s_hist, P, tid);
-}
-
-// ---------------------------------------------------------------------------------------------------
-// The sieve with the key copies handed to the TMA unit (runs whose segments start on 16-byte boundaries and are padded to an even
-// number of entries with EMPTY_MIX: the speculative layouts, see launch_pad_segments).  ncu on the plain sieve: 3.9 warp-instr per key,
-// a third of them in the one-lane-active detours of the suspects, and half of all warp time at block barriers.  So here
+// phase B, sieve (unweighted runs of mostly distinct keys: a genome).  The table variants above pay a compare-and-swap protocol for
+// EVERY key although almost every key of such a partition occurs once.  Here a key first sets its bit in a 2^18-bit map (one shared
+// atomic OR, no retry): with ~3600 keys per partition only ~0.7 % of them find the bit already set.  Only those SUSPECTS and the keys
+// they met are resolved in a small table; every other key occurs once and stays at its input position with count 1.  The input runs
+// are raw runs, whose segments start on 16-byte boundaries and are padded to an even number of entries with EMPTY_MIX (refine_to_run,
+// launch_pad_segments), so the key copies are handed to the TMA unit.  A sieve that copied the keys with plain loads and stores and
+// resolved each suspect on the spot spent 3.9 warp-instr per key (ncu), a third of them in the one-lane-active detours of the
+// suspects, and half of all warp time at block barriers.  So here
 //   * the partition's keys arrive by 1-D bulk loads (one per input run) in one of two key stages, requested half a partition ahead,
 //     and leave by ONE bulk store of the stage (fillers and repeats are patched in the stage); counts go out as plain coalesced
 //     8-byte stores of 1 / 0 while the keys are read, and are patched afterwards where a key repeats;
@@ -1541,9 +1309,12 @@ __global__ void __launch_bounds__(SV_THREADS, 2) count_partitions_sieve_kernel(C
 //     (32-bit CAS; the key of a slot is read from the stage): first claimant = the entry that stays, the others become fillers;
 //   * two 512-thread CTAs per SM, so one CTA's barriers overlap the other's work; output ranges are reserved when the segment
 //     table is fetched (two partitions ahead), so no global atomic sits on the critical path.
-// The output segment is the padded input: entries (EMPTY, 0) are fillers every reader skips.  The in-place variant of this scheme
-// (count_partitions_sieve_in_place_kernel) follows it.
+// The output segment is the padded input: entries (EMPTY, 0) are fillers every reader skips.  A partition with more suspects than
+// the table holds, or more entries than one stage, is appended to P.redo_list and left to the compacting variant.  The in-place
+// variant of this scheme (count_partitions_sieve_in_place_kernel) follows it.
 // ---------------------------------------------------------------------------------------------------
+constexpr uint32_t SV_BM_LOG2 = 18;
+constexpr uint32_t SV_BM_WORDS = 1u << (SV_BM_LOG2 - 5);  // 32 KiB
 constexpr int SVT_THREADS = 512, SVT_G = 8, SVT_NS = 2, SVT_META = 3;
 __host__ __device__ __forceinline__ uint32_t sieve_redo_limit_impl(uint32_t n_parts) { return n_parts / 8 + 64; }
 __device__ __forceinline__ uint32_t sieve_redo_limit(uint32_t n_parts) { return sieve_redo_limit_impl(n_parts); }
@@ -2040,8 +1811,10 @@ __global__ void __launch_bounds__(SVI_THREADS, SVI_CTAS_PER_SM) count_partitions
   if (P.hist) hist_flush(s_hist, P, tid);
 }
 
-// behind every segment of odd length: one EMPTY_MIX entry, so that phase B may copy whole 16-byte units (the layout must have
-// room: the speculative layouts give every partition an even capacity)
+// Every raw run (refine_to_run) has its segments start on 16-byte boundaries and an EMPTY_MIX entry behind every segment of odd
+// length, so that phase B may copy whole 16-byte units.  The speculative layout has room for that entry because it gives every
+// partition an even capacity; the exact layout because its segment starts are the prefix of the lengths rounded up to even
+// (even_lengths_kernel).
 __global__ void pad_segments_kernel(uint64_t *keys, const uint64_t *__restrict__ seg_start, const uint64_t *__restrict__ seg_len, uint32_t n_parts) {
   for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < n_parts; p += gridDim.x * blockDim.x) {
     const uint64_t len = seg_len[p];
@@ -2054,35 +1827,34 @@ cudaError_t launch_pad_segments(uint64_t *keys, const uint64_t *seg_start, const
   pad_segments_kernel<<<(unsigned)std::min<uint64_t>((n_parts + 255) / 256, (uint64_t)num_sms() * 8), 256, 0, s>>>(keys, seg_start, seg_len, n_parts);
   return cudaGetLastError();
 }
+__global__ void even_lengths_kernel(const uint64_t *__restrict__ seg_len, uint64_t *even_len, uint32_t n_parts) {
+  for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < n_parts; p += gridDim.x * blockDim.x) even_len[p] = (seg_len[p] + 1) & ~1ull;
+}
+cudaError_t launch_even_lengths(const uint64_t *seg_len, uint64_t *even_len, uint32_t n_parts, cudaStream_t s) {
+  if (!n_parts) return cudaSuccess;
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  even_lengths_kernel<<<(unsigned)std::min<uint64_t>((n_parts + 255) / 256, (uint64_t)num_sms() * 8), 256, 0, s>>>(seg_len, even_len, n_parts);
+  return cudaGetLastError();
+}
 
 uint32_t sieve_redo_limit_host(uint32_t n_parts) { return sieve_redo_limit_impl(n_parts); }
-cudaError_t launch_count_partitions_sieve(const CountParams &P, bool padded, cudaStream_t s) {
+cudaError_t launch_count_partitions_sieve(const CountParams &P, cudaStream_t s) {
   if (P.n_parts == 0) return cudaSuccess;
   if (!P.redo_list || !P.redo_count || !P.redo_base || !P.redo_len) return cudaErrorInvalidValue;
-  if (padded) {
-    if (P.part_cap) {
-      if (P.R != 1) return cudaErrorInvalidValue;
-      cudaError_t e = cudaFuncSetAttribute(count_partitions_sieve_in_place_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SVI_SMEM);
-      if (e != cudaSuccess) return e;
-      g_launches.fetch_add(1, std::memory_order_relaxed);
-      count_partitions_sieve_in_place_kernel<<<(unsigned)std::min<uint64_t>(P.n_parts, (uint64_t)num_sms() * SVI_CTAS_PER_SM), SVI_THREADS,
-                                               SVI_SMEM, s>>>(P);
-      return cudaGetLastError();
-    }
-    auto kern = P.R == 1 ? count_partitions_sieve_tma_kernel<true> : count_partitions_sieve_tma_kernel<false>;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SVT_SMEM);
+  if (P.part_cap) {
+    if (P.R != 1) return cudaErrorInvalidValue;
+    cudaError_t e = cudaFuncSetAttribute(count_partitions_sieve_in_place_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SVI_SMEM);
     if (e != cudaSuccess) return e;
     g_launches.fetch_add(1, std::memory_order_relaxed);
-    kern<<<(unsigned)std::min<uint64_t>(P.n_parts, (uint64_t)num_sms() * 2), SVT_THREADS, SVT_SMEM, s>>>(P);
+    count_partitions_sieve_in_place_kernel<<<(unsigned)std::min<uint64_t>(P.n_parts, (uint64_t)num_sms() * SVI_CTAS_PER_SM), SVI_THREADS,
+                                             SVI_SMEM, s>>>(P);
     return cudaGetLastError();
   }
-  const size_t smem = (size_t)SV_L_SLOTS * (8 + 4 + 2) + (size_t)SV_BM_WORDS * 4 + (size_t)SV_L_MAX * 2;
-  const unsigned grid = (unsigned)std::min<uint64_t>(P.n_parts, (uint64_t)num_sms() * 2);
-  auto kern = P.R == 1 ? count_partitions_sieve_kernel<true> : count_partitions_sieve_kernel<false>;
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  auto kern = P.R == 1 ? count_partitions_sieve_tma_kernel<true> : count_partitions_sieve_tma_kernel<false>;
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SVT_SMEM);
   if (e != cudaSuccess) return e;
   g_launches.fetch_add(1, std::memory_order_relaxed);
-  kern<<<grid, SV_THREADS, smem, s>>>(P);
+  kern<<<(unsigned)std::min<uint64_t>(P.n_parts, (uint64_t)num_sms() * 2), SVT_THREADS, SVT_SMEM, s>>>(P);
   return cudaGetLastError();
 }
 

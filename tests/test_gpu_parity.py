@@ -493,11 +493,13 @@ def test_sharded_exchange_shapes_on_one_device(world):
             c.close()
 
 
-@pytest.mark.parametrize("shape", ["distinct", "repeats", "triple", "few_partitions", "small"])
+@pytest.mark.parametrize("shape", ["distinct", "repeats", "triple", "few_partitions", "small", "exact_layout", "exact_layout_one_run"])
 def test_phase_b_sieve_variants(shape):
-    """Phase B's sieve (bit map + small side table, keys copied in place; TMA-staged when the runs have padded segments) on
-    inputs it takes whole, inputs with a repeat fraction its side table still holds, and inputs it must hand to the compacting
-    variant (every key repeated; partitions larger than a batch) -- several runs per partition (three calls)."""
+    """Phase B's sieve (bit map + small side table, TMA-staged keys copied in place) on inputs it takes whole, inputs with a
+    repeat fraction its side table still holds, and inputs it must hand to the compacting variant (every key repeated; partitions
+    larger than a batch) -- several runs per partition (three calls).  "exact_layout": ~30 keys per partition and run, too few
+    for the speculative level-2 layout, so the sieve reads raw runs in the exact layout (three runs; "exact_layout_one_run": the
+    first call alone, one run, which is copied rather than counted in place)."""
     rng = np.random.default_rng(4242)
     k = 21
     n = 100_000 if shape == "small" else 2_000_000   # "small": the same kernels at a size compute-sanitizer's racecheck finishes (tools/sanitize.sh)
@@ -511,18 +513,22 @@ def test_phase_b_sieve_variants(shape):
     if shape == "triple":
         g[n:2 * n] = g[:n]
         g[2 * n:] = g[:n]
-    chunks = [g[i * n:(i + 1) * n] for i in range(3)]
+    n_calls = 1 if shape == "exact_layout_one_run" else 3
+    g = g[:n_calls * n]
+    chunks = [g[i * n:(i + 1) * n] for i in range(n_calls)]
     kw = dict(flags=PART, expected_distinct=3 * n)
     if shape == "few_partitions":
         kw = dict(flags=PART, parts_log2=6)   # 64 partitions of ~94 K entries: beyond a batch, beyond one table
+    if shape.startswith("exact_layout"):
+        kw = dict(flags=PART, parts_log2=16)
     with kb.GpuKmerCounter(k, **kw) as c:
         for ch in chunks:
             c.count_batch(ch, None, np.array([0, len(ch)], dtype=np.uint64))
         s = c.finalize()
         got = c.export(1, True)
         hv, hf = c.histogram(1)
-    ok, oc, _ = orc.count_batch(k, g, None, np.array([0, n, 2 * n, 3 * n], dtype=np.uint64))   # the three calls are three records
-    assert s["path"] == 2 and s["n_windows"] == 3 * (n - k + 1) and s["n_distinct"] == len(ok)
+    ok, oc, _ = orc.count_batch(k, g, None, np.arange(n_calls + 1, dtype=np.uint64) * n)   # the calls are records
+    assert s["path"] == 2 and s["n_windows"] == n_calls * (n - k + 1) and s["n_distinct"] == len(ok)
     assert_same(got, (ok, oc))
     ov, of = orc.histogram(oc, 1)
     assert (hv == ov).all() and (hf == of).all()
@@ -530,7 +536,7 @@ def test_phase_b_sieve_variants(shape):
 
 def test_c4_bin_geometry_on_100mbp():
     """The bin counts of the full C4 job (~1000 x 1000: rows of 16 slots, eight lanes per row in the copy-out of both scatter
-    levels, speculative layouts with padded segments, TMA-staged sieve) on an input the oracle counts in seconds: 100 Mbp with
+    levels, speculative layouts, sieve in place) on an input the oracle counts in seconds: 100 Mbp with
     2^20 partitions, the whole table and the histogram against the oracle; then a second, overlapping call (the first result
     re-enters phase B as a weighted run)."""
     import torch

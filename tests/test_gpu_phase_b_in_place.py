@@ -1,4 +1,4 @@
-"""Phase B in place: one raw run in the speculative layout is counted where it lies (count_partitions_sieve_tma_kernel<true, true>).
+"""Phase B in place: one raw run in the speculative layout is counted where it lies (count_partitions_sieve_in_place_kernel).
 The result keeps the run's key array; a repeated key's further entries keep their key with count 0, the slack behind every
 segment gets count 0.  Every case is compared against the oracle, and each runs in a subprocess with KMG_DEBUG_SIEVE set so
 that the route phase B took (in place, or left for the copying route) can be read from its stderr line."""
