@@ -167,6 +167,15 @@ impl GpuKmerCounter {
         self.check(unsafe { sys::kmg_shard_save_kmix(self.ctx, c.as_ptr(), &mut n) })?;
         Ok(n)
     }
+    /// ONE sorted tsv (`tsv == true`) or fasta file from all shards, the same bytes one GPU writes for the same input (every rank
+    /// writes its own byte ranges).  Returns the number of records of the whole file.
+    pub fn write_text_sharded<P: AsRef<Path>>(&mut self, path: P, tsv: bool, min_count: u64) -> Result<u64, GpuError> {
+        let c = CString::new(path.as_ref().to_string_lossy().as_bytes()).expect("path without NUL");
+        let format = if tsv { sys::KMG_TEXT_TSV } else { sys::KMG_TEXT_FASTA };
+        let (mut n, mut bytes) = (0u64, 0u64);
+        self.check(unsafe { sys::kmg_shard_write_text(self.ctx, min_count, format, c.as_ptr(), &mut n, &mut bytes) })?;
+        Ok(n)
+    }
 
     /// `save_index` straight from the device table (all k-mers, never min-count filtered).
     pub fn save_index<P: AsRef<Path>>(&mut self, path: P) -> Result<(), GpuError> {

@@ -179,7 +179,9 @@ kmg_status kmg_adopt_coarse_device(kmg_ctx *ctx, const uint64_t *d_keys, const u
  * partitions it further.  Only sizes, flags and results cross on the host, through a POSIX shared-memory segment named after
  * `group` (created by rank 0, unlinked once everybody is attached) -- no NCCL inside the library.  All kmg_shard_* calls are
  * COLLECTIVE: every rank makes the same sequence of them (a rank without input passes n_bytes / n_records = 0); a rank that
- * fails marks the group aborted, so its peers return KMG_ERR_STATE instead of waiting.  world == 1 degenerates to the plain
+ * fails marks the group aborted, so its peers return KMG_ERR_STATE instead of waiting.  Results of the whole group: summary,
+ * histogram, one .kmix and one sorted text file (kmg_shard_write_text: the key space cut into pieces, each merged by one owner
+ * straight out of its peers' staging buffers).  world == 1 degenerates to the plain
  * single-GPU calls.  Local feeds (kmg_count_ascii, kmg_insert_keys_device ...) are refused on a grouped context.
  *   kmg_shard_join: before the first feed; identical k / batch_bases / expected_keys_total (keys of the WHOLE job; 0 = the
  *   config's expected_distinct) on every rank.  One round moves at most batch_bases bases per rank.
@@ -196,6 +198,13 @@ kmg_status kmg_shard_finalize(kmg_ctx *ctx, kmg_summary *summary);
 kmg_status kmg_shard_histogram(kmg_ctx *ctx, uint64_t min_count, uint64_t *count_vals, uint64_t *freqs, uint64_t cap, uint64_t *n_out);
 /* ONE .kmix from all shards: rank 0 writes header and combined CRC, every rank its own records (src/index.rs:222-279). */
 kmg_status kmg_shard_save_kmix(kmg_ctx *ctx, const char *path, uint64_t *n_records_out);
+/* ONE file holding the records of ALL shards with count >= min_count (0 behaves as 1) in ascending k-mer order, formatted as
+ * KMG_TEXT_FASTA / KMG_TEXT_TSV: byte-identical to what kmg_write_text writes for a single context that counted the same input.
+ * COLLECTIVE, same arguments on every rank; every rank writes its own byte ranges of the file.  *n_records_out / *n_bytes_out:
+ * totals of the whole file, on every rank.  On a context outside a group it is kmg_write_text.  Inside a group "-" (stdout) is
+ * refused with KMG_ERR_INVALID_ARG on every rank; ranks that disagree on min_count / format abort the group. */
+kmg_status kmg_shard_write_text(kmg_ctx *ctx, uint64_t min_count, int format, const char *path,
+                                uint64_t *n_records_out, uint64_t *n_bytes_out);
 /* Diagnostics: keys written to other ranks, keys received, rounds, rounds that took the exact (count + prefix) route. */
 kmg_status kmg_shard_stats(const kmg_ctx *ctx, uint64_t *sent_keys, uint64_t *recv_keys, uint64_t *rounds, uint64_t *exact_rounds);
 

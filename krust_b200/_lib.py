@@ -62,6 +62,7 @@ SIGNATURES = {
     "kmg_shard_finalize": (i32, [vp, C.POINTER(KmgSummary)]),
     "kmg_shard_histogram": (i32, [vp, u64, vp, vp, u64, C.POINTER(u64)]),
     "kmg_shard_save_kmix": (i32, [vp, C.c_char_p, C.POINTER(u64)]),
+    "kmg_shard_write_text": (i32, [vp, u64, i32, C.c_char_p, C.POINTER(u64), C.POINTER(u64)]),
     "kmg_shard_stats": (i32, [vp, C.POINTER(u64), C.POINTER(u64), C.POINTER(u64), C.POINTER(u64)]),
     "kmg_finalize": (i32, [vp, C.POINTER(KmgSummary)]),
     "kmg_export_counts": (i32, [vp, u64, i32, vp, vp, u64, C.POINTER(u64)]),

@@ -329,6 +329,14 @@ class GpuKmerCounter:
         _check(self._L.kmg_shard_save_kmix(self._ctx, os.fspath(path).encode(), C.byref(n)), self._ctx)
         return n.value
 
+    def shard_write_text(self, path, fmt: str = "tsv", min_count: int = 1) -> Tuple[int, int]:
+        """kmg_shard_write_text (collective): ONE sorted fasta / tsv file from all shards of the group, the same bytes as write_text
+        on a single context.  Returns (records, bytes) of the whole file."""
+        code = {"fasta": _lib.KMG_TEXT_FASTA, "tsv": _lib.KMG_TEXT_TSV}[fmt]
+        n_rec, n_bytes = C.c_uint64(0), C.c_uint64(0)
+        _check(self._L.kmg_shard_write_text(self._ctx, min_count, code, os.fspath(path).encode(), C.byref(n_rec), C.byref(n_bytes)), self._ctx)
+        return n_rec.value, n_bytes.value
+
     def shard_stats(self) -> dict:
         a, b, r, x = C.c_uint64(0), C.c_uint64(0), C.c_uint64(0), C.c_uint64(0)
         _check(self._L.kmg_shard_stats(self._ctx, C.byref(a), C.byref(b), C.byref(r), C.byref(x)), self._ctx)

@@ -1823,13 +1823,23 @@ constexpr uint32_t SHARD_HIST_MAX = 2 * 65536;   // (value, frequency) pairs a r
 constexpr uint32_t SHARD_MAGIC = 0x4b4d4753u;
 constexpr double SHARD_TIMEOUT_S = 120.0;
 
+struct PeerBuf {  // a rank's device buffer as its peers open it: raw pointer (threads of one process) or CUDA IPC handle
+  cudaIpcMemHandle_t handle;
+  uint64_t raw_ptr;
+};
 struct ShardRankSlot {
   int32_t pid, device;
-  cudaIpcMemHandle_t handle;
-  uint64_t raw_ptr, recv_entries;
+  PeerBuf send;
+  uint64_t recv_entries;
   uint64_t round_bytes, round_flag;
   uint64_t summary[8];
   uint64_t hist_n;
+  // kmg_shard_write_text: arguments, records of this shard that pass min_count, its staging buffer, where each piece of the current
+  // step starts in its sorted step array, the piece it owns this step (records expected, records merged in order, bytes), bytes written
+  uint64_t text_args[2], text_total;
+  PeerBuf text;
+  uint64_t text_bounds[SHARD_MAX_WORLD + 1];
+  uint64_t text_piece[3], text_written;
 };
 struct ShardShm {
   uint32_t ready, world;
@@ -1870,11 +1880,50 @@ kmg_status shard_barrier(kmg_ctx *c) {
 #define SB(c) do { kmg_status _s = shard_barrier(c); if (_s != KMG_OK) return _s; } while (0)
 #define SCU(c, call) do { cudaError_t _e = (call); if (_e != cudaSuccess) { cuda_fail(c, _e, #call); return shard_fail(c, _e == cudaErrorMemoryAllocation ? KMG_ERR_OOM : KMG_ERR_CUDA, c->err); } } while (0)
 
-void shard_release(kmg_ctx *c) {
-  for (uint32_t r = 0; r < SHARD_MAX_WORLD; ++r) {
-    if (c->sh_peer[r] && c->sh_peer_ipc[r]) cudaIpcCloseMemHandle(c->sh_peer[r]);
-    c->sh_peer[r] = nullptr; c->sh_peer_ipc[r] = false;
+// A device buffer every rank can read: each rank publishes its own in its slot, and after a barrier opens all of them.
+void publish_peer_buffer(PeerBuf &slot, void *mine) {
+  slot.raw_ptr = (uint64_t)(uintptr_t)mine;
+  cudaError_t e = cudaIpcGetMemHandle(&slot.handle, mine);
+  if (e != cudaSuccess) { cudaGetLastError(); memset(&slot.handle, 0, sizeof slot.handle); }  // same-process groups do not need it
+}
+// peers[r] = rank r's buffer as seen from here: threads of one process use plain pointers (+ peer access between different devices),
+// other processes a CUDA IPC mapping (ipc[r]).  Returns why a buffer could not be opened, or "".
+std::string open_peer_buffers(kmg_ctx *c, PeerBuf ShardRankSlot::*which, uint64_t **peers, bool *ipc) {
+  const ShardShm *S = c->shm;
+  const ShardRankSlot &mine = S->ranks[c->sh_rank];
+  for (uint32_t r = 0; r < c->sh_world; ++r) {
+    const ShardRankSlot &o = S->ranks[r];
+    const PeerBuf &b = o.*which;
+    if (r == c->sh_rank) {
+      peers[r] = reinterpret_cast<uint64_t *>((uintptr_t)b.raw_ptr);
+    } else if (o.pid == mine.pid) {
+      if (o.device != c->device) {
+        int can = 0;
+        cudaDeviceCanAccessPeer(&can, c->device, o.device);
+        if (!can) return "no peer access between devices " + std::to_string(c->device) + " and " + std::to_string(o.device);
+        cudaError_t pe = cudaDeviceEnablePeerAccess(o.device, 0);
+        cudaGetLastError();
+        if (pe != cudaSuccess && pe != cudaErrorPeerAccessAlreadyEnabled) return std::string("cudaDeviceEnablePeerAccess: ") + cudaGetErrorString(pe);
+      }
+      peers[r] = reinterpret_cast<uint64_t *>((uintptr_t)b.raw_ptr);
+    } else {
+      void *pp = nullptr;
+      cudaError_t pe = cudaIpcOpenMemHandle(&pp, b.handle, cudaIpcMemLazyEnablePeerAccess);
+      if (pe != cudaSuccess) { cudaGetLastError(); return std::string("cudaIpcOpenMemHandle(rank ") + std::to_string(r) + "): " + cudaGetErrorString(pe); }
+      peers[r] = static_cast<uint64_t *>(pp); ipc[r] = true;
+    }
   }
+  return "";
+}
+void close_peer_buffers(uint64_t **peers, bool *ipc) {
+  for (uint32_t r = 0; r < SHARD_MAX_WORLD; ++r) {
+    if (peers[r] && ipc[r]) cudaIpcCloseMemHandle(peers[r]);
+    peers[r] = nullptr; ipc[r] = false;
+  }
+}
+
+void shard_release(kmg_ctx *c) {
+  close_peer_buffers(c->sh_peer, c->sh_peer_ipc);
   if (c->sh_recv) { cudaFree(c->sh_recv); c->sh_recv = nullptr; }
   if (c->shm) { munmap(c->shm, sizeof(ShardShm)); c->shm = nullptr; }
   c->sh_world = 1; c->sh_rank = 0;
@@ -2067,36 +2116,18 @@ KMG_EXPORT kmg_status kmg_shard_join(kmg_ctx *c, uint32_t world, uint32_t rank, 
   }
   ShardRankSlot &mine = S->ranks[rank];
   mine.pid = (int32_t)getpid(); mine.device = c->device;
-  mine.raw_ptr = (uint64_t)(uintptr_t)c->sh_recv; mine.recv_entries = c->sh_recv_entries;
+  mine.recv_entries = c->sh_recv_entries;
   mine.summary[0] = c->n_coarse; mine.summary[1] = c->n_sub; mine.summary[2] = (uint64_t)c->k;
-  cudaError_t e = cudaIpcGetMemHandle(&mine.handle, c->sh_recv);
-  if (e != cudaSuccess) { cudaGetLastError(); memset(&mine.handle, 0, sizeof mine.handle); }  // same-process groups do not need it
+  publish_peer_buffer(mine.send, c->sh_recv);
   kmg_status st = shard_barrier(c);
   if (st != KMG_OK) { shard_release(c); return st; }
   std::string why;
   for (uint32_t r = 0; r < world && why.empty(); ++r) {
     const ShardRankSlot &o = S->ranks[r];
-    if (o.summary[0] != c->n_coarse || o.summary[1] != c->n_sub || o.summary[2] != (uint64_t)c->k || o.recv_entries != c->sh_recv_entries) {
+    if (o.summary[0] != c->n_coarse || o.summary[1] != c->n_sub || o.summary[2] != (uint64_t)c->k || o.recv_entries != c->sh_recv_entries)
       why = "ranks disagree on k / the partition plan / batch_bases (pass identical arguments on every rank)";
-    } else if (r == rank) {
-      c->sh_peer[r] = c->sh_recv;
-    } else if (o.pid == mine.pid) {  // threads of one process: plain pointers (+ peer access between different devices)
-      if (o.device != c->device) {
-        int can = 0;
-        cudaDeviceCanAccessPeer(&can, c->device, o.device);
-        if (!can) { why = "no peer access between devices " + std::to_string(c->device) + " and " + std::to_string(o.device); break; }
-        cudaError_t pe = cudaDeviceEnablePeerAccess(o.device, 0);
-        if (pe != cudaSuccess && pe != cudaErrorPeerAccessAlreadyEnabled) why = std::string("cudaDeviceEnablePeerAccess: ") + cudaGetErrorString(pe);
-        cudaGetLastError();
-      }
-      c->sh_peer[r] = reinterpret_cast<uint64_t *>((uintptr_t)o.raw_ptr);
-    } else {
-      void *pp = nullptr;
-      cudaError_t pe = cudaIpcOpenMemHandle(&pp, o.handle, cudaIpcMemLazyEnablePeerAccess);
-      if (pe != cudaSuccess) { cudaGetLastError(); why = std::string("cudaIpcOpenMemHandle(rank ") + std::to_string(r) + "): " + cudaGetErrorString(pe); }
-      else { c->sh_peer[r] = static_cast<uint64_t *>(pp); c->sh_peer_ipc[r] = true; }
-    }
   }
+  if (why.empty()) why = open_peer_buffers(c, &ShardRankSlot::send, c->sh_peer, c->sh_peer_ipc);
   if (!why.empty()) __atomic_store_n(&S->abort, 1u, __ATOMIC_RELEASE);
   st = shard_barrier(c);  // every rank has opened its peers (or the group is aborted)
   if (rank == 0) shm_unlink(name.c_str());  // the mapping lives on; no name is left behind
@@ -2480,48 +2511,89 @@ uint32_t crc32_parallel(const uint8_t *p, size_t n) {
   return crc;
 }
 
-// Walk the table in ascending key order WITHOUT a second copy of it: the key space is cut into ranges of at most ~piece_target
-// entries (from a histogram over the top key bits); each range is compacted (count >= min_count), sorted, and handed to
-// fn(d_keys, d_counts, m).  The pieces concatenate to the sorted result.
+// The sorted walkers below cut the key space on the boundaries of KEY_BUCKETS buckets over the top bits of the 2k-bit keys.
+int key_bucket_shift(const kmg_ctx *c) { return 2 * c->k > 12 ? 2 * c->k - 12 : 0; }
+
+// hb[b] = entries of the table (any count) in key bucket b
+kmg_status key_histogram(kmg_ctx *c, uint64_t *hb) {
+  unsigned long long *d_b = nullptr;
+  CU(c, pool_alloc(c, &d_b, KEY_BUCKETS * 8));
+  cudaError_t e = launch_key_buckets(view_of(c), key_bucket_shift(c), d_b, c->stream);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(hb, d_b, KEY_BUCKETS * 8, cudaMemcpyDeviceToHost, c->stream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+  pool_free(c, d_b);
+  if (e != cudaSuccess) return cuda_fail(c, e, "key histogram");
+  return KMG_OK;
+}
+
+// Cuts of the bucket range into pieces of at most max(~piece_target, largest bucket) entries: piece i is buckets [cuts[i], cuts[i+1]).
+// Empty buckets at the end belong to no piece; an empty histogram gives no piece.
+std::vector<int> piece_cuts(const uint64_t *hb, uint64_t piece_target) {
+  uint64_t n_all = 0, piece_cap = 0;
+  for (int b = 0; b < KEY_BUCKETS; ++b) { n_all += hb[b]; piece_cap = std::max<uint64_t>(piece_cap, hb[b]); }
+  piece_cap = std::max<uint64_t>(piece_cap, std::min<uint64_t>(n_all, piece_target));
+  std::vector<int> cuts{0};
+  for (int b0 = 0; b0 < KEY_BUCKETS;) {
+    uint64_t ub = hb[b0];
+    int b1 = b0 + 1;
+    while (b1 < KEY_BUCKETS && ub + hb[b1] <= piece_cap) ub += hb[b1++];
+    if (ub) cuts.push_back(b1);
+    b0 = b1;
+  }
+  return cuts;
+}
+
+// Entries of the largest piece of `cuts` (its sorted part fits a buffer of that size)
+uint64_t largest_piece(const uint64_t *hb, const std::vector<int> &cuts) {
+  uint64_t m = 0;
+  for (size_t i = 0; i + 1 < cuts.size(); ++i) {
+    uint64_t n = 0;
+    for (int b = cuts[i]; b < cuts[i + 1]; ++b) n += hb[b];
+    m = std::max(m, n);
+  }
+  return m;
+}
+
+// Walk the table in ascending key order WITHOUT a second copy of it: each piece of `cuts` is compacted (count >= min_count) into
+// dk / dc (room for cap entries), sorted, and handed to fn(dk, dc, m), empty pieces too.  The pieces concatenate to the sorted result.
+template <class F>
+kmg_status for_each_sorted_piece(kmg_ctx *c, uint64_t min_count, const std::vector<int> &cuts, uint64_t *dk, uint64_t *dc, uint64_t cap,
+                                 F &&fn) {
+  const int shift = key_bucket_shift(c);
+  kmg_status s = KMG_OK;
+  for (size_t i = 0; s == KMG_OK && i + 1 < cuts.size(); ++i) {
+    TableView v = view_of(c);
+    v.range_lo = (uint64_t)cuts[i] << shift;
+    v.range_hi = cuts[i + 1] == KEY_BUCKETS ? ~0ull : ((uint64_t)cuts[i + 1] << shift) - 1;
+    unsigned long long m = 0;
+    cudaError_t e = launch_compact(v, min_count, dk, dc, cap, c->d_stats + 3, c->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&m, c->d_stats + 3, 8, cudaMemcpyDeviceToHost, c->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+    if (e == cudaSuccess && m > cap) return fail(c, KMG_ERR_STATE, "sorted piece larger than its key histogram");
+    if (e == cudaSuccess && m) e = sort_pairs(dk, dc, m, 2 * c->k, c->stream);
+    if (e != cudaSuccess) return cuda_fail(c, e, "sorted piece");
+    s = fn(dk, dc, (uint64_t)m);
+  }
+  return s;
+}
+
+// The whole table of one context, in pieces of about piece_target entries.
 template <class F>
 kmg_status for_each_sorted_piece(kmg_ctx *c, uint64_t min_count, uint64_t piece_target, F &&fn) {
   uint64_t n_all = 0;
   kmg_status s = count_filtered(c, 0, &n_all);
   if (s != KMG_OK || n_all == 0) return s;
-  const int shift = 2 * c->k > 12 ? 2 * c->k - 12 : 0;
-  unsigned long long *d_b = nullptr;
-  CU(c, pool_alloc(c, &d_b, KEY_BUCKETS * 8));
-  std::vector<unsigned long long> hb(KEY_BUCKETS);
-  cudaError_t e = launch_key_buckets(view_of(c), shift, d_b, c->stream);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(hb.data(), d_b, KEY_BUCKETS * 8, cudaMemcpyDeviceToHost, c->stream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-  pool_free(c, d_b);
-  if (e != cudaSuccess) return cuda_fail(c, e, "key histogram");
-  uint64_t piece_cap = std::min<uint64_t>(n_all, piece_target);
-  for (auto v : hb) piece_cap = std::max<uint64_t>(piece_cap, v);
+  std::vector<uint64_t> hb(KEY_BUCKETS);
+  if ((s = key_histogram(c, hb.data())) != KMG_OK) return s;
+  const std::vector<int> cuts = piece_cuts(hb.data(), piece_target);
+  const uint64_t cap = largest_piece(hb.data(), cuts);
   uint64_t *dk = nullptr, *dc = nullptr;
-  CU(c, pool_alloc(c, &dk, piece_cap * 8));
-  e = pool_alloc(c, &dc, piece_cap * 8);
+  CU(c, pool_alloc(c, &dk, cap * 8));
+  cudaError_t e = pool_alloc(c, &dc, cap * 8);
   if (e != cudaSuccess) { pool_free(c, dk); return cuda_fail(c, e, "cudaMalloc(sorted piece)"); }
-  for (int b0 = 0; s == KMG_OK && b0 < KEY_BUCKETS;) {
-    uint64_t ub = hb[b0];
-    int b1 = b0 + 1;
-    while (b1 < KEY_BUCKETS && ub + hb[b1] <= piece_cap) ub += hb[b1++];
-    if (ub) {
-      TableView v = view_of(c);
-      v.range_lo = (uint64_t)b0 << shift;
-      v.range_hi = b1 == KEY_BUCKETS ? ~0ull : ((uint64_t)b1 << shift) - 1;
-      unsigned long long m = 0;
-      e = launch_compact(v, min_count, dk, dc, piece_cap, c->d_stats + 3, c->stream);
-      if (e == cudaSuccess) e = cudaMemcpyAsync(&m, c->d_stats + 3, 8, cudaMemcpyDeviceToHost, c->stream);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-      if (e == cudaSuccess && m > piece_cap) { s = fail(c, KMG_ERR_STATE, "sorted piece larger than its key histogram"); break; }
-      if (e == cudaSuccess && m) e = sort_pairs(dk, dc, m, 2 * c->k, c->stream);
-      if (e != cudaSuccess) { s = cuda_fail(c, e, "sorted piece"); break; }
-      if (m) s = fn(dk, dc, (uint64_t)m);
-    }
-    b0 = b1;
-  }
+  s = for_each_sorted_piece(c, min_count, cuts, dk, dc, cap, [&](const uint64_t *k, const uint64_t *n, uint64_t m) -> kmg_status {
+    return m ? fn(k, n, m) : KMG_OK;
+  });
   pool_free(c, dk); pool_free(c, dc);
   return s;
 }
@@ -2549,6 +2621,38 @@ struct HostStager {
       if (s != KMG_OK) { cudaStreamSynchronize(c->stream); return s; }
       slot ^= 1; len_prev = len_next;
     }
+    return KMG_OK;
+  }
+};
+
+// A sorted (key, count) piece -> its fasta / tsv text in d_text, formatted on the device (line lengths, their exclusive sum = line
+// offsets, then every line written at its offset).  The buffers grow as pieces need and are reused across pieces.
+struct TextFormatter {
+  kmg_ctx *c;
+  int fasta;
+  uint64_t *d_off = nullptr;
+  uint8_t *d_text = nullptr;
+  uint64_t off_cap = 0, text_cap = 0;
+  TextFormatter(kmg_ctx *c_, int fasta_) : c(c_), fasta(fasta_) {}
+  ~TextFormatter() { pool_free(c, d_off); pool_free(c, d_text); }
+  kmg_status format(const uint64_t *dk, const uint64_t *dc, uint64_t m, uint64_t *bytes_out) {
+    if (m + 1 > off_cap) { pool_free(c, d_off); d_off = nullptr; off_cap = std::max<uint64_t>(m + 1, 1ull << 20); CU(c, pool_alloc(c, &d_off, off_cap * 8)); }
+    CU(c, launch_text_len(dc, m, c->k, fasta, d_off, c->stream));
+    CU(c, cudaMemsetAsync(d_off + m, 0, 8, c->stream));
+    if (!c->d_scan_tmp || c->scan_tmp_items < m + 1) {
+      CU(c, cudaStreamSynchronize(c->stream));
+      cudaFree(c->d_scan_tmp); c->d_scan_tmp = nullptr;
+      CU(c, exclusive_sum_u64(nullptr, nullptr, m + 1, nullptr, &c->scan_tmp_bytes, c->stream));
+      CU(c, cudaMalloc(&c->d_scan_tmp, c->scan_tmp_bytes ? c->scan_tmp_bytes : 16));
+      c->scan_tmp_items = m + 1;
+    }
+    CU(c, exclusive_sum_u64(d_off, d_off, m + 1, c->d_scan_tmp, &c->scan_tmp_bytes, c->stream));  // entry m = bytes of the piece
+    uint64_t total = 0;
+    CU(c, cudaMemcpyAsync(&total, d_off + m, 8, cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaStreamSynchronize(c->stream));
+    if (total > text_cap) { pool_free(c, d_text); d_text = nullptr; text_cap = total + total / 8; CU(c, pool_alloc(c, &d_text, text_cap)); }
+    CU(c, launch_text_write(dk, dc, d_off, m, c->k, fasta, d_text, c->stream));
+    *bytes_out = total;
     return KMG_OK;
   }
 };
@@ -2790,32 +2894,16 @@ KMG_EXPORT kmg_status kmg_emit_text(kmg_ctx *c, uint64_t min_count, int format, 
   const int fasta = format == KMG_TEXT_FASTA;
   uint64_t records = 0, bytes = 0;
   HostStager stage(c, 64u << 20);
-  uint64_t *d_off = nullptr;
-  uint8_t *d_text = nullptr;
-  uint64_t off_cap = 0, text_cap = 0;
+  TextFormatter fmt(c, fasta);
   kmg_status s = for_each_sorted_piece(c, min_count, 1ull << 24, [&](const uint64_t *dk, const uint64_t *dc, uint64_t m) -> kmg_status {
-    if (m + 1 > off_cap) { pool_free(c, d_off); d_off = nullptr; off_cap = std::max<uint64_t>(m + 1, 1ull << 20); CU(c, pool_alloc(c, &d_off, off_cap * 8)); }
-    CU(c, launch_text_len(dc, m, c->k, fasta, d_off, c->stream));
-    CU(c, cudaMemsetAsync(d_off + m, 0, 8, c->stream));
-    if (!c->d_scan_tmp || c->scan_tmp_items < m + 1) {
-      CU(c, cudaStreamSynchronize(c->stream));
-      cudaFree(c->d_scan_tmp); c->d_scan_tmp = nullptr;
-      CU(c, exclusive_sum_u64(nullptr, nullptr, m + 1, nullptr, &c->scan_tmp_bytes, c->stream));
-      CU(c, cudaMalloc(&c->d_scan_tmp, c->scan_tmp_bytes ? c->scan_tmp_bytes : 16));
-      c->scan_tmp_items = m + 1;
-    }
-    CU(c, exclusive_sum_u64(d_off, d_off, m + 1, c->d_scan_tmp, &c->scan_tmp_bytes, c->stream));  // entry m = bytes of the piece
     uint64_t total = 0;
-    CU(c, cudaMemcpyAsync(&total, d_off + m, 8, cudaMemcpyDeviceToHost, c->stream));
-    CU(c, cudaStreamSynchronize(c->stream));
-    if (total > text_cap) { pool_free(c, d_text); d_text = nullptr; text_cap = total + total / 8; CU(c, pool_alloc(c, &d_text, text_cap)); }
-    CU(c, launch_text_write(dk, dc, d_off, m, c->k, fasta, d_text, c->stream));
+    kmg_status fs = fmt.format(dk, dc, m, &total);
+    if (fs != KMG_OK) return fs;
     records += m; bytes += total;
-    return stage.drain(d_text, total, [&](const uint8_t *p, size_t len) -> kmg_status {
+    return stage.drain(fmt.d_text, total, [&](const uint8_t *p, size_t len) -> kmg_status {
       return sink(user, p, len) == 0 ? KMG_OK : fail(c, KMG_ERR_IO, "the text sink reported an error");
     });
   });
-  pool_free(c, d_off); pool_free(c, d_text);
   if (n_records_out) *n_records_out = records;
   if (n_bytes_out) *n_bytes_out = bytes;
   return s;
@@ -2835,6 +2923,147 @@ KMG_EXPORT kmg_status kmg_write_text(kmg_ctx *c, uint64_t min_count, int format,
   const bool ok = to_stdout ? fflush(f) == 0 : fclose(f) == 0;
   if (s == KMG_OK && !ok) return fail(c, KMG_ERR_IO, std::string("short write to ") + path);
   return s;
+}
+
+// The same file from all shards of a group, byte for byte.  The shards split the keys by hash, so every key range is spread over
+// all ranks.  The key space is cut into pieces of ~2^24 records from the ranks' summed key histograms; W consecutive pieces make a
+// step.  In each step every rank compacts and sorts its part of the step's key range into a staging buffer its peers can read;
+// rank j then owns piece j of the step: it merges the piece's W sorted parts straight out of the peers' memory
+// (merge_shard_pieces_kernel), formats it on the device and writes it at its offset in the file (the bytes of all earlier pieces).
+KMG_EXPORT kmg_status kmg_shard_write_text(kmg_ctx *c, uint64_t min_count, int format, const char *path, uint64_t *n_records_out,
+                                           uint64_t *n_bytes_out) {
+  if (!c || !path) return KMG_ERR_INVALID_ARG;
+  if (!c->shm) return kmg_write_text(c, min_count, format, path, n_records_out, n_bytes_out);
+  // every rank sees the same path: all of them refuse here, before any barrier
+  if (strcmp(path, "-") == 0) return fail(c, KMG_ERR_INVALID_ARG, "a shard group writes its text to a file: ranks cannot write one stream at given offsets");
+  if (format != KMG_TEXT_FASTA && format != KMG_TEXT_TSV) return shard_fail(c, KMG_ERR_INVALID_ARG, "format must be KMG_TEXT_FASTA or KMG_TEXT_TSV");
+  if (min_count == 0) min_count = 1;
+  SCU(c, cudaSetDevice(c->device));
+  ShardShm *S = c->shm;
+  const uint32_t W = c->sh_world, me = c->sh_rank;
+  ShardRankSlot &mine = S->ranks[me];
+  // 1. arguments, records that pass min_count and key histogram of every shard; rank 0 creates / truncates the file
+  uint64_t n_mine = 0;
+  kmg_status s = count_filtered(c, min_count, &n_mine);
+  if (s == KMG_OK) s = key_histogram(c, S->hist[me]);
+  if (s != KMG_OK) return shard_fail(c, s, c->err);
+  mine.text_args[0] = min_count; mine.text_args[1] = (uint64_t)format; mine.text_total = n_mine;
+  if (me == 0) {
+    FILE *f = fopen(path, "wb");
+    if (!f || fclose(f) != 0) return shard_fail(c, KMG_ERR_IO, std::string("cannot create ") + path);
+  }
+  SB(c);
+  for (uint32_t r = 0; r < W; ++r)
+    if (S->ranks[r].text_args[0] != min_count || S->ranks[r].text_args[1] != (uint64_t)format)
+      return shard_fail(c, KMG_ERR_INVALID_ARG, "ranks disagree on min_count / format (pass identical arguments on every rank)");
+  // 2. the same pieces on every rank; staging buffers sized for the largest part of a step any rank holds, merge buffers for the
+  //    largest piece this rank owns
+  std::vector<uint64_t> sum(KEY_BUCKETS, 0);
+  for (uint32_t r = 0; r < W; ++r)
+    for (int b = 0; b < KEY_BUCKETS; ++b) sum[b] += S->hist[r][b];
+  const std::vector<int> cuts = piece_cuts(sum.data(), 1ull << 24);
+  const size_t n_pieces = cuts.size() - 1;
+  std::vector<int> step_cuts;
+  for (size_t p = 0; p < n_pieces; p += W) step_cuts.push_back(cuts[p]);
+  if (n_pieces) step_cuts.push_back(cuts[n_pieces]);
+  uint64_t stage_cap = 1, own_cap = 1;
+  for (uint32_t r = 0; r < W; ++r) stage_cap = std::max(stage_cap, largest_piece(S->hist[r], step_cuts));
+  for (size_t p = me; p < n_pieces; p += W) own_cap = std::max(own_cap, largest_piece(sum.data(), {cuts[p], cuts[p + 1]}));
+  const int shift = key_bucket_shift(c);
+  uint64_t *stage = nullptr, *dk = nullptr, *dc = nullptr, *d_aux = nullptr;
+  uint64_t *peer[SHARD_MAX_WORLD] = {};
+  bool peer_ipc[SHARD_MAX_WORLD] = {};
+  int fd = -1;
+  uint64_t records = 0, file_bytes = 0;
+  auto run = [&]() -> kmg_status {
+    SCU(c, cudaMalloc(&stage, 2 * stage_cap * 8));  // (key, count) SoA: keys [0, stage_cap), counts [stage_cap, 2 * stage_cap)
+    SCU(c, pool_alloc(c, &dk, own_cap * 8));
+    SCU(c, pool_alloc(c, &dc, own_cap * 8));
+    SCU(c, pool_alloc(c, &d_aux, (SHARD_MAX_WORLD + 2) * 8));  // piece bounds + the merge's placed-record counter
+    publish_peer_buffer(mine.text, stage);
+    SB(c);
+    const std::string why = open_peer_buffers(c, &ShardRankSlot::text, peer, peer_ipc);
+    if (!why.empty()) return shard_fail(c, KMG_ERR_CUDA, why);
+    if ((fd = open(path, O_WRONLY)) < 0) return shard_fail(c, KMG_ERR_IO, std::string("cannot open ") + path + " for writing");
+    HostStager staged(c, 64u << 20);
+    TextFormatter fmt(c, format == KMG_TEXT_FASTA);
+    uint64_t written = 0;
+    size_t step = 0;
+    kmg_status st = for_each_sorted_piece(c, min_count, step_cuts, stage, stage + stage_cap, stage_cap,
+                                          [&](const uint64_t *sk, const uint64_t *, uint64_t m) -> kmg_status {
+      // 3. this rank's part of the step is sorted in its staging buffer: where does each piece start in it
+      const size_t p0 = step++ * W;
+      const uint32_t n_own = (uint32_t)std::min<size_t>(W, n_pieces - p0);
+      uint64_t cut_keys[SHARD_MAX_WORLD + 1], bounds[SHARD_MAX_WORLD + 1];
+      for (uint32_t j = 0; j < n_own; ++j) cut_keys[j] = (uint64_t)cuts[p0 + j] << shift;
+      SCU(c, launch_piece_bounds(sk, m, cut_keys, n_own, d_aux, c->stream));
+      SCU(c, cudaMemcpyAsync(bounds, d_aux, n_own * 8, cudaMemcpyDeviceToHost, c->stream));
+      SCU(c, cudaStreamSynchronize(c->stream));
+      bounds[n_own] = m;
+      memcpy(mine.text_bounds, bounds, (n_own + 1) * 8);
+      SB(c);  // every rank's part of the step is in its staging buffer
+      // 4. the owner merges its piece out of all staging buffers and formats it
+      uint64_t expect = 0, bytes = 0;
+      unsigned long long placed = 0;
+      if (me < n_own) {
+        MergeRuns R{};
+        R.n_runs = W;
+        for (uint32_t q = 0; q < W; ++q) {
+          const uint64_t lo = S->ranks[q].text_bounds[me], hi = S->ranks[q].text_bounds[me + 1];
+          R.keys[q] = peer[q] + lo; R.counts[q] = peer[q] + stage_cap + lo; R.len[q] = hi - lo;
+          expect += hi - lo;
+        }
+        if (expect > own_cap) return shard_fail(c, KMG_ERR_STATE, "merged piece larger than its key histogram");
+        unsigned long long *d_placed = reinterpret_cast<unsigned long long *>(d_aux + SHARD_MAX_WORLD + 1);
+        SCU(c, launch_merge_shard_pieces(R, dk, dc, d_placed, c->stream));
+        SCU(c, cudaMemcpyAsync(&placed, d_placed, 8, cudaMemcpyDeviceToHost, c->stream));
+        kmg_status fs = fmt.format(dk, dc, expect, &bytes);  // ends in a stream synchronize
+        if (fs != KMG_OK) return shard_fail(c, fs, c->err);
+      }
+      mine.text_piece[0] = expect; mine.text_piece[1] = placed; mine.text_piece[2] = bytes;
+      SB(c);  // nobody reads a staging buffer of this step any more: the next step may overwrite them
+      // 5. file offset = bytes of all earlier pieces; every merged piece holds as many ordered records as its parts
+      uint64_t off = file_bytes;
+      for (uint32_t j = 0; j < n_own; ++j) {
+        const uint64_t *tp = S->ranks[j].text_piece;
+        if (tp[0] != tp[1]) return shard_fail(c, KMG_ERR_STATE, "piece " + std::to_string(p0 + j) + ": the merge placed " + std::to_string(tp[1]) + " records in order, its parts hold " + std::to_string(tp[0]));
+        if (j < me) off += tp[2];
+        file_bytes += tp[2]; records += tp[0];
+      }
+      return staged.drain(fmt.d_text, bytes, [&](const uint8_t *p, size_t len) -> kmg_status {
+        for (size_t done = 0; done < len;) {
+          const ssize_t w = pwrite(fd, p + done, len - done, (off_t)off);
+          if (w <= 0) return shard_fail(c, KMG_ERR_IO, std::string("short write to ") + path);
+          done += (size_t)w; off += (uint64_t)w; written += (uint64_t)w;
+        }
+        return KMG_OK;
+      });
+    });
+    if (st != KMG_OK) return shard_fail(c, st, c->err);
+    const int closed = close(fd);
+    fd = -1;
+    if (closed != 0) return shard_fail(c, KMG_ERR_IO, std::string("short write to ") + path);
+    mine.text_written = written;
+    SB(c);
+    // 6. the file holds every record of every shard that passes min_count, and every byte the owners formatted
+    uint64_t want_records = 0, total_written = 0;
+    for (uint32_t r = 0; r < W; ++r) { want_records += S->ranks[r].text_total; total_written += S->ranks[r].text_written; }
+    if (records != want_records) return shard_fail(c, KMG_ERR_STATE, "text file holds " + std::to_string(records) + " records, the shards " + std::to_string(want_records));
+    if (total_written != file_bytes) return shard_fail(c, KMG_ERR_STATE, "bytes written differ from the bytes of the formatted pieces");
+    close_peer_buffers(peer, peer_ipc);
+    SB(c);  // every peer has closed its mapping of this rank's staging buffer
+    return KMG_OK;
+  };
+  s = run();
+  close_peer_buffers(peer, peer_ipc);
+  if (fd >= 0) close(fd);
+  cudaStreamSynchronize(c->stream);
+  cudaFree(stage);
+  pool_free(c, dk); pool_free(c, dc); pool_free(c, d_aux);
+  if (s != KMG_OK) return s;
+  if (n_records_out) *n_records_out = records;
+  if (n_bytes_out) *n_bytes_out = file_bytes;
+  return KMG_OK;
 }
 
 

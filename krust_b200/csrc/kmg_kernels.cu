@@ -1176,6 +1176,101 @@ __global__ void interleave_pairs_kernel(const uint64_t *__restrict__ keys, const
     out[i] = make_ulonglong2(keys[i], counts[i]);
 }
 
+// ---- ONE sorted text file from a shard group (kmg_shard_write_text): every rank holds a sorted step of the key space in a staging
+// buffer its peers can read; the owner of a piece merges the piece's parts straight out of the peers' memory.
+__device__ __forceinline__ uint64_t lower_bound_u64(const uint64_t *a, uint64_t n, uint64_t key) {
+  uint64_t lo = 0, hi = n;
+  while (lo < hi) {
+    const uint64_t mid = (lo + hi) >> 1;
+    if (a[mid] < key) lo = mid + 1; else hi = mid;
+  }
+  return lo;
+}
+struct PieceCuts { uint64_t key[MERGE_MAX_RUNS + 1]; };
+__global__ void piece_bounds_kernel(const uint64_t *__restrict__ keys, uint64_t n, PieceCuts cuts, uint32_t n_cuts, uint64_t *__restrict__ out) {
+  const uint32_t i = threadIdx.x;
+  if (i < n_cuts) out[i] = lower_bound_u64(keys, n, cuts.key[i]);
+}
+
+constexpr int MERGE_THREADS = 256;
+constexpr int MERGE_TILE = 2048;  // output records per CTA: keys and counts staged in 32 KiB of shared memory
+constexpr int MERGE_PER_THREAD = MERGE_TILE / MERGE_THREADS;
+// The runs come from different shards, and a key lives on exactly one shard: no key appears in two runs.  So the record at index i
+// of run r has the global rank i + sum over q != r of lower_bound_q(key), every output position has exactly one split across the
+// runs, and no ties need breaking.  Each CTA writes the fixed output range [d0, d1): it finds where that range starts and ends in
+// every run (binary search over i of the rank above, one warp per (boundary, run), lane q searching run q), loads the sub-ranges
+// with coalesced (peer) loads into shared memory, and puts every record at its rank inside the tile.
+__global__ void __launch_bounds__(MERGE_THREADS) merge_shard_pieces_kernel(MergeRuns R, uint64_t total, uint64_t *__restrict__ keys_out,
+                                                                          uint64_t *__restrict__ counts_out, unsigned long long *placed) {
+  __shared__ uint64_t s_key[MERGE_TILE], s_cnt[MERGE_TILE];
+  __shared__ const uint64_t *s_rk[MERGE_MAX_RUNS], *s_rc[MERGE_MAX_RUNS];
+  __shared__ uint64_t s_len[MERGE_MAX_RUNS], s_lo[MERGE_MAX_RUNS], s_hi[MERGE_MAX_RUNS];
+  __shared__ uint32_t s_off[MERGE_MAX_RUNS + 1];
+  const uint32_t W = R.n_runs;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (threadIdx.x < W) { s_rk[threadIdx.x] = R.keys[threadIdx.x]; s_rc[threadIdx.x] = R.counts[threadIdx.x]; s_len[threadIdx.x] = R.len[threadIdx.x]; }
+  __syncthreads();
+  const uint64_t d0 = blockIdx.x * (uint64_t)MERGE_TILE, d1 = d0 + MERGE_TILE < total ? d0 + MERGE_TILE : total;
+  for (uint32_t job = warp; job < 2 * W; job += MERGE_THREADS / 32) {
+    const uint32_t r = job % W;
+    const uint64_t d = job < W ? d0 : d1;
+    uint64_t lo = 0, hi = s_len[r];
+    while (lo < hi) {  // warp-uniform: every lane sees the same mid and the same sum
+      const uint64_t mid = (lo + hi) >> 1;
+      const uint64_t key = s_rk[r][mid];
+      const uint64_t below = warp_sum(lane < (int)W && lane != (int)r ? lower_bound_u64(s_rk[lane], s_len[lane], key) : 0);
+      if (mid + below < d) lo = mid + 1; else hi = mid;
+    }
+    if (lane == 0) (job < W ? s_lo : s_hi)[r] = lo;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    uint32_t o = 0;
+    for (uint32_t r = 0; r < W; ++r) { s_off[r] = o; o += (uint32_t)(s_hi[r] - s_lo[r]); }
+    s_off[W] = o;  // == d1 - d0
+  }
+  __syncthreads();
+  const uint32_t n = s_off[W];
+  for (uint32_t t = threadIdx.x; t < n; t += MERGE_THREADS) {
+    uint32_t r = 0;
+    while (r + 1 < W && t >= s_off[r + 1]) ++r;
+    const uint64_t i = s_lo[r] + (t - s_off[r]);
+    s_key[t] = s_rk[r][i];
+    s_cnt[t] = s_rc[r][i];
+  }
+  __syncthreads();
+  uint64_t k_[MERGE_PER_THREAD], c_[MERGE_PER_THREAD];
+  uint32_t pos[MERGE_PER_THREAD];
+#pragma unroll
+  for (int j = 0; j < MERGE_PER_THREAD; ++j) {
+    const uint32_t t = threadIdx.x + j * MERGE_THREADS;
+    pos[j] = ~0u;
+    if (t < n) {
+      uint32_t r = 0;
+      while (r + 1 < W && t >= s_off[r + 1]) ++r;
+      const uint64_t key = s_key[t];
+      uint32_t p = t - s_off[r];
+      for (uint32_t q = 0; q < W; ++q)
+        if (q != r) p += (uint32_t)lower_bound_u64(s_key + s_off[q], s_off[q + 1] - s_off[q], key);
+      k_[j] = key; c_[j] = s_cnt[t]; pos[j] = p;
+    }
+  }
+  __syncthreads();
+#pragma unroll
+  for (int j = 0; j < MERGE_PER_THREAD; ++j)
+    if (pos[j] < n) { s_key[pos[j]] = k_[j]; s_cnt[pos[j]] = c_[j]; }
+  __syncthreads();
+  uint64_t asc = 0;
+  for (uint32_t t = threadIdx.x; t < n; t += MERGE_THREADS) {
+    const uint64_t key = s_key[t];
+    keys_out[d0 + t] = key;
+    counts_out[d0 + t] = s_cnt[t];
+    asc += t == 0 || s_key[t - 1] < key;
+  }
+  asc = warp_sum(asc);
+  if (lane == 0 && asc) atomicAdd(placed, (unsigned long long)asc);
+}
+
 // K6: count-of-counts.  Counts below HIST_DENSE_BINS go to dense bins (the first HIST_SMEM_BINS of them
 // privatised in shared memory); larger counts are appended to an overflow list (at most
 // total_windows / HIST_DENSE_BINS entries can ever land there).
@@ -1497,6 +1592,25 @@ cudaError_t launch_interleave_pairs(const uint64_t *d_keys, const uint64_t *d_co
   if (n == 0) return cudaSuccess;
   g_launches.fetch_add(1, std::memory_order_relaxed);
   interleave_pairs_kernel<<<grid_for(n, 256, 8), 256, 0, s>>>(d_keys, d_counts, n, static_cast<ulonglong2 *>(d_out));
+  return cudaGetLastError();
+}
+cudaError_t launch_piece_bounds(const uint64_t *d_keys, uint64_t n, const uint64_t *cut_keys, uint32_t n_cuts, uint64_t *d_out, cudaStream_t s) {
+  if (n_cuts == 0 || n_cuts > MERGE_MAX_RUNS + 1) return n_cuts ? cudaErrorInvalidValue : cudaSuccess;
+  PieceCuts cuts{};
+  for (uint32_t i = 0; i < n_cuts; ++i) cuts.key[i] = cut_keys[i];
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  piece_bounds_kernel<<<1, 32, 0, s>>>(d_keys, n, cuts, n_cuts, d_out);
+  return cudaGetLastError();
+}
+cudaError_t launch_merge_shard_pieces(const MergeRuns &R, uint64_t *d_keys_out, uint64_t *d_counts_out, unsigned long long *d_placed,
+                                      cudaStream_t s) {
+  if (R.n_runs == 0 || R.n_runs > MERGE_MAX_RUNS) return cudaErrorInvalidValue;
+  cudaError_t e = cudaMemsetAsync(d_placed, 0, sizeof(unsigned long long), s);
+  uint64_t total = 0;
+  for (uint32_t r = 0; r < R.n_runs; ++r) total += R.len[r];
+  if (e != cudaSuccess || total == 0) return e;
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  merge_shard_pieces_kernel<<<(unsigned)((total + MERGE_TILE - 1) / MERGE_TILE), MERGE_THREADS, 0, s>>>(R, total, d_keys_out, d_counts_out, d_placed);
   return cudaGetLastError();
 }
 cudaError_t launch_histogram(const TableView &v, uint64_t min_count, unsigned long long *d_bins, uint64_t *d_overflow,

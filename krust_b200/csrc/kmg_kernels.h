@@ -212,6 +212,21 @@ cudaError_t launch_text_len(const uint64_t *d_counts, uint64_t n, int k, int fas
 cudaError_t launch_text_write(const uint64_t *d_keys, const uint64_t *d_counts, const uint64_t *d_offs, uint64_t n, int k, int fasta, uint8_t *d_out,
                               cudaStream_t s);
 cudaError_t launch_interleave_pairs(const uint64_t *d_keys, const uint64_t *d_counts, uint64_t n, void *d_out, cudaStream_t s);
+// text file of a shard group: up to MERGE_MAX_RUNS sorted (key, count) runs, possibly in other GPUs' memory (P2P / IPC mapped),
+// merged into one sorted local run.  The runs' keys must be pairwise distinct (a key lives on one shard only).
+constexpr int MERGE_MAX_RUNS = 8;
+struct MergeRuns {
+  const uint64_t *keys[MERGE_MAX_RUNS];
+  const uint64_t *counts[MERGE_MAX_RUNS];
+  uint64_t len[MERGE_MAX_RUNS];
+  uint32_t n_runs;
+};
+// d_out[i] = lower_bound(d_keys[0, n), cut_keys[i]) for i < n_cuts (<= MERGE_MAX_RUNS + 1): where each piece of a step starts
+cudaError_t launch_piece_bounds(const uint64_t *d_keys, uint64_t n, const uint64_t *cut_keys, uint32_t n_cuts, uint64_t *d_out, cudaStream_t s);
+// out[0, sum of len) = the merged runs; *d_placed (zeroed here) += records written in ascending order (== the total unless two
+// runs shared a key)
+cudaError_t launch_merge_shard_pieces(const MergeRuns &R, uint64_t *d_keys_out, uint64_t *d_counts_out, unsigned long long *d_placed,
+                                      cudaStream_t s);
 uint64_t kernel_launches();  // number of kernels of this library launched so far (process-wide)
 cudaError_t sort_pairs(uint64_t *d_keys, uint64_t *d_counts, uint64_t n, int key_bits, cudaStream_t s);
 

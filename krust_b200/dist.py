@@ -330,6 +330,16 @@ class ShardedKmerCounter:
         dist.barrier(group=self.group)
         return {"records": int(sum(p[0] for p in parts))}
 
+    def write_text(self, path, fmt: str = "tsv", min_count: int = 1) -> Tuple[int, int]:
+        """ONE sorted fasta / tsv file from all shards, byte-identical to what one GPU writes for the same input (collective).
+        Returns (records, bytes) of the whole file on every rank."""
+        if self.world == 1:
+            return self.engine.counter.write_text(path, fmt, min_count)
+        if self.fused and self.engine.joined:
+            return self.engine.counter.shard_write_text(path, fmt, min_count)
+        raise RuntimeError("write_text needs the fused shard group (kmg_shard_*): the generic bucket + all-to-all path has no "
+                           "cross-shard text writer")
+
     def stats(self) -> dict:
         out = {"path": "fused exchange (owners' refine kernels pull their bins from all ranks' send buffers over NVLink)" if self.fused else "bucket + NCCL all_to_all_single + adopt",
                "sent_keys": int(self.sent_keys), "recv_keys": int(self.recv_keys)}
