@@ -113,13 +113,22 @@ impl GpuKmerCounter {
 
     /// `output_counts` for `--format tsv|fasta` (src/run.rs:452-470): sorted lines formatted on the device, streamed into `w`.
     pub fn write_text<W: std::io::Write>(&mut self, w: &mut W, tsv: bool, min_count: u64) -> Result<u64, GpuError> {
+        self.emit_text(w, if tsv { sys::KMG_TEXT_TSV } else { sys::KMG_TEXT_FASTA }, min_count)
+    }
+
+    /// `output_counts` for `--format json` (src/run.rs:471-481): the pretty-printed array of `{kmer, count}` objects plus a
+    /// newline, records in ascending k-mer order, formatted on the device and streamed into `w`.  Returns the records written.
+    pub fn write_json<W: std::io::Write>(&mut self, w: &mut W, min_count: u64) -> Result<u64, GpuError> {
+        self.emit_text(w, sys::KMG_TEXT_JSON, min_count)
+    }
+
+    fn emit_text<W: std::io::Write>(&mut self, w: &mut W, fmt: std::os::raw::c_int, min_count: u64) -> Result<u64, GpuError> {
         unsafe extern "C" fn sink<W: std::io::Write>(user: *mut std::os::raw::c_void, bytes: *const u8, n: usize) -> std::os::raw::c_int {
             let w = &mut *(user as *mut W);
             w.write_all(std::slice::from_raw_parts(bytes, n)).is_err() as std::os::raw::c_int
         }
         self.check(unsafe { sys::kmg_finalize(self.ctx, std::ptr::null_mut()) })?;
         let (mut recs, mut bytes) = (0u64, 0u64);
-        let fmt = if tsv { sys::KMG_TEXT_TSV } else { sys::KMG_TEXT_FASTA };
         self.check(unsafe { sys::kmg_emit_text(self.ctx, min_count, fmt, Some(sink::<W>), w as *mut W as *mut _, &mut recs, &mut bytes) })?;
         Ok(recs)
     }
@@ -170,8 +179,15 @@ impl GpuKmerCounter {
     /// ONE sorted tsv (`tsv == true`) or fasta file from all shards, the same bytes one GPU writes for the same input (every rank
     /// writes its own byte ranges).  Returns the number of records of the whole file.
     pub fn write_text_sharded<P: AsRef<Path>>(&mut self, path: P, tsv: bool, min_count: u64) -> Result<u64, GpuError> {
+        self.shard_write_text(path, if tsv { sys::KMG_TEXT_TSV } else { sys::KMG_TEXT_FASTA }, min_count)
+    }
+    /// ONE json file from all shards, the same bytes `write_json` of one GPU writes for the same input.  Returns the number of
+    /// records of the whole file.
+    pub fn write_json_sharded<P: AsRef<Path>>(&mut self, path: P, min_count: u64) -> Result<u64, GpuError> {
+        self.shard_write_text(path, sys::KMG_TEXT_JSON, min_count)
+    }
+    fn shard_write_text<P: AsRef<Path>>(&mut self, path: P, format: std::os::raw::c_int, min_count: u64) -> Result<u64, GpuError> {
         let c = CString::new(path.as_ref().to_string_lossy().as_bytes()).expect("path without NUL");
-        let format = if tsv { sys::KMG_TEXT_TSV } else { sys::KMG_TEXT_FASTA };
         let (mut n, mut bytes) = (0u64, 0u64);
         self.check(unsafe { sys::kmg_shard_write_text(self.ctx, min_count, format, c.as_ptr(), &mut n, &mut bytes) })?;
         Ok(n)

@@ -199,7 +199,8 @@ kmg_status kmg_shard_histogram(kmg_ctx *ctx, uint64_t min_count, uint64_t *count
 /* ONE .kmix from all shards: rank 0 writes header and combined CRC, every rank its own records (src/index.rs:222-279). */
 kmg_status kmg_shard_save_kmix(kmg_ctx *ctx, const char *path, uint64_t *n_records_out);
 /* ONE file holding the records of ALL shards with count >= min_count (0 behaves as 1) in ascending k-mer order, formatted as
- * KMG_TEXT_FASTA / KMG_TEXT_TSV: byte-identical to what kmg_write_text writes for a single context that counted the same input.
+ * KMG_TEXT_FASTA / KMG_TEXT_TSV / KMG_TEXT_JSON: byte-identical to what kmg_write_text writes for a single context that counted
+ * the same input.
  * COLLECTIVE, same arguments on every rank; every rank writes its own byte ranges of the file.  *n_records_out / *n_bytes_out:
  * totals of the whole file, on every rank.  On a context outside a group it is kmg_write_text.  Inside a group "-" (stdout) is
  * refused with KMG_ERR_INVALID_ARG on every rank; ranks that disagree on min_count / format abort the group. */
@@ -231,12 +232,14 @@ kmg_status kmg_export_shard_device(kmg_ctx *ctx, uint64_t min_count, int sorted,
 kmg_status kmg_histogram(kmg_ctx *ctx, uint64_t min_count, uint64_t *count_vals, uint64_t *freqs,
                          uint64_t cap, uint64_t *n_out);
 
-/* Replaces the fasta / tsv text emitters of output_counts and count_to_writer (src/run.rs:452-470, src/builder.rs:399-442) and
- * unpack_to_string (src/kmer.rs:431-456): entries with count >= min_count (0 behaves as 1) in ascending k-mer order -- the
+/* Replaces the fasta / tsv / json text emitters of output_counts and count_to_writer (src/run.rs:452-481, src/builder.rs:399-442)
+ * and unpack_to_string (src/kmer.rs:431-456): entries with count >= min_count (0 behaves as 1) in ascending k-mer order -- the
  * reference prints HashMap iteration order, parity is defined on the sorted text -- formatted on the device
- * (tsv "{kmer}\t{count}\n", fasta ">{count}\n{kmer}\n") and delivered to `sink` in chunks of at most 64 MiB; a non-zero
- * return from the sink aborts with KMG_ERR_IO.  kmg_write_text writes the same bytes to a file ("-" = stdout). */
-enum { KMG_TEXT_FASTA = 0, KMG_TEXT_TSV = 1 };
+ * (tsv "{kmer}\t{count}\n", fasta ">{count}\n{kmer}\n", json the serde_json::to_string_pretty array of {"kmer", "count"}
+ * objects plus "\n", "[]\n" when no entry passes) and delivered to `sink` in chunks of at most 64 MiB; a non-zero return from
+ * the sink aborts with KMG_ERR_IO.  *n_bytes_out counts every byte delivered, json's "[" and closing "]\n" included.
+ * kmg_write_text writes the same bytes to a file ("-" = stdout). */
+enum { KMG_TEXT_FASTA = 0, KMG_TEXT_TSV = 1, KMG_TEXT_JSON = 2 };
 typedef int (*kmg_text_sink)(void *user, const uint8_t *bytes, size_t n);
 kmg_status kmg_emit_text(kmg_ctx *ctx, uint64_t min_count, int format, kmg_text_sink sink, void *user, uint64_t *n_records_out,
                          uint64_t *n_bytes_out);

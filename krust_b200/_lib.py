@@ -12,7 +12,7 @@ KMG_ABI_VERSION = 1
 KMG_OK, KMG_ERR_INVALID_K, KMG_ERR_INVALID_ARG, KMG_ERR_CUDA, KMG_ERR_OOM, KMG_ERR_TABLE_FULL, KMG_ERR_STATE, \
     KMG_ERR_IO, KMG_ERR_ABI, KMG_ERR_CAPACITY, KMG_ERR_PARSE = range(11)
 KMG_FLAG_FORCE_HASH, KMG_FLAG_FORCE_DIRECT, KMG_FLAG_NO_PREAGG, KMG_FLAG_FORCE_PARTITIONED = 1, 2, 4, 8
-KMG_TEXT_FASTA, KMG_TEXT_TSV = 0, 1
+KMG_TEXT_FASTA, KMG_TEXT_TSV, KMG_TEXT_JSON = 0, 1, 2
 TEXT_SINK = C.CFUNCTYPE(C.c_int, C.c_void_p, C.POINTER(C.c_uint8), C.c_size_t)
 
 

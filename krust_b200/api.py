@@ -65,6 +65,10 @@ def _check(status: int, ctx=None):
     raise GpuError(status, msg)
 
 
+# output formats the device text emitters write (kmg_emit_text / kmg_write_text / kmg_shard_write_text)
+_TEXT_FORMATS = {"fasta": _lib.KMG_TEXT_FASTA, "tsv": _lib.KMG_TEXT_TSV, "json": _lib.KMG_TEXT_JSON}
+
+
 # ----------------------------------------------------------------------------- k-mer primitives (src/kmer.rs)
 class KmerLength:
     """Validated k in 1..=32 (src/kmer.rs:74-145)."""
@@ -330,9 +334,9 @@ class GpuKmerCounter:
         return n.value
 
     def shard_write_text(self, path, fmt: str = "tsv", min_count: int = 1) -> Tuple[int, int]:
-        """kmg_shard_write_text (collective): ONE sorted fasta / tsv file from all shards of the group, the same bytes as write_text
+        """kmg_shard_write_text (collective): ONE sorted fasta / tsv / json file from all shards of the group, the same bytes as write_text
         on a single context.  Returns (records, bytes) of the whole file."""
-        code = {"fasta": _lib.KMG_TEXT_FASTA, "tsv": _lib.KMG_TEXT_TSV}[fmt]
+        code = _TEXT_FORMATS[fmt]
         n_rec, n_bytes = C.c_uint64(0), C.c_uint64(0)
         _check(self._L.kmg_shard_write_text(self._ctx, min_count, code, os.fspath(path).encode(), C.byref(n_rec), C.byref(n_bytes)), self._ctx)
         return n_rec.value, n_bytes.value
@@ -407,9 +411,9 @@ class GpuKmerCounter:
         return vals, freqs
 
     def emit_text(self, writer: IO[bytes], fmt: str = "tsv", min_count: int = 1) -> Tuple[int, int]:
-        """kmg_emit_text: sorted fasta / tsv lines formatted on the device, written to `writer` chunk by chunk.
-        Returns (records, bytes)."""
-        code = {"fasta": _lib.KMG_TEXT_FASTA, "tsv": _lib.KMG_TEXT_TSV}[fmt]
+        """kmg_emit_text: sorted fasta / tsv lines or the json document formatted on the device, written to `writer` chunk by
+        chunk.  Returns (records, bytes); json's bytes include its "[" and closing bracket."""
+        code = _TEXT_FORMATS[fmt]
 
         def sink(_user, ptr, n):
             try:
@@ -424,7 +428,7 @@ class GpuKmerCounter:
         return n_rec.value, n_bytes.value
 
     def write_text(self, path, fmt: str = "tsv", min_count: int = 1) -> Tuple[int, int]:
-        code = {"fasta": _lib.KMG_TEXT_FASTA, "tsv": _lib.KMG_TEXT_TSV}[fmt]
+        code = _TEXT_FORMATS[fmt]
         n_rec, n_bytes = C.c_uint64(0), C.c_uint64(0)
         _check(self._L.kmg_write_text(self._ctx, min_count, code, os.fspath(path).encode(), C.byref(n_rec), C.byref(n_bytes)), self._ctx)
         return n_rec.value, n_bytes.value
@@ -709,21 +713,20 @@ class KmerCounter:
         return _stringify(keys, counts, self._need_k().get())
 
     def count_to_writer(self, path, writer: IO[bytes]):
-        """src/builder.rs:399-442.  fasta / tsv lines are formatted on the GPU (kmg_emit_text), sorted by k-mer; histogram comes
-        from kmg_histogram; json (host formatting, SURVEY.md out of scope) goes through write_counts."""
+        """src/builder.rs:399-442.  fasta / tsv / json are formatted on the GPU (kmg_emit_text), sorted by k-mer; histogram
+        comes from kmg_histogram."""
         k = self._need_k()
+        if self._format not in _TEXT_FORMATS and self._format != OutputFormat.HISTOGRAM:
+            raise ValueError(f"unknown output format {self._format}")
         seq, qual, offsets = read_records(path, self._input_format)
         with GpuKmerCounter(k, min_quality=self._min_quality) as c:
             c.count_batch(seq, qual, offsets)
             c.finalize(False)
-            if self._format in (OutputFormat.FASTA, OutputFormat.TSV):
-                c.emit_text(writer, self._format, self._min_count)
-            elif self._format == OutputFormat.HISTOGRAM:
+            if self._format == OutputFormat.HISTOGRAM:
                 vals, freqs = c.histogram(self._min_count)
                 writer.write(b"".join(b"%d\t%d\n" % (int(v), int(f)) for v, f in zip(vals, freqs)))
             else:
-                keys, counts = c.export(self._min_count, sorted=True)
-                write_counts(writer, keys, counts, k.get(), self._format)
+                c.emit_text(writer, self._format, self._min_count)
 
     def run(self, path):
         """src/builder.rs:366-375 -- to stdout."""

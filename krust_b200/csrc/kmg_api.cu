@@ -2625,19 +2625,20 @@ struct HostStager {
   }
 };
 
-// A sorted (key, count) piece -> its fasta / tsv text in d_text, formatted on the device (line lengths, their exclusive sum = line
-// offsets, then every line written at its offset).  The buffers grow as pieces need and are reused across pieces.
+// A sorted (key, count) piece -> its fasta / tsv / json text in d_text, formatted on the device (record lengths, their exclusive
+// sum = record offsets, then every record written at its offset).  The buffers grow as pieces need and are reused across pieces.
+// first: record 0 of the piece is the first record of the whole output.
 struct TextFormatter {
   kmg_ctx *c;
-  int fasta;
+  int text_format;
   uint64_t *d_off = nullptr;
   uint8_t *d_text = nullptr;
   uint64_t off_cap = 0, text_cap = 0;
-  TextFormatter(kmg_ctx *c_, int fasta_) : c(c_), fasta(fasta_) {}
+  TextFormatter(kmg_ctx *c_, int text_format_) : c(c_), text_format(text_format_) {}
   ~TextFormatter() { pool_free(c, d_off); pool_free(c, d_text); }
-  kmg_status format(const uint64_t *dk, const uint64_t *dc, uint64_t m, uint64_t *bytes_out) {
+  kmg_status format(const uint64_t *dk, const uint64_t *dc, uint64_t m, bool first, uint64_t *bytes_out) {
     if (m + 1 > off_cap) { pool_free(c, d_off); d_off = nullptr; off_cap = std::max<uint64_t>(m + 1, 1ull << 20); CU(c, pool_alloc(c, &d_off, off_cap * 8)); }
-    CU(c, launch_text_len(dc, m, c->k, fasta, d_off, c->stream));
+    CU(c, launch_text_len(dc, m, c->k, text_format, first, d_off, c->stream));
     CU(c, cudaMemsetAsync(d_off + m, 0, 8, c->stream));
     if (!c->d_scan_tmp || c->scan_tmp_items < m + 1) {
       CU(c, cudaStreamSynchronize(c->stream));
@@ -2651,11 +2652,14 @@ struct TextFormatter {
     CU(c, cudaMemcpyAsync(&total, d_off + m, 8, cudaMemcpyDeviceToHost, c->stream));
     CU(c, cudaStreamSynchronize(c->stream));
     if (total > text_cap) { pool_free(c, d_text); d_text = nullptr; text_cap = total + total / 8; CU(c, pool_alloc(c, &d_text, text_cap)); }
-    CU(c, launch_text_write(dk, dc, d_off, m, c->k, fasta, d_text, c->stream));
+    CU(c, launch_text_write(dk, dc, d_off, m, c->k, text_format, first, d_text, c->stream));
     *bytes_out = total;
     return KMG_OK;
   }
 };
+// json framing around the records: "[" in front of them, then "\n]\n" after them, or "]\n" when there is none ("[]\n")
+constexpr char JSON_OPEN[] = "[";
+const char *json_close(uint64_t records) { return records ? "\n]\n" : "]\n"; }
 
 // Stream all (key, count) records of the context to `f` in ascending key order (16-byte records interleaved on the device).
 // *crc_out is the finished CRC-32 of the bytes written here (standard init / xor-out).
@@ -2882,28 +2886,37 @@ KMG_EXPORT kmg_status kmg_shard_stats(const kmg_ctx *c, uint64_t *sent_keys, uin
 }
 
 
-// Text emitters of output_counts / count_to_writer (src/run.rs:452-470, src/builder.rs:399-442) for --format tsv and fasta:
+// Text emitters of output_counts / count_to_writer (src/run.rs:452-481, src/builder.rs:399-442) for --format tsv, fasta and json:
 // records with count >= min_count in ascending k-mer order (the reference prints HashMap order; parity is on the sorted text),
-// formatted ON THE DEVICE (2-bit unpack + decimal count), delivered to `sink` in chunks of at most 64 MiB.
+// formatted ON THE DEVICE (2-bit unpack + decimal count), delivered to `sink` in chunks of at most 64 MiB.  json's framing goes
+// to the sink before the first piece and after the last one.
 KMG_EXPORT kmg_status kmg_emit_text(kmg_ctx *c, uint64_t min_count, int format, kmg_text_sink sink, void *user, uint64_t *n_records_out,
                                     uint64_t *n_bytes_out) {
   if (!c || !sink) return KMG_ERR_INVALID_ARG;
-  if (format != KMG_TEXT_FASTA && format != KMG_TEXT_TSV) return fail(c, KMG_ERR_INVALID_ARG, "format must be KMG_TEXT_FASTA or KMG_TEXT_TSV");
+  if (format != KMG_TEXT_FASTA && format != KMG_TEXT_TSV && format != KMG_TEXT_JSON)
+    return fail(c, KMG_ERR_INVALID_ARG, "format must be KMG_TEXT_FASTA, KMG_TEXT_TSV or KMG_TEXT_JSON");
   CU(c, cudaSetDevice(c->device));
   if (min_count == 0) min_count = 1;
-  const int fasta = format == KMG_TEXT_FASTA;
   uint64_t records = 0, bytes = 0;
+  auto to_sink = [&](const uint8_t *p, size_t len) -> kmg_status {
+    return sink(user, p, len) == 0 ? KMG_OK : fail(c, KMG_ERR_IO, "the text sink reported an error");
+  };
+  auto frame = [&](const char *t) -> kmg_status {
+    bytes += strlen(t);
+    return to_sink(reinterpret_cast<const uint8_t *>(t), strlen(t));
+  };
+  kmg_status s = format == KMG_TEXT_JSON ? frame(JSON_OPEN) : KMG_OK;
   HostStager stage(c, 64u << 20);
-  TextFormatter fmt(c, fasta);
-  kmg_status s = for_each_sorted_piece(c, min_count, 1ull << 24, [&](const uint64_t *dk, const uint64_t *dc, uint64_t m) -> kmg_status {
-    uint64_t total = 0;
-    kmg_status fs = fmt.format(dk, dc, m, &total);
-    if (fs != KMG_OK) return fs;
-    records += m; bytes += total;
-    return stage.drain(fmt.d_text, total, [&](const uint8_t *p, size_t len) -> kmg_status {
-      return sink(user, p, len) == 0 ? KMG_OK : fail(c, KMG_ERR_IO, "the text sink reported an error");
+  TextFormatter fmt(c, format);
+  if (s == KMG_OK)
+    s = for_each_sorted_piece(c, min_count, 1ull << 24, [&](const uint64_t *dk, const uint64_t *dc, uint64_t m) -> kmg_status {
+      uint64_t total = 0;
+      kmg_status fs = fmt.format(dk, dc, m, records == 0, &total);
+      if (fs != KMG_OK) return fs;
+      records += m; bytes += total;
+      return stage.drain(fmt.d_text, total, to_sink);
     });
-  });
+  if (s == KMG_OK && format == KMG_TEXT_JSON) s = frame(json_close(records));
   if (n_records_out) *n_records_out = records;
   if (n_bytes_out) *n_bytes_out = bytes;
   return s;
@@ -2913,7 +2926,7 @@ namespace {
 int file_sink(void *user, const uint8_t *p, size_t n) { return fwrite(p, 1, n, static_cast<FILE *>(user)) == n ? 0 : 1; }
 }  // namespace
 
-// The same into a file ("-" = stdout): what `kmerust <k> <path> --format tsv|fasta --min-count m > file` produces, sorted.
+// The same into a file ("-" = stdout): what `kmerust <k> <path> --format tsv|fasta|json --min-count m > file` produces, sorted.
 KMG_EXPORT kmg_status kmg_write_text(kmg_ctx *c, uint64_t min_count, int format, const char *path, uint64_t *n_records_out, uint64_t *n_bytes_out) {
   if (!c || !path) return KMG_ERR_INVALID_ARG;
   const bool to_stdout = strcmp(path, "-") == 0;
@@ -2930,13 +2943,18 @@ KMG_EXPORT kmg_status kmg_write_text(kmg_ctx *c, uint64_t min_count, int format,
 // step.  In each step every rank compacts and sorts its part of the step's key range into a staging buffer its peers can read;
 // rank j then owns piece j of the step: it merges the piece's W sorted parts straight out of the peers' memory
 // (merge_shard_pieces_kernel), formats it on the device and writes it at its offset in the file (the bytes of all earlier pieces).
+// json: every piece lands after the "[" that rank 0 writes at offset 0; the owner of the first non-empty piece of the file formats
+// its first record without the "," separator; rank 0 writes the closing bracket after the last step.
 KMG_EXPORT kmg_status kmg_shard_write_text(kmg_ctx *c, uint64_t min_count, int format, const char *path, uint64_t *n_records_out,
                                            uint64_t *n_bytes_out) {
   if (!c || !path) return KMG_ERR_INVALID_ARG;
   if (!c->shm) return kmg_write_text(c, min_count, format, path, n_records_out, n_bytes_out);
   // every rank sees the same path: all of them refuse here, before any barrier
   if (strcmp(path, "-") == 0) return fail(c, KMG_ERR_INVALID_ARG, "a shard group writes its text to a file: ranks cannot write one stream at given offsets");
-  if (format != KMG_TEXT_FASTA && format != KMG_TEXT_TSV) return shard_fail(c, KMG_ERR_INVALID_ARG, "format must be KMG_TEXT_FASTA or KMG_TEXT_TSV");
+  if (format != KMG_TEXT_FASTA && format != KMG_TEXT_TSV && format != KMG_TEXT_JSON)
+    return shard_fail(c, KMG_ERR_INVALID_ARG, "format must be KMG_TEXT_FASTA, KMG_TEXT_TSV or KMG_TEXT_JSON");
+  const bool json = format == KMG_TEXT_JSON;
+  const uint64_t head = json ? strlen(JSON_OPEN) : 0;  // bytes in front of the first piece
   if (min_count == 0) min_count = 1;
   SCU(c, cudaSetDevice(c->device));
   ShardShm *S = c->shm;
@@ -2986,8 +3004,16 @@ KMG_EXPORT kmg_status kmg_shard_write_text(kmg_ctx *c, uint64_t min_count, int f
     if (!why.empty()) return shard_fail(c, KMG_ERR_CUDA, why);
     if ((fd = open(path, O_WRONLY)) < 0) return shard_fail(c, KMG_ERR_IO, std::string("cannot open ") + path + " for writing");
     HostStager staged(c, 64u << 20);
-    TextFormatter fmt(c, format == KMG_TEXT_FASTA);
+    TextFormatter fmt(c, format);
     uint64_t written = 0;
+    auto put = [&](const uint8_t *p, size_t len, uint64_t off) -> kmg_status {
+      for (size_t done = 0; done < len;) {
+        const ssize_t w = pwrite(fd, p + done, len - done, (off_t)(off + done));
+        if (w <= 0) return shard_fail(c, KMG_ERR_IO, std::string("short write to ") + path);
+        done += (size_t)w; written += (uint64_t)w;
+      }
+      return KMG_OK;
+    };
     size_t step = 0;
     kmg_status st = for_each_sorted_piece(c, min_count, step_cuts, stage, stage + stage_cap, stage_cap,
                                           [&](const uint64_t *sk, const uint64_t *, uint64_t m) -> kmg_status {
@@ -3008,22 +3034,23 @@ KMG_EXPORT kmg_status kmg_shard_write_text(kmg_ctx *c, uint64_t min_count, int f
       if (me < n_own) {
         MergeRuns R{};
         R.n_runs = W;
+        uint64_t before = records;  // records of the file in front of this piece: earlier steps + earlier pieces of this step
         for (uint32_t q = 0; q < W; ++q) {
           const uint64_t lo = S->ranks[q].text_bounds[me], hi = S->ranks[q].text_bounds[me + 1];
           R.keys[q] = peer[q] + lo; R.counts[q] = peer[q] + stage_cap + lo; R.len[q] = hi - lo;
-          expect += hi - lo;
+          expect += hi - lo; before += lo;
         }
         if (expect > own_cap) return shard_fail(c, KMG_ERR_STATE, "merged piece larger than its key histogram");
         unsigned long long *d_placed = reinterpret_cast<unsigned long long *>(d_aux + SHARD_MAX_WORLD + 1);
         SCU(c, launch_merge_shard_pieces(R, dk, dc, d_placed, c->stream));
         SCU(c, cudaMemcpyAsync(&placed, d_placed, 8, cudaMemcpyDeviceToHost, c->stream));
-        kmg_status fs = fmt.format(dk, dc, expect, &bytes);  // ends in a stream synchronize
+        kmg_status fs = fmt.format(dk, dc, expect, before == 0 && expect > 0, &bytes);  // ends in a stream synchronize
         if (fs != KMG_OK) return shard_fail(c, fs, c->err);
       }
       mine.text_piece[0] = expect; mine.text_piece[1] = placed; mine.text_piece[2] = bytes;
       SB(c);  // nobody reads a staging buffer of this step any more: the next step may overwrite them
-      // 5. file offset = bytes of all earlier pieces; every merged piece holds as many ordered records as its parts
-      uint64_t off = file_bytes;
+      // 5. file offset = json's "[" + bytes of all earlier pieces; every merged piece holds as many ordered records as its parts
+      uint64_t off = head + file_bytes;
       for (uint32_t j = 0; j < n_own; ++j) {
         const uint64_t *tp = S->ranks[j].text_piece;
         if (tp[0] != tp[1]) return shard_fail(c, KMG_ERR_STATE, "piece " + std::to_string(p0 + j) + ": the merge placed " + std::to_string(tp[1]) + " records in order, its parts hold " + std::to_string(tp[0]));
@@ -3031,15 +3058,20 @@ KMG_EXPORT kmg_status kmg_shard_write_text(kmg_ctx *c, uint64_t min_count, int f
         file_bytes += tp[2]; records += tp[0];
       }
       return staged.drain(fmt.d_text, bytes, [&](const uint8_t *p, size_t len) -> kmg_status {
-        for (size_t done = 0; done < len;) {
-          const ssize_t w = pwrite(fd, p + done, len - done, (off_t)off);
-          if (w <= 0) return shard_fail(c, KMG_ERR_IO, std::string("short write to ") + path);
-          done += (size_t)w; off += (uint64_t)w; written += (uint64_t)w;
-        }
-        return KMG_OK;
+        kmg_status ps = put(p, len, off);
+        off += len;
+        return ps;
       });
     });
     if (st != KMG_OK) return shard_fail(c, st, c->err);
+    if (json) {  // every rank knows the group's records now; rank 0 writes the framing around the pieces
+      const char *tail = json_close(records);
+      if (me == 0) {
+        if ((st = put(reinterpret_cast<const uint8_t *>(JSON_OPEN), head, 0)) != KMG_OK) return st;
+        if ((st = put(reinterpret_cast<const uint8_t *>(tail), strlen(tail), head + file_bytes)) != KMG_OK) return st;
+      }
+      file_bytes += head + strlen(tail);
+    }
     const int closed = close(fd);
     fd = -1;
     if (closed != 0) return shard_fail(c, KMG_ERR_IO, std::string("short write to ") + path);

@@ -17,6 +17,7 @@
 #include <cub/device/device_scan.cuh>
 #include <thrust/iterator/transform_iterator.h>
 
+#include "../../include/kmerust_gpu.h"
 #include "kmg_device.cuh"
 
 namespace kmg {
@@ -1145,27 +1146,46 @@ __global__ void deinterleave_pairs_kernel(const ulonglong2 *__restrict__ in, uin
 }
 
 // ---- output formatting on the device (replaces the per-k-mer writeln! of src/run.rs:452-470 / src/builder.rs:406-429 and
-// unpack_to_string, src/kmer.rs:431-456): record i of a sorted piece becomes "{kmer}\t{count}\n" (tsv) or ">{count}\n{kmer}\n" (fasta)
+// unpack_to_string, src/kmer.rs:431-456): record i of a sorted piece becomes "{kmer}\t{count}\n" (tsv), ">{count}\n{kmer}\n" (fasta)
+// or, for json (serde_json::to_string_pretty of the {kmer, count} vector), ",\n" + body with body = "  {\n    \"kmer\": \"{kmer}\",\n
+// \"count\": {count}\n  }".  The separator goes in front of a record, so only the first record of the whole output differs (its
+// prefix is "\n"): `first` says that record 0 of this piece is that one.  The "[" and the trailer are framing the caller writes.
 __device__ __forceinline__ uint32_t dec_digits(uint64_t v) {
   uint32_t d = 1;
   while (v >= 10) { v /= 10; ++d; }
   return d;
 }
-__global__ void text_len_kernel(const uint64_t *__restrict__ counts, uint64_t n, int k, int fasta, uint64_t *__restrict__ lens) {
-  for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x)
-    lens[i] = (uint64_t)k + dec_digits(counts[i]) + (fasta ? 3u : 2u);
+constexpr uint32_t JSON_HEAD = 17;  // `  {\n    "kmer": "`
+constexpr uint32_t JSON_MID = 16;   // `",\n    "count": `
+__global__ void text_len_kernel(const uint64_t *__restrict__ counts, uint64_t n, int k, int format, int first, uint64_t *__restrict__ lens) {
+  for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
+    const uint64_t fixed = format == KMG_TEXT_FASTA ? 3u : format == KMG_TEXT_TSV ? 2u : (i == 0 && first ? 1u : 2u) + JSON_HEAD + JSON_MID + 4u;
+    lens[i] = (uint64_t)k + dec_digits(counts[i]) + fixed;
+  }
 }
 __global__ void text_write_kernel(const uint64_t *__restrict__ keys, const uint64_t *__restrict__ counts, const uint64_t *__restrict__ offs,
-                                  uint64_t n, int k, int fasta, uint8_t *__restrict__ out) {
+                                  uint64_t n, int k, int format, int first, uint8_t *__restrict__ out) {
   for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
     const uint64_t key = keys[i];
     uint64_t cnt = counts[i];
     uint8_t *p = out + offs[i];
     const uint32_t nd = dec_digits(cnt);
-    uint8_t *num = fasta ? p + 1 : p + k + 1;       // where the decimal count goes
-    uint8_t *mer = fasta ? p + 1 + nd + 1 : p;      // where the k-mer goes
-    if (fasta) { p[0] = '>'; p[1 + nd] = '\n'; p[1 + nd + 1 + k] = '\n'; }
-    else { p[k] = '\t'; p[k + 1 + nd] = '\n'; }
+    uint8_t *num, *mer;  // where the decimal count and the k-mer go
+    if (format == KMG_TEXT_FASTA) {
+      num = p + 1; mer = p + 1 + nd + 1;
+      p[0] = '>'; p[1 + nd] = '\n'; p[1 + nd + 1 + k] = '\n';
+    } else if (format == KMG_TEXT_TSV) {
+      num = p + k + 1; mer = p;
+      p[k] = '\t'; p[k + 1 + nd] = '\n';
+    } else {
+      if (!(i == 0 && first)) *p++ = ',';
+      const char head[] = "\n  {\n    \"kmer\": \"", mid[] = "\",\n    \"count\": ", tail[] = "\n  }";
+      for (uint32_t j = 0; j < JSON_HEAD + 1; ++j) p[j] = (uint8_t)head[j];
+      mer = p + JSON_HEAD + 1;
+      for (uint32_t j = 0; j < JSON_MID; ++j) mer[k + j] = (uint8_t)mid[j];
+      num = mer + k + JSON_MID;
+      for (uint32_t j = 0; j < 4; ++j) num[nd + j] = (uint8_t)tail[j];
+    }
     for (int d = (int)nd - 1; d >= 0; --d) { num[d] = (uint8_t)('0' + cnt % 10); cnt /= 10; }
     for (int j = 0; j < k; ++j) mer[j] = "ACGT"[(key >> (2 * (k - 1 - j))) & 3];  // base j = (bits >> 2(k-1-j)) & 3 (src/kmer.rs:431-440)
   }
@@ -1575,17 +1595,17 @@ cudaError_t launch_deinterleave_pairs(const void *d_in, uint64_t n, uint64_t *d_
   deinterleave_pairs_kernel<<<grid_for(n, 256, 8), 256, 0, s>>>(static_cast<const ulonglong2 *>(d_in), n, d_keys, d_counts);
   return cudaGetLastError();
 }
-cudaError_t launch_text_len(const uint64_t *d_counts, uint64_t n, int k, int fasta, uint64_t *d_lens, cudaStream_t s) {
+cudaError_t launch_text_len(const uint64_t *d_counts, uint64_t n, int k, int format, int first, uint64_t *d_lens, cudaStream_t s) {
   if (n == 0) return cudaSuccess;
   g_launches.fetch_add(1, std::memory_order_relaxed);
-  text_len_kernel<<<grid_for(n, 256, 8), 256, 0, s>>>(d_counts, n, k, fasta, d_lens);
+  text_len_kernel<<<grid_for(n, 256, 8), 256, 0, s>>>(d_counts, n, k, format, first, d_lens);
   return cudaGetLastError();
 }
-cudaError_t launch_text_write(const uint64_t *d_keys, const uint64_t *d_counts, const uint64_t *d_offs, uint64_t n, int k, int fasta, uint8_t *d_out,
-                              cudaStream_t s) {
+cudaError_t launch_text_write(const uint64_t *d_keys, const uint64_t *d_counts, const uint64_t *d_offs, uint64_t n, int k, int format, int first,
+                              uint8_t *d_out, cudaStream_t s) {
   if (n == 0) return cudaSuccess;
   g_launches.fetch_add(1, std::memory_order_relaxed);
-  text_write_kernel<<<grid_for(n, 256, 8), 256, 0, s>>>(d_keys, d_counts, d_offs, n, k, fasta, d_out);
+  text_write_kernel<<<grid_for(n, 256, 8), 256, 0, s>>>(d_keys, d_counts, d_offs, n, k, format, first, d_out);
   return cudaGetLastError();
 }
 cudaError_t launch_interleave_pairs(const uint64_t *d_keys, const uint64_t *d_counts, uint64_t n, void *d_out, cudaStream_t s) {

@@ -207,10 +207,11 @@ cudaError_t launch_query_pack(const uint8_t *d_kmers, uint64_t n, int k, uint64_
 cudaError_t launch_query(const TableView &v, HashTable t, const uint64_t *d_seg_start, const uint64_t *d_seg_len, uint32_t n_coarse, uint32_t n_sub,
                          uint32_t shard_world, uint32_t shard_rank, const uint64_t *d_keys, uint64_t n, uint64_t *d_counts, cudaStream_t s);
 cudaError_t launch_deinterleave_pairs(const void *d_in, uint64_t n, uint64_t *d_keys, uint64_t *d_counts, cudaStream_t s);
-// text emitters / index records of a sorted piece (formatting happens on the device)
-cudaError_t launch_text_len(const uint64_t *d_counts, uint64_t n, int k, int fasta, uint64_t *d_lens, cudaStream_t s);
-cudaError_t launch_text_write(const uint64_t *d_keys, const uint64_t *d_counts, const uint64_t *d_offs, uint64_t n, int k, int fasta, uint8_t *d_out,
-                              cudaStream_t s);
+// text emitters / index records of a sorted piece (formatting happens on the device).  format is a KMG_TEXT_* code; first != 0:
+// record 0 of the piece is the first record of the whole output (json puts no "," in front of it)
+cudaError_t launch_text_len(const uint64_t *d_counts, uint64_t n, int k, int format, int first, uint64_t *d_lens, cudaStream_t s);
+cudaError_t launch_text_write(const uint64_t *d_keys, const uint64_t *d_counts, const uint64_t *d_offs, uint64_t n, int k, int format, int first,
+                              uint8_t *d_out, cudaStream_t s);
 cudaError_t launch_interleave_pairs(const uint64_t *d_keys, const uint64_t *d_counts, uint64_t n, void *d_out, cudaStream_t s);
 // text file of a shard group: up to MERGE_MAX_RUNS sorted (key, count) runs, possibly in other GPUs' memory (P2P / IPC mapped),
 // merged into one sorted local run.  The runs' keys must be pairwise distinct (a key lives on one shard only).

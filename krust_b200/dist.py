@@ -331,8 +331,8 @@ class ShardedKmerCounter:
         return {"records": int(sum(p[0] for p in parts))}
 
     def write_text(self, path, fmt: str = "tsv", min_count: int = 1) -> Tuple[int, int]:
-        """ONE sorted fasta / tsv file from all shards, byte-identical to what one GPU writes for the same input (collective).
-        Returns (records, bytes) of the whole file on every rank."""
+        """ONE sorted fasta / tsv / json file from all shards, byte-identical to what one GPU writes for the same input
+        (collective).  Returns (records, bytes) of the whole file on every rank."""
         if self.world == 1:
             return self.engine.counter.write_text(path, fmt, min_count)
         if self.fused and self.engine.joined:

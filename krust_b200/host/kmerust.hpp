@@ -238,10 +238,12 @@ class GpuKmerCounter {
     check(s);
     return true;
   }
-  // fasta / tsv lines formatted on the device, sorted by k-mer (kmg_write_text; "-" = stdout)
+  // fasta / tsv / json records formatted on the device, sorted by k-mer (kmg_write_text; "-" = stdout)
   uint64_t write_text(const std::string &path, OutputFormat fmt, uint64_t min_count) {
+    if (fmt == OutputFormat::Histogram) throw KmeRustError("write_text formats fasta, tsv or json; the histogram comes from histogram()");
+    const int code = fmt == OutputFormat::Tsv ? KMG_TEXT_TSV : fmt == OutputFormat::Json ? KMG_TEXT_JSON : KMG_TEXT_FASTA;
     uint64_t recs = 0, bytes = 0;
-    check(kmg_write_text(ctx_, min_count, fmt == OutputFormat::Tsv ? KMG_TEXT_TSV : KMG_TEXT_FASTA, path.c_str(), &recs, &bytes));
+    check(kmg_write_text(ctx_, min_count, code, path.c_str(), &recs, &bytes));
     return recs;
   }
   std::vector<uint64_t> query(const std::vector<std::string> &kmers, uint64_t *n_invalid = nullptr) {

@@ -122,13 +122,9 @@ int main(int argc, char **argv) {
     std::ios::sync_with_stdio(false);
     if (format == OutputFormat::Histogram) {
       for (auto &kv : counter.histogram(min_count)) std::cout << kv.first << '\t' << kv.second << '\n';
-    } else if (format == OutputFormat::Fasta || format == OutputFormat::Tsv) {
-      std::cout.flush();
-      counter.write_text("-", format, min_count);  // lines are formatted on the device
     } else {
-      std::vector<uint64_t> keys, counts;
-      counter.export_counts(min_count, true, keys, counts);
-      output_counts(std::cout, keys, counts, kl, format);
+      std::cout.flush();
+      counter.write_text("-", format, min_count);  // fasta / tsv / json records are formatted on the device
     }
     std::cout.flush();
   } catch (const KmeRustError &e) {
