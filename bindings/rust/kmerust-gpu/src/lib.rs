@@ -162,6 +162,15 @@ impl GpuKmerCounter {
         let q = qual.map_or(std::ptr::null(), |q| q.as_ptr());
         self.check(unsafe { sys::kmg_shard_count_ascii(self.ctx, seq.as_ptr(), q, offsets.as_ptr(), n) })
     }
+    /// The WHOLE file image, the same on every rank (each process may map the file): every rank parses only its own slice on
+    /// the device.  Returns the records of the whole image.  Join with `expected_keys_total` = `bytes.len()` (FASTA) or half
+    /// of it (FASTQ).  On `KMG_ERR_PARSE` the group is aborted: leave it, drop the counters and count the crate's own reader's
+    /// records with a new group through `count_batch_sharded`.
+    pub fn count_file_image_sharded(&mut self, bytes: &[u8], is_fastq: bool) -> Result<u64, GpuError> {
+        let mut n = 0u64;
+        self.check(unsafe { sys::kmg_shard_count_fastx(self.ctx, bytes.as_ptr(), bytes.len() as u64, is_fastq as i32, &mut n) })?;
+        Ok(n)
+    }
     pub fn histogram_sharded(&mut self, min_count: u64) -> Result<BTreeMap<u64, u64>, GpuError> {
         let mut n = 0u64;
         self.check(unsafe { sys::kmg_shard_histogram(self.ctx, min_count, std::ptr::null_mut(), std::ptr::null_mut(), 0, &mut n) })?;

@@ -192,6 +192,19 @@ kmg_status kmg_shard_leave(kmg_ctx *ctx);
 kmg_status kmg_shard_count_ascii_device(kmg_ctx *ctx, const uint8_t *d_seq, const uint8_t *d_qual, const uint64_t *d_offsets,
                                         uint64_t n_records, uint64_t n_bytes);
 kmg_status kmg_shard_count_ascii(kmg_ctx *ctx, const uint8_t *seq, const uint8_t *qual, const uint64_t *offsets, uint64_t n_records);
+/* kmg_count_fastx for the whole group: every rank passes the SAME whole file image (each process may mmap the file, thread ranks
+ * may share one buffer) and parses only its own slice of it on the device.  With t = len * r / world, rank r's slice begins at
+ * the first line start (FASTA) / record start (FASTQ: a '@' line whose line after next begins with '+') at or after t; every rank
+ * computes all cuts from the same bytes.  A FASTA slice that begins inside a record is preceded by the record's last k-1 bases,
+ * so every window is counted once, by the rank that holds its last base; the union of the shards equals what kmg_count_fastx
+ * gives on one context, whatever the world size.  Each parsed chunk (at most batch_bases - (k-1) raw bytes) is one fused round.
+ * *n_records_out: records of the whole image, on every rank.  Join with expected_keys_total = len (FASTA) or len / 2 (FASTQ).
+ * Every rank returns an error when byte 0 is no header, a line is longer than a chunk, the FASTQ is multi-line or has a quality
+ * of a different length than its sequence (KMG_ERR_PARSE; peers of a rank that fails mid-stream return KMG_ERR_STATE), or the
+ * ranks passed images of different lengths / cuts (KMG_ERR_INVALID_ARG).  The group is then aborted: leave it, destroy the
+ * contexts, and count the input with a new group through kmg_parse_fastx + kmg_shard_count_ascii.  Outside a group it is
+ * kmg_count_fastx. */
+kmg_status kmg_shard_count_fastx(kmg_ctx *ctx, const uint8_t *buf, uint64_t len, int is_fastq, uint64_t *n_records_out);
 /* kmg_finalize + the summary of the WHOLE table (sums over the shards; kernel timings stay this rank's). */
 kmg_status kmg_shard_finalize(kmg_ctx *ctx, kmg_summary *summary);
 /* kmg_histogram merged over the shards (element-wise sum); the size query does the merge, the second call copies it out. */

@@ -59,6 +59,7 @@ SIGNATURES = {
     "kmg_shard_leave": (i32, [vp]),
     "kmg_shard_count_ascii_device": (i32, [vp, vp, vp, vp, u64, u64]),
     "kmg_shard_count_ascii": (i32, [vp, vp, vp, vp, u64]),
+    "kmg_shard_count_fastx": (i32, [vp, vp, u64, i32, C.POINTER(u64)]),
     "kmg_shard_finalize": (i32, [vp, C.POINTER(KmgSummary)]),
     "kmg_shard_histogram": (i32, [vp, u64, vp, vp, u64, C.POINTER(u64)]),
     "kmg_shard_save_kmix": (i32, [vp, C.c_char_p, C.POINTER(u64)]),

@@ -314,6 +314,15 @@ class GpuKmerCounter:
                                              qual.ctypes.data if qual is not None and len(qual) else None,
                                              offsets.ctypes.data if n_rec else None, n_rec), self._ctx)
 
+    def shard_count_fastx(self, data, is_fastq: bool) -> int:
+        """kmg_shard_count_fastx (collective): every rank passes the SAME whole FASTA / FASTQ file image (same input types as
+        count_fastx) and parses its own slice of it on the device.  Returns the records of the whole image."""
+        arr = data if isinstance(data, np.ndarray) else np.frombuffer(data, dtype=np.uint8)
+        assert arr.dtype == np.uint8 and arr.flags.c_contiguous
+        n = C.c_uint64(0)
+        _check(self._L.kmg_shard_count_fastx(self._ctx, arr.ctypes.data if len(arr) else None, len(arr), int(is_fastq), C.byref(n)), self._ctx)
+        return n.value
+
     def shard_finalize(self) -> dict:
         s = KmgSummary()
         _check(self._L.kmg_shard_finalize(self._ctx, C.byref(s)), self._ctx)

@@ -1436,91 +1436,110 @@ KMG_EXPORT kmg_status kmg_count_ascii(kmg_ctx *c, const uint8_t *seq, const uint
 }
 
 
-// FASTA / FASTQ file image (HOST bytes, e.g. an mmap'ed file: src/mmap.rs:33-71) -> counts, with the records found ON THE DEVICE:
-// the raw bytes go over PCIe in chunks cut at line (FASTA) / record (FASTQ) boundaries, a few small kernels classify the lines,
-// compact sequence (+ quality) bytes, mark the record starts, and the usual ingest + scan follow.  Replaces reader::read /
-// read_with_quality (src/reader.rs:82-247: whole file -> Vec<Record> -> Vec<SequenceWithQuality>, two host copies) for
-// well-formed input; multi-line FASTQ, or a line longer than a chunk, is refused with KMG_ERR_PARSE -- nothing has been
-// counted then only if it happens in the first chunk, so callers fall back to kmg_parse_fastx + kmg_count_ascii after kmg_reset.
-KMG_EXPORT kmg_status kmg_count_fastx(kmg_ctx *c, const uint8_t *buf, uint64_t len, int is_fastq, uint64_t *n_records_out) {
-  if (!c || (len && !buf)) return KMG_ERR_INVALID_ARG;
-  if (c->shm) return fail(c, KMG_ERR_STATE, "context belongs to a shard group: feed it with kmg_shard_count_ascii(_device)");
-  if (n_records_out) *n_records_out = 0;
-  if (len == 0) return KMG_OK;
-  const uint8_t marker = is_fastq ? '@' : '>';
-  if (buf[0] != marker) return fail(c, KMG_ERR_PARSE, is_fastq ? "FASTQ record does not start with '@' (record 0)" : "FASTA record does not start with '>' (record 0)");
-  CU(c, cudaSetDevice(c->device));
-  const bool use_q = is_fastq && c->cfg.has_min_quality;
-  const uint64_t K1 = (uint64_t)c->k - 1;
-  const uint64_t CB = std::min<uint64_t>(c->batch_bases, 1ull << 30);
-  // ---- chunk plan: cuts at line starts (FASTA) / record starts (FASTQ)
-  struct Chunk { uint64_t pos, len; };
-  std::vector<Chunk> chunks;
-  for (uint64_t pos = 0; pos < len;) {
-    uint64_t end = std::min(len, pos + CB);
-    if (end < len) {
-      const void *nl = memrchr(buf + pos, '\n', (size_t)(end - pos));
+namespace {
+
+constexpr int FASTQ_SYNC_LINES = 64;  // lines searched for a FASTQ record start at a chunk end (backward) or a rank cut (forward)
+
+// Does the line at p open a FASTQ record?  '@' first, and the line after next begins with '+' (a quality line may begin with '@',
+// but the line after next of a quality line is a sequence line).
+bool fastq_record_start(const uint8_t *buf, uint64_t len, uint64_t p) {
+  if (p >= len || buf[p] != '@') return false;
+  const void *l1 = memchr(buf + p, '\n', (size_t)(len - p));
+  const void *l2 = l1 ? memchr((const uint8_t *)l1 + 1, '\n', (size_t)(buf + len - ((const uint8_t *)l1 + 1))) : nullptr;
+  return l2 && (const uint8_t *)l2 + 1 < buf + len && ((const uint8_t *)l2)[1] == '+';
+}
+
+struct FxChunk { uint64_t pos, len; };
+
+// Staging chunks of buf[begin, end) (begin and end at line starts (FASTA) / record starts (FASTQ), or end == len): each holds at
+// most cb bytes and ends at a line start (FASTA) or a record start (FASTQ).
+kmg_status plan_fastx_chunks(kmg_ctx *c, const uint8_t *buf, uint64_t len, uint64_t begin, uint64_t end, bool is_fastq, uint64_t cb,
+                             std::vector<FxChunk> &chunks) {
+  for (uint64_t pos = begin; pos < end;) {
+    uint64_t stop = std::min(end, pos + cb);
+    if (stop < end) {
+      const void *nl = memrchr(buf + pos, '\n', (size_t)(stop - pos));
       if (!nl) return fail(c, KMG_ERR_PARSE, "a line is longer than a staging chunk (raise batch_bases or use the host splitter)");
-      end = (uint64_t)((const uint8_t *)nl - buf) + 1;
-      if (is_fastq) {  // step back line by line to a line that opens a record: '@' first, and the line after next begins with '+'
-        uint64_t cut = end;
+      stop = (uint64_t)((const uint8_t *)nl - buf) + 1;
+      if (is_fastq) {  // step back line by line to a line that opens a record
+        uint64_t cut = stop;
         bool found = false;
-        for (int tries = 0; tries < 64 && cut > pos; ++tries) {
-          if (buf[cut] == '@') {
-            const void *l1 = memchr(buf + cut, '\n', (size_t)(len - cut));
-            const void *l2 = l1 ? memchr((const uint8_t *)l1 + 1, '\n', (size_t)(buf + len - ((const uint8_t *)l1 + 1))) : nullptr;
-            if (l2 && (const uint8_t *)l2 + 1 < buf + len && ((const uint8_t *)l2)[1] == '+') { found = true; break; }
-          }
+        for (int tries = 0; tries < FASTQ_SYNC_LINES && cut > pos; ++tries) {
+          if (fastq_record_start(buf, len, cut)) { found = true; break; }
           const void *prev = cut >= 2 ? memrchr(buf + pos, '\n', (size_t)(cut - 1 - pos)) : nullptr;  // start of the previous line
           if (!prev) break;
           cut = (uint64_t)((const uint8_t *)prev - buf) + 1;
         }
         if (!found || cut <= pos) return fail(c, KMG_ERR_PARSE, "no FASTQ record boundary found near a chunk end (multi-line FASTQ? use the host splitter)");
-        end = cut;
+        stop = cut;
       }
     }
-    chunks.push_back(Chunk{pos, end - pos});
-    pos = end;
+    chunks.push_back(FxChunk{pos, stop - pos});
+    pos = stop;
   }
-  uint64_t max_len = 0;
-  for (auto &ch : chunks) max_len = std::max(max_len, ch.len);
-  if (max_len >= (1ull << 32)) return fail(c, KMG_ERR_INVALID_ARG, "staging chunks must stay below 4 GiB");
-  // ---- plan the table / partitions for the whole file
-  kmg_status s = KMG_OK;
-  if (use_q && !c->cfg.expected_distinct && c->mode == kmg_ctx::MODE_UNDECIDED && !c->use_dense) c->plan_scale = (double)len / (double)chunks[0].len;
-  else s = decide_mode(c, is_fastq ? len / 2 : len);
-  if (s != KMG_OK) return s;
-  const bool src_pinned = is_pinned_host(buf);
-  s = ensure_staging(c, !src_pinned, false, max_len);
-  if (s != KMG_OK) return s;
-  // ---- parse buffers (pooled)
+  return KMG_OK;
+}
+
+// The device parser's driver over the planned chunks of one file image: pooled parse buffers, raw chunks staged through the
+// context's ring (up to N_STAGE - 1 chunks ahead), per chunk the parse kernels, the scatter of sequence (+ quality) bytes and record
+// marks, the carry of a FASTA record's last k-1 bases into the next chunk, and the error words.  step() leaves the chunk packed in
+// the context's stream and hands it to the caller's scan (scan_packed on one context, shard_scan_round in a group).
+struct FastxFeed {
+  kmg_ctx *c;
+  const uint8_t *buf;
+  const std::vector<FxChunk> &chunks;
+  bool is_fastq, use_q, src_pinned = false;
+  uint64_t K1 = 0, max_len = 0, prev_n = 0, bases = 0;  // prev_n: sequence bases the last chunk left (their tail is the next carry)
   uint8_t *d_kind = nullptr, *d_keep = nullptr, *d_seq = nullptr, *d_qual = nullptr, *d_mark = nullptr, *d_carry = nullptr;
   uint32_t *d_lineno = nullptr, *d_pos_s = nullptr, *d_pos_q = nullptr, *d_misc = nullptr, *h_tot = nullptr;
   void *d_tmp = nullptr;
-  const size_t tmp_bytes = fastx_scan_tmp_bytes(max_len);
-  auto release = [&]() {
-    pool_free(c, d_kind); pool_free(c, d_keep); pool_free(c, d_seq); pool_free(c, d_qual); pool_free(c, d_mark); pool_free(c, d_carry);
-    pool_free(c, d_lineno); pool_free(c, d_pos_s); pool_free(c, d_pos_q); pool_free(c, d_misc); pool_free(c, d_tmp);
-    if (h_tot) cudaFreeHost(h_tot);
-  };
-  cudaError_t e = pool_alloc(c, &d_kind, max_len);
-  if (e == cudaSuccess) e = pool_alloc(c, &d_keep, max_len);
-  if (e == cudaSuccess) e = pool_alloc(c, &d_pos_s, max_len * 4);
-  if (e == cudaSuccess && is_fastq) e = pool_alloc(c, &d_lineno, max_len * 4);
-  if (e == cudaSuccess && is_fastq) e = pool_alloc(c, &d_pos_q, max_len * 4);
-  if (e == cudaSuccess) e = pool_alloc(c, &d_seq, max_len + K1 + 64);
-  if (e == cudaSuccess && use_q) e = pool_alloc(c, &d_qual, max_len + K1 + 64);
-  if (e == cudaSuccess) e = pool_alloc(c, &d_mark, max_len + K1 + 64);
-  if (e == cudaSuccess) e = pool_alloc(c, &d_carry, 2 * 64);
-  if (e == cudaSuccess) e = pool_alloc(c, &d_misc, 64);   // [0..1] n_records (u64), [2..3] totals, [4] error word
-  if (e == cudaSuccess) e = pool_alloc(c, &d_tmp, tmp_bytes);
-  if (e == cudaSuccess) e = cudaHostAlloc(&h_tot, 16, cudaHostAllocDefault);
-  if (e == cudaSuccess) e = cudaMemsetAsync(d_misc, 0, 64, c->stream);
-  if (e != cudaSuccess) { release(); return cuda_fail(c, e, "cudaMalloc(fastx parse buffers)"); }
-  unsigned long long *d_nrec = reinterpret_cast<unsigned long long *>(d_misc);
-  uint32_t *d_err = d_misc + 4;
-  const uint32_t thr = std::min<uint32_t>(255u, (uint32_t)c->cfg.min_quality + 33u);
-  auto stage_chunk = [&](const Chunk &ch, Staging &st) -> kmg_status {
+  size_t tmp_bytes = 0, staged = 0;
+  uint32_t slot0 = 0, thr = 0;
+
+  FastxFeed(kmg_ctx *ctx, const uint8_t *b, const std::vector<FxChunk> &ch, bool fq)
+      : c(ctx), buf(b), chunks(ch), is_fastq(fq), use_q(fq && ctx->cfg.has_min_quality) {}
+  unsigned long long *d_nrec() const { return reinterpret_cast<unsigned long long *>(d_misc); }  // [0..1] n_records (u64)
+  uint32_t *d_err() const { return d_misc + 4; }  // [2..3] totals, [4] error word, [5] pending record start
+
+  kmg_status open() {
+    K1 = (uint64_t)c->k - 1;
+    slot0 = c->next_ascii;
+    for (auto &ch : chunks) max_len = std::max(max_len, ch.len);
+    src_pinned = is_pinned_host(buf);
+    kmg_status s = ensure_staging(c, !src_pinned, false, max_len);
+    if (s != KMG_OK) return s;
+    tmp_bytes = fastx_scan_tmp_bytes(max_len);
+    cudaError_t e = pool_alloc(c, &d_kind, max_len);
+    if (e == cudaSuccess) e = pool_alloc(c, &d_keep, max_len);
+    if (e == cudaSuccess) e = pool_alloc(c, &d_pos_s, max_len * 4);
+    if (e == cudaSuccess && is_fastq) e = pool_alloc(c, &d_lineno, max_len * 4);
+    if (e == cudaSuccess && is_fastq) e = pool_alloc(c, &d_pos_q, max_len * 4);
+    if (e == cudaSuccess) e = pool_alloc(c, &d_seq, max_len + K1 + 64);
+    if (e == cudaSuccess && use_q) e = pool_alloc(c, &d_qual, max_len + K1 + 64);
+    if (e == cudaSuccess) e = pool_alloc(c, &d_mark, max_len + K1 + 64);
+    if (e == cudaSuccess) e = pool_alloc(c, &d_carry, 2 * 64);
+    if (e == cudaSuccess) e = pool_alloc(c, &d_misc, 64);
+    if (e == cudaSuccess) e = pool_alloc(c, &d_tmp, tmp_bytes);
+    if (e == cudaSuccess) e = cudaHostAlloc(&h_tot, 16, cudaHostAllocDefault);
+    if (e == cudaSuccess) e = cudaMemsetAsync(d_misc, 0, 64, c->stream);
+    if (e != cudaSuccess) return cuda_fail(c, e, "cudaMalloc(fastx parse buffers)");
+    thr = std::min<uint32_t>(255u, (uint32_t)c->cfg.min_quality + 33u);
+    return KMG_OK;
+  }
+
+  // The first chunk continues a FASTA record that began before it (a rank's slice in a group): its last n <= k-1 bases and their
+  // record marks, and whether a header line ends right before the chunk (its record then starts with the chunk's first base).
+  kmg_status seed_carry(const uint8_t *seq, const uint8_t *mark, uint64_t n, bool pending) {
+    if (n) {
+      CU(c, cudaMemcpyAsync(d_carry + (K1 - n), seq, n, cudaMemcpyHostToDevice, c->stream));
+      CU(c, cudaMemcpyAsync(d_carry + 64 + (K1 - n), mark, n, cudaMemcpyHostToDevice, c->stream));
+    }
+    if (pending) CU(c, cudaMemsetAsync(d_err() + 1, 1, 1, c->stream));
+    prev_n = n;
+    return KMG_OK;
+  }
+
+  kmg_status stage(const FxChunk &ch, Staging &st) {
     if (st.h2d_pending) { CU(c, cudaEventSynchronize(st.h2d_done)); st.h2d_pending = false; }
     if (st.compute_pending) { CU(c, cudaStreamWaitEvent(c->copy_stream, st.compute_done, 0)); }
     const uint8_t *src = buf + ch.pos;
@@ -1530,83 +1549,129 @@ KMG_EXPORT kmg_status kmg_count_fastx(kmg_ctx *c, const uint8_t *buf, uint64_t l
     CU(c, cudaEventRecord(st.h2d_done, c->copy_stream));
     st.h2d_pending = true;
     return KMG_OK;
-  };
-  const uint32_t slot0 = c->next_ascii;
-  size_t staged = 0;
-  uint64_t prev_n = 0, bases = 0;
-  auto body = [&]() -> kmg_status {
-    for (size_t i = 0; i < chunks.size(); ++i) {
-      for (; staged < chunks.size() && staged < i + N_STAGE; ++staged) {
-        kmg_status ss = stage_chunk(chunks[staged], c->st[(slot0 + staged) % N_STAGE]);
-        if (ss != KMG_OK) return ss;
+  }
+
+  // Chunk i: parse, pack, and -- when it holds sequence bases (with the carry) -- scan(n_words_total).  *scanned tells whether it did.
+  template <class Scan>
+  kmg_status step(size_t i, Scan &&scan, bool *scanned) {
+    *scanned = false;
+    for (; staged < chunks.size() && staged < i + N_STAGE; ++staged) {
+      kmg_status ss = stage(chunks[staged], c->st[(slot0 + staged) % N_STAGE]);
+      if (ss != KMG_OK) return ss;
+    }
+    Staging &st = c->st[(slot0 + i) % N_STAGE];
+    const FxChunk &ch = chunks[i];
+    uint32_t *err = d_err();
+    CU(c, cudaStreamWaitEvent(c->stream, st.h2d_done, 0));
+    // a FASTA chunk that does not open with a header continues the previous chunk's last record: its last k-1 bases (and their
+    // record marks) are put in front, so that the windows spanning the cut are counted -- and none twice (k-1 bases hold no window)
+    const uint64_t carry = (!is_fastq && buf[ch.pos] != '>') ? std::min<uint64_t>(K1, prev_n) : 0;
+    CU(c, cudaMemsetAsync(d_mark, 0, ch.len + K1 + 64, c->stream));
+    CU(c, cudaMemsetAsync(err, 0, 4, c->stream));
+    if (carry) {
+      CU(c, cudaMemcpyAsync(d_seq, d_carry + (K1 - carry), carry, cudaMemcpyDeviceToDevice, c->stream));
+      CU(c, cudaMemcpyAsync(d_mark, d_carry + 64 + (K1 - carry), carry, cudaMemcpyDeviceToDevice, c->stream));
+    }
+    CU(c, launch_fastx_parse(st.d_seq, ch.len, is_fastq, d_kind, d_keep, d_lineno, d_pos_s, d_pos_q, d_tmp, tmp_bytes, carry, d_seq, d_qual, d_mark,
+                             d_nrec(), err, h_tot, c->stream));
+    CU(c, cudaStreamSynchronize(c->stream));
+    const uint32_t total_s = h_tot[0], total_q = h_tot[1], perr = h_tot[2];
+    if (perr & 1u) return fail(c, KMG_ERR_PARSE, "FASTQ record does not start with '@' (multi-line FASTQ is not handled by the device parser)");
+    if (perr & 2u) return fail(c, KMG_ERR_PARSE, "FASTQ record without a '+' separator line where one is expected");
+    if (is_fastq && total_s != total_q) return fail(c, KMG_ERR_PARSE, "sequence and quality lengths differ");
+    // a record whose header closed the previous chunk starts with this chunk's first base (the scatter below may raise the flag anew)
+    if (!is_fastq && total_s) CU(c, launch_fastx_apply_pending(err + 1, d_mark + carry, c->stream));
+    CU(c, launch_fastx_scatter(st.d_seq, ch.len, is_fastq, d_kind, d_lineno, d_keep, d_pos_s, d_pos_q, carry, total_s, d_seq, use_q ? d_qual : nullptr,
+                               d_mark, d_nrec(), err, c->stream));
+    CU(c, cudaEventRecord(st.compute_done, c->stream));  // the raw chunk has been consumed
+    st.compute_pending = true;
+    const uint64_t n = carry + total_s;
+    bases += total_s;
+    prev_n = n;
+    if (!n) return KMG_OK;
+    const uint64_t n_words_total = round_up((n + 31) / 32, TILE_WORDS);
+    kmg_status ps = ensure_packed(c, n_words_total);
+    if (ps != KMG_OK) return ps;
+    CU(c, launch_ingest(d_seq, use_q ? d_qual : nullptr, n, thr, n_words_total, c->d_bases, c->d_valid, c->stream));
+    CU(c, launch_marks_to_bits(d_mark, n, n_words_total, c->d_start, c->stream));
+    if (!is_fastq) {  // keep the tail for the next chunk
+      const uint64_t t = std::min<uint64_t>(K1, n);
+      if (t) {
+        CU(c, cudaMemcpyAsync(d_carry + (K1 - t), d_seq + (n - t), t, cudaMemcpyDeviceToDevice, c->stream));
+        CU(c, cudaMemcpyAsync(d_carry + 64 + (K1 - t), d_mark + (n - t), t, cudaMemcpyDeviceToDevice, c->stream));
       }
-      Staging &st = c->st[(slot0 + i) % N_STAGE];
-      const Chunk &ch = chunks[i];
-      CU(c, cudaStreamWaitEvent(c->stream, st.h2d_done, 0));
-      // a FASTA chunk that does not open with a header continues the previous chunk's last record: its last k-1 bases (and their
-      // record marks) are put in front, so that the windows spanning the cut are counted -- and none twice (k-1 bases hold no window)
-      const uint64_t carry = (!is_fastq && i > 0 && buf[ch.pos] != '>') ? std::min<uint64_t>(K1, prev_n) : 0;
-      CU(c, cudaMemsetAsync(d_mark, 0, ch.len + K1 + 64, c->stream));
-      CU(c, cudaMemsetAsync(d_err, 0, 4, c->stream));
-      if (carry) {
-        CU(c, cudaMemcpyAsync(d_seq, d_carry + (K1 - carry), carry, cudaMemcpyDeviceToDevice, c->stream));
-        CU(c, cudaMemcpyAsync(d_mark, d_carry + 64 + (K1 - carry), carry, cudaMemcpyDeviceToDevice, c->stream));
-      }
-      CU(c, launch_fastx_parse(st.d_seq, ch.len, is_fastq, d_kind, d_keep, d_lineno, d_pos_s, d_pos_q, d_tmp, tmp_bytes, carry, d_seq, d_qual, d_mark,
-                               d_nrec, d_err, h_tot, c->stream));
+    }
+    *scanned = true;
+    ps = scan(n_words_total);
+    if (ps != KMG_OK) return ps;
+    if (is_fastq && use_q) {  // a quality mismatch inside a record shows up at the next record start (checked in the scatter)
+      uint32_t e2 = 0;
+      CU(c, cudaMemcpyAsync(&e2, err, 4, cudaMemcpyDeviceToHost, c->stream));
       CU(c, cudaStreamSynchronize(c->stream));
-      const uint32_t total_s = h_tot[0], total_q = h_tot[1], err = h_tot[2];
-      if (err & 1u) return fail(c, KMG_ERR_PARSE, "FASTQ record does not start with '@' (multi-line FASTQ is not handled by the device parser)");
-      if (err & 2u) return fail(c, KMG_ERR_PARSE, "FASTQ record without a '+' separator line where one is expected");
-      if (is_fastq && total_s != total_q) return fail(c, KMG_ERR_PARSE, "sequence and quality lengths differ");
-      // a record whose header closed the previous chunk starts with this chunk's first base (the scatter below may raise the flag anew)
-      if (!is_fastq && total_s) CU(c, launch_fastx_apply_pending(d_err + 1, d_mark + carry, c->stream));
-      CU(c, launch_fastx_scatter(st.d_seq, ch.len, is_fastq, d_kind, d_lineno, d_keep, d_pos_s, d_pos_q, carry, total_s, d_seq, use_q ? d_qual : nullptr,
-                                 d_mark, d_nrec, d_err, c->stream));
-      CU(c, cudaEventRecord(st.compute_done, c->stream));  // the raw chunk has been consumed
-      st.compute_pending = true;
-      const uint64_t n = carry + total_s;
-      bases += total_s;
-      if (n) {
-        const uint64_t n_words_total = round_up((n + 31) / 32, TILE_WORDS);
-        kmg_status ps = ensure_packed(c, n_words_total);
-        if (ps != KMG_OK) return ps;
-        CU(c, launch_ingest(d_seq, use_q ? d_qual : nullptr, n, thr, n_words_total, c->d_bases, c->d_valid, c->stream));
-        CU(c, launch_marks_to_bits(d_mark, n, n_words_total, c->d_start, c->stream));
-        if (!is_fastq) {  // keep the tail for the next chunk
-          const uint64_t t = std::min<uint64_t>(K1, n);
-          if (t) {
-            CU(c, cudaMemcpyAsync(d_carry + (K1 - t), d_seq + (n - t), t, cudaMemcpyDeviceToDevice, c->stream));
-            CU(c, cudaMemcpyAsync(d_carry + 64 + (K1 - t), d_mark + (n - t), t, cudaMemcpyDeviceToDevice, c->stream));
-          }
-        }
-        ps = scan_packed(c, n_words_total, true);
-        if (ps != KMG_OK) return ps;
-        if (is_fastq && use_q) {  // a quality mismatch inside a record shows up at the next record start (checked in the scatter)
-          uint32_t e2 = 0;
-          CU(c, cudaMemcpyAsync(&e2, d_err, 4, cudaMemcpyDeviceToHost, c->stream));
-          CU(c, cudaStreamSynchronize(c->stream));
-          if (e2 & 8u) return fail(c, KMG_ERR_PARSE, "sequence and quality lengths differ");
-        }
-      }
-      prev_n = n;
+      if (e2 & 8u) return fail(c, KMG_ERR_PARSE, "sequence and quality lengths differ");
     }
     return KMG_OK;
-  };
-  s = body();
-  unsigned long long n_rec = 0;
-  if (s == KMG_OK) {
-    e = cudaMemcpyAsync(&n_rec, d_nrec, 8, cudaMemcpyDeviceToHost, c->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-    if (e != cudaSuccess) s = cuda_fail(c, e, "fastx record count");
-  } else {
-    cudaStreamSynchronize(c->stream); cudaStreamSynchronize(c->copy_stream);
   }
-  c->next_ascii = (slot0 + (uint32_t)chunks.size()) % N_STAGE;
-  for (auto &st : c->st) if (st.h2d_pending && src_pinned) { cudaEventSynchronize(st.h2d_done); st.h2d_pending = false; }
-  release();
+
+  // Records (header lines) the parsed chunks held.
+  kmg_status records(uint64_t *n) {
+    unsigned long long h = 0;
+    CU(c, cudaMemcpyAsync(&h, d_nrec(), 8, cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaStreamSynchronize(c->stream));
+    *n = h;
+    return KMG_OK;
+  }
+
+  // After the last step (or a failed one): the caller's buffer must be reusable when the call returns.
+  void close(bool failed) {
+    if (failed) { cudaStreamSynchronize(c->stream); cudaStreamSynchronize(c->copy_stream); }
+    c->next_ascii = (slot0 + (uint32_t)chunks.size()) % N_STAGE;
+    for (auto &st : c->st) if (st.h2d_pending && src_pinned) { cudaEventSynchronize(st.h2d_done); st.h2d_pending = false; }
+    pool_free(c, d_kind); pool_free(c, d_keep); pool_free(c, d_seq); pool_free(c, d_qual); pool_free(c, d_mark); pool_free(c, d_carry);
+    pool_free(c, d_lineno); pool_free(c, d_pos_s); pool_free(c, d_pos_q); pool_free(c, d_misc); pool_free(c, d_tmp);
+    if (h_tot) cudaFreeHost(h_tot);
+    h_tot = nullptr;
+  }
+};
+
+}  // namespace
+
+// FASTA / FASTQ file image (HOST bytes, e.g. an mmap'ed file: src/mmap.rs:33-71) -> counts, with the records found ON THE DEVICE:
+// the raw bytes go over PCIe in chunks cut at line (FASTA) / record (FASTQ) boundaries, a few small kernels classify the lines,
+// compact sequence (+ quality) bytes, mark the record starts, and the usual ingest + scan follow.  Replaces reader::read /
+// read_with_quality (src/reader.rs:82-247: whole file -> Vec<Record> -> Vec<SequenceWithQuality>, two host copies) for
+// well-formed input; multi-line FASTQ, or a line longer than a chunk, is refused with KMG_ERR_PARSE -- nothing has been
+// counted then only if it happens in the first chunk, so callers fall back to kmg_parse_fastx + kmg_count_ascii after kmg_reset.
+KMG_EXPORT kmg_status kmg_count_fastx(kmg_ctx *c, const uint8_t *buf, uint64_t len, int is_fastq, uint64_t *n_records_out) {
+  if (!c || (len && !buf)) return KMG_ERR_INVALID_ARG;
+  if (c->shm) return fail(c, KMG_ERR_STATE, "context belongs to a shard group: feed it with kmg_shard_count_fastx / kmg_shard_count_ascii(_device)");
+  if (n_records_out) *n_records_out = 0;
+  if (len == 0) return KMG_OK;
+  const uint8_t marker = is_fastq ? '@' : '>';
+  if (buf[0] != marker) return fail(c, KMG_ERR_PARSE, is_fastq ? "FASTQ record does not start with '@' (record 0)" : "FASTA record does not start with '>' (record 0)");
+  CU(c, cudaSetDevice(c->device));
+  const bool use_q = is_fastq && c->cfg.has_min_quality;
+  std::vector<FxChunk> chunks;
+  kmg_status s = plan_fastx_chunks(c, buf, len, 0, len, is_fastq, std::min<uint64_t>(c->batch_bases, 1ull << 30), chunks);
   if (s != KMG_OK) return s;
-  c->n_records += n_rec; c->n_bases += bases;
+  uint64_t max_len = 0;
+  for (auto &ch : chunks) max_len = std::max(max_len, ch.len);
+  if (max_len >= (1ull << 32)) return fail(c, KMG_ERR_INVALID_ARG, "staging chunks must stay below 4 GiB");
+  // ---- plan the table / partitions for the whole file
+  if (use_q && !c->cfg.expected_distinct && c->mode == kmg_ctx::MODE_UNDECIDED && !c->use_dense) c->plan_scale = (double)len / (double)chunks[0].len;
+  else s = decide_mode(c, is_fastq ? len / 2 : len);
+  if (s != KMG_OK) return s;
+  FastxFeed feed(c, buf, chunks, is_fastq);
+  s = feed.open();
+  uint64_t n_rec = 0;
+  for (size_t i = 0; s == KMG_OK && i < chunks.size(); ++i) {
+    bool scanned = false;
+    s = feed.step(i, [&](uint64_t n_words_total) { return scan_packed(c, n_words_total, true); }, &scanned);
+  }
+  if (s == KMG_OK) s = feed.records(&n_rec);
+  feed.close(s != KMG_OK);
+  if (s != KMG_OK) return s;
+  c->n_records += n_rec; c->n_bases += feed.bases;
   if (n_records_out) *n_records_out = n_rec;
   return KMG_OK;
 }
@@ -1840,6 +1905,8 @@ struct ShardRankSlot {
   PeerBuf text;
   uint64_t text_bounds[SHARD_MAX_WORLD + 1];
   uint64_t text_piece[3], text_written;
+  // kmg_shard_count_fastx: the image's length and rank cuts as this rank computed them, its chunk plan's status, its records
+  uint64_t fastx_len, fastx_cuts[SHARD_MAX_WORLD + 1], fastx_status, fastx_records;
 };
 struct ShardShm {
   uint32_t ready, world;
@@ -2269,6 +2336,122 @@ KMG_EXPORT kmg_status kmg_shard_count_ascii(kmg_ctx *c, const uint8_t *seq, cons
   if (src_pinned)
     for (auto &st : c->st)
       if (st.h2d_pending) { CU(c, cudaEventSynchronize(st.h2d_done)); st.h2d_pending = false; }
+  return KMG_OK;
+}
+
+namespace {
+
+// Where a rank's slice of a file image begins, given t = len * r / W: the first line start at or after t (FASTA), or the first
+// record start at or after t within FASTQ_SYNC_LINES lines (FASTQ).  len when the image ends first; false: no record start found.
+bool fastx_rank_cut(const uint8_t *buf, uint64_t len, uint64_t t, bool is_fastq, uint64_t *cut) {
+  auto next_line = [&](uint64_t p) -> uint64_t {
+    const void *nl = memchr(buf + p, '\n', (size_t)(len - p));
+    return nl ? (uint64_t)((const uint8_t *)nl - buf) + 1 : len;
+  };
+  uint64_t p = (t == 0 || t >= len || buf[t - 1] == '\n') ? std::min(t, len) : next_line(t);
+  for (int tries = 0; tries < FASTQ_SYNC_LINES; ++tries) {
+    if (!is_fastq || p >= len || fastq_record_start(buf, len, p)) { *cut = p; return true; }
+    p = next_line(p);
+  }
+  return false;
+}
+
+// The carry of a FASTA slice that begins at the line start p inside a record: the last bases (at most k-1) of that record before
+// p, collected backward line by line with the parser's trim_end (' ' and \t..\r), stopping at the record's header.  A carry that
+// starts at the record's first base carries its record mark; *pending: the record's header is the last line before p that is not
+// blank, so the record starts with the first base of the slice.
+void fasta_carry_at(const uint8_t *buf, uint64_t p, uint64_t K1, std::vector<uint8_t> &seq, std::vector<uint8_t> &mark, bool *pending) {
+  seq.clear();
+  bool at_header = false;
+  for (uint64_t le = p; le > 0 && seq.size() < K1;) {  // the line [ls, le), its '\n' at le - 1
+    const void *nl = le >= 2 ? memrchr(buf, '\n', (size_t)(le - 1)) : nullptr;
+    const uint64_t ls = nl ? (uint64_t)((const uint8_t *)nl - buf) + 1 : 0;
+    if (buf[ls] == '>') { at_header = true; break; }
+    uint64_t t = le;
+    while (t > ls && (buf[t - 1] == ' ' || (buf[t - 1] >= 9 && buf[t - 1] <= 13))) --t;
+    const uint64_t take = std::min<uint64_t>(t - ls, K1 - seq.size());
+    seq.insert(seq.begin(), buf + t - take, buf + t);
+    le = ls;
+  }
+  mark.assign(seq.size(), 0);
+  if (at_header && !seq.empty()) mark[0] = 1;
+  *pending = at_header && seq.empty();
+}
+
+}  // namespace
+
+// One file image counted by the whole group: every rank passes the SAME image and parses only its own slice of it on the device,
+// every parsed chunk is one fused scatter + exchange round.  Slices are cut at line (FASTA) / record (FASTQ) starts that every rank
+// computes from the same bytes; a FASTA slice that begins inside a record gets that record's last k-1 bases in front of its first
+// chunk (collected on the host), so every window is counted by exactly one rank: the one that holds its last base.
+KMG_EXPORT kmg_status kmg_shard_count_fastx(kmg_ctx *c, const uint8_t *buf, uint64_t len, int is_fastq, uint64_t *n_records_out) {
+  if (!c) return KMG_ERR_INVALID_ARG;
+  if (!c->shm) return kmg_count_fastx(c, buf, len, is_fastq, n_records_out);
+  if (n_records_out) *n_records_out = 0;
+  if (len && !buf) return shard_fail(c, KMG_ERR_INVALID_ARG, "buf is NULL");
+  if (len && buf[0] != (is_fastq ? '@' : '>'))
+    return shard_fail(c, KMG_ERR_PARSE, is_fastq ? "FASTQ record does not start with '@' (record 0)" : "FASTA record does not start with '>' (record 0)");
+  SCU(c, cudaSetDevice(c->device));
+  ShardShm *S = c->shm;
+  const uint32_t W = c->sh_world, me = c->sh_rank;
+  const uint64_t K1 = (uint64_t)c->k - 1;
+  // ---- rank cuts (every rank computes all of them) and this rank's chunks: raw chunk + carry <= batch_bases bases, one round each
+  uint64_t cuts[SHARD_MAX_WORLD + 1];
+  cuts[0] = 0; cuts[W] = len;
+  for (uint32_t r = 1; r < W; ++r)
+    if (!fastx_rank_cut(buf, len, len / W * r + len % W * r / W, is_fastq, &cuts[r]))
+      return shard_fail(c, KMG_ERR_PARSE, "no FASTQ record start found near a rank cut (multi-line FASTQ? use the host splitter)");
+  const uint64_t begin = cuts[me], end = cuts[me + 1];
+  std::vector<FxChunk> chunks;
+  const kmg_status plan = plan_fastx_chunks(c, buf, len, begin, end, is_fastq, std::min<uint64_t>(c->batch_bases - K1, 1ull << 30), chunks);
+  // ---- the ranks compare their images (length and cuts) and plans, and agree on the number of rounds
+  ShardRankSlot &mine = S->ranks[me];
+  mine.fastx_len = len;
+  memcpy(mine.fastx_cuts, cuts, (W + 1) * 8);
+  mine.fastx_status = (uint64_t)plan;
+  mine.summary[7] = plan == KMG_OK ? chunks.size() : 0;
+  SB(c);
+  bool same = true, planned = true;
+  uint64_t rounds = 0;
+  for (uint32_t r = 0; r < W; ++r) {
+    const ShardRankSlot &o = S->ranks[r];
+    same = same && o.fastx_len == len && memcmp(o.fastx_cuts, cuts, (W + 1) * 8) == 0;
+    planned = planned && o.fastx_status == (uint64_t)KMG_OK;
+    rounds = std::max<uint64_t>(rounds, o.summary[7]);
+  }
+  SB(c);
+  if (!same) return shard_fail(c, KMG_ERR_INVALID_ARG, "ranks passed different file images (pass the same whole image on every rank)");
+  if (!planned)
+    return shard_fail(c, KMG_ERR_PARSE, plan != KMG_OK ? c->err : "another rank's slice cannot be cut into staging chunks (a line longer than a chunk, or multi-line FASTQ)");
+  // ---- rounds: parse -> pack -> fused scatter + exchange; a rank without chunks left takes part with empty rounds
+  FastxFeed feed(c, buf, chunks, is_fastq);
+  kmg_status s = KMG_OK;
+  if (!chunks.empty()) {
+    s = feed.open();
+    if (s == KMG_OK && !is_fastq && buf[begin] != '>') {
+      std::vector<uint8_t> cseq, cmark;
+      bool pending = false;
+      fasta_carry_at(buf, begin, K1, cseq, cmark, &pending);
+      s = feed.seed_carry(cseq.data(), cmark.data(), cseq.size(), pending);
+    }
+  }
+  for (uint64_t i = 0; s == KMG_OK && i < rounds; ++i) {
+    bool scanned = false;
+    if (i < chunks.size()) s = feed.step(i, [&](uint64_t n_words_total) { return shard_scan_round(c, n_words_total, true); }, &scanned);
+    if (s == KMG_OK && !scanned) s = shard_scan_round(c, 0, false);
+  }
+  uint64_t n_rec = 0;
+  if (s == KMG_OK && !chunks.empty()) s = feed.records(&n_rec);
+  if (!chunks.empty()) feed.close(s != KMG_OK);
+  if (s != KMG_OK) return shard_fail(c, s, c->err);
+  // ---- records of the whole image, on every rank
+  mine.fastx_records = n_rec;
+  SB(c);
+  uint64_t total = 0;
+  for (uint32_t r = 0; r < W; ++r) total += S->ranks[r].fastx_records;
+  SB(c);
+  c->n_records += n_rec; c->n_bases += feed.bases;
+  if (n_records_out) *n_records_out = total;
   return KMG_OK;
 }
 

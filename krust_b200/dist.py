@@ -265,6 +265,17 @@ class ShardedKmerCounter:
             self.count(torch.from_numpy(seq).to(dev, non_blocking=True), torch.from_numpy(np.asarray(offsets).astype(np.int64)).to(dev),
                        None if qual is None else torch.from_numpy(qual).to(dev, non_blocking=True), expected_keys_per_rank=expected_keys_per_rank)
 
+    def count_file_image(self, image, is_fastq: bool) -> int:
+        """The WHOLE FASTA / FASTQ file image, the same on every rank (e.g. each rank's mmap of the file): kmg_shard_count_fastx
+        parses only this rank's slice of it on the device.  Returns the records of the whole image.  At world 1 it is count_fastx."""
+        if self.world == 1:
+            return self.engine.counter.count_fastx(image, is_fastq)
+        if not self.fused:
+            raise RuntimeError("count_file_image needs the fused shard group (kmg_shard_*)")
+        if not self.engine.joined:
+            self._join(max(len(image) // 2 if is_fastq else len(image), 1))   # the size hint kmg_count_fastx plans with
+        return self.engine.counter.shard_count_fastx(image, is_fastq)
+
     def finalize(self) -> dict:
         """Global summary: sums over shards (shards are disjoint), max of max_count."""
         if self.fused and self.engine.joined:
