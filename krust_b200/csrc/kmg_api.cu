@@ -122,6 +122,8 @@ struct kmg_ctx {
   uint64_t sh_recv_entries = 0;
   uint64_t *sh_peer[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};  // every rank's send buffer as seen from here
   bool sh_peer_ipc[8] = {false, false, false, false, false, false, false, false};
+  int sh_pid[8] = {}, sh_device[8] = {};  // every rank's process and device (kmg_shard_join)
+  uint64_t sh_gathers = 0;                // shard_allgather calls since kmg_shard_join: the parity picks the post area's half
   uint64_t sh_sent = 0, sh_recv_keys = 0, sh_rounds = 0, sh_exact_rounds = 0;
   std::vector<uint64_t> sh_hist_vals, sh_hist_freqs;  // merged histogram of the last kmg_shard_histogram
   int feed_kind = 0;        // partitioned path: 1 = runs binned by this context's own coarse function, 2 = blocks adopted from a sender
@@ -1105,20 +1107,22 @@ kmg_status scan_packed(kmg_ctx *c, uint64_t n_words_total, bool has_start) {
   return KMG_OK;
 }
 
-// ingest raw ASCII already on the device into the packed buffers and scan it.
-// d_starts[n_starts] are byte offsets (minus base_offset) of record starts inside this chunk.
-kmg_status count_device_chunk(kmg_ctx *c, const uint8_t *d_seq, const uint8_t *d_qual, const uint64_t *d_starts,
-                              uint64_t n_starts, uint64_t base_offset, uint64_t n_bytes) {
-  if (n_bytes == 0) return KMG_OK;
-  const uint64_t n_words_total = round_up((n_bytes + 31) / 32, TILE_WORDS);
-  kmg_status s = ensure_packed(c, n_words_total);
+// The lowest quality byte a base needs to count under the context's filter: min_quality + 33, saturating (src/run.rs:538).
+uint32_t quality_threshold(const kmg_ctx *c) { return std::min<uint32_t>(255u, (uint32_t)c->cfg.min_quality + 33u); }
+
+// Ingest n_bytes > 0 of raw ASCII already on the device into the context's packed buffers, with the start bits of d_starts[n_starts]
+// (byte offsets, minus base_offset, of record starts inside these bytes).  The scan over them is the caller's.
+kmg_status pack_device_ascii(kmg_ctx *c, const uint8_t *d_seq, const uint8_t *d_qual, const uint64_t *d_starts, uint64_t n_starts,
+                             uint64_t base_offset, uint64_t n_bytes, uint64_t *n_words_total, bool *has_start) {
+  const uint64_t words = round_up((n_bytes + 31) / 32, TILE_WORDS);
+  kmg_status s = ensure_packed(c, words);
   if (s != KMG_OK) return s;
   const bool use_q = c->cfg.has_min_quality && d_qual != nullptr;
-  const uint32_t thr = std::min<uint32_t>(255u, (uint32_t)c->cfg.min_quality + 33u);  // saturating_add (src/run.rs:538)
-  CU(c, launch_ingest(d_seq, use_q ? d_qual : nullptr, n_bytes, thr, n_words_total, c->d_bases, c->d_valid, c->stream));
-  const bool has_start = d_starts != nullptr && n_starts > 0;
-  if (has_start) CU(c, launch_start_bits(d_starts, n_starts, base_offset, n_bytes, n_words_total, c->d_start, c->stream));
-  return scan_packed(c, n_words_total, has_start);
+  CU(c, launch_ingest(d_seq, use_q ? d_qual : nullptr, n_bytes, quality_threshold(c), words, c->d_bases, c->d_valid, c->stream));
+  *has_start = d_starts != nullptr && n_starts > 0;
+  if (*has_start) CU(c, launch_start_bits(d_starts, n_starts, base_offset, n_bytes, words, c->d_start, c->stream));
+  *n_words_total = words;
+  return KMG_OK;
 }
 
 kmg_status ensure_staging(kmg_ctx *c, bool need_pinned, bool need_qual, uint64_t need_bytes) {
@@ -1345,42 +1349,50 @@ KMG_EXPORT kmg_status kmg_count_ascii_device(kmg_ctx *c, const uint8_t *d_seq, c
   if (n_bytes && !d_seq) return fail(c, KMG_ERR_INVALID_ARG, "d_seq is NULL");
   if (((uintptr_t)d_seq & 15) || ((uintptr_t)d_qual & 15)) return fail(c, KMG_ERR_INVALID_ARG, "d_seq / d_qual must be 16-byte aligned");
   CU(c, cudaSetDevice(c->device));
-  // offsets[0] (== 0) needs no start bit; a single record needs none at all
-  kmg_status s = count_device_chunk(c, d_seq, d_qual, n_records > 1 ? d_offsets : nullptr, n_records, 0, n_bytes);
-  if (s != KMG_OK) return s;
+  if (n_bytes) {
+    uint64_t n_words_total = 0;
+    bool has_start = false;
+    // offsets[0] (== 0) needs no start bit; a single record needs none at all
+    kmg_status s = pack_device_ascii(c, d_seq, d_qual, n_records > 1 ? d_offsets : nullptr, n_records, 0, n_bytes, &n_words_total, &has_start);
+    if (s == KMG_OK) s = scan_packed(c, n_words_total, has_start);
+    if (s != KMG_OK) return s;
+  }
   c->n_records += n_records; c->n_bases += n_bytes;
   return KMG_OK;
 }
 
-KMG_EXPORT kmg_status kmg_count_ascii(kmg_ctx *c, const uint8_t *seq, const uint8_t *qual, const uint64_t *offsets, uint64_t n_records) {
-  if (!c) return KMG_ERR_INVALID_ARG;
-  if (c->shm) return fail(c, KMG_ERR_STATE, "context belongs to a shard group: feed it with kmg_shard_count_ascii(_device)");
-  if (n_records == 0) return KMG_OK;
-  if (!offsets || !seq) {
-    if (offsets && offsets[n_records] == offsets[0]) { c->n_records += n_records; return KMG_OK; }
-    return fail(c, KMG_ERR_INVALID_ARG, "seq / offsets must not be NULL");
-  }
+
+namespace {
+
+// The layout checks of kmg_count_ascii and kmg_shard_count_ascii.  A call without records, or with only empty records and no seq,
+// passes with nothing to stage.
+kmg_status check_ascii_layout(kmg_ctx *c, const uint8_t *seq, const uint64_t *offsets, uint64_t n_records) {
+  if (n_records == 0 || (!seq && offsets && offsets[n_records] == offsets[0])) return KMG_OK;
+  if (!offsets || !seq) return fail(c, KMG_ERR_INVALID_ARG, "seq / offsets must not be NULL");
   for (uint64_t r = 0; r < n_records; ++r)
     if (offsets[r + 1] < offsets[r]) return fail(c, KMG_ERR_INVALID_ARG, "offsets must be non-decreasing");
-  CU(c, cudaSetDevice(c->device));
-  const uint64_t begin = offsets[0], end = offsets[n_records];
-  const bool use_q = c->cfg.has_min_quality && qual != nullptr;
-  const bool src_pinned = is_pinned_host(seq + begin) && (!use_q || is_pinned_host(qual + begin));
-  kmg_status s = KMG_OK;
-  if (use_q && !c->cfg.expected_distinct && c->mode == kmg_ctx::MODE_UNDECIDED && !c->use_dense)
-    c->plan_scale = (double)(end - begin) / (double)std::min<uint64_t>(end - begin, c->batch_bases);  // decided after the first chunk's ingest (scan_packed)
-  else s = decide_mode(c, end - begin);  // plan for the whole call, not for its first staging chunk
-  if (s != KMG_OK) return s;
-  s = ensure_staging(c, !src_pinned, use_q, end - begin);
-  if (s != KMG_OK) return s;
-  const uint64_t K1 = (uint64_t)c->k - 1;
-  const uint64_t B = c->batch_bases;  // bytes per chunk including the k-1 overlap
-  const uint64_t step = B - K1;
-  // chunk plan first, then a software pipeline: the H2D copy of chunk i+1 is queued BEFORE chunk i is processed
-  // (processing contains host syncs), so copies overlap the kernels of the previous chunk.
+  return KMG_OK;
+}
+
+// The host ASCII feed of one checked call over the context's staging ring: seq[offsets[0], offsets[n_records]) in chunks of at most
+// batch_bases bytes that overlap by k-1, each with the starts of the records that begin strictly inside it.  The H2D copies run up
+// to N_STAGE - 1 chunks ahead of the kernels (processing contains host syncs).  step() packs a chunk and hands it to the caller's
+// scan (scan_packed on one context, shard_scan_round in a group).
+struct AsciiFeed {
   struct Chunk { uint64_t pos, len, r_lo, nrec; };
+  kmg_ctx *c;
+  const uint8_t *seq, *qual;
+  const uint64_t *offsets;
+  uint64_t begin, end;
+  bool use_q, src_pinned = false;
   std::vector<Chunk> chunks;
-  {
+  uint32_t slot0 = 0;
+  size_t staged = 0;
+
+  AsciiFeed(kmg_ctx *ctx, const uint8_t *s, const uint8_t *q, const uint64_t *off, uint64_t n_records)
+      : c(ctx), seq(s), qual(q), offsets(off), begin(n_records ? off[0] : 0), end(n_records ? off[n_records] : 0),
+        use_q(ctx->cfg.has_min_quality && q != nullptr) {
+    const uint64_t K1 = (uint64_t)c->k - 1, B = c->batch_bases, step = B - K1;  // B: bytes per chunk including the k-1 overlap
     uint64_t r_lo = 0;
     for (uint64_t pos = begin; pos < end; pos += step) {
       const uint64_t len = std::min<uint64_t>(B, end - pos);
@@ -1391,7 +1403,15 @@ KMG_EXPORT kmg_status kmg_count_ascii(kmg_ctx *c, const uint8_t *seq, const uint
       chunks.push_back(Chunk{pos, len, r_lo, r_hi - r_lo});
     }
   }
-  auto stage_chunk = [&](const Chunk &ch, Staging &st) -> kmg_status {
+
+  kmg_status open() {
+    slot0 = c->next_ascii;
+    src_pinned = end > begin && is_pinned_host(seq + begin) && (!use_q || is_pinned_host(qual + begin));
+    return ensure_staging(c, !src_pinned, use_q, end - begin);
+  }
+
+  // chunk i lives in ring slot (slot0 + i) % N_STAGE; reusing a slot waits for its previous chunk's compute_done
+  kmg_status stage(const Chunk &ch, Staging &st) {
     if (st.h2d_pending) { CU(c, cudaEventSynchronize(st.h2d_done)); st.h2d_pending = false; }
     if (st.compute_pending) { CU(c, cudaStreamWaitEvent(c->copy_stream, st.compute_done, 0)); }
     kmg_status es = ensure_offsets(c, st, ch.nrec);
@@ -1411,32 +1431,36 @@ KMG_EXPORT kmg_status kmg_count_ascii(kmg_ctx *c, const uint8_t *seq, const uint
     CU(c, cudaEventRecord(st.h2d_done, c->copy_stream));
     st.h2d_pending = true;
     return KMG_OK;
-  };
-  // ring of N_STAGE slots: chunk i lives in slot (slot0 + i) % N_STAGE, and chunks i+1 .. i+N_STAGE-1 are already
-  // queued on the copy stream while chunk i is processed (slot reuse waits for the previous user's compute_done)
-  const uint32_t slot0 = c->next_ascii;
-  size_t staged = 0;
-  for (size_t i = 0; i < chunks.size(); ++i) {
-    for (; staged < chunks.size() && staged < i + N_STAGE; ++staged)
-      if ((s = stage_chunk(chunks[staged], c->st[(slot0 + staged) % N_STAGE])) != KMG_OK) return s;
+  }
+
+  template <class Scan>
+  kmg_status step(size_t i, Scan &&scan) {
+    for (; staged < chunks.size() && staged < i + N_STAGE; ++staged) {
+      kmg_status ss = stage(chunks[staged], c->st[(slot0 + staged) % N_STAGE]);
+      if (ss != KMG_OK) return ss;
+    }
     Staging &st = c->st[(slot0 + i) % N_STAGE];
     const Chunk &ch = chunks[i];
     CU(c, cudaStreamWaitEvent(c->stream, st.h2d_done, 0));
-    s = count_device_chunk(c, st.d_seq, use_q ? st.d_qual : nullptr, ch.nrec ? st.d_off : nullptr, ch.nrec, ch.pos, ch.len);
+    uint64_t n_words_total = 0;
+    bool has_start = false;
+    kmg_status s = pack_device_ascii(c, st.d_seq, use_q ? st.d_qual : nullptr, ch.nrec ? st.d_off : nullptr, ch.nrec, ch.pos, ch.len,
+                                     &n_words_total, &has_start);
     if (s != KMG_OK) return s;
-    CU(c, cudaEventRecord(st.compute_done, c->stream));
+    CU(c, cudaEventRecord(st.compute_done, c->stream));  // the staging slot is free once the chunk is packed
     st.compute_pending = true;
+    return scan(n_words_total, has_start);
   }
-  c->next_ascii = (slot0 + (uint32_t)chunks.size()) % N_STAGE;
-  c->n_records += n_records; c->n_bases += end - begin;
-  if (src_pinned)  // the copies read the CALLER's buffer: it must be reusable when this call returns
-    for (auto &st : c->st)
-      if (st.h2d_pending) { CU(c, cudaEventSynchronize(st.h2d_done)); st.h2d_pending = false; }
-  return KMG_OK;
-}
 
-
-namespace {
+  // After the last step: the copies read the CALLER's buffer when it is pinned, and it must be reusable when the call returns.
+  kmg_status close() {
+    c->next_ascii = (slot0 + (uint32_t)chunks.size()) % N_STAGE;
+    if (src_pinned)
+      for (auto &st : c->st)
+        if (st.h2d_pending) { CU(c, cudaEventSynchronize(st.h2d_done)); st.h2d_pending = false; }
+    return KMG_OK;
+  }
+};
 
 constexpr int FASTQ_SYNC_LINES = 64;  // lines searched for a FASTQ record start at a chunk end (backward) or a rank cut (forward)
 
@@ -1523,7 +1547,7 @@ struct FastxFeed {
     if (e == cudaSuccess) e = cudaHostAlloc(&h_tot, 16, cudaHostAllocDefault);
     if (e == cudaSuccess) e = cudaMemsetAsync(d_misc, 0, 64, c->stream);
     if (e != cudaSuccess) return cuda_fail(c, e, "cudaMalloc(fastx parse buffers)");
-    thr = std::min<uint32_t>(255u, (uint32_t)c->cfg.min_quality + 33u);
+    thr = quality_threshold(c);
     return KMG_OK;
   }
 
@@ -1635,6 +1659,26 @@ struct FastxFeed {
 };
 
 }  // namespace
+
+KMG_EXPORT kmg_status kmg_count_ascii(kmg_ctx *c, const uint8_t *seq, const uint8_t *qual, const uint64_t *offsets, uint64_t n_records) {
+  if (!c) return KMG_ERR_INVALID_ARG;
+  if (c->shm) return fail(c, KMG_ERR_STATE, "context belongs to a shard group: feed it with kmg_shard_count_ascii(_device)");
+  kmg_status s = check_ascii_layout(c, seq, offsets, n_records);
+  if (s != KMG_OK) return s;
+  if (n_records == 0 || !seq) { c->n_records += n_records; return KMG_OK; }
+  CU(c, cudaSetDevice(c->device));
+  AsciiFeed feed(c, seq, qual, offsets, n_records);
+  const uint64_t bases = feed.end - feed.begin;
+  if (feed.use_q && !c->cfg.expected_distinct && c->mode == kmg_ctx::MODE_UNDECIDED && !c->use_dense)
+    c->plan_scale = (double)bases / (double)std::min<uint64_t>(bases, c->batch_bases);  // decided after the first chunk's ingest (scan_packed)
+  else s = decide_mode(c, bases);  // plan for the whole call, not for its first staging chunk
+  if (s == KMG_OK) s = feed.open();
+  for (size_t i = 0; s == KMG_OK && i < feed.chunks.size(); ++i)
+    s = feed.step(i, [&](uint64_t n_words_total, bool has_start) { return scan_packed(c, n_words_total, has_start); });
+  if (s != KMG_OK) return s;
+  c->n_records += n_records; c->n_bases += bases;
+  return feed.close();
+}
 
 // FASTA / FASTQ file image (HOST bytes, e.g. an mmap'ed file: src/mmap.rs:33-71) -> counts, with the records found ON THE DEVICE:
 // the raw bytes go over PCIe in chunks cut at line (FASTA) / record (FASTQ) boundaries, a few small kernels classify the lines,
@@ -1834,14 +1878,10 @@ KMG_EXPORT kmg_status kmg_extract_keys_device(kmg_ctx *c, const uint8_t *d_seq, 
   CU(c, cudaSetDevice(c->device));
   for (uint32_t i = 0; i < n_shards; ++i) shard_counts_out[i] = 0;
   if (n_bytes == 0) return KMG_OK;
-  const uint64_t n_words_total = round_up((n_bytes + 31) / 32, TILE_WORDS);
-  kmg_status s = ensure_packed(c, n_words_total);
+  uint64_t n_words_total = 0;
+  bool has_start = false;
+  kmg_status s = pack_device_ascii(c, d_seq, d_qual, n_records > 1 ? d_offsets : nullptr, n_records, 0, n_bytes, &n_words_total, &has_start);
   if (s != KMG_OK) return s;
-  const bool use_q = c->cfg.has_min_quality && d_qual != nullptr;
-  const uint32_t thr = std::min<uint32_t>(255u, (uint32_t)c->cfg.min_quality + 33u);
-  CU(c, launch_ingest(d_seq, use_q ? d_qual : nullptr, n_bytes, thr, n_words_total, c->d_bases, c->d_valid, c->stream));
-  const bool has_start = d_offsets != nullptr && n_records > 1;
-  if (has_start) CU(c, launch_start_bits(d_offsets, n_records, 0, n_bytes, n_words_total, c->d_start, c->stream));
   if (n_bytes >= (1ull << 32)) return fail(c, KMG_ERR_INVALID_ARG, "kmg_extract_keys_device handles < 2^32 bytes per call");
   unsigned long long *d_pc = nullptr;
   CU(c, pool_alloc(c, &d_pc, 3 * (size_t)n_shards * 8 + 64));  // pooled: a cudaMalloc / cudaFree pair per call synchronises the device
@@ -1876,8 +1916,10 @@ KMG_EXPORT kmg_status kmg_extract_keys_device(kmg_ctx *c, const uint8_t *d_seq, 
 // region per global bin; the exchange is FUSED into the owner's refine kernel (A2), whose tile loads read the owner's regions
 // straight out of all ranks' send buffers through P2P-mapped pointers (NVLink loads, prefetched a tile ahead), so no key is
 // ever copied: it crosses NVLink once, on its way into the kernel that partitions it further.  Only metadata crosses between
-// the ranks on the host: a POSIX shared-memory segment carries the region sizes, flags, summaries, histograms and a
-// sense-reversing barrier.  No NCCL, no staging copies, no count pass on the fast path.
+// the ranks on the host: a POSIX shared-memory segment carries a sense-reversing barrier and one double-buffered post area,
+// through which every collective exchanges its messages (region sizes, flags, summaries, histograms) with one all-gather
+// (shard_allgather).  The host ASCII feed and the file-image feed are the ones a single context uses (AsciiFeed, FastxFeed);
+// only the scan of a chunk differs.  No NCCL, no staging copies, no count pass on the fast path.
 // (Measured alternative, round 2: the scatter kernel writing into the owners' buffers with P2P STORES.  A sub-tile yields only
 // ~8 keys per bin, and 64-byte NVLink writes cost more than they move: 4.45 ms per 310 M-base round against 2.05 ms for the
 // local scatter; fewer bins made the stores longer but the owner's refine slower -- profiles/r2_summary.md.)
@@ -1888,32 +1930,19 @@ constexpr uint32_t SHARD_HIST_MAX = 2 * 65536;   // (value, frequency) pairs a r
 constexpr uint32_t SHARD_MAGIC = 0x4b4d4753u;
 constexpr double SHARD_TIMEOUT_S = 120.0;
 
+constexpr uint32_t SHARD_POST_WORDS = 1 + 2 * SHARD_HIST_MAX;  // the largest message: a histogram's pair count and its pairs
+
 struct PeerBuf {  // a rank's device buffer as its peers open it: raw pointer (threads of one process) or CUDA IPC handle
   cudaIpcMemHandle_t handle;
   uint64_t raw_ptr;
 };
-struct ShardRankSlot {
-  int32_t pid, device;
-  PeerBuf send;
-  uint64_t recv_entries;
-  uint64_t round_bytes, round_flag;
-  uint64_t summary[8];
-  uint64_t hist_n;
-  // kmg_shard_write_text: arguments, records of this shard that pass min_count, its staging buffer, where each piece of the current
-  // step starts in its sorted step array, the piece it owns this step (records expected, records merged in order, bytes), bytes written
-  uint64_t text_args[2], text_total;
-  PeerBuf text;
-  uint64_t text_bounds[SHARD_MAX_WORLD + 1];
-  uint64_t text_piece[3], text_written;
-  // kmg_shard_count_fastx: the image's length and rank cuts as this rank computed them, its chunk plan's status, its records
-  uint64_t fastx_len, fastx_cuts[SHARD_MAX_WORLD + 1], fastx_status, fastx_records;
-};
+constexpr size_t PEER_BUF_WORDS = sizeof(PeerBuf) / 8;
+static_assert(sizeof(PeerBuf) % 8 == 0, "a PeerBuf is posted as whole words");
+
 struct ShardShm {
   uint32_t ready, world;
   uint32_t bar_count, bar_gen, abort, spec_disabled;
-  ShardRankSlot ranks[SHARD_MAX_WORLD];
-  uint64_t lens[SHARD_MAX_WORLD][SHARD_MAX_BINS];      // [source rank][global bin]: keys source s holds for bin g this round
-  uint64_t hist[SHARD_MAX_WORLD][2 * SHARD_HIST_MAX];  // a rank's (value, frequency) pairs
+  uint64_t post[2][SHARD_MAX_WORLD][SHARD_POST_WORDS];  // [gather parity][rank]: the rank's message of a shard_allgather
 };
 
 namespace {
@@ -1947,28 +1976,47 @@ kmg_status shard_barrier(kmg_ctx *c) {
 #define SB(c) do { kmg_status _s = shard_barrier(c); if (_s != KMG_OK) return _s; } while (0)
 #define SCU(c, call) do { cudaError_t _e = (call); if (_e != cudaSuccess) { cuda_fail(c, _e, #call); return shard_fail(c, _e == cudaErrorMemoryAllocation ? KMG_ERR_OOM : KMG_ERR_CUDA, c->err); } } while (0)
 
-// A device buffer every rank can read: each rank publishes its own in its slot, and after a barrier opens all of them.
+// The one exchange of host metadata between the ranks: every rank posts n_words words, and all[r * n_words, (r + 1) * n_words) is
+// rank r's message afterwards, on every rank.  counted_pairs: a variable-length message, word 0 the number m of pairs that follow as
+// 2m words (n_words = 1 + 2m); every rank's row is copied with its own length, back to back.  Every rank makes the same sequence
+// of calls.
+// One barrier suffices because gathers alternate between the two halves of the post area: a rank writes the half of gather i
+// again only in gather i+2, after it has passed the barrier of gather i+1, and no rank reaches that barrier before it has
+// finished reading gather i.
+kmg_status shard_allgather(kmg_ctx *c, const void *mine, size_t n_words, std::vector<uint64_t> &all, bool counted_pairs = false) {
+  if (n_words > SHARD_POST_WORDS) return shard_fail(c, KMG_ERR_STATE, "shard group message larger than the post area");
+  uint64_t (*post)[SHARD_POST_WORDS] = c->shm->post[c->sh_gathers & 1];
+  memcpy(post[c->sh_rank], mine, n_words * 8);
+  kmg_status st = shard_barrier(c);
+  if (st != KMG_OK) return st;
+  all.clear();
+  for (uint32_t r = 0; r < c->sh_world; ++r) all.insert(all.end(), post[r], post[r] + (counted_pairs ? 1 + 2 * post[r][0] : n_words));
+  c->sh_gathers++;
+  return KMG_OK;
+}
+
+// A device buffer every rank can read: each rank posts its own, and after the gather opens all of them.
 void publish_peer_buffer(PeerBuf &slot, void *mine) {
   slot.raw_ptr = (uint64_t)(uintptr_t)mine;
   cudaError_t e = cudaIpcGetMemHandle(&slot.handle, mine);
   if (e != cudaSuccess) { cudaGetLastError(); memset(&slot.handle, 0, sizeof slot.handle); }  // same-process groups do not need it
 }
-// peers[r] = rank r's buffer as seen from here: threads of one process use plain pointers (+ peer access between different devices),
-// other processes a CUDA IPC mapping (ipc[r]).  Returns why a buffer could not be opened, or "".
-std::string open_peer_buffers(kmg_ctx *c, PeerBuf ShardRankSlot::*which, uint64_t **peers, bool *ipc) {
-  const ShardShm *S = c->shm;
-  const ShardRankSlot &mine = S->ranks[c->sh_rank];
+// peers[r] = rank r's buffer as seen from here, from the PeerBuf at the start of rank r's row of a gather: threads of one process use
+// plain pointers (+ peer access between different devices), other processes a CUDA IPC mapping (ipc[r]).  Returns why a buffer
+// could not be opened, or "".
+std::string open_peer_buffers(kmg_ctx *c, const std::vector<uint64_t> &all, size_t row_words, uint64_t **peers, bool *ipc) {
   for (uint32_t r = 0; r < c->sh_world; ++r) {
-    const ShardRankSlot &o = S->ranks[r];
-    const PeerBuf &b = o.*which;
+    PeerBuf b;
+    memcpy(&b, all.data() + r * row_words, sizeof b);
+    const int dev = c->sh_device[r];
     if (r == c->sh_rank) {
       peers[r] = reinterpret_cast<uint64_t *>((uintptr_t)b.raw_ptr);
-    } else if (o.pid == mine.pid) {
-      if (o.device != c->device) {
+    } else if (c->sh_pid[r] == c->sh_pid[c->sh_rank]) {
+      if (dev != c->device) {
         int can = 0;
-        cudaDeviceCanAccessPeer(&can, c->device, o.device);
-        if (!can) return "no peer access between devices " + std::to_string(c->device) + " and " + std::to_string(o.device);
-        cudaError_t pe = cudaDeviceEnablePeerAccess(o.device, 0);
+        cudaDeviceCanAccessPeer(&can, c->device, dev);
+        if (!can) return "no peer access between devices " + std::to_string(c->device) + " and " + std::to_string(dev);
+        cudaError_t pe = cudaDeviceEnablePeerAccess(dev, 0);
         cudaGetLastError();
         if (pe != cudaSuccess && pe != cudaErrorPeerAccessAlreadyEnabled) return std::string("cudaDeviceEnablePeerAccess: ") + cudaGetErrorString(pe);
       }
@@ -2008,11 +2056,11 @@ kmg_status shard_scan_round(kmg_ctx *c, uint64_t n_words_total, bool has_start) 
   static const bool trace = getenv("KMG_SHARD_TIMING") != nullptr;  // per-round wall times (every phase ends in a sync anyway)
   const double tr0 = now_s();
   // 1. the round's size is known to all (and everybody has finished the round before the previous one: see the buffers' reuse)
-  S->ranks[me].round_bytes = n_words_total * 32;
-  S->ranks[me].round_flag = 0;
-  SB(c);
-  uint64_t max_w = 0;
-  for (uint32_t r = 0; r < W; ++r) max_w = std::max<uint64_t>(max_w, S->ranks[r].round_bytes);
+  std::vector<uint64_t> all;
+  const uint64_t my_bytes = n_words_total * 32;
+  kmg_status gs = shard_allgather(c, &my_bytes, 1, all);
+  if (gs != KMG_OK) return gs;
+  const uint64_t max_w = *std::max_element(all.begin(), all.end());
   if (max_w == 0) return KMG_OK;
   if (max_w >= (1ull << 32) || max_w > c->sh_recv_entries) return shard_fail(c, KMG_ERR_INVALID_ARG, "a sharded round handles at most batch_bases (< 2^32) bases per rank");
   const uint64_t parity = c->sh_rounds & 1;
@@ -2023,7 +2071,10 @@ kmg_status shard_scan_round(kmg_ctx *c, uint64_t n_words_total, bool has_start) 
   ScanInput in;
   in.bases = c->d_bases; in.valid = c->d_valid; in.start = has_start ? c->d_start : nullptr;
   in.n_tiles = n_words_total / TILE_WORDS; in.k = c->k;
-  std::vector<uint64_t> h_start(G), h_len(G);
+  // what this rank posts after its scatter: the overflow flag, then its G region lengths
+  std::vector<uint64_t> h_start(G), post(1 + G);
+  uint64_t *h_len = post.data() + 1;
+  auto len_of = [&](uint32_t s, uint32_t g) { return all[(size_t)s * (G + 1) + 1 + g]; };  // source s's region of global bin g
   const size_t tmr = timer_begin(c, 0);
   bool done = false;
   double tr1 = tr0, tr2 = tr0;
@@ -2041,23 +2092,22 @@ kmg_status shard_scan_round(kmg_ctx *c, uint64_t n_words_total, bool has_start) 
     SCU(c, cudaMemsetAsync(sin.overflow_flag, 0, 4, c->stream));
     SCU(c, cudaMemcpyAsync(d_start, h_start.data(), G * 8, cudaMemcpyHostToDevice, c->stream));
     if (in.n_tiles) SCU(c, launch_scan_partition(sin, G, true, d_cnt, d_start, d_cur, send, c->d_counters, c->stream, /*mixed=*/true));
-    SCU(c, cudaMemcpyAsync(h_len.data(), d_cur, G * 8, cudaMemcpyDeviceToHost, c->stream));
+    SCU(c, cudaMemcpyAsync(h_len, d_cur, G * 8, cudaMemcpyDeviceToHost, c->stream));
     SCU(c, cudaMemcpyAsync(&h_flag, sin.overflow_flag, 4, cudaMemcpyDeviceToHost, c->stream));
     SCU(c, cudaStreamSynchronize(c->stream));
     tr1 = now_s();
-    memcpy(S->lens[me], h_len.data(), G * 8);
-    S->ranks[me].round_flag = h_flag;
-    SB(c);  // every rank's regions are complete in its send buffer
+    post[0] = h_flag;
+    if ((gs = shard_allgather(c, post.data(), 1 + G, all)) != KMG_OK) return gs;  // every rank's regions are complete in its send buffer
     tr2 = now_s();
     bool any = false;
-    for (uint32_t r = 0; r < W; ++r) any |= S->ranks[r].round_flag != 0;
+    for (uint32_t r = 0; r < W; ++r) any |= all[(size_t)r * (G + 1)] != 0;
     if (!any) {
       std::vector<uint64_t> off((size_t)P1 * W + 1), lens((size_t)P1 * W);
       uint64_t n_in = 0;
       for (uint32_t cl = 0; cl < P1; ++cl)
         for (uint32_t s2 = 0; s2 < W; ++s2) {
           const size_t j = (size_t)cl * W + s2;
-          off[j] = (uint64_t)(me * P1 + cl) * cap; lens[j] = S->lens[s2][me * P1 + cl]; n_in += lens[j];
+          off[j] = (uint64_t)(me * P1 + cl) * cap; lens[j] = len_of(s2, me * P1 + cl); n_in += lens[j];
         }
       off[(size_t)P1 * W] = 0;  // unused: lengths are explicit
       for (uint32_t g = 0; g < G; ++g) if (g / P1 != me) c->sh_sent += h_len[g];
@@ -2077,7 +2127,7 @@ kmg_status shard_scan_round(kmg_ctx *c, uint64_t n_words_total, bool has_start) 
     c->sh_exact_rounds++;
     SCU(c, cudaMemsetAsync(c->d_part, 0, 3 * (size_t)MAX_PARTS * sizeof(unsigned long long), c->stream));
     if (in.n_tiles) SCU(c, launch_scan_partition(in, G, false, d_cnt, d_start, d_cur, nullptr, c->d_counters, c->stream));
-    SCU(c, cudaMemcpyAsync(h_len.data(), d_cnt, G * 8, cudaMemcpyDeviceToHost, c->stream));
+    SCU(c, cudaMemcpyAsync(h_len, d_cnt, G * 8, cudaMemcpyDeviceToHost, c->stream));
     SCU(c, cudaStreamSynchronize(c->stream));
     uint64_t run = 0;
     for (uint32_t g = 0; g < G; ++g) { h_start[g] = run; run += h_len[g]; }
@@ -2086,16 +2136,16 @@ kmg_status shard_scan_round(kmg_ctx *c, uint64_t n_words_total, bool has_start) 
     if (in.n_tiles) SCU(c, launch_scan_partition(in, G, true, d_cnt, d_start, d_cur, send, c->d_counters, c->stream, /*mixed=*/true));
     SCU(c, cudaStreamSynchronize(c->stream));
     tr1 = now_s();
-    memcpy(S->lens[me], h_len.data(), G * 8);
-    SB(c);
+    post[0] = 0;
+    if ((gs = shard_allgather(c, post.data(), 1 + G, all)) != KMG_OK) return gs;
     tr2 = now_s();
     std::vector<uint64_t> off((size_t)P1 * W + 1), lens((size_t)P1 * W);
     uint64_t n_in = 0;
     for (uint32_t s2 = 0; s2 < W; ++s2) {
       uint64_t pre = 0;
       for (uint32_t g = 0; g < G; ++g) {
-        if (g / P1 == me) { const size_t j = (size_t)(g - me * P1) * W + s2; off[j] = pre; lens[j] = S->lens[s2][g]; n_in += lens[j]; }
-        pre += S->lens[s2][g];
+        if (g / P1 == me) { const size_t j = (size_t)(g - me * P1) * W + s2; off[j] = pre; lens[j] = len_of(s2, g); n_in += lens[j]; }
+        pre += len_of(s2, g);
       }
     }
     off[(size_t)P1 * W] = 0;
@@ -2181,20 +2231,26 @@ KMG_EXPORT kmg_status kmg_shard_join(kmg_ctx *c, uint32_t world, uint32_t rank, 
     }
     if (S->world != world) { shard_release(c); return fail(c, KMG_ERR_INVALID_ARG, "ranks disagree on the world size"); }
   }
-  ShardRankSlot &mine = S->ranks[rank];
-  mine.pid = (int32_t)getpid(); mine.device = c->device;
-  mine.recv_entries = c->sh_recv_entries;
-  mine.summary[0] = c->n_coarse; mine.summary[1] = c->n_sub; mine.summary[2] = (uint64_t)c->k;
-  publish_peer_buffer(mine.send, c->sh_recv);
-  kmg_status st = shard_barrier(c);
+  // every rank's send buffer, process, device and plan
+  constexpr size_t JW = PEER_BUF_WORDS + 6;
+  uint64_t mine[JW];
+  PeerBuf send;
+  publish_peer_buffer(send, c->sh_recv);
+  memcpy(mine, &send, sizeof send);
+  uint64_t *m = mine + PEER_BUF_WORDS;
+  m[0] = (uint64_t)getpid(); m[1] = (uint64_t)c->device; m[2] = c->n_coarse; m[3] = c->n_sub; m[4] = (uint64_t)c->k; m[5] = c->sh_recv_entries;
+  c->sh_gathers = 0;
+  std::vector<uint64_t> all;
+  kmg_status st = shard_allgather(c, mine, JW, all);
   if (st != KMG_OK) { shard_release(c); return st; }
   std::string why;
-  for (uint32_t r = 0; r < world && why.empty(); ++r) {
-    const ShardRankSlot &o = S->ranks[r];
-    if (o.summary[0] != c->n_coarse || o.summary[1] != c->n_sub || o.summary[2] != (uint64_t)c->k || o.recv_entries != c->sh_recv_entries)
+  for (uint32_t r = 0; r < world; ++r) {
+    const uint64_t *o = all.data() + r * JW + PEER_BUF_WORDS;
+    c->sh_pid[r] = (int)o[0]; c->sh_device[r] = (int)o[1];
+    if (o[2] != c->n_coarse || o[3] != c->n_sub || o[4] != (uint64_t)c->k || o[5] != c->sh_recv_entries)
       why = "ranks disagree on k / the partition plan / batch_bases (pass identical arguments on every rank)";
   }
-  if (why.empty()) why = open_peer_buffers(c, &ShardRankSlot::send, c->sh_peer, c->sh_peer_ipc);
+  if (why.empty()) why = open_peer_buffers(c, all, JW, c->sh_peer, c->sh_peer_ipc);
   if (!why.empty()) __atomic_store_n(&S->abort, 1u, __ATOMIC_RELEASE);
   st = shard_barrier(c);  // every rank has opened its peers (or the group is aborted)
   if (rank == 0) shm_unlink(name.c_str());  // the mapping lives on; no name is left behind
@@ -2227,29 +2283,21 @@ KMG_EXPORT kmg_status kmg_shard_count_ascii_device(kmg_ctx *c, const uint8_t *d_
   if (step == 0) return shard_fail(c, KMG_ERR_INVALID_ARG, "batch_bases is too small for sharded rounds");
   uint64_t my_rounds = 0;
   for (uint64_t pos = 0; pos < n_bytes; pos += step) { if (pos && n_bytes - pos <= K1) break; ++my_rounds; }
-  ShardShm *S = c->shm;
-  S->ranks[c->sh_rank].summary[7] = my_rounds;
-  SB(c);
-  uint64_t rounds = 0;
-  for (uint32_t r = 0; r < c->sh_world; ++r) rounds = std::max<uint64_t>(rounds, S->ranks[r].summary[7]);
-  SB(c);
-  const bool use_q = c->cfg.has_min_quality && d_qual != nullptr;
-  const uint32_t thr = std::min<uint32_t>(255u, (uint32_t)c->cfg.min_quality + 33u);
+  std::vector<uint64_t> all;
+  kmg_status st = shard_allgather(c, &my_rounds, 1, all);
+  if (st != KMG_OK) return st;
+  const uint64_t rounds = *std::max_element(all.begin(), all.end());
   for (uint64_t i = 0; i < rounds; ++i) {
     const uint64_t pos = i * step;
-    uint64_t len = 0;
-    if (i < my_rounds) len = std::min<uint64_t>(step + K1, n_bytes - pos);
+    const uint64_t len = i < my_rounds ? std::min<uint64_t>(step + K1, n_bytes - pos) : 0;
     uint64_t n_words_total = 0;
     bool has_start = false;
     if (len) {
-      n_words_total = round_up((len + 31) / 32, TILE_WORDS);
-      kmg_status st = ensure_packed(c, n_words_total);
+      st = pack_device_ascii(c, d_seq + pos, d_qual ? d_qual + pos : nullptr, n_records > 1 ? d_offsets : nullptr, n_records, pos, len,
+                             &n_words_total, &has_start);
       if (st != KMG_OK) return shard_fail(c, st, c->err);
-      SCU(c, launch_ingest(d_seq + pos, use_q ? d_qual + pos : nullptr, len, thr, n_words_total, c->d_bases, c->d_valid, c->stream));
-      has_start = d_offsets != nullptr && n_records > 1;
-      if (has_start) SCU(c, launch_start_bits(d_offsets, n_records, pos, len, n_words_total, c->d_start, c->stream));
     }
-    kmg_status st = shard_scan_round(c, n_words_total, has_start);
+    st = shard_scan_round(c, n_words_total, has_start);
     if (st != KMG_OK) return st;
   }
   c->n_records += n_records; c->n_bases += n_bytes;
@@ -2260,83 +2308,21 @@ KMG_EXPORT kmg_status kmg_shard_count_ascii_device(kmg_ctx *c, const uint8_t *d_
 KMG_EXPORT kmg_status kmg_shard_count_ascii(kmg_ctx *c, const uint8_t *seq, const uint8_t *qual, const uint64_t *offsets, uint64_t n_records) {
   if (!c) return KMG_ERR_INVALID_ARG;
   if (!c->shm) return kmg_count_ascii(c, seq, qual, offsets, n_records);
-  if (n_records && (!offsets || !seq)) return shard_fail(c, KMG_ERR_INVALID_ARG, "seq / offsets must not be NULL");
-  CU(c, cudaSetDevice(c->device));
-  const uint64_t begin = n_records ? offsets[0] : 0, end = n_records ? offsets[n_records] : 0;
-  const bool use_q = c->cfg.has_min_quality && qual != nullptr;
-  const bool src_pinned = end > begin && is_pinned_host(seq + begin) && (!use_q || is_pinned_host(qual + begin));
-  kmg_status s = ensure_staging(c, !src_pinned, use_q, std::max<uint64_t>(end - begin, 1));
+  kmg_status s = check_ascii_layout(c, seq, offsets, n_records);
   if (s != KMG_OK) return shard_fail(c, s, c->err);
-  const uint64_t K1 = (uint64_t)c->k - 1, B = c->batch_bases, step = B - K1;
-  struct Chunk { uint64_t pos, len, r_lo, nrec; };
-  std::vector<Chunk> chunks;
-  {
-    uint64_t r_lo = 0;
-    for (uint64_t pos = begin; pos < end; pos += step) {
-      const uint64_t len = std::min<uint64_t>(B, end - pos);
-      if (pos != begin && len <= K1) break;
-      while (r_lo < n_records && offsets[r_lo] <= pos) ++r_lo;
-      uint64_t r_hi = r_lo;
-      while (r_hi < n_records && offsets[r_hi] < pos + len) ++r_hi;
-      chunks.push_back(Chunk{pos, len, r_lo, r_hi - r_lo});
-    }
-  }
-  ShardShm *S = c->shm;
-  S->ranks[c->sh_rank].summary[7] = chunks.size();
-  SB(c);
-  uint64_t rounds = 0;
-  for (uint32_t r = 0; r < c->sh_world; ++r) rounds = std::max<uint64_t>(rounds, S->ranks[r].summary[7]);
-  SB(c);
-  auto stage_chunk = [&](const Chunk &ch, Staging &st) -> kmg_status {
-    if (st.h2d_pending) { CU(c, cudaEventSynchronize(st.h2d_done)); st.h2d_pending = false; }
-    if (st.compute_pending) { CU(c, cudaStreamWaitEvent(c->copy_stream, st.compute_done, 0)); }
-    kmg_status es = ensure_offsets(c, st, ch.nrec);
-    if (es != KMG_OK) return es;
-    const uint8_t *src_seq = seq + ch.pos, *src_qual = use_q ? qual + ch.pos : nullptr;
-    if (!src_pinned) {
-      memcpy(st.h_seq, src_seq, ch.len); src_seq = st.h_seq;
-      if (use_q) { memcpy(st.h_qual, src_qual, ch.len); src_qual = st.h_qual; }
-    }
-    CU(c, cudaMemcpyAsync(st.d_seq, src_seq, ch.len, cudaMemcpyHostToDevice, c->copy_stream));
-    if (use_q) CU(c, cudaMemcpyAsync(st.d_qual, src_qual, ch.len, cudaMemcpyHostToDevice, c->copy_stream));
-    if (ch.nrec) {
-      memcpy(st.h_off, offsets + ch.r_lo, ch.nrec * 8);
-      CU(c, cudaMemcpyAsync(st.d_off, st.h_off, ch.nrec * 8, cudaMemcpyHostToDevice, c->copy_stream));
-    }
-    c->h2d_bytes += ch.len * (use_q ? 2 : 1) + ch.nrec * 8;
-    CU(c, cudaEventRecord(st.h2d_done, c->copy_stream));
-    st.h2d_pending = true;
-    return KMG_OK;
-  };
-  const uint32_t thr = std::min<uint32_t>(255u, (uint32_t)c->cfg.min_quality + 33u);
-  const uint32_t slot0 = c->next_ascii;
-  size_t staged = 0;
-  for (uint64_t i = 0; i < rounds; ++i) {
-    uint64_t n_words_total = 0;
-    bool has_start = false;
-    if (i < chunks.size()) {
-      for (; staged < chunks.size() && staged < i + N_STAGE; ++staged)
-        if ((s = stage_chunk(chunks[staged], c->st[(slot0 + staged) % N_STAGE])) != KMG_OK) return shard_fail(c, s, c->err);
-      Staging &st = c->st[(slot0 + i) % N_STAGE];
-      const Chunk &ch = chunks[i];
-      SCU(c, cudaStreamWaitEvent(c->stream, st.h2d_done, 0));
-      n_words_total = round_up((ch.len + 31) / 32, TILE_WORDS);
-      if ((s = ensure_packed(c, n_words_total)) != KMG_OK) return shard_fail(c, s, c->err);
-      SCU(c, launch_ingest(st.d_seq, use_q ? st.d_qual : nullptr, ch.len, thr, n_words_total, c->d_bases, c->d_valid, c->stream));
-      has_start = ch.nrec > 0;
-      if (has_start) SCU(c, launch_start_bits(st.d_off, ch.nrec, ch.pos, ch.len, n_words_total, c->d_start, c->stream));
-      SCU(c, cudaEventRecord(st.compute_done, c->stream));  // the staging slot is free once ingest has packed it
-      st.compute_pending = true;
-    }
-    s = shard_scan_round(c, n_words_total, has_start);
-    if (s != KMG_OK) return s;
-  }
-  c->next_ascii = (slot0 + (uint32_t)chunks.size()) % N_STAGE;
-  c->n_records += n_records; c->n_bases += end - begin;
-  if (src_pinned)
-    for (auto &st : c->st)
-      if (st.h2d_pending) { CU(c, cudaEventSynchronize(st.h2d_done)); st.h2d_pending = false; }
-  return KMG_OK;
+  CU(c, cudaSetDevice(c->device));
+  // the ranks agree on the number of rounds; a rank without chunks left takes part with empty rounds
+  AsciiFeed feed(c, seq, qual, offsets, n_records);
+  if ((s = feed.open()) != KMG_OK) return shard_fail(c, s, c->err);
+  const uint64_t my_rounds = feed.chunks.size();
+  std::vector<uint64_t> all;
+  if ((s = shard_allgather(c, &my_rounds, 1, all)) != KMG_OK) return s;
+  const uint64_t rounds = *std::max_element(all.begin(), all.end());
+  auto scan = [&](uint64_t n_words_total, bool has_start) { return shard_scan_round(c, n_words_total, has_start); };
+  for (uint64_t i = 0; s == KMG_OK && i < rounds; ++i) s = i < my_rounds ? feed.step(i, scan) : scan(0, false);
+  if (s != KMG_OK) return shard_fail(c, s, c->err);
+  c->n_records += n_records; c->n_bases += feed.end - feed.begin;
+  return feed.close();
 }
 
 namespace {
@@ -2392,7 +2378,6 @@ KMG_EXPORT kmg_status kmg_shard_count_fastx(kmg_ctx *c, const uint8_t *buf, uint
   if (len && buf[0] != (is_fastq ? '@' : '>'))
     return shard_fail(c, KMG_ERR_PARSE, is_fastq ? "FASTQ record does not start with '@' (record 0)" : "FASTA record does not start with '>' (record 0)");
   SCU(c, cudaSetDevice(c->device));
-  ShardShm *S = c->shm;
   const uint32_t W = c->sh_world, me = c->sh_rank;
   const uint64_t K1 = (uint64_t)c->k - 1;
   // ---- rank cuts (every rank computes all of them) and this rank's chunks: raw chunk + carry <= batch_bases bases, one round each
@@ -2405,27 +2390,25 @@ KMG_EXPORT kmg_status kmg_shard_count_fastx(kmg_ctx *c, const uint8_t *buf, uint
   std::vector<FxChunk> chunks;
   const kmg_status plan = plan_fastx_chunks(c, buf, len, begin, end, is_fastq, std::min<uint64_t>(c->batch_bases - K1, 1ull << 30), chunks);
   // ---- the ranks compare their images (length and cuts) and plans, and agree on the number of rounds
-  ShardRankSlot &mine = S->ranks[me];
-  mine.fastx_len = len;
-  memcpy(mine.fastx_cuts, cuts, (W + 1) * 8);
-  mine.fastx_status = (uint64_t)plan;
-  mine.summary[7] = plan == KMG_OK ? chunks.size() : 0;
-  SB(c);
+  const size_t FW = W + 4;  // image length, plan status, rounds, cuts
+  uint64_t mine[SHARD_MAX_WORLD + 4] = {len, (uint64_t)plan, plan == KMG_OK ? chunks.size() : 0};
+  memcpy(mine + 3, cuts, (W + 1) * 8);
+  std::vector<uint64_t> all;
+  kmg_status s = shard_allgather(c, mine, FW, all);
+  if (s != KMG_OK) return s;
   bool same = true, planned = true;
   uint64_t rounds = 0;
   for (uint32_t r = 0; r < W; ++r) {
-    const ShardRankSlot &o = S->ranks[r];
-    same = same && o.fastx_len == len && memcmp(o.fastx_cuts, cuts, (W + 1) * 8) == 0;
-    planned = planned && o.fastx_status == (uint64_t)KMG_OK;
-    rounds = std::max<uint64_t>(rounds, o.summary[7]);
+    const uint64_t *o = all.data() + r * FW;
+    same = same && o[0] == len && memcmp(o + 3, cuts, (W + 1) * 8) == 0;
+    planned = planned && o[1] == (uint64_t)KMG_OK;
+    rounds = std::max<uint64_t>(rounds, o[2]);
   }
-  SB(c);
   if (!same) return shard_fail(c, KMG_ERR_INVALID_ARG, "ranks passed different file images (pass the same whole image on every rank)");
   if (!planned)
     return shard_fail(c, KMG_ERR_PARSE, plan != KMG_OK ? c->err : "another rank's slice cannot be cut into staging chunks (a line longer than a chunk, or multi-line FASTQ)");
   // ---- rounds: parse -> pack -> fused scatter + exchange; a rank without chunks left takes part with empty rounds
   FastxFeed feed(c, buf, chunks, is_fastq);
-  kmg_status s = KMG_OK;
   if (!chunks.empty()) {
     s = feed.open();
     if (s == KMG_OK && !is_fastq && buf[begin] != '>') {
@@ -2445,11 +2428,9 @@ KMG_EXPORT kmg_status kmg_shard_count_fastx(kmg_ctx *c, const uint8_t *buf, uint
   if (!chunks.empty()) feed.close(s != KMG_OK);
   if (s != KMG_OK) return shard_fail(c, s, c->err);
   // ---- records of the whole image, on every rank
-  mine.fastx_records = n_rec;
-  SB(c);
+  if ((s = shard_allgather(c, &n_rec, 1, all)) != KMG_OK) return s;
   uint64_t total = 0;
-  for (uint32_t r = 0; r < W; ++r) total += S->ranks[r].fastx_records;
-  SB(c);
+  for (uint64_t n : all) total += n;
   c->n_records += n_rec; c->n_bases += feed.bases;
   if (n_records_out) *n_records_out = total;
   return KMG_OK;
@@ -2958,20 +2939,18 @@ KMG_EXPORT kmg_status kmg_shard_finalize(kmg_ctx *c, kmg_summary *out) {
   kmg_status s = kmg_finalize(c, &loc);
   if (!c->shm) { if (out) *out = loc; return s; }
   if (s != KMG_OK) return shard_fail(c, s, c->err);
-  ShardShm *S = c->shm;
-  uint64_t *m = S->ranks[c->sh_rank].summary;
-  m[0] = loc.n_windows; m[1] = loc.n_distinct; m[2] = loc.n_records; m[3] = loc.n_bases; m[4] = loc.max_count;
-  SB(c);
+  const uint64_t m[5] = {loc.n_windows, loc.n_distinct, loc.n_records, loc.n_bases, loc.max_count};
+  std::vector<uint64_t> all;
+  if ((s = shard_allgather(c, m, 5, all)) != KMG_OK) return s;
   if (out) {
     *out = loc;
     out->n_windows = out->n_distinct = out->n_records = out->n_bases = out->max_count = 0;
     for (uint32_t r = 0; r < c->sh_world; ++r) {
-      const uint64_t *o = S->ranks[r].summary;
+      const uint64_t *o = all.data() + 5 * r;
       out->n_windows += o[0]; out->n_distinct += o[1]; out->n_records += o[2]; out->n_bases += o[3];
       out->max_count = std::max<uint64_t>(out->max_count, o[4]);
     }
   }
-  SB(c);
   return KMG_OK;
 }
 
@@ -2986,15 +2965,13 @@ KMG_EXPORT kmg_status kmg_shard_histogram(kmg_ctx *c, uint64_t min_count, uint64
     kmg_status s = kmg_histogram(c, min_count, nullptr, nullptr, 0, &n);
     if (s != KMG_OK) return shard_fail(c, s, c->err);
     if (n > SHARD_HIST_MAX) return shard_fail(c, KMG_ERR_CAPACITY, "shard histogram has too many distinct count values");
-    ShardShm *S = c->shm;
-    uint64_t *mine = S->hist[c->sh_rank];
-    if (n && (s = kmg_histogram(c, min_count, mine, mine + SHARD_HIST_MAX, n, &n)) != KMG_OK) return shard_fail(c, s, c->err);
-    S->ranks[c->sh_rank].hist_n = n;
-    SB(c);
+    std::vector<uint64_t> mine(1 + 2 * n), posted;  // n, the n values, their n frequencies
+    mine[0] = n;
+    if (n && (s = kmg_histogram(c, min_count, &mine[1], &mine[1 + n], n, &n)) != KMG_OK) return shard_fail(c, s, c->err);
+    if ((s = shard_allgather(c, mine.data(), mine.size(), posted, /*counted_pairs=*/true)) != KMG_OK) return s;
     std::vector<std::pair<uint64_t, uint64_t>> all;
-    for (uint32_t r = 0; r < c->sh_world; ++r)
-      for (uint64_t i = 0; i < S->ranks[r].hist_n; ++i) all.emplace_back(S->hist[r][i], S->hist[r][SHARD_HIST_MAX + i]);
-    SB(c);
+    for (size_t o = 0; o < posted.size(); o += 1 + 2 * posted[o])
+      for (uint64_t i = 0; i < posted[o]; ++i) all.emplace_back(posted[o + 1 + i], posted[o + 1 + posted[o] + i]);
     std::sort(all.begin(), all.end());
     c->sh_hist_vals.clear(); c->sh_hist_freqs.clear();
     for (size_t i = 0; i < all.size();) {
@@ -3026,34 +3003,28 @@ KMG_EXPORT kmg_status kmg_shard_save_kmix(kmg_ctx *c, const char *path, uint64_t
   }
   if (has_gz_suffix(path)) return shard_fail(c, KMG_ERR_INVALID_ARG, "kmg_shard_save_kmix writes uncompressed .kmix files");
   CU(c, cudaSetDevice(c->device));
-  ShardShm *S = c->shm;
   uint64_t n = 0;
   kmg_status s = count_filtered(c, 0, &n);
   if (s != KMG_OK) return shard_fail(c, s, c->err);
-  uint64_t *m = S->ranks[c->sh_rank].summary;
-  m[5] = n;
   if (c->sh_rank == 0 && kmg_kmix_begin(path) != KMG_OK) return shard_fail(c, KMG_ERR_IO, std::string("cannot create ") + path);
-  SB(c);
-  uint64_t before = 0;
-  for (uint32_t r = 0; r < c->sh_rank; ++r) before += S->ranks[r].summary[5];
+  std::vector<uint64_t> recs, crcs;  // every shard's records, then the CRCs of their bytes
+  if ((s = shard_allgather(c, &n, 1, recs)) != KMG_OK) return s;
+  uint64_t before = 0, total = 0;
+  for (uint32_t r = 0; r < c->sh_world; ++r) { if (r < c->sh_rank) before += recs[r]; total += recs[r]; }
   uint64_t n2 = 0;
   uint32_t crc = 0;
   s = kmg_save_kmix_shard(c, path, before, &n2, &crc);
   if (s != KMG_OK) return shard_fail(c, s, c->err);
   if (n2 != n) return shard_fail(c, KMG_ERR_STATE, "shard index writer wrote an unexpected number of records");
-  m[6] = crc;
-  SB(c);
-  uint64_t total = 0;
-  for (uint32_t r = 0; r < c->sh_world; ++r) total += S->ranks[r].summary[5];
-  kmg_status fs = KMG_OK;
+  const uint64_t my_crc = crc;
+  if ((s = shard_allgather(c, &my_crc, 1, crcs)) != KMG_OK) return s;
   if (c->sh_rank == 0) {
-    uint64_t recs[SHARD_MAX_WORLD];
-    uint32_t crcs[SHARD_MAX_WORLD];
-    for (uint32_t r = 0; r < c->sh_world; ++r) { recs[r] = S->ranks[r].summary[5]; crcs[r] = (uint32_t)S->ranks[r].summary[6]; }
-    fs = kmg_kmix_finish(path, (uint32_t)c->k, recs, crcs, c->sh_world);
+    uint32_t crc32s[SHARD_MAX_WORLD];
+    for (uint32_t r = 0; r < c->sh_world; ++r) crc32s[r] = (uint32_t)crcs[r];
+    const kmg_status fs = kmg_kmix_finish(path, (uint32_t)c->k, recs.data(), crc32s, c->sh_world);
     if (fs != KMG_OK) return shard_fail(c, fs, std::string("cannot finish ") + path);
   }
-  SB(c);
+  SB(c);  // no rank returns before rank 0 has finished the file
   if (n_records_out) *n_records_out = total;
   return KMG_OK;
 }
@@ -3140,35 +3111,35 @@ KMG_EXPORT kmg_status kmg_shard_write_text(kmg_ctx *c, uint64_t min_count, int f
   const uint64_t head = json ? strlen(JSON_OPEN) : 0;  // bytes in front of the first piece
   if (min_count == 0) min_count = 1;
   SCU(c, cudaSetDevice(c->device));
-  ShardShm *S = c->shm;
   const uint32_t W = c->sh_world, me = c->sh_rank;
-  ShardRankSlot &mine = S->ranks[me];
   // 1. arguments, records that pass min_count and key histogram of every shard; rank 0 creates / truncates the file
-  uint64_t n_mine = 0;
-  kmg_status s = count_filtered(c, min_count, &n_mine);
-  if (s == KMG_OK) s = key_histogram(c, S->hist[me]);
+  constexpr size_t AW = 3 + KEY_BUCKETS;  // min_count, format, records, key histogram
+  std::vector<uint64_t> mine(AW), args;
+  mine[0] = min_count; mine[1] = (uint64_t)format;
+  kmg_status s = count_filtered(c, min_count, &mine[2]);
+  if (s == KMG_OK) s = key_histogram(c, &mine[3]);
   if (s != KMG_OK) return shard_fail(c, s, c->err);
-  mine.text_args[0] = min_count; mine.text_args[1] = (uint64_t)format; mine.text_total = n_mine;
   if (me == 0) {
     FILE *f = fopen(path, "wb");
     if (!f || fclose(f) != 0) return shard_fail(c, KMG_ERR_IO, std::string("cannot create ") + path);
   }
-  SB(c);
+  if ((s = shard_allgather(c, mine.data(), AW, args)) != KMG_OK) return s;
+  auto hist_of = [&](uint32_t r) { return args.data() + r * AW + 3; };
   for (uint32_t r = 0; r < W; ++r)
-    if (S->ranks[r].text_args[0] != min_count || S->ranks[r].text_args[1] != (uint64_t)format)
+    if (args[r * AW] != min_count || args[r * AW + 1] != (uint64_t)format)
       return shard_fail(c, KMG_ERR_INVALID_ARG, "ranks disagree on min_count / format (pass identical arguments on every rank)");
   // 2. the same pieces on every rank; staging buffers sized for the largest part of a step any rank holds, merge buffers for the
   //    largest piece this rank owns
   std::vector<uint64_t> sum(KEY_BUCKETS, 0);
   for (uint32_t r = 0; r < W; ++r)
-    for (int b = 0; b < KEY_BUCKETS; ++b) sum[b] += S->hist[r][b];
+    for (int b = 0; b < KEY_BUCKETS; ++b) sum[b] += hist_of(r)[b];
   const std::vector<int> cuts = piece_cuts(sum.data(), 1ull << 24);
   const size_t n_pieces = cuts.size() - 1;
   std::vector<int> step_cuts;
   for (size_t p = 0; p < n_pieces; p += W) step_cuts.push_back(cuts[p]);
   if (n_pieces) step_cuts.push_back(cuts[n_pieces]);
   uint64_t stage_cap = 1, own_cap = 1;
-  for (uint32_t r = 0; r < W; ++r) stage_cap = std::max(stage_cap, largest_piece(S->hist[r], step_cuts));
+  for (uint32_t r = 0; r < W; ++r) stage_cap = std::max(stage_cap, largest_piece(hist_of(r), step_cuts));
   for (size_t p = me; p < n_pieces; p += W) own_cap = std::max(own_cap, largest_piece(sum.data(), {cuts[p], cuts[p + 1]}));
   const int shift = key_bucket_shift(c);
   uint64_t *stage = nullptr, *dk = nullptr, *dc = nullptr, *d_aux = nullptr;
@@ -3176,14 +3147,17 @@ KMG_EXPORT kmg_status kmg_shard_write_text(kmg_ctx *c, uint64_t min_count, int f
   bool peer_ipc[SHARD_MAX_WORLD] = {};
   int fd = -1;
   uint64_t records = 0, file_bytes = 0;
+  std::vector<uint64_t> all;
   auto run = [&]() -> kmg_status {
     SCU(c, cudaMalloc(&stage, 2 * stage_cap * 8));  // (key, count) SoA: keys [0, stage_cap), counts [stage_cap, 2 * stage_cap)
     SCU(c, pool_alloc(c, &dk, own_cap * 8));
     SCU(c, pool_alloc(c, &dc, own_cap * 8));
     SCU(c, pool_alloc(c, &d_aux, (SHARD_MAX_WORLD + 2) * 8));  // piece bounds + the merge's placed-record counter
-    publish_peer_buffer(mine.text, stage);
-    SB(c);
-    const std::string why = open_peer_buffers(c, &ShardRankSlot::text, peer, peer_ipc);
+    PeerBuf mine_stage;
+    publish_peer_buffer(mine_stage, stage);
+    kmg_status gs = shard_allgather(c, &mine_stage, PEER_BUF_WORDS, all);
+    if (gs != KMG_OK) return gs;
+    const std::string why = open_peer_buffers(c, all, PEER_BUF_WORDS, peer, peer_ipc);
     if (!why.empty()) return shard_fail(c, KMG_ERR_CUDA, why);
     if ((fd = open(path, O_WRONLY)) < 0) return shard_fail(c, KMG_ERR_IO, std::string("cannot open ") + path + " for writing");
     HostStager staged(c, 64u << 20);
@@ -3209,8 +3183,8 @@ KMG_EXPORT kmg_status kmg_shard_write_text(kmg_ctx *c, uint64_t min_count, int f
       SCU(c, cudaMemcpyAsync(bounds, d_aux, n_own * 8, cudaMemcpyDeviceToHost, c->stream));
       SCU(c, cudaStreamSynchronize(c->stream));
       bounds[n_own] = m;
-      memcpy(mine.text_bounds, bounds, (n_own + 1) * 8);
-      SB(c);  // every rank's part of the step is in its staging buffer
+      kmg_status gst = shard_allgather(c, bounds, n_own + 1, all);  // every rank's part of the step is in its staging buffer
+      if (gst != KMG_OK) return gst;
       // 4. the owner merges its piece out of all staging buffers and formats it
       uint64_t expect = 0, bytes = 0;
       unsigned long long placed = 0;
@@ -3219,7 +3193,7 @@ KMG_EXPORT kmg_status kmg_shard_write_text(kmg_ctx *c, uint64_t min_count, int f
         R.n_runs = W;
         uint64_t before = records;  // records of the file in front of this piece: earlier steps + earlier pieces of this step
         for (uint32_t q = 0; q < W; ++q) {
-          const uint64_t lo = S->ranks[q].text_bounds[me], hi = S->ranks[q].text_bounds[me + 1];
+          const uint64_t lo = all[q * (n_own + 1) + me], hi = all[q * (n_own + 1) + me + 1];
           R.keys[q] = peer[q] + lo; R.counts[q] = peer[q] + stage_cap + lo; R.len[q] = hi - lo;
           expect += hi - lo; before += lo;
         }
@@ -3230,12 +3204,13 @@ KMG_EXPORT kmg_status kmg_shard_write_text(kmg_ctx *c, uint64_t min_count, int f
         kmg_status fs = fmt.format(dk, dc, expect, before == 0 && expect > 0, &bytes);  // ends in a stream synchronize
         if (fs != KMG_OK) return shard_fail(c, fs, c->err);
       }
-      mine.text_piece[0] = expect; mine.text_piece[1] = placed; mine.text_piece[2] = bytes;
-      SB(c);  // nobody reads a staging buffer of this step any more: the next step may overwrite them
+      const uint64_t piece[3] = {expect, placed, bytes};  // records expected, records the merge placed in order, bytes
+      // nobody reads a staging buffer of this step any more after this gather: the next step may overwrite them
+      if ((gst = shard_allgather(c, piece, 3, all)) != KMG_OK) return gst;
       // 5. file offset = json's "[" + bytes of all earlier pieces; every merged piece holds as many ordered records as its parts
       uint64_t off = head + file_bytes;
       for (uint32_t j = 0; j < n_own; ++j) {
-        const uint64_t *tp = S->ranks[j].text_piece;
+        const uint64_t *tp = all.data() + 3 * j;
         if (tp[0] != tp[1]) return shard_fail(c, KMG_ERR_STATE, "piece " + std::to_string(p0 + j) + ": the merge placed " + std::to_string(tp[1]) + " records in order, its parts hold " + std::to_string(tp[0]));
         if (j < me) off += tp[2];
         file_bytes += tp[2]; records += tp[0];
@@ -3258,11 +3233,10 @@ KMG_EXPORT kmg_status kmg_shard_write_text(kmg_ctx *c, uint64_t min_count, int f
     const int closed = close(fd);
     fd = -1;
     if (closed != 0) return shard_fail(c, KMG_ERR_IO, std::string("short write to ") + path);
-    mine.text_written = written;
-    SB(c);
+    if ((gs = shard_allgather(c, &written, 1, all)) != KMG_OK) return gs;
     // 6. the file holds every record of every shard that passes min_count, and every byte the owners formatted
     uint64_t want_records = 0, total_written = 0;
-    for (uint32_t r = 0; r < W; ++r) { want_records += S->ranks[r].text_total; total_written += S->ranks[r].text_written; }
+    for (uint32_t r = 0; r < W; ++r) { want_records += args[r * AW + 2]; total_written += all[r]; }
     if (records != want_records) return shard_fail(c, KMG_ERR_STATE, "text file holds " + std::to_string(records) + " records, the shards " + std::to_string(want_records));
     if (total_written != file_bytes) return shard_fail(c, KMG_ERR_STATE, "bytes written differ from the bytes of the formatted pieces");
     close_peer_buffers(peer, peer_ipc);

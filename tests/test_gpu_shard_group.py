@@ -10,14 +10,16 @@ import numpy as np
 import pytest
 
 import krust_b200 as kb
+from krust_b200 import _lib
 from krust_b200.dist import slice_for_rank
 from oracle import oracle as orc
 
 pytestmark = pytest.mark.gpu
 
 
-def run_group(world, k, seq, offsets, qual=None, min_quality=None, batch_bases=0, host_feed=False, kmix_path=None, uneven=False):
-    """Returns (per-rank results, errors).  Rank r scans slice_for_rank(...) of the stream (or, with `uneven`, rank 0 gets 70 %)."""
+def run_group(world, k, seq, offsets, qual=None, min_quality=None, batch_bases=0, host_feed=False, kmix_path=None, uneven=False, cuts=None):
+    """Returns (per-rank results, errors).  Rank r scans slice_for_rank(...) of the stream (or, with `uneven`, rank 0 gets 70 %; with
+    `cuts`, the byte range cuts[r])."""
     import torch
     dev = torch.device("cuda:0")
     total = len(seq)
@@ -25,6 +27,8 @@ def run_group(world, k, seq, offsets, qual=None, min_quality=None, batch_bases=0
     results, errors = [None] * world, []
 
     def cut(r):
+        if cuts is not None:
+            return cuts[r]
         if not uneven:
             return slice_for_rank(total, world, r, k)
         edges = [0] + [int(total * (0.7 + 0.3 * i / (world - 1))) for i in range(world - 1)] + [total]
@@ -134,6 +138,49 @@ def test_fused_exchange_skew_takes_the_exact_route():
     results, errors = run_group(world, k, seq, offsets, batch_bases=1 << 20)
     check(results, errors, world, oracle)
     assert all(r["stats"]["exact_rounds"] >= 1 for r in results)
+
+
+def test_host_feed_rank_with_an_empty_slice():
+    """A rank whose slice holds one empty record and no bytes (seq NULL, offsets [0, 0]) takes part in every round of the host feed."""
+    world, k = 3, 21
+    seq = _genome(np.random.default_rng(9), 1_500_000)
+    offsets = np.array([0, 400_000, len(seq)], dtype=np.uint64)
+    oracle = orc.count_batch_mt(k, seq, None, offsets)
+    mid = 800_000
+    results, errors = run_group(world, k, seq, offsets, batch_bases=200_000, host_feed=True, cuts=[(0, mid + k - 1), (mid, mid), (mid, len(seq))])
+    check(results, errors, world, oracle)
+    assert results[0]["stats"]["rounds"] >= 4 and len({r["stats"]["rounds"] for r in results}) == 1
+
+
+def test_host_feed_refuses_decreasing_offsets_and_peers_do_not_hang():
+    """Decreasing offsets fail the rank that passes them, as kmg_count_ascii does, and its peer returns instead of waiting."""
+    world, k = 2, 21
+    group = f"d{os.getpid()}-{time.time_ns() & 0xffffff:x}"
+    seq = np.frombuffer(b"ACGT" * 50, dtype=np.uint8)
+    out = [None, None]
+
+    def worker(r):
+        c = kb.GpuKmerCounter(k)
+        try:
+            c.shard_join(world, r, group, 1_000_000)
+            try:
+                c.shard_count_batch(seq, None, np.array([0, 120, 60, 200] if r == 0 else [0, 200], dtype=np.uint64))
+                c.shard_finalize()
+                out[r] = "no error"
+            except kb.GpuError as e:
+                out[r] = e
+        finally:
+            c.close()
+
+    ts = [threading.Thread(target=worker, args=(r,)) for r in range(world)]
+    t0 = time.time()
+    for t in ts:
+        t.start()
+    for t in ts:
+        t.join(timeout=200)
+    assert not any(t.is_alive() for t in ts) and time.time() - t0 < 100
+    assert isinstance(out[0], kb.GpuError) and out[0].status == _lib.KMG_ERR_INVALID_ARG and "offsets must be non-decreasing" in str(out[0])
+    assert isinstance(out[1], kb.GpuError) and "peer rank" in str(out[1])
 
 
 def test_grouped_context_refuses_local_feeds_and_peers_do_not_hang():
