@@ -111,6 +111,69 @@ impl GpuKmerCounter {
         Ok(n)
     }
 
+    /// `count_kmers_from_reader_packed` (src/streaming.rs:295-509) and the stdin / gzip readers (src/reader.rs:102-144): a FASTA /
+    /// FASTQ byte stream (`std::io::stdin().lock()`, a `flate2::read::GzDecoder`, ...) parsed on the device in 64 MiB blocks, in
+    /// host memory bounded by the block and the staging ring.  A stream the device parser refuses (multi-line FASTQ ...) goes on
+    /// through the host splitter: the bytes it did not count plus the rest of the reader.  Returns the records of the stream.
+    pub fn count_reader<R: std::io::Read>(&mut self, mut r: R, is_fastq: bool) -> Result<u64, GpuError> {
+        const BLOCK: usize = 64 << 20;
+        let io_err = |e: std::io::Error| GpuError { status: sys::KMG_ERR_IO, details: e.to_string() };
+        let records = |ctx| {
+            let (mut recs, mut bases) = (0u64, 0u64);
+            unsafe { sys::kmg_progress(ctx, &mut recs, &mut bases) };
+            recs
+        };
+        let r0 = records(self.ctx);
+        self.check(unsafe { sys::kmg_fastx_stream_begin(self.ctx, is_fastq as i32, 0) })?;
+        let mut block = vec![0u8; BLOCK];
+        let mut st = sys::KMG_OK;
+        while st == sys::KMG_OK {
+            let n = match r.read(&mut block) {
+                Ok(0) => break,
+                Ok(n) => n,
+                Err(e) if e.kind() == std::io::ErrorKind::Interrupted => continue,
+                Err(e) => {
+                    unsafe { sys::kmg_reset(self.ctx) };  // abandons the stream
+                    return Err(io_err(e));
+                }
+            };
+            st = unsafe { sys::kmg_fastx_stream_push(self.ctx, block.as_ptr(), n as u64) };
+        }
+        if st == sys::KMG_OK {
+            let mut n = 0u64;
+            st = unsafe { sys::kmg_fastx_stream_end(self.ctx, &mut n) };
+        }
+        if st != sys::KMG_OK {
+            let err = Self::error(self.ctx, st);
+            let mut n_rest = 0u64;
+            if st != sys::KMG_ERR_PARSE
+                || unsafe { sys::kmg_fastx_stream_rest(self.ctx, std::ptr::null_mut(), 0, &mut n_rest) } != sys::KMG_OK
+            {
+                return Err(err);
+            }
+            let mut data = vec![0u8; n_rest as usize];
+            self.check(unsafe { sys::kmg_fastx_stream_rest(self.ctx, data.as_mut_ptr(), n_rest, &mut n_rest) })?;
+            r.read_to_end(&mut data).map_err(io_err)?;
+            let marker = if is_fastq { b'@' } else { b'>' };
+            let max_records = data.iter().filter(|&&b| b == marker).count() as u64 + 1;
+            let (mut seq, mut qual) = (vec![0u8; data.len() + 1], vec![0u8; if is_fastq { data.len() + 1 } else { 0 }]);
+            let mut offsets = vec![0u64; max_records as usize + 1];
+            let (mut n_rec, mut msg) = (0u64, vec![0 as std::os::raw::c_char; 256]);
+            let q = if is_fastq { qual.as_mut_ptr() } else { std::ptr::null_mut() };
+            let ps = unsafe {
+                sys::kmg_parse_fastx(data.as_ptr(), data.len() as u64, is_fastq as i32, seq.as_mut_ptr(), q, offsets.as_mut_ptr(), max_records,
+                                     &mut n_rec, msg.as_mut_ptr(), msg.len())
+            };
+            if ps != sys::KMG_OK {
+                let details = unsafe { CStr::from_ptr(msg.as_ptr()) }.to_string_lossy().into_owned();
+                return Err(GpuError { status: ps, details });
+            }
+            offsets.truncate(n_rec as usize + 1);
+            self.count_batch(&seq, if is_fastq { Some(&qual[..]) } else { None }, &offsets)?;
+        }
+        Ok(records(self.ctx) - r0)
+    }
+
     /// `output_counts` for `--format tsv|fasta` (src/run.rs:452-470): sorted lines formatted on the device, streamed into `w`.
     pub fn write_text<W: std::io::Write>(&mut self, w: &mut W, tsv: bool, min_count: u64) -> Result<u64, GpuError> {
         self.emit_text(w, if tsv { sys::KMG_TEXT_TSV } else { sys::KMG_TEXT_FASTA }, min_count)

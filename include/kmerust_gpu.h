@@ -140,6 +140,34 @@ kmg_status kmg_count_ascii(kmg_ctx *ctx, const uint8_t *seq, const uint8_t *qual
  * kmg_count_ascii after kmg_reset.  *n_records_out: records (header lines) seen. */
 kmg_status kmg_count_fastx(kmg_ctx *ctx, const uint8_t *buf, uint64_t len, int is_fastq, uint64_t *n_records_out);
 
+/* Replaces count_kmers_from_reader_packed (src/streaming.rs:295-509) and the stdin / gzip readers (src/reader.rs:102-144): a
+ * FASTA / FASTQ byte STREAM parsed on the device like kmg_count_fastx, in host memory bounded by the context's four pinned
+ * staging slots whatever the stream's length.  For any split of a byte string into pushes the result (table, histogram, text,
+ * .kmix, and the summary's records / bases / windows) equals kmg_count_fastx on the whole string wherever that call accepts it.
+ *   begin: size_hint = bytes expected (0 = unknown: the table is planned from the first chunk and adapts).  Refused with
+ *     KMG_ERR_STATE on a context of a shard group or with a stream already open.
+ *   push: any number of bytes, cut anywhere; they are copied, so the buffer can be reused on return.  A slot that holds
+ *     min(batch_bases, 2^30) bytes is cut at its last line start (FASTA) / record start (FASTQ), its copy to the device is queued
+ *     and the chunk before it is parsed and counted; the bytes after the cut go to the front of the next slot.  A FASTA slot
+ *     without a newline is cut inside its sequence line (between two non-blank bytes, not before a '>'), so unwrapped lines of
+ *     any length are counted.
+ *   end: parses and counts what is left (a last line without '\n' is fine) and closes the stream; *n_records_out: records of
+ *     the whole stream.
+ *   rest: after a KMG_ERR_PARSE that leaves the context usable, the bytes that were not counted (two-call protocol: bytes ==
+ *     NULL gives the size in *n_out; KMG_ERR_CAPACITY when cap is too small).  That is every byte when byte 0 is no header
+ *     ('>' / '@'), else the bytes from the first byte of the refused chunk on -- a FASTQ chunk refused before it was counted
+ *     (multi-line FASTQ, no '+' line where one is expected, no record start near a slot end) or a FASTA slot without a
+ *     possible cut.  The table then holds exactly the records of the earlier chunks, which all end at record starts: split the
+ *     rest plus the remainder of the input with kmg_parse_fastx and feed it to kmg_count_ascii on the same context.
+ * Every other failure (a quality line whose length differs from its sequence, CUDA errors, a full table) is final, as for
+ * kmg_count_fastx: the stream is closed, rest gives KMG_ERR_STATE and the context needs kmg_reset.  While a stream is open
+ * every other feed, kmg_finalize, export, histogram, text, index and query call returns KMG_ERR_STATE; kmg_progress advances
+ * per counted chunk; kmg_reset and kmg_destroy abandon the stream. */
+kmg_status kmg_fastx_stream_begin(kmg_ctx *ctx, int is_fastq, uint64_t size_hint);
+kmg_status kmg_fastx_stream_push(kmg_ctx *ctx, const uint8_t *bytes, uint64_t n);
+kmg_status kmg_fastx_stream_end(kmg_ctx *ctx, uint64_t *n_records_out);
+kmg_status kmg_fastx_stream_rest(kmg_ctx *ctx, uint8_t *bytes, uint64_t cap, uint64_t *n_out);
+
 /* Pre-packed, zero-copy feed for the Rust reader layer (src/reader.rs, src/streaming.rs, src/mmap.rs): a ring of four pinned
  * batches (zeroed when handed out), each with its own device buffers.  kmg_submit_batch queues the batch's H2D copy on the copy
  * stream at once and scans the batch submitted before it, so copies overlap the kernels while the producer fills the next

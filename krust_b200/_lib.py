@@ -47,6 +47,10 @@ SIGNATURES = {
     "kmg_reset": (i32, [vp]),
     "kmg_count_ascii": (i32, [vp, vp, vp, vp, u64]),
     "kmg_count_fastx": (i32, [vp, vp, u64, i32, C.POINTER(u64)]),
+    "kmg_fastx_stream_begin": (i32, [vp, i32, u64]),
+    "kmg_fastx_stream_push": (i32, [vp, vp, u64]),
+    "kmg_fastx_stream_end": (i32, [vp, C.POINTER(u64)]),
+    "kmg_fastx_stream_rest": (i32, [vp, vp, u64, C.POINTER(u64)]),
     "kmg_acquire_batch": (i32, [vp, C.POINTER(KmgBatch)]),
     "kmg_submit_batch": (i32, [vp, C.POINTER(KmgBatch)]),
     "kmg_count_ascii_device": (i32, [vp, vp, vp, vp, u64, u64]),

@@ -10,6 +10,7 @@ from __future__ import annotations
 import ctypes as C
 import gzip
 import os
+import stat
 import sys
 import zlib
 from typing import Dict, IO, Iterable, Iterator, Optional, Sequence, Tuple
@@ -245,6 +246,47 @@ class GpuKmerCounter:
         n = C.c_uint64(0)
         _check(self._L.kmg_count_fastx(self._ctx, arr.ctypes.data if len(arr) else None, len(arr), int(is_fastq), C.byref(n)), self._ctx)
         return n.value
+
+    def count_stream(self, readable, is_fastq: bool, size_hint: int = 0, block: int = 64 << 20) -> int:
+        """kmg_fastx_stream_*: a FASTA / FASTQ byte stream (sys.stdin.buffer, gzip.open(...), any object with readinto or read)
+        parsed on the device, pushed in blocks of `block` bytes; host memory stays bounded by the block and the staging ring.
+        size_hint: bytes expected (0 = unknown).  A stream the device parser refuses (multi-line FASTQ ...) goes on through the
+        host splitter: the bytes it did not count plus the rest of the stream are split with parse_fastx and fed to count_batch.
+        Returns the records of the whole stream.  An exception from the reader abandons the stream with kmg_reset."""
+        L, ctx = self._L, self._ctx
+        r0 = self.progress()[0]
+        _check(L.kmg_fastx_stream_begin(ctx, int(is_fastq), int(size_hint)), ctx)
+        buf = bytearray(block)
+        addr = C.addressof((C.c_char * block).from_buffer(buf))
+        view = memoryview(buf)
+        st = _lib.KMG_OK
+        try:
+            while st == _lib.KMG_OK:
+                if hasattr(readable, "readinto"):
+                    n = readable.readinto(view) or 0
+                else:
+                    data = readable.read(block)
+                    n = len(data)
+                    view[:n] = data
+                if n == 0:
+                    break
+                st = L.kmg_fastx_stream_push(ctx, addr, n)
+        except BaseException:
+            L.kmg_reset(ctx)
+            raise
+        if st == _lib.KMG_OK:
+            st = L.kmg_fastx_stream_end(ctx, C.byref(C.c_uint64(0)))
+        if st != _lib.KMG_OK:
+            msg = (L.kmg_last_error(ctx) or b"").decode() or L.kmg_status_string(st).decode()
+            n_rest = C.c_uint64(0)
+            if st != _lib.KMG_ERR_PARSE or L.kmg_fastx_stream_rest(ctx, None, 0, C.byref(n_rest)) != _lib.KMG_OK:
+                raise SequenceParseError(msg) if st == _lib.KMG_ERR_PARSE else GpuError(st, msg)
+            rest = np.empty(n_rest.value, dtype=np.uint8)
+            _check(L.kmg_fastx_stream_rest(ctx, rest.ctypes.data, n_rest.value, C.byref(n_rest)), ctx)
+            tail = readable.read()
+            seq, qual, offsets = parse_fastx(rest.tobytes() + (tail or b""), is_fastq)
+            self.count_batch(seq, qual, offsets)
+        return self.progress()[0] - r0
 
     def count_records(self, records: Iterable[bytes], quals: Optional[Iterable[bytes]] = None):
         records = [bytes(r) for r in records]
@@ -527,26 +569,36 @@ def count_kmers_from_sequences(sequences: Iterable[bytes], k: KmerLength) -> Dic
 
 
 def _read_file_image(path, fmt: str):
-    """(bytes of the decompressed file, is_fastq)."""
+    """(bytes of an uncompressed file, is_fastq)."""
     p = os.fspath(path)
-    if p == "-":
-        return sys.stdin.buffer.read(), SequenceFormat.resolve(fmt, None) == SequenceFormat.FASTQ
     try:
         with open(p, "rb") as f:
             data = f.read()
     except OSError as e:
         raise KmeRustError(f"failed to read sequences from '{p}': {e}") from e
-    if p.lower().endswith(".gz"):
-        try:
-            data = gzip.decompress(data)
-        except (OSError, EOFError, zlib.error) as e:
-            raise KmeRustError(f"failed to read sequences from '{p}': {e}") from e
     return data, SequenceFormat.resolve(fmt, p) == SequenceFormat.FASTQ
 
 
 def _feed_file(c: "GpuKmerCounter", path, fmt: str):
-    """File -> counter: records are found on the device (kmg_count_fastx); inputs the device parser refuses (multi-line FASTQ,
-    broken records) go through the host splitter, which reports the reference's parse errors."""
+    """File -> counter: records are found on the device -- stdin ("-") and .gz files as a stream (count_stream), other files as
+    one image (kmg_count_fastx); inputs the device parser refuses (multi-line FASTQ, broken records) go through the host splitter,
+    which reports the reference's parse errors."""
+    p = os.fspath(path)
+    if p == "-":
+        try:
+            st = os.fstat(sys.stdin.buffer.fileno())
+            hint = st.st_size if stat.S_ISREG(st.st_mode) else 0
+        except (OSError, ValueError, AttributeError):
+            hint = 0
+        c.count_stream(sys.stdin.buffer, SequenceFormat.resolve(fmt, None) == SequenceFormat.FASTQ, hint)
+        return
+    if p.lower().endswith(".gz"):
+        try:
+            with gzip.open(p, "rb") as g:
+                c.count_stream(g, SequenceFormat.resolve(fmt, p) == SequenceFormat.FASTQ)
+        except (OSError, EOFError, zlib.error) as e:
+            raise KmeRustError(f"failed to read sequences from '{p}': {e}") from e
+        return
     data, is_fastq = _read_file_image(path, fmt)
     try:
         c.count_fastx(data, is_fastq)

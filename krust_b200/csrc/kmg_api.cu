@@ -116,6 +116,9 @@ struct kmg_ctx {
   size_t scan_tmp_bytes = 0;
   uint64_t scan_tmp_items = 0, fine_cursor_items = 0;
   bool in_resplit = false;
+  struct FxStream *fxs = nullptr;    // an open FASTA / FASTQ stream (kmg_fastx_stream_begin .. _end)
+  std::vector<uint8_t> fx_rest;      // the bytes a refused stream did not count (kmg_fastx_stream_rest)
+  bool fx_rest_ok = false;
   struct ShardShm *shm = nullptr;     // sharded mode (kmg_shard_join): the group's shared segment
   uint32_t sh_world = 1, sh_rank = 0;
   uint64_t *sh_recv = nullptr;        // this rank's SEND buffer: two halves of sh_recv_entries keys (owners pull their regions over NVLink)
@@ -161,6 +164,7 @@ struct kmg_ctx {
 namespace {
 
 void shard_release(kmg_ctx *c);  // defined with the shard group code below
+void fx_stream_close(kmg_ctx *c, bool failed);  // abandons an open FASTA / FASTQ stream (defined with kmg_fastx_stream_begin)
 kmg_status scan_pending_batch(kmg_ctx *c);  // pre-packed feed: scan the batch whose copy is in flight (defined with kmg_submit_batch)
 
 kmg_status fail(kmg_ctx *ctx, kmg_status s, const std::string &msg) {
@@ -175,6 +179,12 @@ kmg_status cuda_fail(kmg_ctx *ctx, cudaError_t e, const char *what) {
   do {                                                           \
     cudaError_t _e = (call);                                     \
     if (_e != cudaSuccess) return cuda_fail(ctx, _e, #call);     \
+  } while (0)
+
+// every feed and every call that reads the table waits for an open FASTA / FASTQ stream to end
+#define NO_OPEN_STREAM(ctx)                                                                                                        \
+  do {                                                                                                                             \
+    if ((ctx)->fxs) return fail(ctx, KMG_ERR_STATE, "a FASTA / FASTQ stream is open on this context: end it with kmg_fastx_stream_end (or kmg_reset)"); \
   } while (0)
 
 inline uint64_t round_up(uint64_t x, uint64_t m) { return (x + m - 1) / m * m; }
@@ -1234,6 +1244,7 @@ KMG_EXPORT void kmg_destroy(kmg_ctx *c) {
   if (c->stream) cudaStreamSynchronize(c->stream);
   if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
   timers_collect(c);
+  if (c->fxs) fx_stream_close(c, true);
   if (c->shm || c->sh_recv) shard_release(c);
   for (auto &r : c->runs) free_run(c, r);
   if (c->has_result) free_run(c, c->result);
@@ -1321,6 +1332,9 @@ KMG_EXPORT kmg_status kmg_create(const kmg_config *cfg, kmg_ctx **out) {
 KMG_EXPORT kmg_status kmg_reset(kmg_ctx *c) {
   if (!c) return KMG_ERR_INVALID_ARG;
   CU(c, cudaSetDevice(c->device));
+  if (c->fxs) fx_stream_close(c, true);  // an open stream is abandoned with everything else
+  std::vector<uint8_t>().swap(c->fx_rest);
+  c->fx_rest_ok = false;
   CU(c, cudaStreamSynchronize(c->copy_stream));
   c->pending_slot = -1;  // a submitted but unscanned pre-packed batch is forgotten with everything else
   if (c->use_dense) CU(c, cudaMemsetAsync(c->dense, 0, c->dense_n * 8, c->stream));
@@ -1345,6 +1359,7 @@ KMG_EXPORT kmg_status kmg_reset(kmg_ctx *c) {
 KMG_EXPORT kmg_status kmg_count_ascii_device(kmg_ctx *c, const uint8_t *d_seq, const uint8_t *d_qual, const uint64_t *d_offsets,
                                              uint64_t n_records, uint64_t n_bytes) {
   if (!c) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   if (c->shm) return fail(c, KMG_ERR_STATE, "context belongs to a shard group: feed it with kmg_shard_count_ascii(_device)");
   if (n_bytes && !d_seq) return fail(c, KMG_ERR_INVALID_ARG, "d_seq is NULL");
   if (((uintptr_t)d_seq & 15) || ((uintptr_t)d_qual & 15)) return fail(c, KMG_ERR_INVALID_ARG, "d_seq / d_qual must be 16-byte aligned");
@@ -1475,6 +1490,29 @@ bool fastq_record_start(const uint8_t *buf, uint64_t len, uint64_t p) {
 
 struct FxChunk { uint64_t pos, len; };
 
+const char *const FX_NO_NEWLINE = "a line is longer than a staging chunk (raise batch_bases or use the host splitter)";
+const char *const FX_NO_RECORD = "no FASTQ record boundary found near a chunk end (multi-line FASTQ? use the host splitter)";
+
+// The last chunk boundary in buf[pos, stop) above pos (the lines after it are read up to len): the start of the last line
+// (FASTA), or the last line start within FASTQ_SYNC_LINES lines that opens a record (FASTQ).  nullptr, or why there is none.
+const char *last_fastx_cut(const uint8_t *buf, uint64_t len, uint64_t pos, uint64_t stop, bool is_fastq, uint64_t *cut) {
+  const void *nl = memrchr(buf + pos, '\n', (size_t)(stop - pos));
+  if (!nl) return FX_NO_NEWLINE;
+  uint64_t p = (uint64_t)((const uint8_t *)nl - buf) + 1;
+  if (is_fastq) {  // step back line by line to a line that opens a record
+    bool found = false;
+    for (int tries = 0; tries < FASTQ_SYNC_LINES && p > pos; ++tries) {
+      if (fastq_record_start(buf, len, p)) { found = true; break; }
+      const void *prev = p >= 2 ? memrchr(buf + pos, '\n', (size_t)(p - 1 - pos)) : nullptr;  // start of the previous line
+      if (!prev) break;
+      p = (uint64_t)((const uint8_t *)prev - buf) + 1;
+    }
+    if (!found || p <= pos) return FX_NO_RECORD;
+  }
+  *cut = p;
+  return nullptr;
+}
+
 // Staging chunks of buf[begin, end) (begin and end at line starts (FASTA) / record starts (FASTQ), or end == len): each holds at
 // most cb bytes and ends at a line start (FASTA) or a record start (FASTQ).
 kmg_status plan_fastx_chunks(kmg_ctx *c, const uint8_t *buf, uint64_t len, uint64_t begin, uint64_t end, bool is_fastq, uint64_t cb,
@@ -1482,21 +1520,8 @@ kmg_status plan_fastx_chunks(kmg_ctx *c, const uint8_t *buf, uint64_t len, uint6
   for (uint64_t pos = begin; pos < end;) {
     uint64_t stop = std::min(end, pos + cb);
     if (stop < end) {
-      const void *nl = memrchr(buf + pos, '\n', (size_t)(stop - pos));
-      if (!nl) return fail(c, KMG_ERR_PARSE, "a line is longer than a staging chunk (raise batch_bases or use the host splitter)");
-      stop = (uint64_t)((const uint8_t *)nl - buf) + 1;
-      if (is_fastq) {  // step back line by line to a line that opens a record
-        uint64_t cut = stop;
-        bool found = false;
-        for (int tries = 0; tries < FASTQ_SYNC_LINES && cut > pos; ++tries) {
-          if (fastq_record_start(buf, len, cut)) { found = true; break; }
-          const void *prev = cut >= 2 ? memrchr(buf + pos, '\n', (size_t)(cut - 1 - pos)) : nullptr;  // start of the previous line
-          if (!prev) break;
-          cut = (uint64_t)((const uint8_t *)prev - buf) + 1;
-        }
-        if (!found || cut <= pos) return fail(c, KMG_ERR_PARSE, "no FASTQ record boundary found near a chunk end (multi-line FASTQ? use the host splitter)");
-        stop = cut;
-      }
+      const char *why = last_fastx_cut(buf, len, pos, stop, is_fastq, &stop);
+      if (why) return fail(c, KMG_ERR_PARSE, why);
     }
     chunks.push_back(FxChunk{pos, stop - pos});
     pos = stop;
@@ -1504,15 +1529,18 @@ kmg_status plan_fastx_chunks(kmg_ctx *c, const uint8_t *buf, uint64_t len, uint6
   return KMG_OK;
 }
 
-// The device parser's driver over the planned chunks of one file image: pooled parse buffers, raw chunks staged through the
-// context's ring (up to N_STAGE - 1 chunks ahead), per chunk the parse kernels, the scatter of sequence (+ quality) bytes and record
-// marks, the carry of a FASTA record's last k-1 bases into the next chunk, and the error words.  step() leaves the chunk packed in
-// the context's stream and hands it to the caller's scan (scan_packed on one context, shard_scan_round in a group).
+// The device parser's driver over chunks that are cut at line (FASTA) / record (FASTQ) starts -- or, in a stream, inside a FASTA
+// sequence line between two non-blank bytes: pooled parse buffers, per chunk the parse kernels, the scatter of sequence
+// (+ quality) bytes and record marks, the carry of a FASTA record's last k-1 bases into the next chunk, and the error words.
+// parse() takes a chunk whose bytes are in (or on their way to) a staging slot and leaves it packed in the context's stream for the
+// caller's scan (scan_packed on one context, shard_scan_round in a group).  Over the planned chunks of one file image, step()
+// stages the raw chunks through the context's ring itself, up to N_STAGE - 1 chunks ahead; a stream fills the slots (FxStream).
 struct FastxFeed {
   kmg_ctx *c;
-  const uint8_t *buf;
-  const std::vector<FxChunk> &chunks;
+  const uint8_t *buf;                  // the file image, or nullptr for a stream
+  const std::vector<FxChunk> *chunks;  // the image's planned chunks
   bool is_fastq, use_q, src_pinned = false;
+  bool refused = false;  // the last parse() refused its chunk's layout before anything of the chunk was counted
   uint64_t K1 = 0, max_len = 0, prev_n = 0, bases = 0;  // prev_n: sequence bases the last chunk left (their tail is the next carry)
   uint8_t *d_kind = nullptr, *d_keep = nullptr, *d_seq = nullptr, *d_qual = nullptr, *d_mark = nullptr, *d_carry = nullptr;
   uint32_t *d_lineno = nullptr, *d_pos_s = nullptr, *d_pos_q = nullptr, *d_misc = nullptr, *h_tot = nullptr;
@@ -1520,17 +1548,19 @@ struct FastxFeed {
   size_t tmp_bytes = 0, staged = 0;
   uint32_t slot0 = 0, thr = 0;
 
-  FastxFeed(kmg_ctx *ctx, const uint8_t *b, const std::vector<FxChunk> &ch, bool fq)
+  FastxFeed(kmg_ctx *ctx, bool fq, const uint8_t *b = nullptr, const std::vector<FxChunk> *ch = nullptr)
       : c(ctx), buf(b), chunks(ch), is_fastq(fq), use_q(fq && ctx->cfg.has_min_quality) {}
   unsigned long long *d_nrec() const { return reinterpret_cast<unsigned long long *>(d_misc); }  // [0..1] n_records (u64)
   uint32_t *d_err() const { return d_misc + 4; }  // [2..3] totals, [4] error word, [5] pending record start
 
-  kmg_status open() {
+  // stream_len: the largest chunk of a stream (the slots are filled by the caller, from pinned memory)
+  kmg_status open(uint64_t stream_len = 0) {
     K1 = (uint64_t)c->k - 1;
     slot0 = c->next_ascii;
-    for (auto &ch : chunks) max_len = std::max(max_len, ch.len);
-    src_pinned = is_pinned_host(buf);
-    kmg_status s = ensure_staging(c, !src_pinned, false, max_len);
+    max_len = stream_len;
+    if (chunks) for (auto &ch : *chunks) max_len = std::max(max_len, ch.len);
+    src_pinned = buf && is_pinned_host(buf);
+    kmg_status s = ensure_staging(c, buf && !src_pinned, false, max_len);  // a stream pins the slots it uses itself
     if (s != KMG_OK) return s;
     tmp_bytes = fastx_scan_tmp_bytes(max_len);
     cudaError_t e = pool_alloc(c, &d_kind, max_len);
@@ -1563,49 +1593,63 @@ struct FastxFeed {
     return KMG_OK;
   }
 
-  kmg_status stage(const FxChunk &ch, Staging &st) {
-    if (st.h2d_pending) { CU(c, cudaEventSynchronize(st.h2d_done)); st.h2d_pending = false; }
+  // Queue the copy of len bytes at src (pinned) into the slot's device buffer once the slot's previous chunk has been consumed.
+  kmg_status copy_to_slot(Staging &st, const uint8_t *src, uint64_t len) {
     if (st.compute_pending) { CU(c, cudaStreamWaitEvent(c->copy_stream, st.compute_done, 0)); }
-    const uint8_t *src = buf + ch.pos;
-    if (!src_pinned) { memcpy(st.h_seq, src, ch.len); src = st.h_seq; }
-    CU(c, cudaMemcpyAsync(st.d_seq, src, ch.len, cudaMemcpyHostToDevice, c->copy_stream));
-    c->h2d_bytes += ch.len;
+    CU(c, cudaMemcpyAsync(st.d_seq, src, len, cudaMemcpyHostToDevice, c->copy_stream));
+    c->h2d_bytes += len;
     CU(c, cudaEventRecord(st.h2d_done, c->copy_stream));
     st.h2d_pending = true;
     return KMG_OK;
   }
 
-  // Chunk i: parse, pack, and -- when it holds sequence bases (with the carry) -- scan(n_words_total).  *scanned tells whether it did.
+  kmg_status stage(const FxChunk &ch, Staging &st) {
+    if (st.h2d_pending) { CU(c, cudaEventSynchronize(st.h2d_done)); st.h2d_pending = false; }
+    const uint8_t *src = buf + ch.pos;
+    if (!src_pinned) { memcpy(st.h_seq, src, ch.len); src = st.h_seq; }
+    return copy_to_slot(st, src, ch.len);
+  }
+
+  // Chunk i of the image: staged ahead, then parsed.
   template <class Scan>
   kmg_status step(size_t i, Scan &&scan, bool *scanned) {
     *scanned = false;
-    for (; staged < chunks.size() && staged < i + N_STAGE; ++staged) {
-      kmg_status ss = stage(chunks[staged], c->st[(slot0 + staged) % N_STAGE]);
+    for (; staged < chunks->size() && staged < i + N_STAGE; ++staged) {
+      kmg_status ss = stage((*chunks)[staged], c->st[(slot0 + staged) % N_STAGE]);
       if (ss != KMG_OK) return ss;
     }
-    Staging &st = c->st[(slot0 + i) % N_STAGE];
-    const FxChunk &ch = chunks[i];
+    const FxChunk &ch = (*chunks)[i];
+    return parse(c->st[(slot0 + i) % N_STAGE], ch.len, buf[ch.pos] == '>', scan, scanned);
+  }
+
+  // The chunk of len bytes whose copy into st was queued last (opens_header: its first byte is '>'): parse, pack, and -- when it
+  // holds sequence bases (with the carry) -- scan(n_words_total).  *scanned tells whether it did.
+  template <class Scan>
+  kmg_status parse(Staging &st, uint64_t len, bool opens_header, Scan &&scan, bool *scanned) {
+    *scanned = false;
+    refused = false;
     uint32_t *err = d_err();
     CU(c, cudaStreamWaitEvent(c->stream, st.h2d_done, 0));
     // a FASTA chunk that does not open with a header continues the previous chunk's last record: its last k-1 bases (and their
     // record marks) are put in front, so that the windows spanning the cut are counted -- and none twice (k-1 bases hold no window)
-    const uint64_t carry = (!is_fastq && buf[ch.pos] != '>') ? std::min<uint64_t>(K1, prev_n) : 0;
-    CU(c, cudaMemsetAsync(d_mark, 0, ch.len + K1 + 64, c->stream));
+    const uint64_t carry = (!is_fastq && !opens_header) ? std::min<uint64_t>(K1, prev_n) : 0;
+    CU(c, cudaMemsetAsync(d_mark, 0, len + K1 + 64, c->stream));
     CU(c, cudaMemsetAsync(err, 0, 4, c->stream));
     if (carry) {
       CU(c, cudaMemcpyAsync(d_seq, d_carry + (K1 - carry), carry, cudaMemcpyDeviceToDevice, c->stream));
       CU(c, cudaMemcpyAsync(d_mark, d_carry + 64 + (K1 - carry), carry, cudaMemcpyDeviceToDevice, c->stream));
     }
-    CU(c, launch_fastx_parse(st.d_seq, ch.len, is_fastq, d_kind, d_keep, d_lineno, d_pos_s, d_pos_q, d_tmp, tmp_bytes, carry, d_seq, d_qual, d_mark,
+    CU(c, launch_fastx_parse(st.d_seq, len, is_fastq, d_kind, d_keep, d_lineno, d_pos_s, d_pos_q, d_tmp, tmp_bytes, carry, d_seq, d_qual, d_mark,
                              d_nrec(), err, h_tot, c->stream));
     CU(c, cudaStreamSynchronize(c->stream));
     const uint32_t total_s = h_tot[0], total_q = h_tot[1], perr = h_tot[2];
+    refused = (perr & 3u) != 0;
     if (perr & 1u) return fail(c, KMG_ERR_PARSE, "FASTQ record does not start with '@' (multi-line FASTQ is not handled by the device parser)");
     if (perr & 2u) return fail(c, KMG_ERR_PARSE, "FASTQ record without a '+' separator line where one is expected");
     if (is_fastq && total_s != total_q) return fail(c, KMG_ERR_PARSE, "sequence and quality lengths differ");
     // a record whose header closed the previous chunk starts with this chunk's first base (the scatter below may raise the flag anew)
     if (!is_fastq && total_s) CU(c, launch_fastx_apply_pending(err + 1, d_mark + carry, c->stream));
-    CU(c, launch_fastx_scatter(st.d_seq, ch.len, is_fastq, d_kind, d_lineno, d_keep, d_pos_s, d_pos_q, carry, total_s, d_seq, use_q ? d_qual : nullptr,
+    CU(c, launch_fastx_scatter(st.d_seq, len, is_fastq, d_kind, d_lineno, d_keep, d_pos_s, d_pos_q, carry, total_s, d_seq, use_q ? d_qual : nullptr,
                                d_mark, d_nrec(), err, c->stream));
     CU(c, cudaEventRecord(st.compute_done, c->stream));  // the raw chunk has been consumed
     st.compute_pending = true;
@@ -1649,7 +1693,7 @@ struct FastxFeed {
   // After the last step (or a failed one): the caller's buffer must be reusable when the call returns.
   void close(bool failed) {
     if (failed) { cudaStreamSynchronize(c->stream); cudaStreamSynchronize(c->copy_stream); }
-    c->next_ascii = (slot0 + (uint32_t)chunks.size()) % N_STAGE;
+    if (chunks) c->next_ascii = (slot0 + (uint32_t)chunks->size()) % N_STAGE;
     for (auto &st : c->st) if (st.h2d_pending && src_pinned) { cudaEventSynchronize(st.h2d_done); st.h2d_pending = false; }
     pool_free(c, d_kind); pool_free(c, d_keep); pool_free(c, d_seq); pool_free(c, d_qual); pool_free(c, d_mark); pool_free(c, d_carry);
     pool_free(c, d_lineno); pool_free(c, d_pos_s); pool_free(c, d_pos_q); pool_free(c, d_misc); pool_free(c, d_tmp);
@@ -1662,6 +1706,7 @@ struct FastxFeed {
 
 KMG_EXPORT kmg_status kmg_count_ascii(kmg_ctx *c, const uint8_t *seq, const uint8_t *qual, const uint64_t *offsets, uint64_t n_records) {
   if (!c) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   if (c->shm) return fail(c, KMG_ERR_STATE, "context belongs to a shard group: feed it with kmg_shard_count_ascii(_device)");
   kmg_status s = check_ascii_layout(c, seq, offsets, n_records);
   if (s != KMG_OK) return s;
@@ -1688,6 +1733,7 @@ KMG_EXPORT kmg_status kmg_count_ascii(kmg_ctx *c, const uint8_t *seq, const uint
 // counted then only if it happens in the first chunk, so callers fall back to kmg_parse_fastx + kmg_count_ascii after kmg_reset.
 KMG_EXPORT kmg_status kmg_count_fastx(kmg_ctx *c, const uint8_t *buf, uint64_t len, int is_fastq, uint64_t *n_records_out) {
   if (!c || (len && !buf)) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   if (c->shm) return fail(c, KMG_ERR_STATE, "context belongs to a shard group: feed it with kmg_shard_count_fastx / kmg_shard_count_ascii(_device)");
   if (n_records_out) *n_records_out = 0;
   if (len == 0) return KMG_OK;
@@ -1705,7 +1751,7 @@ KMG_EXPORT kmg_status kmg_count_fastx(kmg_ctx *c, const uint8_t *buf, uint64_t l
   if (use_q && !c->cfg.expected_distinct && c->mode == kmg_ctx::MODE_UNDECIDED && !c->use_dense) c->plan_scale = (double)len / (double)chunks[0].len;
   else s = decide_mode(c, is_fastq ? len / 2 : len);
   if (s != KMG_OK) return s;
-  FastxFeed feed(c, buf, chunks, is_fastq);
+  FastxFeed feed(c, is_fastq, buf, &chunks);
   s = feed.open();
   uint64_t n_rec = 0;
   for (size_t i = 0; s == KMG_OK && i < chunks.size(); ++i) {
@@ -1717,6 +1763,222 @@ KMG_EXPORT kmg_status kmg_count_fastx(kmg_ctx *c, const uint8_t *buf, uint64_t l
   if (s != KMG_OK) return s;
   c->n_records += n_rec; c->n_bases += feed.bases;
   if (n_records_out) *n_records_out = n_rec;
+  return KMG_OK;
+}
+
+// ---- FASTA / FASTQ byte streams (kmg_fastx_stream_*): the file-image parser over input that arrives in pieces ----------------
+// Pushed bytes fill the ring slot `cur` in place.  A full slot is cut at its last line / record start (plan_fastx_chunks' rules;
+// a FASTA slot without a newline inside its sequence line), the copy of the chunk in front of the cut is queued at once, and then
+// the chunk before it (`pend`) is parsed and scanned, so the copy of chunk i overlaps the kernels of chunk i-1; the bytes after
+// the cut open the other slot.  The stream alternates between two slots of the ring (pinned on first use): host memory is those
+// two slots whatever the stream's length.
+struct FxStream {
+  FastxFeed feed;
+  uint64_t cb = 0;         // bytes a slot holds when it is cut
+  uint32_t slot[2] = {0, 1};  // the ring slots the stream alternates between
+  uint32_t cur = 0;        // the slot being filled
+  uint64_t fill = 0;
+  int pend = -1;           // the slot whose chunk has been queued for the device but not parsed
+  uint64_t pend_len = 0;
+  bool started = false;    // byte 0 has been checked
+  bool mid_line = false;   // the slot being filled continues a FASTA sequence line that the last cut split
+  uint64_t plan_len = 0;   // size hint that scales the quality-filtered plan of the first chunk (as kmg_count_fastx does)
+  uint64_t rec0 = 0, bases0 = 0;           // the context's records / bases before the stream
+  unsigned long long *h_nrec = nullptr;    // pinned: records of the chunks parsed so far, read back without a synchronisation
+  FxStream(kmg_ctx *c, bool fq) : feed(c, fq) {}
+};
+
+namespace {
+
+void fx_stream_close(kmg_ctx *c, bool failed) {
+  FxStream *x = c->fxs;
+  x->feed.close(failed);
+  c->next_ascii = (x->cur + 1) % N_STAGE;
+  if (x->h_nrec) cudaFreeHost(x->h_nrec);
+  delete x;
+  c->fxs = nullptr;
+}
+
+// A refusal that leaves the context usable: the bytes from the refused chunk on -- the pending chunk if it is the refused one,
+// the slot being filled, the caller's bytes this push has not consumed -- become the stream's rest, and the stream closes.
+kmg_status fx_stream_refuse(kmg_ctx *c, const uint8_t *more, uint64_t n_more) {
+  FxStream *x = c->fxs;
+  std::vector<uint8_t>().swap(c->fx_rest);
+  if (x->pend >= 0) c->fx_rest.insert(c->fx_rest.end(), c->st[x->pend].h_seq, c->st[x->pend].h_seq + x->pend_len);
+  c->fx_rest.insert(c->fx_rest.end(), c->st[x->cur].h_seq, c->st[x->cur].h_seq + x->fill);
+  if (n_more) c->fx_rest.insert(c->fx_rest.end(), more, more + n_more);
+  // the records and bases of exactly the chunks counted before the refused one (the refused chunk reached no scatter)
+  const std::string why = c->err;
+  uint64_t n_rec = 0;
+  if (x->feed.records(&n_rec) != KMG_OK) { fx_stream_close(c, true); return KMG_ERR_CUDA; }
+  c->n_records = x->rec0 + n_rec; c->n_bases = x->bases0 + x->feed.bases;
+  c->err = why;
+  c->fx_rest_ok = true;
+  fx_stream_close(c, true);
+  return KMG_ERR_PARSE;
+}
+
+// A failed step: a layout refusal before anything of the chunk was counted keeps the context usable, everything else is final.
+kmg_status fx_stream_fail(kmg_ctx *c, kmg_status s, const uint8_t *more, uint64_t n_more) {
+  if (s == KMG_ERR_PARSE && c->fxs->feed.refused) return fx_stream_refuse(c, more, n_more);
+  fx_stream_close(c, true);
+  return s;
+}
+
+// Parse and scan the pending chunk; the context's progress then counts the bases of every parsed chunk and the records of all
+// chunks before it.
+kmg_status fx_stream_parse_pending(kmg_ctx *c) {
+  FxStream *x = c->fxs;
+  if (x->pend < 0) return KMG_OK;
+  Staging &st = c->st[x->pend];
+  if (x->plan_len) { c->plan_scale = (double)x->plan_len / (double)x->pend_len; x->plan_len = 0; }
+  bool scanned = false;
+  kmg_status s = x->feed.parse(st, x->pend_len, st.h_seq[0] == '>', [&](uint64_t n_words_total) { return scan_packed(c, n_words_total, true); },
+                               &scanned);
+  if (s != KMG_OK) return s;
+  x->pend = -1;
+  c->n_records = x->rec0 + *x->h_nrec;  // copied behind the previous chunk, complete since the parse synchronised
+  CU(c, cudaMemcpyAsync(x->h_nrec, x->feed.d_nrec(), 8, cudaMemcpyDeviceToHost, c->stream));
+  c->n_bases = x->bases0 + x->feed.bases;
+  return KMG_OK;
+}
+
+// The slot being filled holds cb bytes: cut it, queue the chunk's copy, count the pending chunk, move the rest to the next slot.
+// more / n_more: the bytes of the current push not consumed yet (part of the rest if the stream is refused).
+kmg_status fx_stream_flush(kmg_ctx *c, const uint8_t *more, uint64_t n_more) {
+  FxStream *x = c->fxs;
+  Staging &st = c->st[x->cur];
+  const uint8_t *b = st.h_seq;
+  uint64_t cut = 0;
+  const char *why = last_fastx_cut(b, x->fill, 0, x->fill, x->feed.is_fastq, &cut);
+  bool mid = false;
+  if (why == FX_NO_NEWLINE && !x->feed.is_fastq) {
+    // a sequence line longer than a slot is cut between two non-blank bytes, not before a '>' (the next chunk must not open a
+    // header); a slot that opens a header line holds no such position
+    why = "a FASTA header line is longer than a staging chunk, or a sequence line holds no cut between two non-blank bytes";
+    if (x->mid_line || b[0] != '>') {
+      auto blank = [](uint8_t v) { return v == ' ' || (v >= 9 && v <= 13); };
+      for (uint64_t p = x->fill - 1; p > 0; --p)
+        if (!blank(b[p - 1]) && !blank(b[p]) && b[p] != '>') { cut = p; why = nullptr; mid = true; break; }
+    }
+  }
+  kmg_status s = KMG_OK;
+  if (why) {
+    if ((s = fx_stream_parse_pending(c)) != KMG_OK) return fx_stream_fail(c, s, more, n_more);
+    fail(c, KMG_ERR_PARSE, why);
+    return fx_stream_refuse(c, more, n_more);
+  }
+  if ((s = x->feed.copy_to_slot(st, b, cut)) != KMG_OK) return fx_stream_fail(c, s, more, n_more);
+  if ((s = fx_stream_parse_pending(c)) != KMG_OK) return fx_stream_fail(c, s, more, n_more);
+  const uint32_t nxt = x->cur == x->slot[0] ? x->slot[1] : x->slot[0];
+  Staging &ns = c->st[nxt];
+  if (ns.h2d_pending) {
+    const cudaError_t e = cudaEventSynchronize(ns.h2d_done);  // the slot's last chunk has left the host
+    if (e != cudaSuccess) { cuda_fail(c, e, "cudaEventSynchronize(h2d_done)"); return fx_stream_fail(c, KMG_ERR_CUDA, more, n_more); }
+    ns.h2d_pending = false;
+  }
+  memcpy(ns.h_seq, b + cut, x->fill - cut);
+  x->pend = (int)x->cur; x->pend_len = cut;
+  x->cur = nxt; x->fill -= cut; x->mid_line = mid;
+  return KMG_OK;
+}
+
+}  // namespace
+
+KMG_EXPORT kmg_status kmg_fastx_stream_begin(kmg_ctx *c, int is_fastq, uint64_t size_hint) {
+  if (!c) return KMG_ERR_INVALID_ARG;
+  if (c->shm) return fail(c, KMG_ERR_STATE, "context belongs to a shard group: a stream is counted on a context of its own");
+  if (c->fxs) return fail(c, KMG_ERR_STATE, "a FASTA / FASTQ stream is already open on this context");
+  CU(c, cudaSetDevice(c->device));
+  std::vector<uint8_t>().swap(c->fx_rest);
+  c->fx_rest_ok = false;
+  kmg_status s = scan_pending_batch(c);  // the pre-packed feed's last batch uses the ring's events
+  if (s != KMG_OK) return s;
+  // a slot holds a chunk of min(batch_bases, 2^30) bytes; a known small stream gets smaller slots (1 MiB at least)
+  uint64_t cb = std::min<uint64_t>(c->batch_bases, 1ull << 30);
+  if (size_hint) cb = std::min<uint64_t>(cb, std::max<uint64_t>(round_up(size_hint, 64), 1ull << 20));
+  const bool use_q = is_fastq && c->cfg.has_min_quality;
+  FxStream *x = new FxStream(c, is_fastq != 0);
+  x->cb = cb;
+  if (size_hint) {  // plan the table / partitions for the whole stream, as kmg_count_fastx does for a file
+    if (use_q && !c->cfg.expected_distinct && c->mode == kmg_ctx::MODE_UNDECIDED && !c->use_dense) x->plan_len = size_hint;
+    else s = decide_mode(c, is_fastq ? size_hint / 2 : size_hint);
+  }
+  if (s == KMG_OK) s = x->feed.open(cb);
+  cudaError_t e = cudaSuccess;
+  if (s == KMG_OK) {
+    x->slot[0] = x->cur = c->next_ascii;
+    x->slot[1] = (c->next_ascii + 1) % N_STAGE;
+    e = cudaHostAlloc(&x->h_nrec, 8, cudaHostAllocDefault);
+    for (uint32_t i : x->slot) {
+      Staging &st = c->st[i];
+      if (e == cudaSuccess && !st.h_seq) e = cudaHostAlloc(&st.h_seq, c->staging_cap, cudaHostAllocDefault);
+    }
+    Staging &st = c->st[x->cur];
+    if (e == cudaSuccess && st.h2d_pending) e = cudaEventSynchronize(st.h2d_done);
+    if (e == cudaSuccess) { *x->h_nrec = 0; st.h2d_pending = false; }
+    else s = cuda_fail(c, e, "stream ring");
+  }
+  x->rec0 = c->n_records; x->bases0 = c->n_bases;
+  c->fxs = x;
+  if (s != KMG_OK) fx_stream_close(c, true);
+  return s;
+}
+
+KMG_EXPORT kmg_status kmg_fastx_stream_push(kmg_ctx *c, const uint8_t *bytes, uint64_t n) {
+  if (!c) return KMG_ERR_INVALID_ARG;
+  if (!c->fxs) return fail(c, KMG_ERR_STATE, "no FASTA / FASTQ stream is open on this context (kmg_fastx_stream_begin)");
+  if (n && !bytes) return fail(c, KMG_ERR_INVALID_ARG, "bytes is NULL");
+  CU(c, cudaSetDevice(c->device));
+  FxStream *x = c->fxs;
+  if (n && !x->started) {
+    x->started = true;
+    if (bytes[0] != (x->feed.is_fastq ? '@' : '>')) {
+      fail(c, KMG_ERR_PARSE, x->feed.is_fastq ? "FASTQ record does not start with '@' (record 0)" : "FASTA record does not start with '>' (record 0)");
+      return fx_stream_refuse(c, bytes, n);
+    }
+  }
+  while (n) {
+    const uint64_t take = std::min<uint64_t>(n, x->cb - x->fill);
+    memcpy(c->st[x->cur].h_seq + x->fill, bytes, take);
+    x->fill += take; bytes += take; n -= take;
+    if (x->fill == x->cb) {
+      const kmg_status s = fx_stream_flush(c, bytes, n);
+      if (s != KMG_OK) return s;
+    }
+  }
+  return KMG_OK;
+}
+
+KMG_EXPORT kmg_status kmg_fastx_stream_end(kmg_ctx *c, uint64_t *n_records_out) {
+  if (!c) return KMG_ERR_INVALID_ARG;
+  if (n_records_out) *n_records_out = 0;
+  if (!c->fxs) return fail(c, KMG_ERR_STATE, "no FASTA / FASTQ stream is open on this context (kmg_fastx_stream_begin)");
+  CU(c, cudaSetDevice(c->device));
+  FxStream *x = c->fxs;
+  Staging &st = c->st[x->cur];
+  kmg_status s = x->fill ? x->feed.copy_to_slot(st, st.h_seq, x->fill) : KMG_OK;
+  if (s == KMG_OK) s = fx_stream_parse_pending(c);
+  if (s == KMG_OK && x->fill) {  // the last chunk: whatever is left, a last line without '\n' included
+    x->pend = (int)x->cur; x->pend_len = x->fill; x->fill = 0;
+    s = fx_stream_parse_pending(c);
+  }
+  uint64_t n_rec = 0;
+  if (s == KMG_OK) s = x->feed.records(&n_rec);
+  if (s != KMG_OK) return fx_stream_fail(c, s, nullptr, 0);
+  c->n_records = x->rec0 + n_rec; c->n_bases = x->bases0 + x->feed.bases;
+  fx_stream_close(c, false);
+  if (n_records_out) *n_records_out = n_rec;
+  return KMG_OK;
+}
+
+KMG_EXPORT kmg_status kmg_fastx_stream_rest(kmg_ctx *c, uint8_t *bytes, uint64_t cap, uint64_t *n_out) {
+  if (!c || !n_out) return KMG_ERR_INVALID_ARG;
+  if (!c->fx_rest_ok) return fail(c, KMG_ERR_STATE, "no refused stream: the rest exists after a KMG_ERR_PARSE that left the context usable");
+  *n_out = c->fx_rest.size();
+  if (!bytes) return KMG_OK;
+  if (cap < c->fx_rest.size()) return fail(c, KMG_ERR_CAPACITY, "rest needs " + std::to_string(c->fx_rest.size()) + " bytes");
+  if (!c->fx_rest.empty()) memcpy(bytes, c->fx_rest.data(), c->fx_rest.size());
   return KMG_OK;
 }
 
@@ -1745,6 +2007,7 @@ kmg_status scan_pending_batch(kmg_ctx *c) {
 
 KMG_EXPORT kmg_status kmg_acquire_batch(kmg_ctx *c, kmg_batch *b) {
   if (!c || !b) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   CU(c, cudaSetDevice(c->device));
   const uint64_t words = round_up((c->batch_bases + 31) / 32, TILE_WORDS);
   if (!c->packed_feed_ready) {
@@ -1787,6 +2050,7 @@ KMG_EXPORT kmg_status kmg_acquire_batch(kmg_ctx *c, kmg_batch *b) {
 
 KMG_EXPORT kmg_status kmg_submit_batch(kmg_ctx *c, const kmg_batch *b) {
   if (!c || !b) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   if (c->shm) return fail(c, KMG_ERR_STATE, "context belongs to a shard group: feed it with kmg_shard_count_ascii(_device)");
   if (b->slot >= (uint32_t)N_STAGE || !c->packed_feed_ready || b->bases2bit != c->st[b->slot].hp_bases)
     return fail(c, KMG_ERR_STATE, "batch was not obtained from kmg_acquire_batch");
@@ -1813,6 +2077,7 @@ KMG_EXPORT kmg_status kmg_submit_batch(kmg_ctx *c, const kmg_batch *b) {
 
 KMG_EXPORT kmg_status kmg_insert_keys_device(kmg_ctx *c, const uint64_t *d_keys, const uint64_t *d_counts, uint64_t n) {
   if (!c) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   if (c->shm) return fail(c, KMG_ERR_STATE, "context belongs to a shard group: feed it with kmg_shard_count_ascii(_device)");
   if (n == 0) return KMG_OK;
   if (!d_keys) return fail(c, KMG_ERR_INVALID_ARG, "d_keys is NULL");
@@ -1834,6 +2099,7 @@ KMG_EXPORT kmg_status kmg_insert_keys_device(kmg_ctx *c, const uint64_t *d_keys,
 
 KMG_EXPORT kmg_status kmg_partition_plan(kmg_ctx *c, uint64_t expected_keys, uint32_t *n_coarse, uint32_t *n_sub) {
   if (!c) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   CU(c, cudaSetDevice(c->device));
   if (c->mode == kmg_ctx::MODE_UNDECIDED) {
     if (c->use_dense) return fail(c, KMG_ERR_STATE, "context uses the direct-indexed path; create it with KMG_FLAG_FORCE_PARTITIONED");
@@ -1850,6 +2116,7 @@ KMG_EXPORT kmg_status kmg_partition_plan(kmg_ctx *c, uint64_t expected_keys, uin
 
 KMG_EXPORT kmg_status kmg_adopt_coarse_device(kmg_ctx *c, const uint64_t *d_keys, const uint64_t *bin_counts, uint32_t n_bins, uint64_t n) {
   if (!c || !bin_counts) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   if (c->shm) return fail(c, KMG_ERR_STATE, "context belongs to a shard group: feed it with kmg_shard_count_ascii(_device)");
   if (c->mode != kmg_ctx::MODE_PARTITIONED) return fail(c, KMG_ERR_STATE, "call kmg_partition_plan first");
   if (n_bins != c->n_coarse) return fail(c, KMG_ERR_INVALID_ARG, "n_bins must equal the context's coarse partition count");
@@ -1873,6 +2140,7 @@ KMG_EXPORT kmg_status kmg_extract_keys_device(kmg_ctx *c, const uint8_t *d_seq, 
                                               uint64_t n_records, uint64_t n_bytes, uint32_t n_shards, uint64_t *d_keys_out,
                                               uint64_t cap, uint64_t *shard_counts_out) {
   if (!c || !shard_counts_out) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   if (n_shards < 1 || n_shards > (uint32_t)MAX_PARTS) return fail(c, KMG_ERR_INVALID_ARG, "n_shards must be in 1..=8192");
   if (((uintptr_t)d_seq & 15) || ((uintptr_t)d_qual & 15)) return fail(c, KMG_ERR_INVALID_ARG, "d_seq / d_qual must be 16-byte aligned");
   CU(c, cudaSetDevice(c->device));
@@ -2168,6 +2436,7 @@ kmg_status shard_scan_round(kmg_ctx *c, uint64_t n_words_total, bool has_start) 
 
 KMG_EXPORT kmg_status kmg_shard_join(kmg_ctx *c, uint32_t world, uint32_t rank, const char *group, uint64_t expected_keys_total) {
   if (!c || !group || !*group) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   if (world < 1 || world > SHARD_MAX_WORLD || rank >= world) return fail(c, KMG_ERR_INVALID_ARG, "world must be 1..=8 and rank < world");
   if (c->shm || c->sh_world > 1) return fail(c, KMG_ERR_STATE, "context already belongs to a shard group");
   if (c->mode != kmg_ctx::MODE_UNDECIDED) return fail(c, KMG_ERR_STATE, "kmg_shard_join must come before the first feeding call");
@@ -2408,7 +2677,7 @@ KMG_EXPORT kmg_status kmg_shard_count_fastx(kmg_ctx *c, const uint8_t *buf, uint
   if (!planned)
     return shard_fail(c, KMG_ERR_PARSE, plan != KMG_OK ? c->err : "another rank's slice cannot be cut into staging chunks (a line longer than a chunk, or multi-line FASTQ)");
   // ---- rounds: parse -> pack -> fused scatter + exchange; a rank without chunks left takes part with empty rounds
-  FastxFeed feed(c, buf, chunks, is_fastq);
+  FastxFeed feed(c, is_fastq, buf, &chunks);
   if (!chunks.empty()) {
     s = feed.open();
     if (s == KMG_OK && !is_fastq && buf[begin] != '>') {
@@ -2438,6 +2707,7 @@ KMG_EXPORT kmg_status kmg_shard_count_fastx(kmg_ctx *c, const uint8_t *buf, uint
 
 KMG_EXPORT kmg_status kmg_finalize(kmg_ctx *c, kmg_summary *out) {
   if (!c) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   CU(c, cudaSetDevice(c->device));
   { kmg_status _fs = scan_pending_batch(c); if (_fs != KMG_OK) return _fs; }
   CU(c, cudaStreamSynchronize(c->copy_stream));
@@ -2494,6 +2764,7 @@ kmg_status count_filtered(kmg_ctx *c, uint64_t min_count, uint64_t *n, uint64_t 
 kmg_status export_device(kmg_ctx *c, uint64_t min_count, int sorted, uint64_t shard_mod, uint64_t shard_rem, uint64_t *d_keys,
                          uint64_t *d_counts, uint64_t cap, uint64_t *n_out) {
   if (!c || !n_out) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   if (shard_mod > 1 && shard_rem >= shard_mod) return fail(c, KMG_ERR_INVALID_ARG, "shard must be < n_shards");
   CU(c, cudaSetDevice(c->device));
   uint64_t n = 0;
@@ -2513,6 +2784,7 @@ kmg_status export_device(kmg_ctx *c, uint64_t min_count, int sorted, uint64_t sh
 kmg_status export_host(kmg_ctx *c, uint64_t min_count, int sorted, uint64_t shard_mod, uint64_t shard_rem, uint64_t *keys,
                        uint64_t *counts, uint64_t cap, uint64_t *n_out) {
   if (!c || !n_out) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   if (shard_mod > 1 && shard_rem >= shard_mod) return fail(c, KMG_ERR_INVALID_ARG, "shard must be < n_shards");
   CU(c, cudaSetDevice(c->device));
   uint64_t n = 0;
@@ -2561,6 +2833,7 @@ KMG_EXPORT kmg_status kmg_export_shard_device(kmg_ctx *c, uint64_t min_count, in
 
 KMG_EXPORT kmg_status kmg_histogram(kmg_ctx *c, uint64_t min_count, uint64_t *count_vals, uint64_t *freqs, uint64_t cap, uint64_t *n_out) {
   if (!c || !n_out) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   CU(c, cudaSetDevice(c->device));
   { kmg_status _fs = scan_pending_batch(c); if (_fs != KMG_OK) return _fs; }
   CU(c, cudaStreamSynchronize(c->copy_stream));
@@ -2866,6 +3139,7 @@ bool has_gz_suffix(const char *path) { const size_t l = strlen(path); return l >
 
 KMG_EXPORT kmg_status kmg_save_kmix(kmg_ctx *c, const char *path) {
   if (!c || !path) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   // src/index.rs:159-168 gzips when the path ends in .gz; this writer does not compress -- refuse rather than write raw bytes
   // under a .gz name (the reference's load_index would reject that file)
   if (has_gz_suffix(path)) return fail(c, KMG_ERR_INVALID_ARG, "kmg_save_kmix writes uncompressed .kmix files; gzip on the host side for a .gz path");
@@ -2903,6 +3177,7 @@ KMG_EXPORT kmg_status kmg_kmix_begin(const char *path) {
 }
 KMG_EXPORT kmg_status kmg_save_kmix_shard(kmg_ctx *c, const char *path, uint64_t record_offset, uint64_t *n_records_out, uint32_t *crc_out) {
   if (!c || !path || !n_records_out || !crc_out) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   CU(c, cudaSetDevice(c->device));
   FILE *f = fopen(path, "r+b");
   if (!f) return fail(c, KMG_ERR_IO, std::string("cannot open ") + path + " (call kmg_kmix_begin first)");
@@ -3047,6 +3322,7 @@ KMG_EXPORT kmg_status kmg_shard_stats(const kmg_ctx *c, uint64_t *sent_keys, uin
 KMG_EXPORT kmg_status kmg_emit_text(kmg_ctx *c, uint64_t min_count, int format, kmg_text_sink sink, void *user, uint64_t *n_records_out,
                                     uint64_t *n_bytes_out) {
   if (!c || !sink) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   if (format != KMG_TEXT_FASTA && format != KMG_TEXT_TSV && format != KMG_TEXT_JSON)
     return fail(c, KMG_ERR_INVALID_ARG, "format must be KMG_TEXT_FASTA, KMG_TEXT_TSV or KMG_TEXT_JSON");
   CU(c, cudaSetDevice(c->device));
@@ -3083,6 +3359,7 @@ int file_sink(void *user, const uint8_t *p, size_t n) { return fwrite(p, 1, n, s
 // The same into a file ("-" = stdout): what `kmerust <k> <path> --format tsv|fasta|json --min-count m > file` produces, sorted.
 KMG_EXPORT kmg_status kmg_write_text(kmg_ctx *c, uint64_t min_count, int format, const char *path, uint64_t *n_records_out, uint64_t *n_bytes_out) {
   if (!c || !path) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   const bool to_stdout = strcmp(path, "-") == 0;
   FILE *f = to_stdout ? stdout : fopen(path, "wb");
   if (!f) return fail(c, KMG_ERR_IO, std::string("cannot open ") + path + " for writing");
@@ -3282,6 +3559,7 @@ kmg_status query_device_keys(kmg_ctx *c, const uint64_t *d_keys, uint64_t n, uin
 // counts_out[i] = count of the canonical packed key keys[i] (0 when absent).  HOST arrays.
 KMG_EXPORT kmg_status kmg_query_keys(kmg_ctx *c, const uint64_t *keys, uint64_t n, uint64_t *counts_out) {
   if (!c || (n && (!keys || !counts_out))) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   if (n == 0) return KMG_OK;
   CU(c, cudaSetDevice(c->device));
   uint64_t *d_keys = nullptr;
@@ -3296,6 +3574,7 @@ KMG_EXPORT kmg_status kmg_query_keys(kmg_ctx *c, const uint64_t *keys, uint64_t 
 // query subcommand does on the host) and looked up.  A k-mer with a byte outside ACGTacgt counts 0 and sets *n_invalid_out.
 KMG_EXPORT kmg_status kmg_query_ascii(kmg_ctx *c, const uint8_t *kmers, uint64_t n, uint64_t *counts_out, uint64_t *n_invalid_out) {
   if (!c || (n && (!kmers || !counts_out))) return KMG_ERR_INVALID_ARG;
+  NO_OPEN_STREAM(c);
   if (n_invalid_out) *n_invalid_out = 0;
   if (n == 0) return KMG_OK;
   CU(c, cudaSetDevice(c->device));

@@ -238,6 +238,44 @@ class GpuKmerCounter {
     check(s);
     return true;
   }
+  // A FASTA / FASTQ byte stream (stdin through fread, a .gz file through gzread) parsed on the device in blocks of 64 MiB; host
+  // memory stays bounded by the block and the staging ring (kmg_fastx_stream_*).  A stream the device parser refuses (multi-line
+  // FASTQ ...) goes on through the host splitter: the bytes it did not count plus the rest of the input are split with
+  // kmg_parse_fastx and counted with count().  Returns the records of the whole stream.
+  uint64_t count_stream(FILE *f, bool is_fastq, uint64_t size_hint = 0) {
+    return count_stream_from([f](uint8_t *b, size_t cap) -> long { const size_t n = fread(b, 1, cap, f); return ferror(f) ? -1 : (long)n; },
+                             is_fastq, size_hint);
+  }
+  uint64_t count_stream(gzFile g, bool is_fastq, uint64_t size_hint = 0) {
+    return count_stream_from([g](uint8_t *b, size_t cap) -> long { return (long)gzread(g, b, (unsigned)cap); }, is_fastq, size_hint);
+  }
+  // read(buf, cap): bytes read, 0 at the end, < 0 on a read error
+  template <class Read>
+  uint64_t count_stream_from(Read &&read, bool is_fastq, uint64_t size_hint) {
+    constexpr size_t BLOCK = 64u << 20;
+    const uint64_t r0 = progress().sequences_processed;
+    check(kmg_fastx_stream_begin(ctx_, is_fastq, size_hint));
+    std::vector<uint8_t> block(BLOCK);
+    kmg_status s = KMG_OK;
+    long n = 0;
+    while (s == KMG_OK && (n = read(block.data(), BLOCK)) > 0) s = kmg_fastx_stream_push(ctx_, block.data(), (uint64_t)n);
+    if (n < 0) { kmg_reset(ctx_); throw SequenceReadError("failed to read sequences from the input stream"); }
+    if (s == KMG_OK) { uint64_t recs = 0; s = kmg_fastx_stream_end(ctx_, &recs); }
+    if (s != KMG_OK) {
+      const std::string msg = kmg_last_error(ctx_);
+      uint64_t n_rest = 0;
+      if (s != KMG_ERR_PARSE || kmg_fastx_stream_rest(ctx_, nullptr, 0, &n_rest) != KMG_OK) {
+        if (s == KMG_ERR_PARSE) throw SequenceParseError(msg);
+        throw GpuError(s, msg);
+      }
+      std::vector<uint8_t> data(n_rest);
+      check(kmg_fastx_stream_rest(ctx_, data.data(), n_rest, &n_rest));
+      while ((n = read(block.data(), BLOCK)) > 0) data.insert(data.end(), block.data(), block.data() + n);
+      if (n < 0) throw SequenceReadError("failed to read sequences from the input stream");
+      count(parse_records(data, is_fastq));
+    }
+    return progress().sequences_processed - r0;
+  }
   // fasta / tsv / json records formatted on the device, sorted by k-mer (kmg_write_text; "-" = stdout)
   uint64_t write_text(const std::string &path, OutputFormat fmt, uint64_t min_count) {
     if (fmt == OutputFormat::Histogram) throw KmeRustError("write_text formats fasta, tsv or json; the histogram comes from histogram()");

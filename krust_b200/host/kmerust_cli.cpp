@@ -108,12 +108,21 @@ int main(int argc, char **argv) {
   try {
     const KmerLength kl = KmerLength::create(k);
     GpuKmerCounter counter(kl, min_quality);
-    bool fed = false;
-    if (path != "-") {  // file image -> device parser; refused inputs (multi-line FASTQ ...) take the host splitter below
+    const bool is_fastq = resolved == SequenceFormat::Fastq;
+    if (path == "-") {  // stdin and .gz files stream through the device parser, in host memory bounded by its staging ring
+      struct stat sb;
+      const uint64_t hint = fstat(fileno(stdin), &sb) == 0 && S_ISREG(sb.st_mode) ? (uint64_t)sb.st_size : 0;
+      counter.count_stream(stdin, is_fastq, hint);
+    } else if (ends_with(lower(path), ".gz")) {
+      gzFile g = gzopen(path.c_str(), "rb");
+      if (!g) throw SequenceReadError("failed to read sequences from '" + path + "'");
+      gzbuffer(g, 1u << 20);
+      try { counter.count_stream(g, is_fastq); } catch (...) { gzclose(g); throw; }
+      gzclose(g);
+    } else {  // file image -> device parser; refused inputs (multi-line FASTQ ...) take the host splitter
       const std::vector<uint8_t> image = slurp(path);
-      fed = counter.count_file_image(image.data(), image.size(), resolved == SequenceFormat::Fastq);
+      if (!counter.count_file_image(image.data(), image.size(), is_fastq)) counter.count(read_with_quality(path, resolved));
     }
-    if (!fed) counter.count(read_with_quality(path, resolved));
     kmg_summary s = counter.finalize();
     if (!save.empty()) {  // the index holds ALL k-mers; --min-count only filters stdout (src/main.rs:155-212)
       try { counter.save_kmix(save); } catch (const KmeRustError &e) { die("Failed to save index:", e.what()); }
