@@ -1603,13 +1603,22 @@ __global__ void __launch_bounds__(SVT_THREADS, 2) count_partitions_sieve_tma_ker
 // The passes are those of the TMA sieve above.  Without a bulk store the stage only has to live until the queue is resolved, so a
 // CTA has one key stage and keeps no keys in registers across its barriers (pass 2 and the queue re-read the stage); the next
 // partition's bulk load is issued right after barrier D.  The shared memory a second stage would take holds more partitions in
-// flight instead: four 256-thread CTAs per SM, whose chains of a bulk load and four block barriers per partition overlap.  The bit
-// map is 2^16 bits: a partition of ~3500 keys has ~90 suspects and a queue of ~300 entries, well inside SVT_Q and SVT_L_MAX.
+// flight instead: four 256-thread CTAs per SM, whose chains of a bulk load and four block barriers per partition overlap.
+// The map is 2^16 bits (2048 words), and a key sets TWO bits of one word with one atomic OR: word (lo >> 5) & 2047, bits lo & 31
+// and (lo >> 16) & 31 of the key's low half lo.  A key is a suspect iff both were already set.  Of two equal keys, the one whose OR
+// comes second sees both bits of the other, so every repeat makes a suspect; a distinct key is a (false) suspect only when both
+// its bits were set by other keys of its word.  Bits 0-20 of lo vary freely inside a partition (sub_of_mix takes at most 11 top
+// bits of lo, the coarse bin comes from the high half).  A partition of ~3500 keys has ~22 suspects and a queue of ~50 entries
+// (one bit per key: ~90 and ~250), well inside SVT_Q and SVT_L_MAX.  The queue is dealt out across the warps (entry e to lane
+// e / 8 of warp e % 8), so that no warp carries a chain of probes that the others wait for at barrier D, and the entry that claims
+// a slot of L notes the slot in its queue entry: after barrier D only the claimed slots are read and cleaned.
 // ---------------------------------------------------------------------------------------------------
 constexpr int SVI_THREADS = 256, SVI_G = 16, SVI_BATCH = 8, SVI_CTAS_PER_SM = 4;
 constexpr uint32_t SVI_BM_WORDS = 1u << (16 - 5);  // 8 KiB
 static_assert(SVI_THREADS * SVI_G == (int)SVT_CAP, "one stage per partition");
+static_assert(SVT_CAP <= 0x8000u && SVT_L_SLOTS <= 0x8000u, "a queue entry holds a stage index or a flagged slot of L");
 constexpr size_t SVI_SMEM = (size_t)SVT_CAP * 8 + (size_t)SVI_BM_WORDS * 4 + (size_t)SVT_L_SLOTS * 8 + (size_t)SVT_Q * 2;
+__device__ __forceinline__ uint32_t svi_map_bits(uint32_t lo) { return __funnelshift_l(0u, 1u, lo) | __funnelshift_l(0u, 1u, lo >> 16); }
 
 __global__ void __launch_bounds__(SVI_THREADS, SVI_CTAS_PER_SM) count_partitions_sieve_in_place_kernel(CountParams P) {
   extern __shared__ __align__(128) unsigned char svi_raw[];
@@ -1710,11 +1719,13 @@ __global__ void __launch_bounds__(SVI_THREADS, SVI_CTAS_PER_SM) count_partitions
           const bool lv = idx < np;           // not the pad entry behind a segment of odd length
           live |= (lv ? 1u : 0u) << (h + j);
           if (idx < P.part_cap) __stcs(P.out_counts + base + idx, lv ? 1ull : 0ull);
-          old[j] = lv ? atomicOr(&bm[(lo[j] >> 5) & (SVI_BM_WORDS - 1)], __funnelshift_l(0u, 1u, lo[j])) : 0u;
+          old[j] = lv ? atomicOr(&bm[(lo[j] >> 5) & (SVI_BM_WORDS - 1)], svi_map_bits(lo[j])) : 0u;
         }
 #pragma unroll
-        for (int j = 0; j < SVI_BATCH; ++j)  // a suspect (its bit was already set) marks the filter
-          if (__funnelshift_r(old[j], 0u, lo[j]) & 1u) atomicOr(&s_bloom[(lo[j] >> 5) & (SVT_BLOOM_WORDS - 1)], __funnelshift_l(0u, 1u, lo[j]));
+        for (int j = 0; j < SVI_BATCH; ++j) {  // a suspect (both its bits were already set) marks the filter
+          const uint32_t m = svi_map_bits(lo[j]);
+          if ((old[j] & m) == m) atomicOr(&s_bloom[(lo[j] >> 5) & (SVT_BLOOM_WORDS - 1)], __funnelshift_l(0u, 1u, lo[j]));
+        }
       }
       for (uint32_t i = (uint32_t)G * T + tid; i < P.part_cap; i += T) __stcs(P.out_counts + base + i, 0ull);  // the capacity may exceed one stage
       __syncthreads();  // B: bit map and filter complete
@@ -1745,8 +1756,9 @@ __global__ void __launch_bounds__(SVI_THREADS, SVI_CTAS_PER_SM) count_partitions
       __syncthreads();  // C: the queue is complete
       const uint32_t nq = s_nq;
       // ---- resolve the queue: entry e claims a slot of L for its key or meets the entry that did
+      const uint32_t e0 = (uint32_t)(tid & 31) * (T / 32) + (uint32_t)(tid >> 5);  // this thread's first entry
       if (nq <= SVT_Q)
-        for (uint32_t e = tid; e < nq; e += T) {
+        for (uint32_t e = e0; e < nq; e += T) {
           const uint32_t idx = Q[e];
           const unsigned long long k = st[idx];
           uint32_t s = (uint32_t)(k >> 32) & (SVT_L_SLOTS - 1);
@@ -1758,6 +1770,7 @@ __global__ void __launch_bounds__(SVI_THREADS, SVI_CTAS_PER_SM) count_partitions
               cur = atomicCAS(&Lslot[s], 0u, idx + 1u);
               if (cur == 0u) {
                 if (atomicAdd(&s_nL, 1u) >= SVT_L_MAX) atomicExch(&s_fail, 1u);
+                Q[e] = (uint16_t)(0x8000u | s);  // read back after barrier D
                 break;
               }
             }
@@ -1773,22 +1786,19 @@ __global__ void __launch_bounds__(SVI_THREADS, SVI_CTAS_PER_SM) count_partitions
       __syncthreads();  // D: L's counters are final; nobody reads the stage any more
       if (tid == 0) issue(sl_next);
       const bool fail = nq > SVT_Q || s_fail != 0;
-      {  // the entries that own a slot of L carry their key's count; L is cleaned (one slot quad per thread)
-        static_assert(SVT_L_SLOTS == 4 * T, "one uint4 of L per thread");
-        uint4 *ls4 = reinterpret_cast<uint4 *>(Lslot) + tid, *lc4 = reinterpret_cast<uint4 *>(Lcnt) + tid;
-        const uint4 ls = *ls4, lc = *lc4;
-        if (!fail && (lc.x | lc.y | lc.z | lc.w)) {
-          const uint32_t own[4] = {ls.x, ls.y, ls.z, ls.w}, more[4] = {lc.x, lc.y, lc.z, lc.w};
-#pragma unroll
-          for (int u = 0; u < 4; ++u) {
-            if (!more[u]) continue;
-            const unsigned long long cnt = 1ull + more[u];
-            P.out_counts[base + own[u] - 1u] = cnt;
+      // the entries that own a slot of L carry their key's count, and their threads clean the slot
+      if (nq <= SVT_Q)
+        for (uint32_t e = e0; e < nq; e += T) {
+          const uint32_t q = Q[e];
+          if (!(q & 0x8000u)) continue;
+          const uint32_t s = q & (SVT_L_SLOTS - 1), more = Lcnt[s];
+          if (!fail && more) {
+            const unsigned long long cnt = 1ull + more;
+            P.out_counts[base + Lslot[s] - 1u] = cnt;
             if (P.hist) hist_add(s_hist, P, cnt);
           }
+          Lslot[s] = 0; Lcnt[s] = 0;
         }
-        if (ls.x | ls.y | ls.z | ls.w) { *ls4 = make_uint4(0u, 0u, 0u, 0u); *lc4 = make_uint4(0u, 0u, 0u, 0u); }
-      }
       if (tid == 0) {
         if (!fail) {
           P.out_seg_len[p] = npad;
